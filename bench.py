@@ -7,7 +7,7 @@ HBM: BASELINE.json configs[1], 1024 clips x 900 frames x 160x120 uint16 per GPU,
 filtered fp32 + uint8 label image + region lists for every frame.  Clips are independent, so
 N GPUs each take their own 1024 clips (weak scaling, no collective on the data path).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--clips C] [--frames T]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--clips C] [--frames T] [--dump-outputs DIR]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference      # CPU port of the reference path on the host cores
 """
@@ -268,6 +268,36 @@ def check_parity(hout, port, n_clips, frames, max_regions=16):
     return int(live.sum())
 
 
+DUMP_FRAMES = 256  # frames written by --dump-outputs: about 40 MB in all
+
+
+def dump_outputs(out, total, directory, seed=0):
+    """Write what one extraction step returned for a fixed, seeded sample of DUMP_FRAMES frames of the batch, so that two
+    builds can be compared output for output: filtered images and label images (float32), and the frame records and region
+    lists (float64, one file per field; region slots past the frame's stored regions carry no result and are written as
+    zero)."""
+    import torch
+
+    from classifier_pipeline_b200.batch import BatchExtractor
+
+    idx = np.sort(np.random.default_rng(seed).choice(total, min(total, DUMP_FRAMES), replace=False))
+    d_idx = torch.from_numpy(idx).to(out["info"].device)
+    info = BatchExtractor.info_numpy(out["info"].index_select(0, d_idx))
+    regions = BatchExtractor.regions_numpy(out["regions"].index_select(0, d_idx))
+    live = np.arange(regions.shape[1])[None, :] < np.minimum(info["n_components"], regions.shape[1])[:, None]
+    arrays = {"frame_index": idx.astype(np.float64),
+              "filtered": out["filtered"].index_select(0, d_idx).cpu().numpy().astype(np.float32),
+              "labels": out["labels"].index_select(0, d_idx).cpu().numpy().astype(np.float32)}
+    for name in info.dtype.names:
+        if name != "reserved":
+            arrays["info_" + name] = info[name].astype(np.float64)
+    for name in regions.dtype.names:
+        arrays["region_" + name] = np.where(live, regions[name], 0).astype(np.float64)
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
+
+
 def workload_config(C, T):
     """The workload both arms (`--impl b200` and `--impl reference`) are quoted on."""
     return {
@@ -474,7 +504,13 @@ def main():
     ap.add_argument("--no-motion", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the denoise / parse_clips / streaming legs")
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write a seeded sample of the last timed step's outputs as DIR/<name>.npy "
+                    "(rank 0's clips)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of --impl b200")
     if args.warmup < 3 and args.impl == "b200":
         args.warmup = max(args.warmup, 1)
     if args.impl == "reference":
@@ -535,6 +571,8 @@ def main():
         barrier()
     ms_total = start.elapsed_time(stop)
     kernel_ms = float(np.mean([a.elapsed_time(b) for a, b in kernel_events]))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(out, total, args.dump_outputs)
     # per-kernel durations of a step: CUDA events recorded by the library around its own launches, on its own stream
     # (torch events only see torch's current stream), averaged over a few extra steps outside the timed region
     import ctypes

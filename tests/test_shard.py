@@ -2,6 +2,7 @@
 per-rank host tracking of its own clips) on 2 CPU processes with the gloo backend."""
 import json
 import os
+import socket
 import subprocess
 import sys
 
@@ -50,12 +51,19 @@ dist.destroy_process_group()
 """
 
 
+def free_port():
+    """A port no other process on the host listens on (a fixed one can be taken on a shared machine)."""
+    with socket.socket() as s:
+        s.bind(("127.0.0.1", 0))
+        return s.getsockname()[1]
+
+
 def test_two_ranks_gloo(tmp_path):
     from tests.tracking_helpers import track_clip_from_golden
 
     script = tmp_path / "worker.py"
     script.write_text(WORKER.format(root=ROOT))
-    env = dict(os.environ, MASTER_ADDR="127.0.0.1", MASTER_PORT="29517", WORLD_SIZE="2", PYTHONPATH=ROOT)
+    env = dict(os.environ, MASTER_ADDR="127.0.0.1", MASTER_PORT=str(free_port()), WORLD_SIZE="2", PYTHONPATH=ROOT)
     procs = [subprocess.Popen([sys.executable, str(script)], env=dict(env, RANK=str(r), LOCAL_RANK=str(r)), stdout=subprocess.PIPE,
                               stderr=subprocess.PIPE, text=True) for r in range(2)]
     outs = []
