@@ -265,9 +265,15 @@ class BatchPreprocessor:
             seg[i] = idx[pad_segment_samples(int(seg_len[i]), self.tiles, seed)]
         return lim, smp, seg, seg_track.astype(np.int32)
 
-    def run_tables(self, d_thermal, d_filtered, limit_regions, samples, segment_samples, n_tracks, crop_rectangle, out=None):
+    def run_tables(self, d_thermal, d_filtered, limit_regions, samples, segment_samples, n_tracks, crop_rectangle, out=None,
+                   row_map=None, frame_medians=None, frame_info=None):
         """Launch on prepared tables (host numpy or CUDA uint8/int32 tensors).  Returns the CUDA float32
-        tensor (n_segments, rows*size, per_row*size, 2) plus the device tables."""
+        tensor (n_segments, rows*size, per_row*size, 2) plus the device tables.
+
+        On an extraction's own buffers (``DeviceBatch``): ``row_map`` (host int64, one entry per thermal row) gives the filtered
+        row of every thermal row the tables name; ``frame_medians`` (CUDA float32 per thermal row, ``cpt_frame_medians``) and
+        ``frame_info`` (the extraction's CUDA INFO_DTYPE records, with CLIP_FRAME_STATS) are reused instead of re-reading the
+        frames.  The tables must then be host arrays."""
         torch = self.torch
         ctx = self.ex.ctx
         ctx.use_torch_stream()
@@ -290,18 +296,25 @@ class BatchPreprocessor:
             d_out = torch.empty(shape, dtype=torch.float32, device=self.device)
             if out is not None:
                 out["segments"] = d_out
-        ctx.preprocess_limits(d_filtered, d_lim, n_lim if self.diff_norm else 0, d_tracks, n_tracks)  # (always resets the rows)
+        d_lim_rows = d_smp_rows = None
+        if row_map is not None:
+            row_map = np.asarray(row_map, dtype=np.int64)
+            d_lim_rows = torch.from_numpy(row_map[limit_regions["frame"]]).to(self.device)
+            d_smp_rows = torch.from_numpy(row_map[samples["frame"]]).to(self.device)
+        # (always resets the rows)
+        ctx.preprocess_limits_ex(d_filtered, d_lim_rows, d_lim, n_lim if self.diff_norm else 0, d_tracks, n_tracks)
         if self.thermal_diff_norm:
-            ctx.preprocess_thermal_limits(d_thermal, d_lim, n_lim, d_tracks, n_tracks)
-        ctx.preprocess_medians(d_thermal, d_smp, n_smp, d_tracks)
+            ctx.preprocess_thermal_limits_ex(d_thermal, d_lim_rows, d_lim, n_lim, d_tracks, n_tracks, frame_medians, frame_info)
+        ctx.preprocess_medians_ex(d_thermal, frame_medians, d_smp, n_smp, d_tracks)
         fn = int(self.preprocess_fn) | (0 if self.diff_norm else native.PREPROCESS_PER_TILE)
-        ctx.preprocess_segments(d_thermal, d_filtered, d_smp, d_tracks, d_seg, n_seg, self.tiles, self.frames_per_row,
-                                self.frame_size, crop_rectangle, fn, d_out)
+        ctx.preprocess_segments_ex(d_thermal, d_filtered, d_smp_rows, d_smp, d_tracks, d_seg, n_seg, self.tiles, self.frames_per_row,
+                                   self.frame_size, crop_rectangle, fn, d_out)
         return dict(segments=d_out, tracks=d_tracks, samples=d_smp)
 
-    def run(self, d_thermal, d_filtered, tracks, crop_rectangle, seed=None, out=None):
+    def run(self, d_thermal, d_filtered, tracks, crop_rectangle, seed=None, out=None, row_map=None, frame_medians=None, frame_info=None):
         lim, smp, seg, seg_track = self.build_tables(tracks, seed=seed)
-        res = self.run_tables(d_thermal, d_filtered, lim, smp, seg, len(tracks), crop_rectangle, out=out)
+        res = self.run_tables(d_thermal, d_filtered, lim, smp, seg, len(tracks), crop_rectangle, out=out, row_map=row_map,
+                              frame_medians=frame_medians, frame_info=frame_info)
         res["segment_track"] = seg_track
         return res
 
@@ -309,3 +322,49 @@ class BatchPreprocessor:
     def tracks_numpy(t):
         a = t.cpu().numpy()
         return a.reshape(-1).view(native.TRACK_NORM_DTYPE)
+
+
+def tracked_row_map(clips, n_input):
+    """thermal row -> filtered row of every tracked frame of the CLIP_DTYPE records ``clips`` (frame t of clip i is thermal
+    row ``frame_offset + t`` and filtered row ``out_offset + t``); -1 for the other rows of the ``n_input``-row input (init
+    frames, leading background frames)."""
+    row_map = np.full(int(n_input), -1, np.int64)
+    for c in np.asarray(clips, dtype=native.CLIP_DTYPE).reshape(-1):
+        f0, o0, n = int(c["frame_offset"]), int(c["out_offset"]), int(c["n_frames"])
+        row_map[f0 : f0 + n] = np.arange(o0, o0 + n)
+    return row_map
+
+
+class DeviceBatch:
+    """The device buffers one ``ClipTrackExtractor.parse_clips(keep_on_device=True)`` launch leaves behind, shared by the
+    ``ClipDeviceFrames`` handles of its clips: the thermal input (uint16, one row per frame read, init and leading
+    background frames included), the filtered output (float32, one row per tracked frame), the frame medians (float32 per
+    thermal row) and the frame records (INFO_DTYPE bytes per filtered row).  ``row_map[thermal row]`` is the filtered row of
+    a tracked frame and -1 for every other row.  The memory is freed when the last handle is released."""
+
+    def __init__(self, engine, thermal, filtered, medians, info, row_map):
+        self.engine = engine
+        self.thermal, self.filtered, self.medians, self.info = thermal, filtered, medians, info
+        self.row_map = np.asarray(row_map, dtype=np.int64)
+
+
+class ClipDeviceFrames:
+    """One clip's frames inside a ``DeviceBatch``: frame number ``n`` (``Clip.current_frame``) is thermal row
+    ``thermal_row0 + n``, median row ``median_row0 + n`` and filtered row ``filtered_row0 + n`` for ``first_kept <= n <
+    n_frames`` (``first_kept`` > 0 only when the clip's frame buffer keeps the last ``max_frames`` frames)."""
+
+    def __init__(self, batch, thermal_row0, filtered_row0, n_frames, first_kept=0):
+        self.batch = batch
+        self.thermal_row0 = int(thermal_row0)
+        self.median_row0 = int(thermal_row0)
+        self.filtered_row0 = int(filtered_row0)
+        self.n_frames = int(n_frames)
+        self.first_kept = int(first_kept)
+
+    @property
+    def live(self):
+        return self.batch is not None
+
+    def release(self):
+        """Drop this clip's reference to the batch buffers (freed once every clip of the batch has released them)."""
+        self.batch = None

@@ -15,12 +15,17 @@ namespace cpt {
 constexpr int kMedianBins = 2048;
 constexpr int kMedianThreads = 256;
 
-// bins: kMedianBins uint32 of shared scratch; red: 80 ints of shared scratch.  Every thread of the CTA must call.
+// bins: kMedianBins uint32 of shared scratch; red: 80 ints of shared scratch.  Every thread of the CTA must call; the CTA
+// has kThreads threads (64..256; a crop of a few hundred pixels wants fewer than a whole frame).  px may point to shared or
+// global memory.
+template <int kThreads = kMedianThreads>
 __device__ inline int rect_median_sum(const uint16_t *px, int W, int x0, int y0, int w, int h, uint32_t *bins, int *red) {
+    static_assert(kThreads % 32 == 0 && kThreads >= 64 && kThreads <= 256 && kMedianBins % kThreads == 0, "CTA size");
+    constexpr int kWarps = kThreads / 32;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, n = w * h;
     // ---- range of the rectangle
     int mn = 65535, mx = 0;
-    for (int i = tid; i < n; i += kMedianThreads) {
+    for (int i = tid; i < n; i += kThreads) {
         const int yy = i / w, xx = i - yy * w;
         const int v = px[(y0 + yy) * W + x0 + xx];
         mn = min(mn, v);
@@ -31,21 +36,21 @@ __device__ inline int rect_median_sum(const uint16_t *px, int W, int x0, int y0,
     __syncthreads();  // scratch may still be read by a previous call
     if (lane == 0) { red[warp] = mn; red[8 + warp] = mx; }
     __syncthreads();
-    mn = red[lane & 7];
-    mx = red[8 + (lane & 7)];
+    mn = red[lane % kWarps];
+    mx = red[8 + lane % kWarps];
     mn = __reduce_min_sync(0xffffffffu, mn);
     mx = __reduce_max_sync(0xffffffffu, mx);
     const int r_lo = (n - 1) / 2, r_hi = n / 2;
     if (mx - mn < kMedianBins) {
-        for (int i = tid; i < kMedianBins; i += kMedianThreads) bins[i] = 0;
+        for (int i = tid; i < kMedianBins; i += kThreads) bins[i] = 0;
         __syncthreads();
-        for (int i = tid; i < n; i += kMedianThreads) {
+        for (int i = tid; i < n; i += kThreads) {
             const int yy = i / w, xx = i - yy * w;
             atomicAdd(&bins[px[(y0 + yy) * W + x0 + xx] - mn], 1u);
         }
         __syncthreads();
-        // thread t owns bins [8t, 8t + 8): block-wide inclusive scan of the per-thread counts
-        constexpr int kPer = kMedianBins / kMedianThreads;
+        // thread t owns bins [kPer t, kPer (t + 1)): block-wide inclusive scan of the per-thread counts
+        constexpr int kPer = kMedianBins / kThreads;
         uint32_t c[kPer], loc = 0;
 #pragma unroll
         for (int j = 0; j < kPer; ++j) { c[j] = bins[tid * kPer + j]; loc += c[j]; }
@@ -80,9 +85,9 @@ __device__ inline int rect_median_sum(const uint16_t *px, int W, int x0, int y0,
     }
     // ---- wide range: radix select on the high byte, then on the low byte inside the selected bucket(s)
     uint32_t *h0 = bins, *h1 = bins + 256;
-    for (int i = tid; i < 512; i += kMedianThreads) bins[i] = 0;
+    for (int i = tid; i < 512; i += kThreads) bins[i] = 0;
     __syncthreads();
-    for (int i = tid; i < n; i += kMedianThreads) {
+    for (int i = tid; i < n; i += kThreads) {
         const int yy = i / w, xx = i - yy * w;
         atomicAdd(&h0[px[(y0 + yy) * W + x0 + xx] >> 8], 1u);
     }
@@ -100,9 +105,9 @@ __device__ inline int rect_median_sum(const uint16_t *px, int W, int x0, int y0,
     }
     __syncthreads();
     const int b_lo = red[40], b_hi = red[41];
-    for (int i = tid; i < 512; i += kMedianThreads) bins[i] = 0;
+    for (int i = tid; i < 512; i += kThreads) bins[i] = 0;
     __syncthreads();
-    for (int i = tid; i < n; i += kMedianThreads) {
+    for (int i = tid; i < n; i += kThreads) {
         const int yy = i / w, xx = i - yy * w;
         const int v = px[(y0 + yy) * W + x0 + xx], hb = v >> 8;
         if (hb == b_lo) atomicAdd(&h0[v & 0xff], 1u);

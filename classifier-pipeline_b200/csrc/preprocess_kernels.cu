@@ -12,6 +12,11 @@
 //                            image (preprocess_movement / square_clip, preprocess.py:151-202,
 //                            imageprocessing.py:85-104): one CTA per (segment, tile); the crop is read from
 //                            HBM/L2 once, the only large traffic is the coalesced float2 output rows.
+// The *_ex entry points run the same kernels on an extraction's own buffers, where a frame's thermal row (its row of the
+// input) and its filtered row (its row of every per-frame output) differ, and reuse the per-frame statistics the extraction
+// has already computed:
+//   sample_crop_median_kernel        pass 1 with the frame medians of cpt_frame_medians: only the crop is read
+//   track_thermal_limits_stats_kernel  thermal_diff_norm limits from cpt_frame_info.thermal_min / thermal_max: no frame read
 #include <cfloat>
 
 #include "cptrack_internal.cuh"
@@ -103,13 +108,15 @@ __global__ void track_thermal_on_kernel(cpt_track_norm *tracks, int n_tracks) {
 // one warp per non-blank region of a track (a crop is a few hundred pixels: a warp's worth of work, and many warps in
 // flight hide the cold reads; a 128-thread CTA per region with two block reductions took 1.6 ms for 450 k regions)
 constexpr int kLimitsThreads = 256;
-__global__ void __launch_bounds__(kLimitsThreads) track_limits_kernel(const float *filtered, int W, int H, const cpt_sample *regions,
-                                                                      int n_regions, cpt_track_norm *tracks) {
+// filtered_rows (may be NULL: the region's frame): the filtered row of every region
+__global__ void __launch_bounds__(kLimitsThreads) track_limits_kernel(const float *filtered, const int64_t *filtered_rows, int W, int H,
+                                                                      const cpt_sample *regions, int n_regions, cpt_track_norm *tracks) {
     const int idx = blockIdx.x * (kLimitsThreads / 32) + (threadIdx.x >> 5), lane = threadIdx.x & 31;
     if (idx >= n_regions) return;
     const cpt_sample r = regions[idx];
-    if (r.width <= 0 || r.height <= 0 || r.frame < 0) return;  // (a row without a frame or an area is nobody's region)
-    const float *f = filtered + (size_t)r.frame * W * H;
+    const int64_t row = filtered_rows ? filtered_rows[idx] : r.frame;
+    if (r.width <= 0 || r.height <= 0 || r.frame < 0 || row < 0) return;  // (a row without a frame or an area is nobody's region)
+    const float *f = filtered + (size_t)row * W * H;
     float mn = FLT_MAX, mx = -FLT_MAX;
     const int n = r.width * r.height;
     const uint32_t rcp = 0xffffffffu / (uint32_t)r.width + 1u;  // i / width == umulhi(i, rcp) (wraps to 0 for width == 1)
@@ -157,6 +164,30 @@ __global__ void __launch_bounds__(256) sample_median_kernel(const uint16_t *ther
     }
 }
 
+// pass 1 when the frame medians are known (cpt_frame_medians over the same thermal rows): sample.median is looked up and only
+// the crop is read for the clip_thermals_at_zero test -- a few hundred pixels instead of the 19 200 of a frame, so a small CTA
+// that reads them straight from L2 (no staging; the two passes of median.cuh touch the crop twice)
+constexpr int kCropMedianThreads = 128;
+__global__ void __launch_bounds__(kCropMedianThreads) sample_crop_median_kernel(const uint16_t *thermal, int W, int H,
+                                                                               const float *frame_medians, cpt_sample *samples,
+                                                                               cpt_track_norm *tracks) {
+    __shared__ uint32_t bins[kMedianBins];
+    __shared__ int red[80];
+    cpt_sample *sp = samples + blockIdx.x;
+    const cpt_sample r = *sp;
+    if (r.frame < 0) return;
+    const float median = __ldg(frame_medians + r.frame);
+    const bool has_crop = r.width > 0 && r.height > 0;
+    int crop2 = 0;
+    if (has_crop)
+        crop2 = rect_median_sum<kCropMedianThreads>(thermal + (size_t)r.frame * W * H, W, r.x, r.y, r.width, r.height, bins, red);
+    if (threadIdx.x == 0) {
+        sp->median = median;
+        // the same integer test as sample_median_kernel: 2 * median is exact (a multiple of 0.5 below 2^16)
+        if (has_crop && crop2 <= __float2int_rn(2.0f * median)) atomicAnd(&tracks[r.track].clip_at_zero, 0);
+    }
+}
+
 // get_limits with thermal_diff_norm: one CTA per non-blank region of a track -- the extrema of frame.thermal - median over
 // the whole frame (interpreter.py:338-345; float32 arithmetic on integer / half-integer values: exact)
 __global__ void __launch_bounds__(256) track_thermal_limits_kernel(const uint16_t *thermal, int W, int H, const cpt_sample *regions,
@@ -199,6 +230,22 @@ __global__ void __launch_bounds__(256) track_thermal_limits_kernel(const uint16_
     }
 }
 
+// the same limits from the extraction's per-frame statistics: frame extrema from cpt_frame_info (indexed by the filtered row,
+// like every per-frame output) and the median from cpt_frame_medians (indexed by the thermal row); one thread per region
+__global__ void track_thermal_limits_stats_kernel(const cpt_sample *regions, const int64_t *filtered_rows, int n_regions,
+                                                  const float *frame_medians, const cpt_frame_info *info, cpt_track_norm *tracks) {
+    const int idx = blockIdx.x * blockDim.x + threadIdx.x;
+    if (idx >= n_regions) return;
+    const cpt_sample r = regions[idx];
+    const int64_t row = filtered_rows ? filtered_rows[idx] : r.frame;
+    if (r.width <= 0 || r.height <= 0 || r.frame < 0 || row < 0) return;
+    const float median = __ldg(frame_medians + r.frame);
+    cpt_track_norm *t = tracks + r.track;
+    atomic_min_float(&t->thermal_min, __fsub_rn((float)info[row].thermal_min, median));
+    atomic_max_float(&t->thermal_max, __fsub_rn((float)info[row].thermal_max, median));
+    t->has_thermal_limits = 1;
+}
+
 // ------------------------------------------------------------------------------------------------
 struct ResizeTaps {
     int i0, i1;
@@ -239,6 +286,7 @@ __device__ __forceinline__ float normalize255(float v, float mn, float mx) {
 struct SegmentArgs {
     const uint16_t *thermal;
     const float *filtered;
+    const int64_t *filtered_rows;    // [n_samples] filtered row of every sample, or NULL: the sample's frame
     const cpt_sample *samples;
     const cpt_track_norm *tracks;
     const int32_t *segment_samples;  // [n_segments][tiles]
@@ -261,12 +309,13 @@ __global__ void __launch_bounds__(kTileThreads) segment_tiles_kernel(const Segme
     const int seg = blockIdx.x / a.tiles, tile = blockIdx.x - seg * a.tiles;
     const int sidx = a.segment_samples[blockIdx.x];
     const cpt_sample r = a.samples[sidx];
-    if (r.frame < 0 || r.width <= 0 || r.height <= 0) return;  // (malformed table: the tile is left as it is)
+    const int64_t frow = a.filtered_rows ? a.filtered_rows[sidx] : r.frame;
+    if (r.frame < 0 || frow < 0 || r.width <= 0 || r.height <= 0) return;  // (malformed table: the tile is left as it is)
     const cpt_track_norm tn = a.tracks[r.track];
     const int size = a.size, n = size * size, tid = threadIdx.x;
     const int sw = r.width, sh = r.height;
     const uint16_t *th = a.thermal + (size_t)r.frame * a.W * a.H + r.y * a.W + r.x;
-    const float *fl = a.filtered + (size_t)r.frame * a.W * a.H + r.y * a.W + r.x;
+    const float *fl = a.filtered + (size_t)frow * a.W * a.H + r.y * a.W + r.x;
 
     // ---- target size and paste offsets (imageprocessing.py:24-59)
     const double scale = fmin((double)size / (double)sh, (double)size / (double)sw);
@@ -352,8 +401,8 @@ using cpt::fail;
 
 extern "C" {
 
-int cpt_preprocess_limits(cpt_ctx *c, const float *d_filtered, const cpt_sample *d_regions, int n_regions,
-                          cpt_track_norm *d_tracks, int n_tracks) {
+int cpt_preprocess_limits_ex(cpt_ctx *c, const float *d_filtered, const int64_t *d_filtered_rows, const cpt_sample *d_regions,
+                             int n_regions, cpt_track_norm *d_tracks, int n_tracks) {
     if (!c || !d_tracks) return fail(CPT_ERR_INVALID, "null argument");
     if (n_regions < 0 || n_tracks < 0) return fail(CPT_ERR_INVALID, "negative count");
     if (n_tracks == 0) return CPT_OK;
@@ -362,7 +411,35 @@ int cpt_preprocess_limits(cpt_ctx *c, const float *d_filtered, const cpt_sample 
     if (n_regions > 0) {
         if (!d_filtered || !d_regions) return fail(CPT_ERR_INVALID, "null filtered / regions");
         cpt::track_limits_kernel<<<(n_regions + cpt::kLimitsThreads / 32 - 1) / (cpt::kLimitsThreads / 32), cpt::kLimitsThreads, 0, c->stream>>>(
-            d_filtered, c->g.W, c->g.H, d_regions, n_regions, d_tracks);
+            d_filtered, d_filtered_rows, c->g.W, c->g.H, d_regions, n_regions, d_tracks);
+    }
+    CUDA_TRY(cudaGetLastError());
+    return CPT_OK;
+}
+
+int cpt_preprocess_limits(cpt_ctx *c, const float *d_filtered, const cpt_sample *d_regions, int n_regions,
+                          cpt_track_norm *d_tracks, int n_tracks) {
+    return cpt_preprocess_limits_ex(c, d_filtered, nullptr, d_regions, n_regions, d_tracks, n_tracks);
+}
+
+int cpt_preprocess_thermal_limits_ex(cpt_ctx *c, const uint16_t *d_thermal, const int64_t *d_filtered_rows, const cpt_sample *d_regions,
+                                     int n_regions, cpt_track_norm *d_tracks, int n_tracks, const float *d_frame_medians,
+                                     const cpt_frame_info *d_frame_info) {
+    if (!c || !d_tracks) return fail(CPT_ERR_INVALID, "null argument");
+    if (n_regions < 0 || n_tracks < 0) return fail(CPT_ERR_INVALID, "negative count");
+    if (n_tracks == 0) return CPT_OK;
+    CUDA_TRY(cudaSetDevice(c->device));
+    cpt::track_thermal_on_kernel<<<(n_tracks + 255) / 256, 256, 0, c->stream>>>(d_tracks, n_tracks);
+    if (n_regions > 0) {
+        if (!d_regions) return fail(CPT_ERR_INVALID, "null regions");
+        if (d_frame_medians && d_frame_info) {
+            cpt::track_thermal_limits_stats_kernel<<<(n_regions + 255) / 256, 256, 0, c->stream>>>(d_regions, d_filtered_rows, n_regions,
+                                                                                              d_frame_medians, d_frame_info, d_tracks);
+        } else {
+            if (!d_thermal) return fail(CPT_ERR_INVALID, "null thermal");
+            const size_t smem = (((size_t)c->g.npx * sizeof(uint16_t) + 15) & ~(size_t)15) + cpt::kMedianBins * sizeof(uint32_t);
+            cpt::track_thermal_limits_kernel<<<n_regions, 256, smem, c->stream>>>(d_thermal, c->g.W, c->g.H, d_regions, d_tracks);
+        }
     }
     CUDA_TRY(cudaGetLastError());
     return CPT_OK;
@@ -370,15 +447,22 @@ int cpt_preprocess_limits(cpt_ctx *c, const float *d_filtered, const cpt_sample 
 
 int cpt_preprocess_thermal_limits(cpt_ctx *c, const uint16_t *d_thermal, const cpt_sample *d_regions, int n_regions,
                                   cpt_track_norm *d_tracks, int n_tracks) {
-    if (!c || !d_tracks) return fail(CPT_ERR_INVALID, "null argument");
-    if (n_regions < 0 || n_tracks < 0) return fail(CPT_ERR_INVALID, "negative count");
-    if (n_tracks == 0) return CPT_OK;
+    return cpt_preprocess_thermal_limits_ex(c, d_thermal, nullptr, d_regions, n_regions, d_tracks, n_tracks, nullptr, nullptr);
+}
+
+int cpt_preprocess_medians_ex(cpt_ctx *c, const uint16_t *d_thermal, const float *d_frame_medians, cpt_sample *d_samples, int n_samples,
+                              cpt_track_norm *d_tracks) {
+    if (!c) return fail(CPT_ERR_INVALID, "null ctx");
+    if (n_samples < 0) return fail(CPT_ERR_INVALID, "negative count");
+    if (n_samples == 0) return CPT_OK;
+    if (!d_thermal || !d_samples || !d_tracks) return fail(CPT_ERR_INVALID, "null argument");
     CUDA_TRY(cudaSetDevice(c->device));
-    cpt::track_thermal_on_kernel<<<(n_tracks + 255) / 256, 256, 0, c->stream>>>(d_tracks, n_tracks);
-    if (n_regions > 0) {
-        if (!d_thermal || !d_regions) return fail(CPT_ERR_INVALID, "null thermal / regions");
+    if (d_frame_medians) {
+        cpt::sample_crop_median_kernel<<<n_samples, cpt::kCropMedianThreads, 0, c->stream>>>(d_thermal, c->g.W, c->g.H, d_frame_medians,
+                                                                                          d_samples, d_tracks);
+    } else {
         const size_t smem = (((size_t)c->g.npx * sizeof(uint16_t) + 15) & ~(size_t)15) + cpt::kMedianBins * sizeof(uint32_t);
-        cpt::track_thermal_limits_kernel<<<n_regions, 256, smem, c->stream>>>(d_thermal, c->g.W, c->g.H, d_regions, d_tracks);
+        cpt::sample_median_kernel<<<n_samples, 256, smem, c->stream>>>(d_thermal, c->g.W, c->g.H, d_samples, d_tracks);
     }
     CUDA_TRY(cudaGetLastError());
     return CPT_OK;
@@ -386,22 +470,13 @@ int cpt_preprocess_thermal_limits(cpt_ctx *c, const uint16_t *d_thermal, const c
 
 int cpt_preprocess_medians(cpt_ctx *c, const uint16_t *d_thermal, cpt_sample *d_samples, int n_samples,
                            cpt_track_norm *d_tracks) {
-    if (!c) return fail(CPT_ERR_INVALID, "null ctx");
-    if (n_samples < 0) return fail(CPT_ERR_INVALID, "negative count");
-    if (n_samples == 0) return CPT_OK;
-    if (!d_thermal || !d_samples || !d_tracks) return fail(CPT_ERR_INVALID, "null argument");
-    CUDA_TRY(cudaSetDevice(c->device));
-    const size_t smem = (((size_t)c->g.npx * sizeof(uint16_t) + 15) & ~(size_t)15) + cpt::kMedianBins * sizeof(uint32_t);
-    cpt::sample_median_kernel<<<n_samples, 256, smem, c->stream>>>(d_thermal, c->g.W, c->g.H,
-                                                                                                   d_samples, d_tracks);
-    CUDA_TRY(cudaGetLastError());
-    return CPT_OK;
+    return cpt_preprocess_medians_ex(c, d_thermal, nullptr, d_samples, n_samples, d_tracks);
 }
 
-int cpt_preprocess_segments(cpt_ctx *c, const uint16_t *d_thermal, const float *d_filtered, const cpt_sample *d_samples,
-                            const cpt_track_norm *d_tracks, const int32_t *d_segment_samples, int n_segments,
-                            int tiles_per_segment, int frames_per_row, int frame_size, const int32_t *crop_rectangle,
-                            int preprocess_fn, float *d_out) {
+int cpt_preprocess_segments_ex(cpt_ctx *c, const uint16_t *d_thermal, const float *d_filtered, const int64_t *d_filtered_rows,
+                               const cpt_sample *d_samples, const cpt_track_norm *d_tracks, const int32_t *d_segment_samples,
+                               int n_segments, int tiles_per_segment, int frames_per_row, int frame_size,
+                               const int32_t *crop_rectangle, int preprocess_fn, float *d_out) {
     if (!c) return fail(CPT_ERR_INVALID, "null ctx");
     if (n_segments < 0) return fail(CPT_ERR_INVALID, "negative count");
     if (n_segments == 0) return CPT_OK;
@@ -411,10 +486,9 @@ int cpt_preprocess_segments(cpt_ctx *c, const uint16_t *d_thermal, const float *
         return fail(CPT_ERR_INVALID, "bad tiling (frame_size must be in [1,%d])", cpt::kMaxTile);
     if (preprocess_fn & ~(CPT_PREPROCESS_INC3 | CPT_PREPROCESS_PER_TILE)) return fail(CPT_ERR_INVALID, "preprocess_fn: unknown flag");
     if ((long long)n_segments * tiles_per_segment > 0x7fffffffll) return fail(CPT_ERR_INVALID, "too many tiles for one launch");
-    if (n_segments == 0) return CPT_OK;
     CUDA_TRY(cudaSetDevice(c->device));
     cpt::SegmentArgs a{};
-    a.thermal = d_thermal; a.filtered = d_filtered; a.samples = d_samples; a.tracks = d_tracks;
+    a.thermal = d_thermal; a.filtered = d_filtered; a.filtered_rows = d_filtered_rows; a.samples = d_samples; a.tracks = d_tracks;
     a.segment_samples = d_segment_samples; a.out = d_out;
     a.W = c->g.W; a.H = c->g.H;
     a.tiles = tiles_per_segment; a.per_row = frames_per_row; a.size = frame_size;
@@ -426,6 +500,14 @@ int cpt_preprocess_segments(cpt_ctx *c, const uint16_t *d_thermal, const float *
     cpt::segment_tiles_kernel<<<(unsigned)(n_segments * tiles_per_segment), cpt::kTileThreads, smem, c->stream>>>(a);
     CUDA_TRY(cudaGetLastError());
     return CPT_OK;
+}
+
+int cpt_preprocess_segments(cpt_ctx *c, const uint16_t *d_thermal, const float *d_filtered, const cpt_sample *d_samples,
+                            const cpt_track_norm *d_tracks, const int32_t *d_segment_samples, int n_segments,
+                            int tiles_per_segment, int frames_per_row, int frame_size, const int32_t *crop_rectangle,
+                            int preprocess_fn, float *d_out) {
+    return cpt_preprocess_segments_ex(c, d_thermal, d_filtered, nullptr, d_samples, d_tracks, d_segment_samples, n_segments,
+                                      tiles_per_segment, frames_per_row, frame_size, crop_rectangle, preprocess_fn, d_out);
 }
 
 }  // extern "C"

@@ -7,6 +7,11 @@ inference (TFLite / Keras / OpenVINO) are outside this path: subclass and implem
 launches (track limits, medians + clip test, fused crop/resize/normalise/tile); ``preprocess_tracks``
 does the same for every track of a clip in one go, and ``BatchPreprocessor`` (``..batch``) is the
 device-resident form used after a batched extraction.
+
+A clip parsed with ``parse_clips(..., keep_on_device=True)`` carries ``clip.device_frames``: its frames are then read from
+the extraction's device buffers instead of being uploaded, the frame medians (and, for ``thermal_diff_norm``, the frame
+extrema) the extraction computed are reused, and ``preprocess_clips`` makes the classifier inputs of every track of many
+clips in one set of launches.
 """
 import logging
 
@@ -153,13 +158,15 @@ class Interpreter:
             filtered_limits = (lo, np.float32(n["filtered_max"]) if n["has_limits"] else 0)
         return thermal_limits, filtered_limits
 
-    def _run(self, clip, jobs):
-        eng = self._engine_for(clip)
+    @staticmethod
+    def _needed(jobs):
         needed = []
         for track, _ in jobs:
-            needed.extend(r.frame_number for r in track.bounds_history if not r.blank and r.width > 0 and r.height > 0)
-        needed = [n for n in sorted(set(needed)) if clip.get_frame(n) is not None]
-        d_t, d_f, index = self._upload(eng, clip, needed)
+            needed.extend(int(r.frame_number) for r in track.bounds_history if not r.blank and r.width > 0 and r.height > 0)
+        return sorted(set(needed))  # (Python ints: frame numbers of tracks loaded from metadata are np.uint16)
+
+    def _tables(self, clip, jobs, index):
+        """Per track (region rows, segment frames) with frame numbers mapped through ``index`` to device rows."""
         tables = []
         for track, segments in jobs:
             seg_frames = []
@@ -169,6 +176,41 @@ class Interpreter:
                     raise Exception("Clasifying clip {} track {} can't get frame {}".format(clip.get_id(), track.get_id(), missing[0]))
                 seg_frames.append(np.array([index[int(n)] for n in s.frame_indices], dtype=np.int64))
             tables.append((self._region_rows(track, index), seg_frames))
+        return tables
+
+    @staticmethod
+    def _device_batch(clip):
+        """The live ``DeviceBatch`` of a clip parsed with keep_on_device, None for any other clip."""
+        h = getattr(clip, "device_frames", None)
+        if h is None:
+            return None
+        if not h.live:
+            raise Exception("Clasifying clip {}: its device frames were released".format(clip.get_id()))
+        return h.batch
+
+    def _run(self, clip, jobs):
+        batch = self._device_batch(clip)
+        if batch is not None:
+            return self._run_device(batch, clip.crop_rectangle, [(clip, jobs)])
+        eng = self._engine_for(clip)
+        needed = [n for n in self._needed(jobs) if clip.get_frame(n) is not None]
+        d_t, d_f, index = self._upload(eng, clip, needed)
+        return self._launch(eng, d_t, d_f, self._tables(clip, jobs, index), clip.crop_rectangle)
+
+    def _device_index(self, handle, jobs):
+        """frame number -> thermal row of the frames the jobs' regions name that the clip's handle holds."""
+        return {n: int(handle.thermal_row0) + n for n in self._needed(jobs) if handle.first_kept <= n < handle.n_frames}
+
+    def _run_device(self, batch, crop, clip_jobs):
+        """The tracks of several clips of one keep_on_device batch in one set of launches on the batch's own buffers: frame
+        number n of a clip is thermal row ``thermal_row0 + n``; ``row_map`` takes each thermal row to its filtered row."""
+        tables = []
+        for clip, jobs in clip_jobs:
+            tables.extend(self._tables(clip, jobs, self._device_index(clip.device_frames, jobs)))
+        return self._launch(batch.engine, batch.thermal, batch.filtered, tables, crop, row_map=batch.row_map,
+                            frame_medians=batch.medians, frame_info=batch.info)
+
+    def _launch(self, eng, d_t, d_f, tables, crop, **device_stats):
         fn = 0
         if self.preprocess_fn is not None:
             from . import preprocess as _pp
@@ -179,8 +221,7 @@ class Interpreter:
                 fn = 1
         bp = BatchPreprocessor(eng, frame_size=self.params.frame_size, frames_per_row=self.params.square_width, preprocess_fn=fn,
                                diff_norm=self.params.diff_norm, thermal_diff_norm=self.params.thermal_diff_norm)
-        crop = clip.crop_rectangle
-        return bp.run(d_t, d_f, tables, (crop.x, crop.y, crop.width, crop.height), seed=self.seed)
+        return bp.run(d_t, d_f, tables, (crop.x, crop.y, crop.width, crop.height), seed=self.seed, **device_stats)
 
     def _fn_on_device(self):
         from . import preprocess as _pp
@@ -196,7 +237,10 @@ class Interpreter:
     def preprocess_tracks(self, clip, jobs):
         """``preprocess_segments`` for several (track, segments) pairs of one clip in one set of launches."""
         jobs = [(t, list(s)) for t, s in jobs]
-        res = self._run(clip, jobs)
+        return self._collect(self._run(clip, jobs), jobs)
+
+    def _collect(self, res, jobs):
+        """Launch results -> per job (frame_indices per segment, data, masses), on the host."""
         d_seg = res["segments"]
         if self._channel_index != [0, 1]:
             import torch
@@ -215,3 +259,30 @@ class Interpreter:
     def preprocess(self, clip, track, **args):
         segments = self.frames_for_prediction(clip, track, **args)
         return self.preprocess_segments(clip, track, segments, args.get("predict_from_last"))
+
+    def preprocess_clips(self, clips, **args):
+        """``preprocess`` for every track of every clip: per clip, per track in ``clip.tracks``, ``(frame_indices, data,
+        masses)``.  The clips parsed in one ``parse_clips(..., keep_on_device=True)`` batch (with the same crop rectangle) go
+        through one set of launches on the extraction's buffers; a clip without ``device_frames`` takes the per-clip path.
+        Segments are selected in clip and track order first, so the random draws are those of ``preprocess`` called in a loop."""
+        clip_jobs = []
+        for clip in clips:
+            self._device_batch(clip)  # (a released handle fails before anything runs)
+            clip_jobs.append([(t, list(self.frames_for_prediction(clip, t, **args))) for t in clip.tracks])
+        out = [None] * len(clips)
+        groups = {}
+        for i, clip in enumerate(clips):
+            batch = self._device_batch(clip)
+            if batch is None:
+                out[i] = [self.preprocess_segments(clip, t, segments) for t, segments in clip_jobs[i]]
+                continue
+            c = clip.crop_rectangle
+            groups.setdefault((id(batch), c.x, c.y, c.width, c.height), (batch, c, []))[2].append(i)
+        for batch, crop, members in groups.values():
+            res = self._collect(self._run_device(batch, crop, [(clips[i], clip_jobs[i]) for i in members]),
+                                [j for i in members for j in clip_jobs[i]])
+            at = 0
+            for i in members:
+                out[i] = res[at : at + len(clip_jobs[i])]
+                at += len(clip_jobs[i])
+        return out

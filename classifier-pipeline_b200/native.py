@@ -144,6 +144,10 @@ SYMBOLS = {
     "cpt_preprocess_thermal_limits": (_i, [_vp, _vp, _vp, _i, _vp, _i]),
     "cpt_preprocess_medians": (_i, [_vp, _vp, _vp, _i, _vp]),
     "cpt_preprocess_segments": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp, _i, _vp]),
+    "cpt_preprocess_limits_ex": (_i, [_vp, _vp, _vp, _vp, _i, _vp, _i]),
+    "cpt_preprocess_thermal_limits_ex": (_i, [_vp, _vp, _vp, _vp, _i, _vp, _i, _vp, _vp]),
+    "cpt_preprocess_medians_ex": (_i, [_vp, _vp, _vp, _vp, _i, _vp]),
+    "cpt_preprocess_segments_ex": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp, _i, _vp]),
     "cpt_minmax_f32": (_i, [_vp, _vp, _i64, _vp]),
     "cpt_normalize_f32": (_i, [_vp, _vp, _i64, _d, _d, _d, _i, _vp]),
     "cpt_resize_pad_f32": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _f, _i, _vp]),
@@ -301,6 +305,28 @@ class Context:
         check(self.lib.cpt_preprocess_segments(
             self._h, _ptr(d_thermal), _ptr(d_filtered), _ptr(d_samples), _ptr(d_tracks), _ptr(d_segment_samples), int(n_segments),
             int(tiles), int(per_row), int(frame_size), crop, int(preprocess_fn), _ptr(d_out)))
+
+    # the same passes on an extraction's buffers (include/cptrack.h, cpt_preprocess_*_ex): d_filtered_rows int64 per entry
+    # (None: the entry's frame), d_frame_medians float32 per thermal row, d_frame_info the extraction's INFO_DTYPE records
+    def preprocess_limits_ex(self, d_filtered, d_filtered_rows, d_regions, n_regions, d_tracks, n_tracks):
+        check(self.lib.cpt_preprocess_limits_ex(self._h, _ptr(d_filtered), _ptr(d_filtered_rows), _ptr(d_regions), int(n_regions),
+                                                _ptr(d_tracks), int(n_tracks)))
+
+    def preprocess_thermal_limits_ex(self, d_thermal, d_filtered_rows, d_regions, n_regions, d_tracks, n_tracks, d_frame_medians=None,
+                                     d_frame_info=None):
+        check(self.lib.cpt_preprocess_thermal_limits_ex(self._h, _ptr(d_thermal), _ptr(d_filtered_rows), _ptr(d_regions), int(n_regions),
+                                                        _ptr(d_tracks), int(n_tracks), _ptr(d_frame_medians), _ptr(d_frame_info)))
+
+    def preprocess_medians_ex(self, d_thermal, d_frame_medians, d_samples, n_samples, d_tracks):
+        check(self.lib.cpt_preprocess_medians_ex(self._h, _ptr(d_thermal), _ptr(d_frame_medians), _ptr(d_samples), int(n_samples),
+                                                 _ptr(d_tracks)))
+
+    def preprocess_segments_ex(self, d_thermal, d_filtered, d_filtered_rows, d_samples, d_tracks, d_segment_samples, n_segments, tiles,
+                               per_row, frame_size, crop_rectangle, preprocess_fn, d_out):
+        crop = None if crop_rectangle is None else (ctypes.c_int32 * 4)(*[int(v) for v in crop_rectangle])
+        check(self.lib.cpt_preprocess_segments_ex(
+            self._h, _ptr(d_thermal), _ptr(d_filtered), _ptr(d_filtered_rows), _ptr(d_samples), _ptr(d_tracks), _ptr(d_segment_samples),
+            int(n_segments), int(tiles), int(per_row), int(frame_size), crop, int(preprocess_fn), _ptr(d_out)))
 
     def minmax_f32(self, d_in, n, d_out2):
         check(self.lib.cpt_minmax_f32(self._h, _ptr(d_in), int(n), _ptr(d_out2)))

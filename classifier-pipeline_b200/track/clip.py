@@ -36,6 +36,7 @@ class Clip:
         self.video_start_time = None
         self.location = None
         self.frame_buffer = None
+        self.device_frames = None  # batch.ClipDeviceFrames after parse_clips(keep_on_device=True)
         self.device = None
         self._background = None
         self.background_calculated = False

@@ -18,7 +18,7 @@ import numpy as np
 
 from .. import engine as _engine
 from .. import native
-from ..batch import linear_clips
+from ..batch import ClipDeviceFrames, DeviceBatch, linear_clips, tracked_row_map
 from ..cptv import CptvReader
 from ..piclassifier.cptvmotiondetector import is_affected_by_ffc
 from ..piclassifier.motiondetector import WeightedBackground
@@ -102,18 +102,23 @@ class ClipTrackExtractor(ClipTracker):
                                   device=self.device)
 
     # ------------------------------------------------------------------ whole clips
-    def parse_clip(self, clip, process_background=False):
-        """Loads a cptv file and extracts its tracks.  Returns True."""
+    def parse_clip(self, clip, process_background=False, *, keep_on_device=False):
+        """Loads a cptv file and extracts its tracks.  Returns True.  ``keep_on_device``: as in ``parse_clips``."""
         self._tracking_time = None
         start = time.time()
-        self.parse_clips([clip], process_background=process_background)
+        self.parse_clips([clip], process_background=process_background, keep_on_device=keep_on_device)
         self._tracking_time = time.time() - start
         return True
 
-    def parse_clips(self, clips, process_background=False):
+    def parse_clips(self, clips, process_background=False, *, keep_on_device=False):
         """Batched ``parse_clip``: decode every clip, ONE kernel launch for all of them, then the
         host-side matcher per clip.  Track ids restart at 1 for every clip, as they do when the
-        reference processes the clips one after another."""
+        reference processes the clips one after another.
+
+        ``keep_on_device=True`` keeps the batch's frames in device memory for ``Interpreter.preprocess_clips``: the thermal
+        input, the filtered output (also with ``keep_frames=False``), the frame medians (also with ``calc_stats=False``) and
+        the frame records.  Each clip gets ``clip.device_frames``, a ``batch.ClipDeviceFrames`` handle; ``release()`` it when
+        the clip's classifier inputs are made.  With ``keep_frames=False`` no filtered or label image is copied to the host."""
         from .track import Track
 
         jobs = []
@@ -145,8 +150,9 @@ class ClipTrackExtractor(ClipTracker):
         device_frames = None
         if device_decode and jobs:
             jobs, device_frames = self._decode_on_device(jobs, readers, process_background)
-        results = self._run_batch(jobs, device_frames)
+        results = self._run_batch(jobs, device_frames, keep_on_device=keep_on_device)
         for (clip, background_alg, frames), res in zip(jobs, results):
+            clip.device_frames = res.get("device_frames")
             self.background_alg = background_alg
             Track._track_id = 1
             for t, frame in enumerate(frames):
@@ -193,8 +199,9 @@ class ClipTrackExtractor(ClipTracker):
             frame_offsets.append(first + skip)
         return out_jobs, (d_frames, init_offsets, frame_offsets)
 
-    def _run_batch(self, jobs, device_frames=None):
-        """One launch over every clip of ``jobs``; per clip a dict of host arrays for its frames."""
+    def _run_batch(self, jobs, device_frames=None, keep_on_device=False):
+        """One launch over every clip of ``jobs``; per clip a dict of host arrays for its frames (and, with
+        ``keep_on_device``, its ``ClipDeviceFrames`` handle)."""
         import torch
 
         if not jobs:
@@ -208,7 +215,8 @@ class ClipTrackExtractor(ClipTracker):
         counts = [len(frames) for _, _, frames in jobs]
         total = sum(counts)
         keep_images = self.keep_frames or self.calculate_filtered
-        clips = linear_clips(counts, 0, 0, flags=self._flags())
+        # keep_on_device: the frame records carry the thermal extrema the thermal_diff_norm limits reuse
+        clips = linear_clips(counts, 0, 0, flags=self._flags() | (native.CLIP_FRAME_STATS if keep_on_device else 0))
         for i, (clip, background_alg, frames) in enumerate(jobs):
             clips["background_thresh"][i] = clip.background_thresh
             clips["weight_table"][i] = ctx.weight_table(background_alg.weight_add, max_frames=max(max(counts), 1024))
@@ -232,12 +240,17 @@ class ClipTrackExtractor(ClipTracker):
             d_frames = torch.from_numpy(h_frames.view(np.int16)).to(eng.device).view(torch.uint16)
             n_input = total + len(jobs)
         denoise = bool(getattr(self.config, "denoise", False))  # the device NLM + variance passes read the filtered images
-        out = eng.extract_device(d_frames, clips, keep_filtered=keep_images or denoise, keep_labels=keep_images, keep_state=True, out={})
-        medians = None
-        if self.calc_stats and total:
+        out = eng.extract_device(d_frames, clips, keep_filtered=keep_images or denoise or keep_on_device, keep_labels=keep_images,
+                                 keep_state=True, out={})
+        medians = d_med = None
+        if (self.calc_stats or keep_on_device) and total:
             d_med = torch.empty((n_input,), dtype=torch.float32, device=eng.device)
             ctx.frame_medians(d_frames, n_input, d_med)
-            medians = d_med.cpu().numpy()
+            if self.calc_stats:
+                medians = d_med.cpu().numpy()
+        batch = None
+        if keep_on_device:
+            batch = DeviceBatch(eng, d_frames, out["filtered"], d_med, out["info"], tracked_row_map(clips, n_input))
         info = eng.info_numpy(out["info"])
         # (only the region slots some frame uses travel: the API engines have 255 per frame)
         used = min(int(info["n_components"][:total].max()) if total else 0, eng.max_regions)
@@ -261,6 +274,9 @@ class ClipTrackExtractor(ClipTracker):
                 labels=None if labels is None else labels[o0 : o0 + n],
                 medians=None if medians is None else medians[f0 : f0 + n],
             ))
+            if batch is not None:
+                kept = clip.frame_buffer.max_frames if clip.frame_buffer is not None else None
+                results[-1]["device_frames"] = ClipDeviceFrames(batch, f0, o0, n, first_kept=max(n - kept, 0) if kept else 0)
         return results
 
     def _consume_frame(self, clip, frame, res, t):

@@ -233,6 +233,28 @@ int cpt_preprocess_segments(cpt_ctx *ctx, const uint16_t *d_thermal, const float
                             int tiles_per_segment, int frames_per_row, int frame_size, const int32_t *crop_rectangle,
                             int preprocess_fn, float *d_out);
 
+/* The same passes on an extraction's own buffers (ClipTrackExtractor.parse_clips(keep_on_device=True)).  There a tracked frame
+ * lives at different rows: its thermal row (sample.frame; the row of d_frames it was read from, also its row of
+ * cpt_frame_medians) and its filtered row (out_offset + n, its row of d_filtered and of every other per-frame output).
+ *   d_filtered_rows    one int64 per entry of d_regions / d_samples: the entry's filtered row (NULL: the same as sample.frame)
+ *   d_frame_medians    float32 per thermal row as cpt_frame_medians writes them (NULL: recompute them from the frames).  Given,
+ *                      the medians pass looks sample.median up and reads only the crop for the clip_thermals_at_zero test
+ *   d_frame_info       the extraction's cpt_frame_info per filtered row, computed with CPT_CLIP_FRAME_STATS.  With
+ *                      d_frame_medians as well, the thermal_diff_norm limits are (thermal_min - median, thermal_max - median)
+ *                      folded per track without reading a frame; otherwise the frames are read as cpt_preprocess_thermal_limits does
+ * Results are bit-identical to the entry points above on the same frames. */
+int cpt_preprocess_limits_ex(cpt_ctx *ctx, const float *d_filtered, const int64_t *d_filtered_rows, const cpt_sample *d_regions,
+                             int n_regions, cpt_track_norm *d_tracks, int n_tracks);
+int cpt_preprocess_thermal_limits_ex(cpt_ctx *ctx, const uint16_t *d_thermal, const int64_t *d_filtered_rows, const cpt_sample *d_regions,
+                                     int n_regions, cpt_track_norm *d_tracks, int n_tracks, const float *d_frame_medians,
+                                     const cpt_frame_info *d_frame_info);
+int cpt_preprocess_medians_ex(cpt_ctx *ctx, const uint16_t *d_thermal, const float *d_frame_medians, cpt_sample *d_samples, int n_samples,
+                              cpt_track_norm *d_tracks);
+int cpt_preprocess_segments_ex(cpt_ctx *ctx, const uint16_t *d_thermal, const float *d_filtered, const int64_t *d_filtered_rows,
+                               const cpt_sample *d_samples, const cpt_track_norm *d_tracks, const int32_t *d_segment_samples,
+                               int n_segments, int tiles_per_segment, int frames_per_row, int frame_size,
+                               const int32_t *crop_rectangle, int preprocess_fn, float *d_out);
+
 /* ---- ml_tools/imageprocessing.py helpers on single images (device buffers) ----
  * normalize() (imageprocessing.py:151-169): cpt_minmax_f32 writes {min, max} of d_in to d_out2; cpt_normalize_f32
  * computes new_max * (float32(data) - min) / (max - min) (max == min: zeros if max == 0, else data / max) in fp32
