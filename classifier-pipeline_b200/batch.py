@@ -162,13 +162,18 @@ class BatchPreprocessor:
     clip-at-zero test, then one CTA per (segment, tile) that crops, resizes, normalises and writes the
     tile into the segment image.  Frames stay in HBM (the extraction's thermal input and filtered output)."""
 
-    def __init__(self, extractor, frame_size=32, frames_per_row=5, tiles=None, preprocess_fn=0, diff_norm=True, thermal_diff_norm=False):
+    def __init__(self, extractor, frame_size=32, frames_per_row=5, preprocess_fn=0, diff_norm=True, thermal_diff_norm=False):
+        # preprocess_movement pads every segment to frames_per_row * 5 samples (preprocess.py:161) and square_clip lays out the
+        # first frames_per_row ** 2 of them, frames_per_row to a row (imageprocessing.py:85-104); past 5 per row a padded
+        # segment has fewer samples than cells and the reference's square_clip fails with an IndexError
+        if not 1 <= int(frames_per_row) <= 5:
+            raise ValueError("frames_per_row (HyperParams.square_width) must be in [1, 5], got {}".format(frames_per_row))
         self.ex = extractor
         self.torch = extractor.torch
         self.device = extractor.device
         self.frame_size = frame_size
-        self.frames_per_row = frames_per_row
-        self.tiles = tiles if tiles is not None else frames_per_row * 5  # preprocess.py:161: frames_per_row * 5
+        self.frames_per_row = int(frames_per_row)
+        self.tiles = self.frames_per_row * 5  # samples drawn and padded per segment: the columns of the segment table
         self.preprocess_fn = preprocess_fn
         # HyperParams.diff_norm / thermal_diff_norm (interpreter.py:315-363,405-408): track-wide limits for the filtered / the
         # thermal channel; with diff_norm off both channels are normalised per tile
@@ -265,10 +270,16 @@ class BatchPreprocessor:
             seg[i] = idx[pad_segment_samples(int(seg_len[i]), self.tiles, seed)]
         return lim, smp, seg, seg_track.astype(np.int32)
 
+    def output_shape(self, n_segments):
+        """Shape of the segment images: the first ``frames_per_row ** 2`` samples of each segment, ``frames_per_row`` to a row,
+        both channels."""
+        side = self.frames_per_row * self.frame_size
+        return (int(n_segments), side, side, 2)
+
     def run_tables(self, d_thermal, d_filtered, limit_regions, samples, segment_samples, n_tracks, crop_rectangle, out=None,
                    row_map=None, frame_medians=None, frame_info=None):
         """Launch on prepared tables (host numpy or CUDA uint8/int32 tensors).  Returns the CUDA float32
-        tensor (n_segments, rows*size, per_row*size, 2) plus the device tables.
+        tensor ``output_shape(n_segments)`` plus the device tables.
 
         On an extraction's own buffers (``DeviceBatch``): ``row_map`` (host int64, one entry per thermal row) gives the filtered
         row of every thermal row the tables name; ``frame_medians`` (CUDA float32 per thermal row, ``cpt_frame_medians``) and
@@ -287,10 +298,14 @@ class BatchPreprocessor:
         n_smp = len(samples) if isinstance(samples, np.ndarray) else samples.numel() // native.SAMPLE_DTYPE.itemsize
         n_seg = segment_samples.shape[0]
         d_lim, d_smp = dev(limit_regions), dev(samples)
-        d_seg = torch.from_numpy(np.ascontiguousarray(segment_samples, dtype=np.int32)).to(self.device) if isinstance(segment_samples, np.ndarray) else segment_samples
+        # only the first frames_per_row ** 2 columns are tiles of the image (at the default 5: all 25)
+        launched = self.frames_per_row ** 2
+        if isinstance(segment_samples, np.ndarray):
+            d_seg = torch.from_numpy(np.ascontiguousarray(segment_samples[:, :launched], dtype=np.int32)).to(self.device)
+        else:
+            d_seg = segment_samples[:, :launched].contiguous()
         d_tracks = torch.empty((max(n_tracks, 1), native.TRACK_NORM_DTYPE.itemsize), dtype=torch.uint8, device=self.device)
-        rows = (self.tiles + self.frames_per_row - 1) // self.frames_per_row
-        shape = (n_seg, rows * self.frame_size, self.frames_per_row * self.frame_size, 2)
+        shape = self.output_shape(n_seg)
         d_out = None if out is None else out.get("segments")
         if d_out is None or tuple(d_out.shape) != shape:
             d_out = torch.empty(shape, dtype=torch.float32, device=self.device)
@@ -307,7 +322,7 @@ class BatchPreprocessor:
             ctx.preprocess_thermal_limits_ex(d_thermal, d_lim_rows, d_lim, n_lim, d_tracks, n_tracks, frame_medians, frame_info)
         ctx.preprocess_medians_ex(d_thermal, frame_medians, d_smp, n_smp, d_tracks)
         fn = int(self.preprocess_fn) | (0 if self.diff_norm else native.PREPROCESS_PER_TILE)
-        ctx.preprocess_segments_ex(d_thermal, d_filtered, d_smp_rows, d_smp, d_tracks, d_seg, n_seg, self.tiles, self.frames_per_row,
+        ctx.preprocess_segments_ex(d_thermal, d_filtered, d_smp_rows, d_smp, d_tracks, d_seg, n_seg, launched, self.frames_per_row,
                                    self.frame_size, crop_rectangle, fn, d_out)
         return dict(segments=d_out, tracks=d_tracks, samples=d_smp)
 

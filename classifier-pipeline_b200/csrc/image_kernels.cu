@@ -24,10 +24,11 @@ __global__ void __launch_bounds__(256) minmax_kernel(const float *in, long long 
         mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, off));
     }
     if ((threadIdx.x & 31) == 0) {
-        // ordered-int trick: non-negative floats order as ints, negative floats order reversed as unsigned
+        // ordered-int trick: floats with the sign bit clear order as ints, floats with it set order reversed as unsigned.
+        // The branch tests the sign bit, not v >= 0: -0.0 compares equal to 0 but its bits are INT_MIN as an int.
         int *o = reinterpret_cast<int *>(out);
-        if (mn >= 0.0f) atomicMin(o, __float_as_int(mn)); else atomicMax(reinterpret_cast<unsigned *>(o), __float_as_uint(mn));
-        if (mx >= 0.0f) atomicMax(o + 1, __float_as_int(mx)); else atomicMin(reinterpret_cast<unsigned *>(o + 1), __float_as_uint(mx));
+        if (__float_as_int(mn) >= 0) atomicMin(o, __float_as_int(mn)); else atomicMax(reinterpret_cast<unsigned *>(o), __float_as_uint(mn));
+        if (__float_as_int(mx) >= 0) atomicMax(o + 1, __float_as_int(mx)); else atomicMin(reinterpret_cast<unsigned *>(o + 1), __float_as_uint(mx));
     }
 }
 
