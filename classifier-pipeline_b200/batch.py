@@ -28,6 +28,20 @@ def linear_clips(n_frames, background_thresh, weight_table, flags=native.CLIP_UP
     return clips
 
 
+def _total_frames(clips):
+    """Frames the per-frame outputs of a batch of CLIP_DTYPE records hold: max over clips of ``out_offset + n_frames``."""
+    return int((clips["out_offset"] + clips["n_frames"]).max()) if len(clips) else 0
+
+
+def _pinned_out(out, name, shape, dtype):
+    """``out[name]``, replaced by a new pinned host array unless it already has this shape and dtype."""
+    a = out.get(name)
+    if a is None or a.shape != tuple(shape) or a.dtype != np.dtype(dtype):
+        a = native.pinned_empty(shape, dtype)
+        out[name] = a
+    return a
+
+
 class BatchExtractor:
     """Owns a native context and the output buffers of one device."""
 
@@ -56,7 +70,7 @@ class BatchExtractor:
             self.ctx.use_torch_stream()
         if isinstance(clips, np.ndarray):
             n_clips = len(clips)
-            total = int((clips["out_offset"] + clips["n_frames"]).max()) if n_clips else 0
+            total = _total_frames(clips)
             d_clips = torch.from_numpy(clips.view(np.uint8).reshape(-1).copy()).to(self.device)
         else:
             raise TypeError("clips must be a numpy CLIP_DTYPE array")
@@ -99,18 +113,12 @@ class BatchExtractor:
     def extract_host(self, h_frames, clips, keep_filtered=False, keep_labels=False, chunk_clips=0, out=None):
         """Host uint16 frames in, host records out: H2D / kernel / D2H pipelined inside the library."""
         h_frames = np.ascontiguousarray(h_frames, dtype=np.uint16)
-        total = int((clips["out_offset"] + clips["n_frames"]).max()) if len(clips) else 0
+        total = _total_frames(clips)
         out = out if out is not None else {}
-        def buf(name, shape, dtype):
-            a = out.get(name)
-            if a is None or a.shape != tuple(shape) or a.dtype != np.dtype(dtype):
-                a = native.pinned_empty(shape, dtype)
-                out[name] = a
-            return a
-        regions = buf("regions", (max(total, 1), self.max_regions), native.REGION_DTYPE)
-        info = buf("info", (max(total, 1),), native.INFO_DTYPE)
-        filtered = buf("filtered", (max(total, 1), self.height, self.width), np.float32) if keep_filtered else None
-        labels = buf("labels", (max(total, 1), self.height, self.width), np.uint8) if keep_labels else None
+        regions = _pinned_out(out, "regions", (max(total, 1), self.max_regions), native.REGION_DTYPE)
+        info = _pinned_out(out, "info", (max(total, 1),), native.INFO_DTYPE)
+        filtered = _pinned_out(out, "filtered", (max(total, 1), self.height, self.width), np.float32) if keep_filtered else None
+        labels = _pinned_out(out, "labels", (max(total, 1), self.height, self.width), np.uint8) if keep_labels else None
         clips = np.ascontiguousarray(clips)
         self.ctx.extract_batch_host(h_frames, clips, total, regions, info, filtered, labels, chunk_clips)
         out["total_frames"] = total
@@ -127,18 +135,10 @@ class BatchExtractor:
         clips = np.ascontiguousarray(clips)
         if len(clip_first) != len(clips) + 1:
             raise ValueError("clip_first must hold len(clips) + 1 rows")
-        total = int((clips["out_offset"] + clips["n_frames"]).max()) if len(clips) else 0
+        total = _total_frames(clips)
         out = out if out is not None else {}
-
-        def buf(name, shape, dtype):
-            a = out.get(name)
-            if a is None or a.shape != tuple(shape) or a.dtype != np.dtype(dtype):
-                a = native.pinned_empty(shape, dtype)
-                out[name] = a
-            return a
-
-        regions = buf("regions", (max(total, 1), self.max_regions), native.REGION_DTYPE)
-        info = buf("info", (max(total, 1),), native.INFO_DTYPE)
+        regions = _pinned_out(out, "regions", (max(total, 1), self.max_regions), native.REGION_DTYPE)
+        info = _pinned_out(out, "info", (max(total, 1),), native.INFO_DTYPE)
         self.ctx.extract_batch_cptv_host(h_stream, table, clip_first, clips, total, regions, info, chunk_clips)
         out["total_frames"] = total
         return out

@@ -7,6 +7,7 @@
 #include <cstdarg>
 #include <cstdio>
 #include <cstring>
+#include <functional>
 #include <vector>
 
 #include "cptrack_internal.cuh"
@@ -147,18 +148,6 @@ cpt_ctx *cpt_ctx_create(int device, int width, int height, int edge_pixels, int 
     return c;
 }
 
-static void free_stage(cpt_ctx *c) {
-    for (int i = 0; i < 2; ++i) {
-        cudaFree(c->stage_frames[i]); c->stage_frames[i] = nullptr;
-        cudaFree(c->stage_regions[i]); c->stage_regions[i] = nullptr;
-        cudaFree(c->stage_info[i]); c->stage_info[i] = nullptr;
-        cudaFree(c->stage_filtered[i]); c->stage_filtered[i] = nullptr;
-        cudaFree(c->stage_labels[i]); c->stage_labels[i] = nullptr;
-    }
-    c->stage_frames_bytes = 0;
-    c->stage_out_frames = 0;
-}
-
 void cpt_ctx_destroy(cpt_ctx *c) {
     if (!c) return;
     cudaSetDevice(c->device);
@@ -166,29 +155,11 @@ void cpt_ctx_destroy(cpt_ctx *c) {
     for (auto &t : c->tables) {
         cudaFree(t.d_thr);
     }
-    cudaFree(c->scratch);
-    cudaFree(c->qbytes);
-    cudaFree(c->prec);
-    cudaFree(c->fhdr);
-    cudaFree(c->maskbits);
-    cudaFree(c->fallback);
     for (int i = 0; i < 6; ++i)
         if (c->ev_k[i]) cudaEventDestroy(c->ev_k[i]);
     cudaFree(c->work_counter);
     cudaFree(c->zero_frame);
     cudaFree(c->debug);
-    cudaFree(c->d_clips);
-    cudaFree(c->detect_scratch);
-    cudaFree(c->cptv_scratch);
-    cudaFree(c->u8_frames[0]);
-    cudaFree(c->u8_frames[1]);
-    for (int i = 0; i < 2; ++i) {
-        cudaFree(c->pk_stream[i]); cudaFree(c->pk_table[i]); cudaFree(c->pk_first[i]);
-        cudaFreeHost(c->pk_h_table[i]); cudaFreeHost(c->pk_h_first[i]);
-    }
-    cudaFree(c->pk_change);
-    cudaFree(c->scratch_filtered);
-    free_stage(c);
     if (c->events)
         for (int i = 0; i < 2; ++i) {
             cudaEventDestroy(c->ev_h2d[i]);
@@ -198,7 +169,7 @@ void cpt_ctx_destroy(cpt_ctx *c) {
     cudaStreamDestroy(c->own_stream);
     cudaStreamDestroy(c->copy_stream);
     cudaStreamDestroy(c->d2h_stream);
-    delete c;
+    delete c;  // (the scratch and staging buffers free themselves)
 }
 
 int cpt_ctx_set_stream(cpt_ctx *c, void *cuda_stream) {
@@ -389,14 +360,7 @@ static int launch_extract(cpt_ctx *c, const uint16_t *d_frames, const cpt_clip *
                           const cpt_outputs *out, void *d_state, cudaStream_t stream, long long total_frames) {
     if (n_clips == 0) return CPT_OK;
     int grid = std::min(n_clips, c->num_sms);
-    if (!out->d_filtered && c->scratch_ctas < (size_t)grid) {
-        CUDA_TRY(cudaStreamSynchronize(stream));
-        cudaFree(c->scratch);
-        c->scratch = nullptr;
-        size_t ctas = (size_t)std::max(grid, c->num_sms);
-        CUDA_TRY(cudaMalloc(&c->scratch, ctas * 8 * c->g.npx * sizeof(float)));
-        c->scratch_ctas = ctas;
-    }
+    if (!out->d_filtered) CUDA_TRY(c->scratch.ensure((size_t)c->num_sms * 8 * c->g.npx));
     cpt::KernelArgs a{};
     a.g = c->g;
     a.frames = d_frames;
@@ -406,7 +370,7 @@ static int launch_extract(cpt_ctx *c, const uint16_t *d_frames, const cpt_clip *
     a.info = out->d_info;
     a.filtered = out->d_filtered;
     a.labels = out->d_labels;
-    a.scratch = out->d_filtered ? nullptr : c->scratch;
+    a.scratch = out->d_filtered ? nullptr : static_cast<float *>(c->scratch);
     a.state = (uint8_t *)d_state;
     for (int i = 0; i < 4; ++i) a.tables[i] = c->tables[i].device();
     a.work_counter = c->work_counter;
@@ -421,16 +385,7 @@ static int launch_extract(cpt_ctx *c, const uint16_t *d_frames, const cpt_clip *
         // passes over all frames (the recurrence does not depend on the masks)
         if (total_frames < 1 || !out->d_filtered)
             return fail(CPT_ERR_INVALID, "denoise needs cpt_outputs.total_frames and d_filtered");
-        const size_t need = (size_t)total_frames * c->g.npx;
-        if (c->u8_bytes < need) {
-            CUDA_TRY(cudaStreamSynchronize(stream));
-            cudaFree(c->u8_frames[0]); cudaFree(c->u8_frames[1]);
-            c->u8_frames[0] = c->u8_frames[1] = nullptr;
-            c->u8_bytes = 0;
-            CUDA_TRY(cudaMalloc(&c->u8_frames[0], need));
-            CUDA_TRY(cudaMalloc(&c->u8_frames[1], need));
-            c->u8_bytes = need;
-        }
+        for (auto &u8 : c->u8_frames) CUDA_TRY(u8.ensure((size_t)total_frames * c->g.npx));
         a.u8_frames = c->u8_frames[0];
         a.defer_variance = 1;
     }
@@ -445,21 +400,12 @@ static int launch_extract(cpt_ctx *c, const uint16_t *d_frames, const cpt_clip *
     const bool split = split_allowed && !c->force_single && (d_state == nullptr || out->no_resume) && out->d_filtered != nullptr &&
                        total_frames > 0 && c->g.W % 8 == 0;
     if (split) {
-        const size_t qb_frame = (size_t)c->g.H * c->g.qpr;
-        if (c->split_frames < (size_t)total_frames || c->split_clips < (size_t)n_clips) {
-            CUDA_TRY(cudaStreamSynchronize(stream));
-            cudaFree(c->qbytes); cudaFree(c->prec); cudaFree(c->fhdr); cudaFree(c->maskbits); cudaFree(c->fallback);
-            c->qbytes = nullptr; c->prec = nullptr; c->fhdr = nullptr; c->maskbits = nullptr; c->fallback = nullptr;
-            c->split_frames = c->split_clips = 0;
-            const size_t nf = std::max(c->split_frames, (size_t)total_frames), nc = std::max(c->split_clips, (size_t)n_clips);
-            CUDA_TRY(cudaMalloc(&c->qbytes, nf * qb_frame));
-            CUDA_TRY(cudaMalloc(&c->prec, (nf + nc) * c->g.n_strips * sizeof(cpt::StripRec)));
-            CUDA_TRY(cudaMalloc(&c->fhdr, nf * sizeof(cpt::FrameHdr)));
-            CUDA_TRY(cudaMalloc(&c->maskbits, nf * cpt::kMaxWords * sizeof(uint32_t)));
-            CUDA_TRY(cudaMalloc(&c->fallback, (nf + 1) * sizeof(int)));
-            c->split_frames = nf;
-            c->split_clips = nc;
-        }
+        const size_t nf = (size_t)total_frames, nc = (size_t)n_clips;
+        CUDA_TRY(c->qbytes.ensure(nf * c->g.H * c->g.qpr));
+        CUDA_TRY(c->prec.ensure((nf + nc) * c->g.n_strips));
+        CUDA_TRY(c->fhdr.ensure(nf));
+        CUDA_TRY(c->maskbits.ensure(nf * cpt::kMaxWords));
+        CUDA_TRY(c->fallback.ensure(nf + 1));
         a.qbytes = c->qbytes;
         a.prec = c->prec;
         a.fhdr = c->fhdr;
@@ -527,20 +473,49 @@ int cpt_extract_batch(cpt_ctx *c, const uint16_t *d_frames, const cpt_clip *d_cl
     return launch_extract(c, d_frames, d_clips, n_clips, out, d_state, c->stream, out->total_frames);
 }
 
-// Host-staged calls that do not return the filtered images still run the split plan (it keeps the whole GPU busy with
-// (clip, strip) units where the single persistent kernel has one CTA per clip): the images go to a scratch buffer.
-static int ensure_filtered_scratch(cpt_ctx *c, size_t out_frames) {
-    if (c->scratch_filtered_frames >= out_frames) return CPT_OK;
-    CUDA_TRY(cudaDeviceSynchronize());
-    cudaFree(c->scratch_filtered);
-    c->scratch_filtered = nullptr;
-    c->scratch_filtered_frames = 0;
-    CUDA_TRY(cudaMalloc(&c->scratch_filtered, out_frames * c->g.npx * sizeof(float)));
-    c->scratch_filtered_frames = out_frames;
-    return CPT_OK;
+// One chunk of a host-staged call: clips [c0, c1), the input they read -- frames of the raw call, frame table rows of the
+// packed call -- [in_lo, in_hi), the output frames they write [out_lo, out_hi) and, packed call only, the payload bytes of
+// their rows [byte_lo, byte_hi)
+struct Chunk {
+    int c0, c1;
+    int64_t in_lo, in_hi, out_lo, out_hi;
+    uint64_t byte_lo, byte_hi;
+};
+
+static std::vector<Chunk> make_chunks(int n_clips, int chunk_clips) {
+    std::vector<Chunk> chunks;
+    for (int c0 = 0; c0 < n_clips; c0 = chunks.back().c1) chunks.push_back(Chunk{c0, c0 + std::min(chunk_clips, n_clips - c0)});
+    return chunks;
 }
 
-static int ensure_stage(cpt_ctx *c, size_t frames_bytes, size_t out_frames, bool filtered, bool labels) {
+using ChunkStep = std::function<int(int ch, int b)>;
+
+// The pipeline of both host-staged calls, double-buffered over the chunks: chunk ch uses staging buffers b = ch & 1.
+// `upload` enqueues the chunk's input on copy_stream; `decode` (packed call only) turns it into frames in stage_frames[b]
+// on c->stream.  The extraction runs on c->stream and its outputs go back to the host on d2h_stream.  The clips come
+// validated and the chunks with their input spans; this finds the output spans and rebases the clips to both.
+static int run_host_staged(cpt_ctx *c, const cpt_clip *h_clips, std::vector<Chunk> &chunks, cpt_region *h_regions,
+                           cpt_frame_info *h_info, float *h_filtered, uint8_t *h_labels, const ChunkStep &upload,
+                           const ChunkStep &decode) {
+    const size_t npx = c->g.npx;
+    const int n_clips = chunks.back().c1;
+    std::vector<cpt_clip> rebased(h_clips, h_clips + n_clips);
+    size_t max_in = 1, max_out = 1;
+    for (Chunk &k : chunks) {
+        k.out_lo = INT64_MAX;
+        k.out_hi = 0;
+        for (int i = k.c0; i < k.c1; ++i) {
+            k.out_lo = std::min(k.out_lo, h_clips[i].out_offset);
+            k.out_hi = std::max(k.out_hi, h_clips[i].out_offset + h_clips[i].n_frames);
+        }
+        for (int i = k.c0; i < k.c1; ++i) {
+            rebased[i].frame_offset -= k.in_lo;
+            rebased[i].init_offset -= k.in_lo;
+            rebased[i].out_offset -= k.out_lo;
+        }
+        max_in = std::max(max_in, (size_t)(k.in_hi - k.in_lo));
+        max_out = std::max(max_out, (size_t)(k.out_hi - k.out_lo));
+    }
     if (!c->events) {
         for (int i = 0; i < 2; ++i) {
             CUDA_TRY(cudaEventCreateWithFlags(&c->ev_h2d[i], cudaEventDisableTiming));
@@ -549,24 +524,50 @@ static int ensure_stage(cpt_ctx *c, size_t frames_bytes, size_t out_frames, bool
         }
         c->events = true;
     }
-    bool need = frames_bytes > c->stage_frames_bytes || out_frames > c->stage_out_frames ||
-                (filtered && !c->stage_has_filtered) || (labels && !c->stage_has_labels);
-    if (!need) return CPT_OK;
-    CUDA_TRY(cudaDeviceSynchronize());
-    free_stage(c);
-    filtered = filtered || c->stage_has_filtered;
-    labels = labels || c->stage_has_labels;
-    for (int i = 0; i < 2; ++i) {
-        CUDA_TRY(cudaMalloc(&c->stage_frames[i], frames_bytes));
-        CUDA_TRY(cudaMalloc(&c->stage_regions[i], out_frames * c->g.max_regions * sizeof(cpt_region)));
-        CUDA_TRY(cudaMalloc(&c->stage_info[i], out_frames * sizeof(cpt_frame_info)));
-        if (filtered) CUDA_TRY(cudaMalloc(&c->stage_filtered[i], out_frames * c->g.npx * sizeof(float)));
-        if (labels) CUDA_TRY(cudaMalloc(&c->stage_labels[i], out_frames * c->g.npx));
+    for (int b = 0; b < 2; ++b) {
+        CUDA_TRY(c->stage_frames[b].ensure(max_in * npx));
+        CUDA_TRY(c->stage_regions[b].ensure(max_out * c->g.max_regions));
+        CUDA_TRY(c->stage_info[b].ensure(max_out));
+        if (h_filtered) CUDA_TRY(c->stage_filtered[b].ensure(max_out * npx));
+        if (h_labels) CUDA_TRY(c->stage_labels[b].ensure(max_out * npx));
     }
-    c->stage_frames_bytes = frames_bytes;
-    c->stage_out_frames = out_frames;
-    c->stage_has_filtered = filtered;
-    c->stage_has_labels = labels;
+    // calls that do not return the filtered images still run the split plan (it keeps the whole GPU busy with (clip, strip)
+    // units where the single persistent kernel has one CTA per clip): the images go to a scratch buffer
+    if (!h_filtered) CUDA_TRY(c->scratch_filtered.ensure(max_out * npx));
+    CUDA_TRY(c->d_clips.ensure(n_clips));
+    CUDA_TRY(cudaMemcpyAsync(c->d_clips, rebased.data(), sizeof(cpt_clip) * n_clips, cudaMemcpyHostToDevice, c->stream));
+    CUDA_TRY(cudaStreamSynchronize(c->stream));
+    for (int ch = 0; ch < (int)chunks.size(); ++ch) {
+        const Chunk &k = chunks[ch];
+        const int b = ch & 1;
+        // staging buffers b are free once the kernels of chunk ch-2 have run and its outputs have been copied back
+        if (ch >= 2) CUDA_TRY(cudaStreamWaitEvent(c->copy_stream, c->ev_compute[b], 0));
+        if (int rc = upload(ch, b)) return rc;
+        CUDA_TRY(cudaEventRecord(c->ev_h2d[b], c->copy_stream));
+        CUDA_TRY(cudaStreamWaitEvent(c->stream, c->ev_h2d[b], 0));
+        if (ch >= 2) CUDA_TRY(cudaStreamWaitEvent(c->stream, c->ev_d2h[b], 0));
+        if (decode)
+            if (int rc = decode(ch, b)) return rc;
+        int denoise = 0;  // (CPT_CLIP_DENOISE clips: the NLM, mask and component passes follow the chunk's launch)
+        for (int i = k.c0; i < k.c1; ++i) denoise |= (h_clips[i].flags & CPT_CLIP_DENOISE) ? 1 : 0;
+        const int64_t nf = k.out_hi - k.out_lo;
+        cpt_outputs out{c->stage_regions[b], c->stage_info[b], h_filtered ? c->stage_filtered[b] : c->scratch_filtered,
+                        h_labels ? static_cast<uint8_t *>(c->stage_labels[b]) : nullptr, nf, denoise, 1};
+        if (int rc = launch_extract(c, c->stage_frames[b], c->d_clips + k.c0, k.c1 - k.c0, &out, nullptr, c->stream, nf)) return rc;
+        CUDA_TRY(cudaEventRecord(c->ev_compute[b], c->stream));
+        CUDA_TRY(cudaStreamWaitEvent(c->d2h_stream, c->ev_compute[b], 0));
+        CUDA_TRY(cudaMemcpyAsync(h_regions + (size_t)k.out_lo * c->g.max_regions, c->stage_regions[b],
+                                 (size_t)nf * c->g.max_regions * sizeof(cpt_region), cudaMemcpyDeviceToHost, c->d2h_stream));
+        CUDA_TRY(cudaMemcpyAsync(h_info + k.out_lo, c->stage_info[b], (size_t)nf * sizeof(cpt_frame_info), cudaMemcpyDeviceToHost, c->d2h_stream));
+        if (h_filtered)
+            CUDA_TRY(cudaMemcpyAsync(h_filtered + (size_t)k.out_lo * npx, c->stage_filtered[b], (size_t)nf * npx * sizeof(float),
+                                     cudaMemcpyDeviceToHost, c->d2h_stream));
+        if (h_labels)
+            CUDA_TRY(cudaMemcpyAsync(h_labels + (size_t)k.out_lo * npx, c->stage_labels[b], (size_t)nf * npx, cudaMemcpyDeviceToHost, c->d2h_stream));
+        CUDA_TRY(cudaEventRecord(c->ev_d2h[b], c->d2h_stream));
+    }
+    CUDA_TRY(cudaStreamSynchronize(c->d2h_stream));
+    CUDA_TRY(cudaStreamSynchronize(c->stream));
     return CPT_OK;
 }
 
@@ -578,82 +579,28 @@ int cpt_extract_batch_host(cpt_ctx *c, const uint16_t *h_frames, const cpt_clip 
     if (n_clips == 0) return CPT_OK;
     if (!h_frames || !h_clips || !h_regions || !h_info) return fail(CPT_ERR_INVALID, "null host buffer");
     CUDA_TRY(cudaSetDevice(c->device));
-    if (chunk_clips <= 0) chunk_clips = c->num_sms;
-    const size_t npx = c->g.npx;
-    const int n_chunks = (n_clips + chunk_clips - 1) / chunk_clips;
-    // per chunk: the span of input frames and of output frames its clips touch
-    struct Span { int64_t in_lo, in_hi, out_lo, out_hi; };
-    std::vector<Span> spans(n_chunks);
-    std::vector<cpt_clip> rebased(h_clips, h_clips + n_clips);
-    size_t max_in = 0, max_out = 0;
-    for (int ch = 0; ch < n_chunks; ++ch) {
-        int c0 = ch * chunk_clips, c1 = std::min(n_clips, c0 + chunk_clips);
-        Span sp{INT64_MAX, 0, INT64_MAX, 0};
-        for (int i = c0; i < c1; ++i) {
+    std::vector<Chunk> chunks = make_chunks(n_clips, chunk_clips > 0 ? chunk_clips : c->num_sms);
+    for (Chunk &sp : chunks) {
+        // the chunk's input: from the first frame its clips read to past the last
+        sp.in_lo = INT64_MAX;
+        for (int i = sp.c0; i < sp.c1; ++i) {
             const cpt_clip &k = h_clips[i];
             if (k.flags & CPT_CLIP_RESUME) return fail(CPT_ERR_INVALID, "CPT_CLIP_RESUME is not supported by the host-staged call");
             if (k.n_frames < 0 || k.frame_offset < 0 || k.init_offset < 0 || k.out_offset < 0 || k.ring_frames != 0)
                 return fail(CPT_ERR_INVALID, "clip %d: bad offsets", i);
             if (k.out_offset + k.n_frames > total_frames) return fail(CPT_ERR_INVALID, "clip %d: outputs exceed total_frames", i);
-            sp.in_lo = std::min(sp.in_lo, std::min(k.frame_offset, k.init_offset));
-            sp.in_hi = std::max(sp.in_hi, std::max(k.frame_offset + k.n_frames, k.init_offset + 1));
-            sp.out_lo = std::min(sp.out_lo, k.out_offset);
-            sp.out_hi = std::max(sp.out_hi, k.out_offset + k.n_frames);
+            sp.in_lo = std::min({sp.in_lo, k.frame_offset, k.init_offset});
+            sp.in_hi = std::max({sp.in_hi, k.frame_offset + k.n_frames, k.init_offset + 1});
         }
-        for (int i = c0; i < c1; ++i) {
-            rebased[i].frame_offset -= sp.in_lo;
-            rebased[i].init_offset -= sp.in_lo;
-            rebased[i].out_offset -= sp.out_lo;
-        }
-        spans[ch] = sp;
-        max_in = std::max(max_in, (size_t)(sp.in_hi - sp.in_lo));
-        max_out = std::max(max_out, (size_t)std::max<int64_t>(sp.out_hi - sp.out_lo, 1));
     }
-    int rc = ensure_stage(c, max_in * npx * sizeof(uint16_t), max_out, h_filtered != nullptr, h_labels != nullptr);
-    if (rc) return rc;
-    if (!h_filtered && (rc = ensure_filtered_scratch(c, max_out))) return rc;
-    if (c->d_clips_cap < (size_t)n_clips) {
-        cudaFree(c->d_clips);
-        c->d_clips = nullptr;
-        CUDA_TRY(cudaMalloc(&c->d_clips, sizeof(cpt_clip) * n_clips));
-        c->d_clips_cap = n_clips;
-    }
-    CUDA_TRY(cudaMemcpyAsync(c->d_clips, rebased.data(), sizeof(cpt_clip) * n_clips, cudaMemcpyHostToDevice, c->stream));
-    CUDA_TRY(cudaStreamSynchronize(c->stream));
-    for (int ch = 0; ch < n_chunks; ++ch) {
-        const int b = ch & 1;
-        const int c0 = ch * chunk_clips, c1 = std::min(n_clips, c0 + chunk_clips);
-        const Span &sp = spans[ch];
-        // frames buffer b is free once the kernel of chunk ch-2 has run
-        if (ch >= 2) CUDA_TRY(cudaStreamWaitEvent(c->copy_stream, c->ev_compute[b], 0));
-        CUDA_TRY(cudaMemcpyAsync(c->stage_frames[b], h_frames + (size_t)sp.in_lo * npx,
-                                 (size_t)(sp.in_hi - sp.in_lo) * npx * sizeof(uint16_t), cudaMemcpyHostToDevice, c->copy_stream));
-        CUDA_TRY(cudaEventRecord(c->ev_h2d[b], c->copy_stream));
-        CUDA_TRY(cudaStreamWaitEvent(c->stream, c->ev_h2d[b], 0));
-        if (ch >= 2) CUDA_TRY(cudaStreamWaitEvent(c->stream, c->ev_d2h[b], 0));
-        int chunk_denoise = 0;  // (CPT_CLIP_DENOISE clips: the NLM, mask and component passes follow the chunk's launch)
-        for (int i = c0; i < c1; ++i) chunk_denoise |= (h_clips[i].flags & CPT_CLIP_DENOISE) ? 1 : 0;
-        cpt_outputs out{c->stage_regions[b], c->stage_info[b], h_filtered ? c->stage_filtered[b] : c->scratch_filtered,
-                        h_labels ? c->stage_labels[b] : nullptr, sp.out_hi - sp.out_lo, chunk_denoise, 1};
-        rc = launch_extract(c, (const uint16_t *)c->stage_frames[b], c->d_clips + c0, c1 - c0, &out, nullptr, c->stream,
-                            sp.out_hi - sp.out_lo);
-        if (rc) return rc;
-        CUDA_TRY(cudaEventRecord(c->ev_compute[b], c->stream));
-        CUDA_TRY(cudaStreamWaitEvent(c->d2h_stream, c->ev_compute[b], 0));
-        const size_t nf = (size_t)(sp.out_hi - sp.out_lo);
-        CUDA_TRY(cudaMemcpyAsync(h_regions + (size_t)sp.out_lo * c->g.max_regions, c->stage_regions[b],
-                                 nf * c->g.max_regions * sizeof(cpt_region), cudaMemcpyDeviceToHost, c->d2h_stream));
-        CUDA_TRY(cudaMemcpyAsync(h_info + sp.out_lo, c->stage_info[b], nf * sizeof(cpt_frame_info), cudaMemcpyDeviceToHost, c->d2h_stream));
-        if (h_filtered)
-            CUDA_TRY(cudaMemcpyAsync(h_filtered + (size_t)sp.out_lo * npx, c->stage_filtered[b], nf * npx * sizeof(float),
-                                     cudaMemcpyDeviceToHost, c->d2h_stream));
-        if (h_labels)
-            CUDA_TRY(cudaMemcpyAsync(h_labels + (size_t)sp.out_lo * npx, c->stage_labels[b], nf * npx, cudaMemcpyDeviceToHost, c->d2h_stream));
-        CUDA_TRY(cudaEventRecord(c->ev_d2h[b], c->d2h_stream));
-    }
-    CUDA_TRY(cudaStreamSynchronize(c->d2h_stream));
-    CUDA_TRY(cudaStreamSynchronize(c->stream));
-    return CPT_OK;
+    const size_t npx = c->g.npx;
+    auto upload = [&](int ch, int b) -> int {
+        const Chunk &sp = chunks[ch];
+        CUDA_TRY(cudaMemcpyAsync(c->stage_frames[b], h_frames + (size_t)sp.in_lo * npx, (size_t)(sp.in_hi - sp.in_lo) * npx * sizeof(uint16_t),
+                                 cudaMemcpyHostToDevice, c->copy_stream));
+        return CPT_OK;
+    };
+    return run_host_staged(c, h_clips, chunks, h_regions, h_info, h_filtered, h_labels, upload, nullptr);
 }
 
 // Host-staged extraction from PACKED clips: the inflated CPTV frame payloads travel over PCIe (about one byte per pixel
@@ -668,17 +615,15 @@ int cpt_extract_batch_cptv_host(cpt_ctx *c, const uint8_t *h_stream, uint64_t st
     CUDA_TRY(cudaSetDevice(c->device));
     if (chunk_clips <= 0) chunk_clips = c->num_sms;
     const size_t npx = c->g.npx;
-    const int n_chunks = (n_clips + chunk_clips - 1) / chunk_clips;
-    // per chunk: the rows of the frame table, the bytes of the stream and the output frames its clips touch
-    struct Span { int64_t row_lo, row_hi, out_lo, out_hi; uint64_t byte_lo, byte_hi; };
-    std::vector<Span> spans(n_chunks);
-    std::vector<cpt_clip> rebased(h_clips, h_clips + n_clips);
-    size_t max_rows = 0, max_out = 0, max_bytes = 0;
-    for (int ch = 0; ch < n_chunks; ++ch) {
-        const int c0 = ch * chunk_clips, c1 = std::min(n_clips, c0 + chunk_clips);
-        Span sp{h_clip_first[c0], h_clip_first[c1], INT64_MAX, 0, UINT64_MAX, 0};
-        if (sp.row_lo < 0 || sp.row_hi < sp.row_lo) return fail(CPT_ERR_INVALID, "clip table rows must ascend");
-        for (int64_t r = sp.row_lo; r < sp.row_hi; ++r) {
+    std::vector<Chunk> chunks = make_chunks(n_clips, chunk_clips);
+    size_t max_rows = 1, max_bytes = 0;
+    for (Chunk &sp : chunks) {
+        // the chunk's input: the frame table rows of its clips and the payload bytes of those rows
+        sp.in_lo = h_clip_first[sp.c0];
+        sp.in_hi = h_clip_first[sp.c1];
+        if (sp.in_lo < 0 || sp.in_hi < sp.in_lo) return fail(CPT_ERR_INVALID, "clip table rows must ascend");
+        sp.byte_lo = UINT64_MAX;
+        for (int64_t r = sp.in_lo; r < sp.in_hi; ++r) {
             // every payload must lie inside the stream (a malformed file must not make the device read out of bounds)
             const cpt_cptv_frame &f = h_table[r];
             if (f.bit_width < 1 || f.bit_width > 24) return fail(CPT_ERR_INVALID, "frame %lld: unsupported bit width %d", (long long)r, f.bit_width);
@@ -688,7 +633,8 @@ int cpt_extract_batch_cptv_host(cpt_ctx *c, const uint8_t *h_stream, uint64_t st
             sp.byte_lo = std::min(sp.byte_lo, f.payload_offset);
             sp.byte_hi = std::max(sp.byte_hi, f.payload_offset + size);
         }
-        for (int i = c0; i < c1; ++i) {
+        if (sp.in_hi == sp.in_lo) sp.byte_lo = 0;
+        for (int i = sp.c0; i < sp.c1; ++i) {
             const cpt_clip &k = h_clips[i];
             if (k.flags & CPT_CLIP_RESUME) return fail(CPT_ERR_UNSUPPORTED, "clip %d: CPT_CLIP_RESUME is not supported by the host-staged calls", i);
             if (k.n_frames < 0 || k.out_offset < 0 || k.ring_frames != 0) return fail(CPT_ERR_INVALID, "clip %d: bad offsets", i);
@@ -696,101 +642,45 @@ int cpt_extract_batch_cptv_host(cpt_ctx *c, const uint8_t *h_stream, uint64_t st
                 k.init_offset >= std::max(h_clip_first[i + 1], h_clip_first[i] + 1))
                 return fail(CPT_ERR_INVALID, "clip %d: frames outside the clip's rows of the frame table", i);
             if (k.out_offset + k.n_frames > total_frames) return fail(CPT_ERR_INVALID, "clip %d: outputs exceed total_frames", i);
-            sp.out_lo = std::min(sp.out_lo, k.out_offset);
-            sp.out_hi = std::max(sp.out_hi, k.out_offset + k.n_frames);
         }
-        if (sp.row_hi == sp.row_lo) { sp.byte_lo = sp.byte_hi = 0; }
-        if (sp.out_lo == INT64_MAX) sp.out_lo = 0;
-        for (int i = c0; i < c1; ++i) {
-            rebased[i].frame_offset -= sp.row_lo;
-            rebased[i].init_offset -= sp.row_lo;
-            rebased[i].out_offset -= sp.out_lo;
-        }
-        spans[ch] = sp;
-        max_rows = std::max(max_rows, (size_t)(sp.row_hi - sp.row_lo));
-        max_out = std::max(max_out, (size_t)std::max<int64_t>(sp.out_hi - sp.out_lo, 1));
+        max_rows = std::max(max_rows, (size_t)(sp.in_hi - sp.in_lo));
         max_bytes = std::max(max_bytes, (size_t)(sp.byte_hi - sp.byte_lo));
     }
-    int rc = ensure_stage(c, std::max<size_t>(max_rows, 1) * npx * sizeof(uint16_t), max_out, false, false);
-    if (rc) return rc;
-    if ((rc = ensure_filtered_scratch(c, max_out))) return rc;
-    // packed staging: stream bytes (+4: the unpacker's 32-bit window may read past the last payload), frame table rows, the
-    // clips' first rows; the decoder's int32 change images
-    const size_t need_bytes = max_bytes + 4, need_rows = std::max<size_t>(max_rows, 1);
-    if (c->pk_bytes < need_bytes || c->pk_rows < need_rows || c->pk_clips < (size_t)chunk_clips + 1) {
-        CUDA_TRY(cudaDeviceSynchronize());
-        for (int i = 0; i < 2; ++i) {
-            cudaFree(c->pk_stream[i]); cudaFree(c->pk_table[i]); cudaFree(c->pk_first[i]);
-            cudaFreeHost(c->pk_h_table[i]); cudaFreeHost(c->pk_h_first[i]);
-            c->pk_stream[i] = nullptr; c->pk_table[i] = nullptr; c->pk_first[i] = nullptr; c->pk_h_table[i] = nullptr; c->pk_h_first[i] = nullptr;
-        }
-        cudaFree(c->pk_change);
-        c->pk_change = nullptr;
-        c->pk_bytes = c->pk_rows = c->pk_clips = 0;
-        for (int i = 0; i < 2; ++i) {
-            CUDA_TRY(cudaMalloc(&c->pk_stream[i], need_bytes));
-            CUDA_TRY(cudaMalloc(&c->pk_table[i], need_rows * sizeof(cpt_cptv_frame)));
-            CUDA_TRY(cudaMalloc(&c->pk_first[i], ((size_t)chunk_clips + 1) * sizeof(int32_t)));
-            CUDA_TRY(cudaHostAlloc((void **)&c->pk_h_table[i], need_rows * sizeof(cpt_cptv_frame), cudaHostAllocDefault));
-            CUDA_TRY(cudaHostAlloc((void **)&c->pk_h_first[i], ((size_t)chunk_clips + 1) * sizeof(int32_t), cudaHostAllocDefault));
-        }
-        CUDA_TRY(cudaMalloc(&c->pk_change, need_rows * npx * sizeof(int32_t)));
-        c->pk_bytes = need_bytes; c->pk_rows = need_rows; c->pk_clips = (size_t)chunk_clips + 1;
+    // packed staging: payload bytes (+4: the unpacker's 32-bit window may read past the last payload), frame table rows,
+    // the clips' first rows; the decoder's int32 change images
+    for (int b = 0; b < 2; ++b) {
+        CUDA_TRY(c->pk_stream[b].ensure(max_bytes + 4));
+        CUDA_TRY(c->pk_table[b].ensure(max_rows));
+        CUDA_TRY(c->pk_h_table[b].ensure(max_rows));
+        CUDA_TRY(c->pk_first[b].ensure((size_t)chunk_clips + 1));
+        CUDA_TRY(c->pk_h_first[b].ensure((size_t)chunk_clips + 1));
     }
-    if (c->d_clips_cap < (size_t)n_clips) {
-        cudaFree(c->d_clips);
-        c->d_clips = nullptr;
-        CUDA_TRY(cudaMalloc(&c->d_clips, sizeof(cpt_clip) * n_clips));
-        c->d_clips_cap = n_clips;
-    }
-    CUDA_TRY(cudaMemcpyAsync(c->d_clips, rebased.data(), sizeof(cpt_clip) * n_clips, cudaMemcpyHostToDevice, c->stream));
-    CUDA_TRY(cudaStreamSynchronize(c->stream));
-    for (int ch = 0; ch < n_chunks; ++ch) {
-        const int b = ch & 1;
-        const int c0 = ch * chunk_clips, c1 = std::min(n_clips, c0 + chunk_clips);
-        const Span &sp = spans[ch];
-        const int rows = (int)(sp.row_hi - sp.row_lo);
-        // staging buffers b (host tables, packed bytes, decoded frames) are free once the kernels of chunk ch-2 have run
-        if (ch >= 2) {
-            CUDA_TRY(cudaEventSynchronize(c->ev_compute[b]));
-            CUDA_TRY(cudaStreamWaitEvent(c->copy_stream, c->ev_compute[b], 0));
-        }
+    CUDA_TRY(c->pk_change.ensure(max_rows * npx));
+    auto upload = [&](int ch, int b) -> int {
+        const Chunk &sp = chunks[ch];
+        const int rows = (int)(sp.in_hi - sp.in_lo);
+        // the host tables of buffers b are rewritten here: the copies of chunk ch-2 out of them must have run
+        if (ch >= 2) CUDA_TRY(cudaEventSynchronize(c->ev_compute[b]));
         for (int r = 0; r < rows; ++r) {
-            c->pk_h_table[b][r] = h_table[sp.row_lo + r];
+            c->pk_h_table[b][r] = h_table[sp.in_lo + r];
             c->pk_h_table[b][r].payload_offset -= sp.byte_lo;
         }
-        for (int i = c0; i <= c1; ++i) c->pk_h_first[b][i - c0] = (int32_t)(h_clip_first[i] - sp.row_lo);
+        for (int i = sp.c0; i <= sp.c1; ++i) c->pk_h_first[b][i - sp.c0] = (int32_t)(h_clip_first[i] - sp.in_lo);
         if (rows > 0) {
             CUDA_TRY(cudaMemcpyAsync(c->pk_stream[b], h_stream + sp.byte_lo, (size_t)(sp.byte_hi - sp.byte_lo), cudaMemcpyHostToDevice, c->copy_stream));
             CUDA_TRY(cudaMemcpyAsync(c->pk_table[b], c->pk_h_table[b], (size_t)rows * sizeof(cpt_cptv_frame), cudaMemcpyHostToDevice, c->copy_stream));
         }
-        CUDA_TRY(cudaMemcpyAsync(c->pk_first[b], c->pk_h_first[b], (size_t)(c1 - c0 + 1) * sizeof(int32_t), cudaMemcpyHostToDevice, c->copy_stream));
-        CUDA_TRY(cudaEventRecord(c->ev_h2d[b], c->copy_stream));
-        CUDA_TRY(cudaStreamWaitEvent(c->stream, c->ev_h2d[b], 0));
-        if (ch >= 2) CUDA_TRY(cudaStreamWaitEvent(c->stream, c->ev_d2h[b], 0));
-        if (rows > 0) {
-            rc = cpt::cptv_decode_launch(c, c->pk_stream[b], c->pk_table[b], rows, c->pk_first[b], c1 - c0, (uint16_t *)c->stage_frames[b],
-                                         c->pk_change, c->stream);
-            if (rc) return rc;
-        }
-        int chunk_denoise = 0;
-        for (int i = c0; i < c1; ++i) chunk_denoise |= (h_clips[i].flags & CPT_CLIP_DENOISE) ? 1 : 0;
-        cpt_outputs out{c->stage_regions[b], c->stage_info[b], c->scratch_filtered, nullptr, sp.out_hi - sp.out_lo, chunk_denoise, 1};
-        rc = launch_extract(c, (const uint16_t *)c->stage_frames[b], c->d_clips + c0, c1 - c0, &out, nullptr, c->stream, sp.out_hi - sp.out_lo);
-        if (rc) return rc;
-        CUDA_TRY(cudaEventRecord(c->ev_compute[b], c->stream));
-        CUDA_TRY(cudaStreamWaitEvent(c->d2h_stream, c->ev_compute[b], 0));
-        const size_t nf = (size_t)std::max<int64_t>(sp.out_hi - sp.out_lo, 0);
-        if (nf) {
-            CUDA_TRY(cudaMemcpyAsync(h_regions + (size_t)sp.out_lo * c->g.max_regions, c->stage_regions[b], nf * c->g.max_regions * sizeof(cpt_region),
-                                     cudaMemcpyDeviceToHost, c->d2h_stream));
-            CUDA_TRY(cudaMemcpyAsync(h_info + sp.out_lo, c->stage_info[b], nf * sizeof(cpt_frame_info), cudaMemcpyDeviceToHost, c->d2h_stream));
-        }
-        CUDA_TRY(cudaEventRecord(c->ev_d2h[b], c->d2h_stream));
-    }
-    CUDA_TRY(cudaStreamSynchronize(c->d2h_stream));
-    CUDA_TRY(cudaStreamSynchronize(c->stream));
-    return CPT_OK;
+        CUDA_TRY(cudaMemcpyAsync(c->pk_first[b], c->pk_h_first[b], (size_t)(sp.c1 - sp.c0 + 1) * sizeof(int32_t), cudaMemcpyHostToDevice, c->copy_stream));
+        return CPT_OK;
+    };
+    auto decode = [&](int ch, int b) -> int {
+        const Chunk &sp = chunks[ch];
+        const int rows = (int)(sp.in_hi - sp.in_lo);
+        if (rows == 0) return CPT_OK;
+        return cpt::cptv_decode_launch(c, c->pk_stream[b], c->pk_table[b], rows, c->pk_first[b], sp.c1 - sp.c0, c->stage_frames[b],
+                                       c->pk_change, c->stream);
+    };
+    return run_host_staged(c, h_clips, chunks, h_regions, h_info, nullptr, nullptr, upload, decode);
 }
 
 int cpt_background_process(cpt_ctx *c, void *d_state, const int32_t *d_record_index, int n_records,

@@ -86,16 +86,8 @@ int cpt_cptv_decode(cpt_ctx *c, const uint8_t *d_stream, const cpt_cptv_frame *d
     if (n_frames == 0 || n_clips == 0) return CPT_OK;
     if (!d_stream || !d_table || !d_clip_first || !d_frames) return fail(CPT_ERR_INVALID, "null argument");
     CUDA_TRY(cudaSetDevice(c->device));
-    const size_t need = (size_t)n_frames * c->g.npx * sizeof(int32_t);
-    if (c->cptv_scratch_bytes < need) {
-        CUDA_TRY(cudaStreamSynchronize(c->stream));
-        cudaFree(c->cptv_scratch);
-        c->cptv_scratch = nullptr;
-        c->cptv_scratch_bytes = 0;
-        CUDA_TRY(cudaMalloc(&c->cptv_scratch, need));
-        c->cptv_scratch_bytes = need;
-    }
-    return cpt::cptv_decode_launch(c, d_stream, d_table, n_frames, d_clip_first, n_clips, d_frames, (int32_t *)c->cptv_scratch, c->stream);
+    CUDA_TRY(c->cptv_scratch.ensure((size_t)n_frames * c->g.npx));
+    return cpt::cptv_decode_launch(c, d_stream, d_table, n_frames, d_clip_first, n_clips, d_frames, c->cptv_scratch, c->stream);
 }
 
 }  // extern "C"

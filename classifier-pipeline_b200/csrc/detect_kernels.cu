@@ -295,15 +295,8 @@ int cpt_detect_objects_ex(cpt_ctx *c, const uint8_t *d_image, int width, int hei
     const size_t off_count = off_label + (size_t)(max_components + 1) * 4;
     const size_t off_hist = off_count + 256;
     const size_t total = off_hist + 256 * sizeof(unsigned int);
-    if (c->detect_scratch_bytes < total) {
-        CUDA_TRY(cudaStreamSynchronize(c->stream));
-        cudaFree(c->detect_scratch);
-        c->detect_scratch = nullptr;
-        c->detect_scratch_bytes = 0;
-        CUDA_TRY(cudaMalloc(&c->detect_scratch, total));
-        c->detect_scratch_bytes = total;
-    }
-    uint8_t *base = (uint8_t *)c->detect_scratch;
+    CUDA_TRY(c->detect_scratch.ensure(total));
+    uint8_t *base = c->detect_scratch;
     uint8_t *grey_a = base, *grey_b = base + img_bytes, *mask_a = base + 2 * img_bytes, *mask_b = base + 3 * img_bytes;
     int *parent = (int *)(base + off_parent), *slot_of = (int *)(base + off_slot);
     cpt::CompStats *stats = (cpt::CompStats *)(base + off_stats);
