@@ -1,5 +1,4 @@
 // cptrack.cu -- C ABI (include/cptrack.h) over the sm_100a kernels.
-#include <cstdlib>
 #include <cuda_runtime.h>
 
 #include <algorithm>
@@ -395,9 +394,8 @@ static int launch_extract(cpt_ctx *c, const uint16_t *d_frames, const cpt_clip *
     // kernel with its three warp roles.
     const bool timed = c->time_kernels && c->ev_k[0];
     if (timed) CUDA_TRY(cudaEventRecord(c->ev_k[0], stream));
-    static const bool split_allowed = [] { const char *e = getenv("CPT_SPLIT"); return !(e && e[0] == '0'); }();
     // (the sweep kernel stages frame rows with 16-byte bulk copies: rows must be a multiple of 8 pixels)
-    const bool split = split_allowed && !c->force_single && (d_state == nullptr || out->no_resume) && out->d_filtered != nullptr &&
+    const bool split = !c->force_single && (d_state == nullptr || out->no_resume) && out->d_filtered != nullptr &&
                        total_frames > 0 && c->g.W % 8 == 0;
     if (split) {
         const size_t nf = (size_t)total_frames, nc = (size_t)n_clips;

@@ -1,10 +1,10 @@
-// cptrack_kernels.cuh -- sm_100a kernels for thermal-clip track extraction (DESIGN.md section 3.1).
+// cptrack_kernels.cuh -- sm_100a kernels for thermal-clip track extraction (DESIGN.md section 3.1): launch sizes,
+// shared-memory layouts and the per-frame rules both launch plans share.
 //
 // The per-clip recurrence of the reference (WeightedBackground: background + per-pixel weight counter, the 45-frame
 // sliding sum that replaces np.mean(get_last_x(45)), piclassifier/motiondetector.py:178-248 and
-// track/cliptrackextractor.py:168-176) runs in one persistent CTA per clip with its whole state resident in shared
-// memory; frames stream through once from HBM and each frame emits filtered fp32 (K1), the uint8 label image (K5) and
-// a compact region list (K5/K6).  Stages of a frame (SURVEY.md section 8a):
+// track/cliptrackextractor.py:168-176) streams through the frames from HBM, and each frame emits filtered fp32 (K1), the
+// uint8 label image (K5) and a compact region list (K5/K6).  Stages of a frame (SURVEY.md section 8a):
 //   fused sweep   weighted background update of the previous frame (K7), then F = P - B, sliding sum, sum P,
 //                 min/max F, per-quad maxima of F                                               (K1, K7, K8)
 //   scalars       avg_change, normalisation range, mapped threshold, bound below which no pixel can fire  (K2)
@@ -14,52 +14,34 @@
 //   close         C[y] = M[y-1] | (M[y] & M[y-2]) on 32-bit row words                           (K4)
 //   label         run-based union-find on the bit rows, OpenCV label order                      (K5)
 //   regions       bbox / area / centroid sums per component, delta-frame variance               (K5, K6)
-// Two launch plans share these device functions:
+// Two launch plans run these stages and must give the same bits:
 //   split path (batch launches that keep the filtered images and resume from no state): strip_sweep_kernel (strip_sweep.cu:
 //     the recurrence, one CTA per (clip, strip of rows)) -> frame_scalars_kernel -> frame_regions_kernel (one small CTA per
 //     frame: marks .. regions in place; the rare very busy mask goes on a list for frame_components_kernel) ->
 //     region_variance_kernel
 //   single kernel (streaming, resumed clips, regions-only): extract_clips_kernel, the stages as three warp roles
 //     (sweep / mask / component warps) running concurrently on consecutive frames of the clip
+// Each rule that decides those bits has one copy both plans call: here the scalars of a frame (frame_scalars_of), the
+// rounded background average (rounded_background_average), the frame's info record (frame_info_of), the normalise
+// (norm_u8, norm_u8_int) and the union-find; in extract_kernel.cu the work-list emission (emit_norm_groups,
+// emit_blur_groups), normalise, blur and components of a frame and the region variance.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
 
 #include "../../include/cptrack.h"
 
-#ifndef CPT_EXP
-#define CPT_EXP 0
-#endif
-
 namespace cpt {
 
 // warp-specialised pipeline over consecutive frames: sweep warps (the recurrence), mask warps (scalars, work lists,
-// normalise, blur) and component warps (labelling)
-// Sweep-warp count (tools/gpu_exp.sh builds -DCPT_EXP=<n> variants for A/B runs; the measured alternatives are in
-// DESIGN.md section 7).  640 = 16 row groups (7 or 8 quads per thread); 480 / 800 / 960 = 12 / 20 / 24 balanced groups of
-// 10 / 6 / 5 quads (800 and 960: split path only -- the single persistent kernel cannot hold that many warps next to
-// its mask and component warps, so those builds shrink the two roles to placeholders).
-#if CPT_EXP == 10
-constexpr int kPThreads = 640;
-#elif CPT_EXP == 5
-constexpr int kPThreads = 800;
-#elif CPT_EXP == 4
-constexpr int kPThreads = 960;
-#elif CPT_EXP == 2
-constexpr int kPThreads = 480;
-#else
+// normalise, blur) and component warps (labelling).
 // 19 sweep warps: 15 rows x 40 quads per iteration at 160 pixels (the last 8 threads idle).  120 rows / 15 row groups = 8
-// quads for every thread once the two border rows are balanced (Geometry::balanced): no warp is ever ahead of another.
+// quads for every thread once the two border rows are balanced (Geometry::balanced): no warp is ever ahead of another
+// (other sweep-warp counts were measured slower, DESIGN.md section 7).
 constexpr int kPThreads = 608;
-#endif
 constexpr int kPWarps = kPThreads / 32;
-#if CPT_EXP == 5 || CPT_EXP == 4
-constexpr int kMThreads = 32;
-constexpr int kCThreads = 32;
-#else
 constexpr int kMThreads = 128;                  // 4 mask warps
 constexpr int kCThreads = 256;                  // 8 component warps
-#endif
 constexpr int kCWarps = kCThreads / 32;
 constexpr int kThreads = kPThreads + kMThreads + kCThreads;
 constexpr int kWarps = kThreads / 32;
@@ -67,14 +49,7 @@ constexpr int kWarps = kThreads / 32;
 // frame_components_kernel (full-size tables) redoes the frames whose masks are too busy for it
 constexpr int kFThreads = 128;   // frame_regions_kernel
 constexpr int kGThreads = 256;   // frame_components_kernel
-#ifndef CPT_VAR_THREADS
-#define CPT_VAR_THREADS 256
-#endif
-#ifndef CPT_VAR_BATCH
-#define CPT_VAR_BATCH 1
-#endif
-constexpr int kVarThreads = CPT_VAR_THREADS;  // region_variance_kernel: one warp per frame
-constexpr int kVarBatch = CPT_VAR_BATCH;      // pixels per lane whose loads are in flight together
+constexpr int kVarThreads = 256;  // region_variance_kernel: one warp per frame
 constexpr int kMaxPx = 19200;
 constexpr int kQIter = (kMaxPx / 4 + kPThreads - 1) / kPThreads;  // 6 quads of 4 pixels per pixel thread
 constexpr int kMaxW = 160;
@@ -260,20 +235,11 @@ struct __align__(16) Smem {
 // shared memory of frame_regions_kernel (one frame per CTA, one band of rows at a time: hot quads -> work lists -> normalise
 // -> blur + threshold)
 constexpr int kBandHalo = 4;    // rows of normalised values a blur output can reach above / below a hot quad
-#ifndef CPT_BAND_ROWS
-#define CPT_BAND_ROWS 24
-#endif
-#ifndef CPT_LEAN_PARENTS
-#define CPT_LEAN_PARENTS 1024
-#endif
-#ifndef CPT_F_MINBLOCKS
-#define CPT_F_MINBLOCKS 13
-#endif
-constexpr int kBandRows = CPT_BAND_ROWS;   // hot rows one band covers
-constexpr int kFMinBlocks = CPT_F_MINBLOCKS;  // frame_regions_kernel CTAs per SM the register allocation allows
+constexpr int kBandRows = 24;     // hot rows one band covers
+constexpr int kFMinBlocks = 13;   // frame_regions_kernel CTAs per SM the register allocation allows
 constexpr int kBandURows = kBandRows + 2 * kBandHalo;
 constexpr int kBandList = kBandURows * (kMaxW / 8);  // every group of every row of the band: the lists cannot overflow
-constexpr int kLeanParents = CPT_LEAN_PARENTS;  // run ids of the in-CTA components stage: rows of the mask's extent * runs per row
+constexpr int kLeanParents = 1024;  // run ids of the in-CTA components stage: rows of the mask's extent * runs per row
 constexpr int kLeanSlots = 32;      // components it numbers; slot kLeanSlots is the overflow sink (more: the fallback kernel)
 struct __align__(16) MaskSmem {
     union {
@@ -361,6 +327,84 @@ __device__ __forceinline__ uint32_t norm_u8(int v, float range_f) {
 // n / r by multiplication: m = ceil(2^(24+l) / r), l = ceil(log2 r)  (Granlund-Montgomery).
 __device__ __forceinline__ uint32_t norm_u8_int(int v, uint32_t m, int shift) {
     return (uint32_t)(((unsigned long long)(uint32_t)(255 * v) * m) >> shift);
+}
+
+// WeightedBackground.average after an update that changed the background: int(round(np.average(background))),
+// motiondetector.py:232, of the background summed over the ncrop crop pixels -- half to even, in integers.
+__device__ __forceinline__ double rounded_background_average(uint32_t bsum, uint32_t ncrop) {
+    uint32_t qa = bsum / ncrop;
+    const uint32_t ra = bsum - qa * ncrop;
+    if (2u * ra > ncrop || (2u * ra == ncrop && (qa & 1u))) qa += 1u;
+    return (double)qa;
+}
+
+struct FrameScalars {
+    int ac, gmn, gmx, fth;
+    float thr;
+    uint32_t nmagic;
+    int nshift;
+};
+
+// K2 scalars of one frame (track/cliptracker.py:93-122, imageprocessing.py:151-169) from its sums: avg_change, the
+// normalisation range, the mapped threshold (fp32 as numpy >= 2 evaluates it), the bound F >= fth below which a pixel cannot
+// reach the threshold (INT32_MIN: no usable bound) and the Granlund-Montgomery constants of the integer normalise.
+__device__ __forceinline__ FrameScalars frame_scalars_of(uint32_t psum, int fmin, int fmax, double average, int background_thresh, int npx) {
+    FrameScalars r;
+    // avg_change = int(round(np.average(thermal) - background average)), cliptracker.py:103-105
+    const double avg_int = rint(average);
+    if (avg_int == average && average >= 0.0 && average < 65536.0) {
+        // integer average (always, once the background has changed): round_half_even((sum - avg * n) / n) in integers;
+        // identical to the fp64 expression because the only ties are exact.  |sum - avg * n| < 2^31.
+        const int num = (int)psum - (int)avg_int * npx;
+        int qd = num / npx, rem = num - qd * npx;
+        if (rem < 0) { rem += npx; qd -= 1; }
+        if (2 * rem > npx || (2 * rem == npx && (qd & 1))) qd += 1;
+        r.ac = qd;
+    } else {
+        r.ac = (int)rint((double)psum / (double)npx - average);
+    }
+    r.gmx = max(fmax - r.ac, 0);
+    r.gmn = max(fmin - r.ac, 0);
+    r.fth = INT32_MIN;
+    r.nmagic = 0;  // 0: the fp32 divide; else (255 v) / range == (255 v * nmagic) >> nshift for 255 v < 2^24
+    r.nshift = 0;
+    if (r.gmx == r.gmn) {
+        r.thr = (float)background_thresh;  // cliptracker.py:118-119
+    } else {
+        const float range = (float)r.gmx - (float)r.gmn;
+        r.thr = __fmul_rn(__fdiv_rn((float)background_thresh, range), 255.0f);
+        const unsigned rr = (unsigned)(r.gmx - r.gmn);
+        if (255ull * rr < (1ull << 24)) {
+            // every product is exact in fp32 here, so trunc(fl(255 v / r)) == (255 v) / r and a quad can only produce
+            // foreground if one of its pixels has U > floor(thr):  U >= ith + 1  <=>  v >= ceil((ith + 1) r / 255),
+            // v = max(F - ac, 0) - gmn, i.e. F >= fth (the bound is >= 1, so the clamp never matters)
+            const int it = (int)floorf(r.thr);
+            if (it >= 0 && it < 255) r.fth = (int)(((unsigned)(it + 1) * rr + 254u) / 255u) + r.ac + r.gmn;
+            // Granlund-Montgomery: l = ceil(log2 r), m = ceil(2^(24 + l) / r) < 2^25.  The fp64 quotient is exact for powers
+            // of two and otherwise at least 1/r >= 2^-17 away from an integer: its ceiling is m.
+            const int l = (rr <= 1u) ? 0 : 32 - __clz((int)(rr - 1u));
+            r.nshift = 24 + l;
+            r.nmagic = (uint32_t)ceil(ldexp(1.0, r.nshift) / (double)rr);
+        }
+    }
+    return r;
+}
+
+// The frame's info record from its scalars and sums; the thermal extrema and sum |filtered| only with
+// CPT_CLIP_FRAME_STATS.  dn_marker goes to reserved[1], the denoise marker (0: not a denoise clip; 1: a clip's first
+// frame; 2: the previous filtered image is frame o - 1).  frame_scalars_kernel knows it here; the single kernel passes 0
+// and its mask warps write the marker once they have emitted the frame's normalised image.
+__device__ __forceinline__ cpt_frame_info frame_info_of(const FrameScalars &fs, double average, uint32_t psum, int fmin, int fmax,
+                                                        bool want_stats, int pmin, int pmax, uint32_t fabs_sum, int dn_marker) {
+    cpt_frame_info fi;
+    fi.background_average = average;
+    fi.threshold = fs.thr; fi.norm_min = fs.gmn; fi.norm_max = fs.gmx; fi.avg_change = fs.ac;
+    fi.filtered_min = fmin; fi.filtered_max = fmax; fi.n_components = 0;
+    fi.thermal_min = want_stats ? pmin : 0; fi.thermal_max = want_stats ? pmax : 0;
+    fi.thermal_sum = psum; fi.abs_filtered_sum = want_stats ? fabs_sum : 0u; fi.thermal_median = 0.f;
+    fi.reserved[0] = 0;
+    fi.reserved[1] = dn_marker;
+    return fi;
 }
 
 // normalize(F, new_max=255) of get_delta_frame (track/cliptracker.py:249-261): fp64 arithmetic

@@ -6,9 +6,8 @@
 //   component warps (8):  frame t:   close, run-based labelling, statistics, variance (K4, K5, K6)
 //   Messages (frame sums + per-quad maxima, then the thresholded bit image) are double buffered and handed over
 //   with named barriers (full / empty per buffer); everything else the roles touch is disjoint shared memory.
-// extract_sweep_kernel: the same sweep warps on their own, plus a scalar warp (one frame behind: info record, byte
-//   threshold for the hot-quad ballots) and a producer warp (TMA bulk copies of the frame rows into a shared-memory ring);
-//   frame_regions_kernel / frame_components_kernel / region_variance_kernel then do the per-frame stages one CTA (warp) per frame.
+// Split path: after strip_sweep_kernel and frame_scalars_kernel (strip_sweep.cu), frame_regions_kernel /
+//   frame_components_kernel / region_variance_kernel do the per-frame stages one CTA (warp) per frame.
 #include "cptrack_kernels.cuh"
 
 namespace cpt {
@@ -519,6 +518,43 @@ __device__ __forceinline__ void normalise_group(SM &s, const float *F, int grp, 
     normalise_values(s, f0, f1, grp, ac, gmn, gmx, nmagic, nshift, u_global, u_off);
 }
 
+// Work lists, one row at a time: near = the row's hot-quad bits OR-ed over the rows around it (bit q: quad q), rowmask = the
+// row's quads.  Group g of the row is listed, as row_grp + g, if either of its quads (bits 2g, 2g + 1) is marked; count is
+// the list's length in shared memory (one atomic per row).  kCapped: entries from kListCap on are counted, not stored (the
+// single kernel turns an overflow into dense work; frame_regions_kernel's lists hold every group of a band).
+// emit_norm_groups: the groups to normalise, the marks widened by two quads.
+template <bool kCapped>
+__device__ __forceinline__ void emit_norm_groups(unsigned long long near, unsigned long long rowmask, int row_grp, int *count,
+                                                 uint16_t *list) {
+    if (!near) return;
+    const unsigned long long mk = (near | (near << 1) | (near >> 1) | (near << 2) | (near >> 2)) & rowmask;
+    unsigned long long grp_bits = (mk | (mk >> 1)) & 0x5555555555555555ull;
+    int base = atomicAdd(count, __popcll(grp_bits));
+    while (grp_bits) {
+        const int bit = __ffsll((long long)grp_bits) - 1;
+        grp_bits &= grp_bits - 1;
+        if (kCapped && base >= kListCap) { ++base; continue; }
+        list[base++] = (uint16_t)(row_grp + (bit >> 1));
+    }
+}
+
+// emit_blur_groups: the groups to blur, the marks widened by one quad; an entry carries the group's two quad marks in
+// bits 14-15 (blur_group's q2).
+template <bool kCapped>
+__device__ __forceinline__ void emit_blur_groups(unsigned long long near, unsigned long long rowmask, int row_grp, int *count,
+                                                 uint16_t *list) {
+    if (!near) return;
+    const unsigned long long mk = (near | (near << 1) | (near >> 1)) & rowmask;
+    unsigned long long grp_bits = (mk | (mk >> 1)) & 0x5555555555555555ull;
+    int base = atomicAdd(count, __popcll(grp_bits));
+    while (grp_bits) {
+        const int bit = __ffsll((long long)grp_bits) - 1;
+        grp_bits &= grp_bits - 1;
+        if (kCapped && base >= kListCap) { ++base; continue; }
+        list[base++] = (uint16_t)((row_grp + (bit >> 1)) | ((uint32_t)((mk >> bit) & 3ull) << 14));
+    }
+}
+
 // L2 policy of the bulk prefetch of the next frame: a fraction of its lines is kept (evict_last) until the frame is read
 // again, 45 frames later, as P_old
 __device__ __forceinline__ unsigned long long l2_policy_keep() {
@@ -1016,88 +1052,35 @@ __device__ void sweep_warps(const KernelArgs &a, Smem &s, const cpt_clip &clip, 
     }
 }
 
-// K2 / K7 scalars of one frame from the sweep's message (one thread): WeightedBackground.average, avg_change, the
-// normalisation range, the mapped threshold, the bound F >= fth below which a pixel cannot reach the threshold and the
-// byte threshold for the stored quad maxima.  Writes the frame's info record and s.bcast_i[0..5, 8, 13, 14].
+// K2 / K7 scalars of one frame from the sweep's message (one thread): WeightedBackground.average, the frame's scalars
+// (frame_scalars_of) and the byte threshold for the stored quad maxima.  Writes the frame's info record and
+// s.bcast_i[0..5, 8, 13, 14].
 __device__ __forceinline__ void frame_scalars(const KernelArgs &a, Smem &s, const cpt_clip &clip, FrameMsg &fm, size_t o,
                                               bool is_frame, bool want_stats, double &average) {
     const Geometry &g = a.g;
-    const int npx = g.npx;
     const uint32_t v0 = fm.red[0];
     const int v1 = (int)fm.red[1], v2 = (int)fm.red[2];
-    const uint32_t bsum = fm.red[6], changed = fm.red[7];
-    if (fm.update && changed) {
-        // int(round(np.average(background))), motiondetector.py:232 -- half to even, in integers
-        uint32_t qa = bsum / (uint32_t)g.ncrop;
-        const uint32_t ra = bsum - qa * (uint32_t)g.ncrop;
-        if (2u * ra > (uint32_t)g.ncrop || (2u * ra == (uint32_t)g.ncrop && (qa & 1u))) qa += 1u;
-        average = (double)qa;
-    }
+    if (fm.update && fm.red[7]) average = rounded_background_average(fm.red[6], (uint32_t)g.ncrop);  // the background changed
     if (is_frame) {
-        // avg_change = int(round(np.average(thermal) - background average)), cliptracker.py:103-105
-        int ac;
-        const double avg_int = rint(average);
-        if (avg_int == average && average >= 0.0 && average < 65536.0) {
-            // integer average (always, once the background has changed): round_half_even((sum - avg*n) / n)
-            // in integers; identical to the fp64 expression because the only ties are exact
-            // |sum - avg * n| < 2^31: 32-bit arithmetic
-            int num = (int)v0 - (int)avg_int * npx;
-            int qd = num / npx, rem = num - qd * npx;
-            if (rem < 0) { rem += npx; qd -= 1; }
-            if (2 * rem > npx || (2 * rem == npx && (qd & 1))) qd += 1;
-            ac = (int)qd;
-        } else {
-            ac = (int)rint((double)v0 / (double)npx - average);
-        }
-        int gmx = max(v2 - ac, 0), gmn = max(v1 - ac, 0);
-        float thr;
-        int fth = INT32_MIN;
-        uint32_t nmagic = 0;  // 0: the fp32 divide; else (255 v) / r == (255 v * nmagic) >> nshift for 255 v < 2^24
-        int nshift = 0;
-        if (gmx == gmn) {
-            thr = (float)clip.background_thresh;  // cliptracker.py:118-119
-        } else {
-            float range = (float)gmx - (float)gmn;
-            thr = __fmul_rn(__fdiv_rn((float)clip.background_thresh, range), 255.0f);
-            unsigned r = (unsigned)(gmx - gmn);
-            if (255ull * r < (1ull << 24)) {
-                // every product is exact in fp32 here, so trunc(fl(255 v / r)) == (255 v) / r and a quad can
-                // only produce foreground if one of its pixels has U > floor(thr):
-                // U >= ith + 1  <=>  v >= ceil((ith + 1) r / 255), v = max(F - ac, 0) - gmn,
-                // i.e. F >= fth (the bound is >= 1, so the clamp never matters)
-                int it = (int)floorf(thr);
-                if (it >= 0 && it < 255) fth = (int)(((unsigned)(it + 1) * r + 254u) / 255u) + ac + gmn;
-                // Granlund-Montgomery: l = ceil(log2 r), m = ceil(2^(24 + l) / r) < 2^25.  The fp64 quotient is exact
-                // for powers of two and otherwise at least 1/r >= 2^-17 away from an integer: its ceiling is m.
-                const int l = (r <= 1u) ? 0 : 32 - __clz((int)(r - 1u));
-                nshift = 24 + l;
-                nmagic = (uint32_t)ceil(ldexp(1.0, nshift) / (double)r);
-            }
-        }
-        s.bcast_i[0] = ac; s.bcast_i[1] = gmn; s.bcast_i[2] = gmx;
+        const FrameScalars fs = frame_scalars_of(v0, v1, v2, average, clip.background_thresh, g.npx);
+        s.bcast_i[0] = fs.ac; s.bcast_i[1] = fs.gmn; s.bcast_i[2] = fs.gmx;
         s.bcast_i[3] = v1; s.bcast_i[4] = v2;
-        s.bcast_i[5] = __float_as_int(thr);
-        s.bcast_i[13] = (int)nmagic; s.bcast_i[14] = nshift;
+        s.bcast_i[5] = __float_as_int(fs.thr);
+        s.bcast_i[13] = (int)fs.nmagic; s.bcast_i[14] = fs.nshift;
         // byte threshold for the quad maxima the sweep stored relative to qref (0: no usable bound, dense work):
         // stored v = clamp(max F - qref, -128, 127) + 128, hot <=> v >= clamp(fth - qref, -127, 127) + 128.
         // v == 0 means max F <= qref - 128 < fth; v == 255 means max F >= qref + 127 >= fth unless the
         // threshold was clamped from above, which only widens the marks.
         {
             int tu = 0;
-            if (fth != INT32_MIN) {
-                const long long dq = (long long)fth - (long long)fm.qref;
+            if (fs.fth != INT32_MIN) {
+                const long long dq = (long long)fs.fth - (long long)fm.qref;
                 if (dq >= -127) tu = (int)min(dq, 127ll) + 128;
             }
             s.bcast_i[8] = tu;
         }
-        if (fth != INT32_MIN) *(volatile int32_t *)&s.fth_latest = fth;
-        cpt_frame_info fi;
-        fi.threshold = thr; fi.norm_min = gmn; fi.norm_max = gmx; fi.avg_change = ac;
-        fi.filtered_min = v1; fi.filtered_max = v2; fi.n_components = 0;
-        fi.thermal_min = want_stats ? (int)fm.red[3] : 0; fi.thermal_max = want_stats ? (int)fm.red[4] : 0;
-        fi.thermal_sum = v0; fi.abs_filtered_sum = want_stats ? fm.red[5] : 0u; fi.thermal_median = 0.f;
-        fi.background_average = average; fi.reserved[0] = 0; fi.reserved[1] = 0;
-        a.info[o] = fi;
+        if (fs.fth != INT32_MIN) *(volatile int32_t *)&s.fth_latest = fs.fth;
+        a.info[o] = frame_info_of(fs, average, v0, v1, v2, want_stats, (int)fm.red[3], (int)fm.red[4], fm.red[5], 0);
     }
     frame_msg_reset(fm);
 }
@@ -1153,7 +1136,7 @@ __device__ void mask_warps(const KernelArgs &a, Smem &s, const cpt_clip &clip, i
         have_prev = 1;
         if (denoise) {
             // K3 sits between K2 and K4: emit the whole normalised image; cv2.fastNlMeansDenoising, blur, threshold,
-            // close and components run as separate wide passes over all frames (nlm_denoise_kernel, mask_components_kernel)
+            // close and components run as separate wide passes over all frames (nlm_quads_kernel, mask_components_kernel)
             uint8_t *u_frame = a.u8_frames + o * npx;
             for (int grp = mtid; grp < g.groups; grp += kMThreads) normalise_group(s, fcur, grp, ac, gmn, gmx, nmagic, nshift, u_frame);
             if (mtid == 0) a.info[o].reserved[1] = (t > 0 || prev_in_output) ? 2 : 1;  // 2: the previous filtered image is frame o - 1
@@ -1207,31 +1190,8 @@ __device__ void mask_warps(const KernelArgs &a, Smem &s, const cpt_clip &clip, i
                     near_u |= h;
                     if (dy >= -2 && dy <= 2) near_b |= h;
                 }
-                const int row_grp = rrow * g.gpr;
-                if (near_u) {
-                    const unsigned long long mk = (near_u | (near_u << 1) | (near_u >> 1) | (near_u << 2) | (near_u >> 2)) & rowmask;
-                    // group g of the row is wanted if either of its quads (bits 2g, 2g + 1) is marked
-                    unsigned long long grp_bits = (mk | (mk >> 1)) & 0x5555555555555555ull;
-                    int base = atomicAdd(&s.bcast_i[11], __popcll(grp_bits));
-                    while (grp_bits) {
-                        const int bit = __ffsll((long long)grp_bits) - 1;
-                        grp_bits &= grp_bits - 1;
-                        if (base < kListCap) s.list_u[base] = (uint16_t)(row_grp + (bit >> 1));
-                        ++base;
-                    }
-                }
-                if (near_b) {
-                    const unsigned long long mk = (near_b | (near_b << 1) | (near_b >> 1)) & rowmask;
-                    unsigned long long grp_bits = (mk | (mk >> 1)) & 0x5555555555555555ull;
-                    int base = atomicAdd(&s.bcast_i[12], __popcll(grp_bits));
-                    while (grp_bits) {
-                        const int bit = __ffsll((long long)grp_bits) - 1;
-                        grp_bits &= grp_bits - 1;
-                        const uint32_t quads = (uint32_t)((mk >> bit) & 3ull);
-                        if (base < kListCap) s.list_b[base] = (uint16_t)((row_grp + (bit >> 1)) | (quads << 14));
-                        ++base;
-                    }
-                }
+                emit_norm_groups<true>(near_u, rowmask, rrow * g.gpr, &s.bcast_i[11], s.list_u);
+                emit_blur_groups<true>(near_b, rowmask, rrow * g.gpr, &s.bcast_i[12], s.list_b);
             }
             bar_sync(BAR_M, kMThreads);
             n_u = s.bcast_i[11];
@@ -1580,7 +1540,7 @@ __global__ void __launch_bounds__(kFThreads, kFMinBlocks) frame_regions_kernel(c
     const float *fcur = a.filtered + (size_t)o * g.npx;
     if (dn_marker) {
         // denoise clips: K3 sits between K2 and K4 -- emit the whole normalised image; cv2.fastNlMeansDenoising, blur,
-        // threshold, close and components follow as wide passes (nlm_denoise_kernel, mask_components_kernel)
+        // threshold, close and components follow as wide passes (nlm_quads_kernel, mask_components_kernel)
         uint8_t *u_frame = a.u8_frames + (size_t)o * g.npx;
         for (int grp = tid; grp < g.groups; grp += kFThreads) normalise_group(s, fcur, grp, ac, gmn, gmx, nmagic, nshift, u_frame);
         return;
@@ -1711,17 +1671,7 @@ __global__ void __launch_bounds__(kFThreads, kFMinBlocks) frame_regions_kernel(c
                     const int rr = y + dy;
                     if (rr >= lo && rr <= hi) nearq |= s.hot64[rr];
                 }
-                if (nearq) {
-                    const unsigned long long mk = (nearq | (nearq << 1) | (nearq >> 1) | (nearq << 2) | (nearq >> 2)) & rowmask;
-                    unsigned long long grp_bits = (mk | (mk >> 1)) & 0x5555555555555555ull;
-                    int base = atomicAdd(&s.count[bp][0], __popcll(grp_bits));
-                    const int row_grp = tid * g.gpr;  // (band row)
-                    while (grp_bits) {
-                        const int bit = __ffsll((long long)grp_bits) - 1;
-                        grp_bits &= grp_bits - 1;
-                        s.list_u[base++] = (uint16_t)(row_grp + (bit >> 1));
-                    }
-                }
+                emit_norm_groups<false>(nearq, rowmask, tid * g.gpr, &s.count[bp][0], s.list_u);  // (band row)
             }
         } else {
             const int y = br0 + tid - kFThreads / 2;
@@ -1732,17 +1682,7 @@ __global__ void __launch_bounds__(kFThreads, kFMinBlocks) frame_regions_kernel(c
                     const int rr = y + dy;
                     if (rr >= lo && rr <= hi) nearq |= s.hot64[rr];
                 }
-                if (nearq) {
-                    const unsigned long long mk = (nearq | (nearq << 1) | (nearq >> 1)) & rowmask;
-                    unsigned long long grp_bits = (mk | (mk >> 1)) & 0x5555555555555555ull;
-                    int base = atomicAdd(&s.count[bp][1], __popcll(grp_bits));
-                    const int row_grp = y * g.gpr;  // (frame row)
-                    while (grp_bits) {
-                        const int bit = __ffsll((long long)grp_bits) - 1;
-                        grp_bits &= grp_bits - 1;
-                        s.list_b[base++] = (uint16_t)((row_grp + (bit >> 1)) | ((uint32_t)((mk >> bit) & 3ull) << 14));
-                    }
-                }
+                emit_blur_groups<false>(nearq, rowmask, y * g.gpr, &s.count[bp][1], s.list_b);  // (frame row)
             }
         }
         __syncthreads();
@@ -1789,29 +1729,13 @@ __device__ __forceinline__ void region_variance_warp(const Geometry &g, cpt_regi
     if (l < 0 || tp < 0 || bw < 1 || bh < 1 || l + bw > g.W || tp + bh > g.H) return;  // not a record of this launch
     double s1 = 0.0, s2 = 0.0;
     const uint32_t rcp = 0xffffffffu / (uint32_t)bw + 1u;  // i / bw == umulhi(i, rcp) for i * bw < 2^32
-    // pixels lane, lane + 32, ... in this order; the loads of eight of them are in flight together (a bounding box is cold:
-    // one DRAM round trip per batch instead of one per pixel)
-    constexpr int kBatch = kVarBatch;
-    for (int i0 = lane; i0 < npix; i0 += 32 * kBatch) {
-        float fcv[kBatch], fpv[kBatch];
-#pragma unroll
-        for (int k = 0; k < kBatch; ++k) {
-            const int i = i0 + 32 * k;
-            fcv[k] = 0.0f; fpv[k] = 0.0f;
-            if (i < npix) {
-                const int yy = bw == 1 ? i : (int)__umulhi((uint32_t)i, rcp), xx = i - yy * bw, p = (tp + yy) * g.W + l + xx;  // (rcp wraps to 0 for bw == 1)
-                fcv[k] = __ldg(fcur + p);
-                fpv[k] = __ldg(fprev + p);
-            }
-        }
-#pragma unroll
-        for (int k = 0; k < kBatch; ++k) {
-            if (i0 + 32 * k < npix) {
-                const float d = fabsf(norm255((int)fcv[k], cur_fmin, cur_fmax, exact) - norm255((int)fpv[k], prev_fmin, prev_fmax, exact));
-                s1 += (double)d;
-                s2 += (double)d * (double)d;
-            }
-        }
+    // pixels lane, lane + 32, ... in this order
+    for (int i = lane; i < npix; i += 32) {
+        const int yy = bw == 1 ? i : (int)__umulhi((uint32_t)i, rcp), xx = i - yy * bw, p = (tp + yy) * g.W + l + xx;  // (rcp wraps to 0 for bw == 1)
+        const float fc = __ldg(fcur + p), fp = __ldg(fprev + p);
+        const float d = fabsf(norm255((int)fc, cur_fmin, cur_fmax, exact) - norm255((int)fp, prev_fmin, prev_fmax, exact));
+        s1 += (double)d;
+        s2 += (double)d * (double)d;
     }
     for (int off = 16; off; off >>= 1) {
         s1 += __shfl_xor_sync(0xffffffffu, s1, off);

@@ -5,24 +5,19 @@
 //     w = table[dist >> 6],  est += w * ext[p + o],  wsum += w;      out = (est + wsum / 2) / wsum
 // with table[a] = rint(19096 * exp(-(a * 64 / 49) / 9)), zero below 0.001 * 19096 -- only a <= 47 is non-zero.
 // Compute bound by design (441 offsets x 49 template pixels per output pixel).  nlm_quads_kernel, the kernel every
-// ordinary image takes: a thread owns 4 adjacent columns x 10 rows, its 40 estimates and weight sums live in registers for
+// image takes: a thread owns 4 adjacent columns x 10 rows, its 40 estimates and weight sums live in registers for
 // all 441 offsets; per offset it walks down 10 + 6 rows of its columns -- per row three words of the image and of the
 // shifted image (funnel shifts bring the shifted bytes into line), |a - b| on four bytes at a time, the squares summed
 // by dp4a into the four 7-wide horizontal sums, a 7-deep register ring for the vertical running sum -- and then looks
 // up the weight of each of its 10 x 4 pixels: about 27 instructions per pixel and offset, no barrier inside the search.
-// nlm_denoise_kernel (one CTA per 16x16 tile, squared differences box-summed through shared memory, two barriers per
-// offset) is the first version; it remains for images wider than the quad kernel's tile logic is sized for.
 #include <algorithm>
 #include <cmath>
-#include <cstdlib>
 
 #include "cptrack_internal.cuh"
 
 namespace cpt {
 
-constexpr int kNlmTile = 16, kNlmT = 3, kNlmS = 10, kNlmB = kNlmT + kNlmS;  // template / search / border radii
-constexpr int kNlmExt = kNlmTile + 2 * kNlmB;                               // 42
-constexpr int kNlmSq = kNlmTile + 2 * kNlmT;                                // 22
+constexpr int kNlmT = 3, kNlmS = 10, kNlmB = kNlmT + kNlmS;  // template / search / border radii
 constexpr int kNlmWeights = 64;
 
 __constant__ int c_nlm_weights[kNlmWeights];
@@ -33,73 +28,20 @@ __device__ __forceinline__ int nlm_reflect(int p, int n) {
     return p;
 }
 
-// info != nullptr: only the frames the extraction kernel marked for denoising (reserved[1] != 0) are processed
-__global__ void __launch_bounds__(256) nlm_denoise_kernel(const uint8_t *src, int W, int H, uint8_t *dst, const cpt_frame_info *info) {
-    if (info && info[blockIdx.z].reserved[1] == 0) return;
-    __shared__ uint8_t ext[kNlmExt][kNlmExt + 2];
-    __shared__ uint32_t sq[kNlmSq][kNlmSq + 1];
-    __shared__ uint32_t hs[kNlmSq][kNlmTile + 1];
-    const int tid = threadIdx.x, tx = tid & 15, ty = tid >> 4;
-    const int x0 = blockIdx.x * kNlmTile, y0 = blockIdx.y * kNlmTile;
-    const uint8_t *img = src + (size_t)blockIdx.z * W * H;
-    for (int i = tid; i < kNlmExt * kNlmExt; i += 256) {
-        const int ey = i / kNlmExt, ex = i - ey * kNlmExt;
-        ext[ey][ex] = img[nlm_reflect(y0 + ey - kNlmB, H) * W + nlm_reflect(x0 + ex - kNlmB, W)];
-    }
-    __syncthreads();
-    uint32_t est = 0, wsum = 0;
-    for (int oy = -kNlmS; oy <= kNlmS; ++oy)
-        for (int ox = -kNlmS; ox <= kNlmS; ++ox) {
-            // squared differences over the tile grown by the template radius
-            for (int i = tid; i < kNlmSq * kNlmSq; i += 256) {
-                const int sy = i / kNlmSq, sx = i - sy * kNlmSq;
-                const int d = (int)ext[sy + kNlmS + oy][sx + kNlmS + ox] - (int)ext[sy + kNlmS][sx + kNlmS];
-                sq[sy][sx] = (uint32_t)(d * d);
-            }
-            __syncthreads();
-            // horizontal 7-sums
-            for (int i = tid; i < kNlmSq * kNlmTile; i += 256) {
-                const int sy = i >> 4, sx = i & 15;
-                uint32_t acc = 0;
-#pragma unroll
-                for (int j = 0; j < 2 * kNlmT + 1; ++j) acc += sq[sy][sx + j];
-                hs[sy][sx] = acc;
-            }
-            __syncthreads();
-            uint32_t dist = 0;
-#pragma unroll
-            for (int j = 0; j < 2 * kNlmT + 1; ++j) dist += hs[ty + j][tx];
-            const uint32_t a = dist >> 6;
-            if (a < (uint32_t)kNlmWeights) {
-                const uint32_t w = (uint32_t)c_nlm_weights[a];
-                est += w * ext[ty + kNlmB + oy][tx + kNlmB + ox];
-                wsum += w;
-            }
-            // (hs is rewritten only after the next offset's first barrier, sq only after this offset's second)
-        }
-    const int x = x0 + tx, y = y0 + ty;
-    if (x < W && y < H) dst[(size_t)blockIdx.z * W * H + y * W + x] = (uint8_t)((est + wsum / 2) / wsum);
-}
-
-
 // ---- the quad kernel -------------------------------------------------------------------------------------------------
 constexpr int kNqCols = 160;                       // pixels per tile row: 40 threads x 4
 constexpr int kNqQuads = kNqCols / 4;
-#ifndef CPT_NLM_ROWS
-#define CPT_NLM_ROWS 10
-#endif
-#ifndef CPT_NLM_MINBLOCKS
-#define CPT_NLM_MINBLOCKS 3
-#endif
-constexpr int kNqRowsT = CPT_NLM_ROWS;             // rows per thread
+constexpr int kNqRowsT = 10;                       // rows per thread
 constexpr int kNqStrips = 4;                       // threads per column quad: 4 strips of kNqRowsT rows
 constexpr int kNqRows = kNqRowsT * kNqStrips;      // 40 rows per tile: three tiles cover the 120 rows of a Lepton frame exactly
 constexpr int kNqThreads = kNqQuads * kNqStrips;   // 160
 constexpr int kNqPad = 16;                         // columns left / right of the tile in shared memory (>= 13, a multiple of 4)
 constexpr int kNqExtW = kNqCols + 2 * kNqPad;      // 192 bytes per row
 constexpr int kNqExtH = kNqRows + 2 * kNlmB;       // 58 rows
+constexpr int kNqMinBlocks = 3;                    // CTAs per SM the register allocation allows
 
-__global__ void __launch_bounds__(kNqThreads, CPT_NLM_MINBLOCKS) nlm_quads_kernel(const uint8_t *src, int W, int H, uint8_t *dst, const cpt_frame_info *info) {
+// info != nullptr: only the frames the extraction kernel marked for denoising (reserved[1] != 0) are processed
+__global__ void __launch_bounds__(kNqThreads, kNqMinBlocks) nlm_quads_kernel(const uint8_t *src, int W, int H, uint8_t *dst, const cpt_frame_info *info) {
     if (info && info[blockIdx.z].reserved[1] == 0) return;
     __shared__ __align__(16) uint8_t ext[kNqExtH][kNqExtW];
     __shared__ int wtab[kNlmWeights];
@@ -217,14 +159,8 @@ int nlm_launch(cpt_ctx *c, const uint8_t *d_src, int width, int height, long lon
         const uint8_t *s0 = d_src + (size_t)f0 * width * height;
         uint8_t *d0 = d_dst + (size_t)f0 * width * height;
         const cpt_frame_info *i0 = info ? info + f0 : nullptr;
-        static const bool tiles_only = [] { const char *e = getenv("CPT_NLM_TILES"); return e && e[0] == '1'; }();  // (A/B and tests)
-        if (!tiles_only) {
-            dim3 grid((width + kNqCols - 1) / kNqCols, (height + kNqRows - 1) / kNqRows, nz);
-            nlm_quads_kernel<<<grid, kNqThreads, 0, stream>>>(s0, width, height, d0, i0);
-        } else {
-            dim3 grid((width + kNlmTile - 1) / kNlmTile, (height + kNlmTile - 1) / kNlmTile, nz);
-            nlm_denoise_kernel<<<grid, 256, 0, stream>>>(s0, width, height, d0, i0);
-        }
+        dim3 grid((width + kNqCols - 1) / kNqCols, (height + kNqRows - 1) / kNqRows, nz);
+        nlm_quads_kernel<<<grid, kNqThreads, 0, stream>>>(s0, width, height, d0, i0);
     }
     CUDA_TRY(cudaGetLastError());
     return CPT_OK;

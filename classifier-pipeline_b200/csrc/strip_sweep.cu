@@ -32,21 +32,15 @@ namespace {
 
 using namespace prim;
 
-#ifndef CPT_LEAD
-#define CPT_LEAD 7
-#endif
-constexpr int kLead = CPT_LEAD;                      // frames the copy warp runs ahead of the slowest consumer warp
+constexpr int kLead = 7;                             // frames the copy warp runs ahead of the slowest consumer warp
 constexpr int kRingSlots = kMeanFrames + kLead;      // 52 frames of the strip's rows
 constexpr int kSlotBytes = kStripPxMax * 2;          // 3840
 constexpr int kConsWarps = kStripPxMax / 4 / 32;     // 15
 constexpr int kConsThreads = kConsWarps * 32;        // 480
-constexpr int kBarRing = kLead < 8 ? 8 : 16;          // full / done barriers and stat rows are reused every kBarRing passes
+constexpr int kBarRing = 8;                          // full / done barriers and stat rows are reused every kBarRing passes
 static_assert(kBarRing > kLead, "a barrier is reused only after every warp has passed its previous use");
 static_assert(kStripThreads == kConsThreads + 64, "consumer warps + the copy warp + the fold warp");
-#ifndef CPT_STRIP_TABLE
-#define CPT_STRIP_TABLE 4096
-#endif
-constexpr int kStripTable = CPT_STRIP_TABLE;         // first entries of the clip's keep-test table
+constexpr int kStripTable = 4096;                    // first entries of the clip's keep-test table
 constexpr int kRefLag = kLead + 1;                    // a frame's quad bytes are stored against the strip minimum kRefLag frames earlier
 constexpr int kRefDefault = kQuadRefBias;            // reference of the first kRefLag frames (filtered starts near 0)
 
@@ -541,61 +535,6 @@ size_t strip_sweep_smem_bytes() { return sizeof(StripSmem); }
 // ================================================================================================
 // frame_scalars_kernel: one warp per clip, lanes = 32 consecutive passes.
 // ================================================================================================
-namespace {
-
-struct FrameScalars {
-    int ac, gmn, gmx, fth;
-    float thr;
-    uint32_t nmagic;
-    int nshift;
-};
-
-// K2 scalars of one frame (track/cliptracker.py:93-122, imageprocessing.py:151-169) from its sums: avg_change, the
-// normalisation range, the mapped threshold (fp32 as numpy >= 2 evaluates it), the bound F >= fth below which a pixel cannot
-// reach the threshold and the Granlund-Montgomery constants of the integer normalise.
-__device__ __forceinline__ FrameScalars frame_scalars_of(uint32_t psum, int fmin, int fmax, double average, int background_thresh, int npx) {
-    FrameScalars r;
-    // avg_change = int(round(np.average(thermal) - background average)), cliptracker.py:103-105
-    const double avg_int = rint(average);
-    if (avg_int == average && average >= 0.0 && average < 65536.0) {
-        // integer average (always, once the background has changed): round_half_even((sum - avg * n) / n) in integers;
-        // identical to the fp64 expression because the only ties are exact.  |sum - avg * n| < 2^31.
-        const int num = (int)psum - (int)avg_int * npx;
-        int qd = num / npx, rem = num - qd * npx;
-        if (rem < 0) { rem += npx; qd -= 1; }
-        if (2 * rem > npx || (2 * rem == npx && (qd & 1))) qd += 1;
-        r.ac = qd;
-    } else {
-        r.ac = (int)rint((double)psum / (double)npx - average);
-    }
-    r.gmx = max(fmax - r.ac, 0);
-    r.gmn = max(fmin - r.ac, 0);
-    r.fth = INT32_MIN;
-    r.nmagic = 0;  // 0: the fp32 divide; else (255 v) / range == (255 v * nmagic) >> nshift for 255 v < 2^24
-    r.nshift = 0;
-    if (r.gmx == r.gmn) {
-        r.thr = (float)background_thresh;  // cliptracker.py:118-119
-    } else {
-        const float range = (float)r.gmx - (float)r.gmn;
-        r.thr = __fmul_rn(__fdiv_rn((float)background_thresh, range), 255.0f);
-        const unsigned rr = (unsigned)(r.gmx - r.gmn);
-        if (255ull * rr < (1ull << 24)) {
-            // every product is exact in fp32 here, so trunc(fl(255 v / r)) == (255 v) / r and a quad can only produce
-            // foreground if one of its pixels has U > floor(thr):  U >= ith + 1  <=>  v >= ceil((ith + 1) r / 255),
-            // v = max(F - ac, 0) - gmn, i.e. F >= fth (the bound is >= 1, so the clamp never matters)
-            const int it = (int)floorf(r.thr);
-            if (it >= 0 && it < 255) r.fth = (int)(((unsigned)(it + 1) * rr + 254u) / 255u) + r.ac + r.gmn;
-            // Granlund-Montgomery: l = ceil(log2 r), m = ceil(2^(24 + l) / r) < 2^25
-            const int l = (rr <= 1u) ? 0 : 32 - __clz((int)(rr - 1u));
-            r.nshift = 24 + l;
-            r.nmagic = (uint32_t)ceil(ldexp(1.0, r.nshift) / (double)rr);
-        }
-    }
-    return r;
-}
-
-}  // namespace
-
 __global__ void __launch_bounds__(128) frame_scalars_kernel(const KernelArgs a) {
     const Geometry &g = a.g;
     const int lane = threadIdx.x & 31;
@@ -661,10 +600,7 @@ __global__ void __launch_bounds__(128) frame_scalars_kernel(const KernelArgs a) 
             mine = (double)bsum / (double)g.ncrop;
             sets = true;
         } else if (valid && upd && changed) {
-            uint32_t qa = bsum / (uint32_t)g.ncrop;
-            const uint32_t ra = bsum - qa * (uint32_t)g.ncrop;
-            if (2u * ra > (uint32_t)g.ncrop || (2u * ra == (uint32_t)g.ncrop && (qa & 1u))) qa += 1u;
-            mine = (double)qa;
+            mine = rounded_background_average(bsum, (uint32_t)g.ncrop);
             sets = true;
         }
         const uint32_t set_mask = __ballot_sync(0xffffffffu, sets);
@@ -676,15 +612,7 @@ __global__ void __launch_bounds__(128) frame_scalars_kernel(const KernelArgs a) 
         frames_seen += __popc(__ballot_sync(0xffffffffu, valid && upd));
         if (is_frame) {
             const FrameScalars fs = frame_scalars_of(psum, fmin, fmax, avg_here, clip.background_thresh, npx);
-            cpt_frame_info fi;
-            fi.background_average = avg_here;
-            fi.threshold = fs.thr; fi.norm_min = fs.gmn; fi.norm_max = fs.gmx; fi.avg_change = fs.ac;
-            fi.filtered_min = fmin; fi.filtered_max = fmax; fi.n_components = 0;
-            fi.thermal_min = want_stats ? pmin : 0; fi.thermal_max = want_stats ? pmax : 0;
-            fi.thermal_sum = psum; fi.abs_filtered_sum = want_stats ? fabs_sum : 0u; fi.thermal_median = 0.f;
-            fi.reserved[0] = 0;
-            fi.reserved[1] = denoise ? ((t > 0) ? 2 : 1) : 0;  // 2: the previous filtered image is frame o - 1
-            a.info[o] = fi;
+            a.info[o] = frame_info_of(fs, avg_here, psum, fmin, fmax, want_stats, pmin, pmax, fabs_sum, denoise ? ((t > 0) ? 2 : 1) : 0);
             FrameHdr h;
             h.nmagic = fs.nmagic; h.nshift = fs.nshift;
             h.flags = kHdrValid | (t == 0 ? kHdrFirst : 0u) | (denoise ? kHdrDenoise : 0u);

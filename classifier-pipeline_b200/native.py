@@ -10,7 +10,7 @@ import os
 import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-LIB_PATH = os.environ.get("CPT_LIB") or os.path.join(_HERE, "libcptrack.so")  # CPT_LIB: an experimental build (tools/)
+LIB_PATH = os.environ.get("CPT_LIB") or os.path.join(_HERE, "libcptrack.so")  # CPT_LIB: load another build instead (A/B of two builds in one session)
 
 CLIP_UPDATE_BACKGROUND = 1
 CLIP_RESUME = 2

@@ -7,7 +7,7 @@ python -m pytest tests -m gpu -x -q > gpurun_out/pytest_$tag.log 2>&1; echo "pyt
 python bench.py --impl reference --steps 2 --warmup 1 > gpurun_out/bench_ref_$tag.json 2> gpurun_out/bench_$tag.err; cat gpurun_out/bench_ref_$tag.json
 python bench.py > gpurun_out/bench_$tag.json 2>> gpurun_out/bench_$tag.err; echo "bench rc=$?"; cat gpurun_out/bench_$tag.json
 python tools/phase_timing.py 148 300 0 2>/dev/null | grep -v 'warning\|__attribute\|\^\|^$' > gpurun_out/phases_$tag.txt; cat gpurun_out/phases_$tag.txt
-KERNELS='regex:extract_clips|strip_sweep|frame_scalars|frame_regions|frame_components|region_variance|mask_components|nlm_denoise|cptv_|segment_tiles|sample_median|track_limits|track_norm_reset|motion_step|frame_median|background_step'
+KERNELS='regex:extract_clips|strip_sweep|frame_scalars|frame_regions|frame_components|region_variance|mask_components|nlm_quads|cptv_|segment_tiles|sample_median|track_limits|track_norm_reset|motion_step|frame_median|background_step'
 ncu --metrics gpu__time_duration.sum --clock-control none -k "$KERNELS" -c 2000 --csv --log-file gpurun_out/launches_$tag.csv \
     python bench.py --steps 3 --warmup 1 --clips 296 --frames 300 --tracks 2000 --no-cpu-baseline > gpurun_out/ncu_bench_$tag.log 2>&1
 for k in strip_sweep frame_regions region_variance; do

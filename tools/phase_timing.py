@@ -1,4 +1,6 @@
-"""Build a -DCPT_PHASE_TIMING copy of the library and print where the cycles of a frame go (GPU box)."""
+"""Build a -DCPT_PHASE_TIMING copy of the library and print where the cycles of a frame go (GPU box).
+
+usage: python tools/phase_timing.py [clips] [frames] [single]   (single = 1: the single persistent kernel, else the split plan)"""
 import ctypes
 import os
 import subprocess
@@ -11,13 +13,13 @@ sys.path.insert(0, ROOT)
 PKG = os.path.join(ROOT, "classifier-pipeline_b200")
 
 
-def main(clips=148, frames=300, exp=0, split=1):
+def main(clips=148, frames=300, single=0):
     import torch
     from classifier_pipeline_b200 import native
 
     dbg = os.path.join(PKG, "libcptrack_timing.so")
     srcs = [os.path.join(PKG, "csrc", f) for f in sorted(os.listdir(os.path.join(PKG, "csrc"))) if f.endswith(".cu")]
-    subprocess.run(["nvcc", "-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-DCPT_PHASE_TIMING", "-DCPT_EXP={}".format(exp),
+    subprocess.run(["nvcc", "-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-DCPT_PHASE_TIMING",
                     "-Xcompiler", "-fPIC", "-shared", "-o", dbg] + srcs, check=True)
     native.LIB_PATH = dbg
     from classifier_pipeline_b200.batch import BatchExtractor, linear_clips
@@ -28,7 +30,7 @@ def main(clips=148, frames=300, exp=0, split=1):
     d_frames, models = make_clips_torch(clips, frames, torch.device("cuda", 0))
     cl = linear_clips([frames] * clips, np.array([MODELS[m][2] for m in models]), np.array([slots[m] for m in models]))
     out = {}
-    if not split:
+    if single:
         native.check(ex.ctx.lib.cpt_debug_force_single_kernel(ex.ctx._h, 1))
     ex.extract_device(d_frames, cl, out=out)
     torch.cuda.synchronize()
@@ -38,7 +40,7 @@ def main(clips=148, frames=300, exp=0, split=1):
     torch.cuda.synchronize()
     native.check(ex.ctx.lib.cpt_debug_phase_cycles(ex.ctx._h, buf, 0))
     total = clips * frames
-    if split:
+    if not single:
         # frame_regions_kernel, thread 0 of every CTA (cycles include the waits at the CTA's barriers)
         names = {7: "header + info", 15: "quad bytes -> hot rows", 4: "band record + work lists", 5: "normalise", 8: "blur + threshold",
                  9: "components (close .. labels)"}
