@@ -253,6 +253,70 @@ __device__ void components_of_frame(const KernelArgs &a, SM &s, const Geometry &
     bar_sync(kBar, kT);
     CPT_TICK2(ctid == 0, 23);  // roots + barrier
     const int ncomp = s.ncomp;
+    if (ncomp > CPT_MAX_COMPONENTS) {
+        // More components than slots, and the slots above went in scheduling order.  Hand them again, to the components that
+        // come first in OpenCV label order: each root's parent entry takes the least key of its runs (keys are unique per
+        // component: the pixels of a 2x2 block are all 8-connected), a bitmap over the keys ranks them, and the first
+        // CPT_MAX_COMPONENTS ranks are the slots.  The bitmap lives in c_area until the slot tables are reset.
+        static_assert(((kMaxH + 1) / 2) * ((kMaxW + 1) / 2) <= 32 * kCompSlots && ((kMaxH + 1) / 2) * ((kMaxW + 1) / 2) < 0x7fff,
+                      "a bit per key fits in c_area, and a key in a parent entry");
+        uint32_t *keybits = reinterpret_cast<uint32_t *>(s.c_area);
+        const int nkw = (((g.H + 1) >> 1) * g.block_w + 31) >> 5;
+        for (int i = ctid; i < nkw; i += kT) keybits[i] = 0u;
+#pragma unroll
+        for (int it = 0; it < kIter; ++it) {
+            const int id0 = rc[it].y * kRunsPerRow + rc[it].base, n = __popc(rc[it].stw);
+            for (int k = 0; k < n; ++k)
+                if (s.parent[id0 + k] & kSlotFlag) s.parent[id0 + k] = (uint16_t)(kSlotFlag | 0x7fffu);
+        }
+        bar_sync(kBar, kT);
+#pragma unroll
+        for (int it = 0; it < kIter; ++it) {
+            uint32_t bitsleft = rc[it].stw;
+            int id = rc[it].y * kRunsPerRow + rc[it].base;
+            while (bitsleft) {
+                const int b = __ffs(bitsleft) - 1;
+                bitsleft &= bitsleft - 1;
+                const int root = uf_find(s.parent, id++);
+                const unsigned short key = (unsigned short)(kSlotFlag | ((rc[it].y >> 1) * g.block_w + ((rc[it].wi * 32 + b) >> 1)));
+                unsigned short *p = reinterpret_cast<unsigned short *>(s.parent + root);
+                for (unsigned short old = *(volatile unsigned short *)p; key < old;) {
+                    const unsigned short seen = atomicCAS(p, old, key);
+                    if (seen == old) break;
+                    old = seen;
+                }
+            }
+        }
+        bar_sync(kBar, kT);
+#pragma unroll
+        for (int it = 0; it < kIter; ++it) {
+            const int id0 = rc[it].y * kRunsPerRow + rc[it].base, n = __popc(rc[it].stw);
+            for (int k = 0; k < n; ++k) {
+                const int p = s.parent[id0 + k];
+                if (p & kSlotFlag) atomicOr(&keybits[(p & 0x7fff) >> 5], 1u << (p & 31));
+            }
+        }
+        bar_sync(kBar, kT);
+#pragma unroll
+        for (int it = 0; it < kIter; ++it) {
+            const int id0 = rc[it].y * kRunsPerRow + rc[it].base, n = __popc(rc[it].stw);
+            for (int k = 0; k < n; ++k) {
+                const int p = s.parent[id0 + k];
+                if (!(p & kSlotFlag)) continue;
+                const int key = p & 0x7fff;
+                int rank = __popc(keybits[key >> 5] & ((1u << (key & 31)) - 1u));
+                for (int q = 0; q < (key >> 5); ++q) rank += __popc(keybits[q]);
+                s.parent[id0 + k] = (uint16_t)(kSlotFlag | min(rank, CPT_MAX_COMPONENTS));
+            }
+        }
+        bar_sync(kBar, kT);
+        for (int slot = ctid; slot < CPT_MAX_COMPONENTS; slot += kT) {
+            s.c_key[slot] = INT32_MAX; s.c_area[slot] = 0; s.c_sx[slot] = 0; s.c_sy[slot] = 0;
+            s.c_l[slot] = INT32_MAX; s.c_t[slot] = INT32_MAX; s.c_r[slot] = -1; s.c_b[slot] = -1;
+            s.acc_s[slot] = 0.0; s.acc_s2[slot] = 0.0;
+        }
+        bar_sync(kBar, kT);
+    }
     // ---- per-run statistics into the slot tables
 #pragma unroll
     for (int it = 0; it < kIter; ++it) {
