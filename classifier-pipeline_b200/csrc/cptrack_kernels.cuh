@@ -217,7 +217,6 @@ struct __align__(16) Smem {
     int32_t bcast_i[16];
     int32_t msg[2][4];         // pixel warps -> component warps, per mask buffer: filtered min, max
     double bcast_d[4];
-    double acc_s[kCompSlots], acc_s2[kCompSlots];  // per-component sum / sum of squares of the delta frame
     uint32_t wthr[kSmemWeights];                   // first entries of the clip's keep-test table
     // per owned quad q = it * kPThreads + ptid (= owned row * qpr + column quad): max F - qref saturated to int8,
     // written by the sweep warps at the end of a frame, turned into hot64 by the mask warps
@@ -276,16 +275,9 @@ static_assert(kMaxH * (kMaxW / 8) <= (1 << 14), "a blur list entry keeps the gro
 struct __align__(16) CompSmem {
     uint16_t parent[kMaxRuns];
     uint32_t C[kMaxWords];
-    union {
-        // the mask (read by the close) and the run-start bits / per-word run counts (read by the unions) ...
-        struct {
-            uint32_t M[1][kMaxWords];
-            uint32_t ST[kMaxWords];
-            uint8_t base[kMaxWords + 8];
-        };
-        // ... then the variance sums (components_of_frame zeroes them after the unions)
-        struct { double acc_s[kCompSlots], acc_s2[kCompSlots]; };
-    };
+    uint32_t M[1][kMaxWords];
+    uint32_t ST[kMaxWords];
+    uint8_t base[kMaxWords + 8];
     int32_t c_key[kCompSlots], c_area[kCompSlots], c_sx[kCompSlots], c_sy[kCompSlots];
     int32_t c_l[kCompSlots], c_t[kCompSlots], c_r[kCompSlots], c_b[kCompSlots];
     uint8_t c_rank[kCompSlots];
@@ -415,11 +407,12 @@ __device__ __forceinline__ float norm255_f64(float f, double mn, double mx) {
 }
 
 // ---- run bookkeeping on the closed mask ------------------------------------------------------
+// Id of the run that holds pixel x of a row whose first word in the tables is w0 (row `row` of the table, rpr ids per row):
+// the runs that start in the earlier words of the row (base) and in bits 0 .. x & 31 of word x >> 5.
 template <class SM>
-__device__ __forceinline__ int run_id(const SM &s, const Geometry &g, int x, int y) {
-    int w = y * g.row_words + (x >> 5), b = x & 31;
-    uint32_t below = s.ST[w] & (0xffffffffu >> (31 - b));
-    return y * kRunsPerRow + (int)s.base[w] + __popc(below) - 1;
+__device__ __forceinline__ int run_id(const SM &s, int w0, int row, int rpr, int x) {
+    const int w = w0 + (x >> 5), b = x & 31;
+    return row * rpr + (int)s.base[w] + __popc(s.ST[w] & (0xffffffffu >> (31 - b))) - 1;
 }
 
 __device__ __forceinline__ int uf_find(volatile uint16_t *parent, int a) {

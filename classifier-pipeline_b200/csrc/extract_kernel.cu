@@ -115,51 +115,193 @@ __device__ __forceinline__ float norm255(int f, int mn, int mx, bool exact_f32) 
     return (float)(255.0 * ((double)f - (double)mn) / ((double)mx - (double)mn));
 }
 
+// norm255's exact_f32 for the two frames of a delta frame
+__device__ __forceinline__ bool norm255_exact(int cur_fmin, int cur_fmax, int prev_fmin, int prev_fmax) {
+    return 255ll * max(cur_fmax - cur_fmin, prev_fmax - prev_fmin) < (1ll << 24) &&
+           max(max(abs(cur_fmax), abs(cur_fmin)), max(abs(prev_fmax), abs(prev_fmin))) < (1 << 24);
+}
+
+// K6 for one region record: variance of |norm255(F_t) - norm255(F_t-1)| over the component's bounding box (l, tp, bw, bh);
+// one warp, lane 0 stores it to *var.  Every frame's variances are summed in this one order (pixels lane, lane + 32, ...
+// of the box, then one shuffle tree), whichever kernel computes them.  kLdg: the images are read-only for the whole launch
+// (region_variance_kernel); the extraction kernel reads images its own launch wrote, through coherent loads.
+template <bool kLdg>
+__device__ __forceinline__ void region_variance(const Geometry &g, int l, int tp, int bw, int bh, const float *fcur,
+                                                const float *fprev, int cur_fmin, int cur_fmax, int prev_fmin, int prev_fmax,
+                                                bool exact, int lane, double *var) {
+    const int npix = bw * bh;
+    double s1 = 0.0, s2 = 0.0;
+    const uint32_t rcp = 0xffffffffu / (uint32_t)bw + 1u;  // i / bw == umulhi(i, rcp) for i * bw < 2^32
+    for (int i = lane; i < npix; i += 32) {
+        const int yy = bw == 1 ? i : (int)__umulhi((uint32_t)i, rcp), xx = i - yy * bw, p = (tp + yy) * g.W + l + xx;  // (rcp wraps to 0 for bw == 1)
+        const float fc = kLdg ? __ldg(fcur + p) : fcur[p], fp = kLdg ? __ldg(fprev + p) : fprev[p];
+        const float d = fabsf(norm255((int)fc, cur_fmin, cur_fmax, exact) - norm255((int)fp, prev_fmin, prev_fmax, exact));
+        s1 += (double)d;
+        s2 += (double)d * (double)d;
+    }
+    for (int off = 16; off; off >>= 1) {
+        s1 += __shfl_xor_sync(0xffffffffu, s1, off);
+        s2 += __shfl_xor_sync(0xffffffffu, s2, off);
+    }
+    if (lane == 0) {
+        const double cnt = (double)npix, mean = s1 / cnt, v = s2 / cnt - mean * mean;
+        *var = v > 0.0 ? v : 0.0;
+    }
+}
+
 // ================================================================================================
-// component warps: one frame's mask -> regions
+// components of a frame's mask (K4 second half, K5): the passes of both drivers, components_of_frame (component warps,
+// frame_components_kernel, mask_components_kernel: full-size tables) and components_lean (frame_regions_kernel).
+// Tables C, ST and base hold one entry per word w of the closed mask, word wi of its row of rw words.
 // ================================================================================================
+// closed word C[y] = M[y-1] | (M[y] & M[y-2]) (C[0] = M[0]) of mask word w, image row y
+__device__ __forceinline__ uint32_t closed_word(const uint32_t *M, int w, int y, int rw) {
+    const uint32_t m0 = M[w];
+    return y == 0 ? m0 : M[w - rw] | (m0 & (y >= 2 ? M[w - 2 * rw] : 0u));
+}
+
+// run-start bits of closed word c = C[w] into ST[w], and the runs that start in the earlier words of its row into base[w]
+template <class SM>
+__device__ __forceinline__ uint32_t word_run_starts(SM &s, int w, int wi, uint32_t c, int &base) {
+    uint32_t carry = 0;
+    base = 0;
+    for (int q = 0; q < wi; ++q) {
+        const uint32_t cq = s.C[w - wi + q];
+        base += __popc(cq & ~((cq << 1) | carry));
+        carry = cq >> 31;
+    }
+    const uint32_t stw = c & ~((c << 1) | carry);
+    s.ST[w] = stw;
+    s.base[w] = (uint8_t)base;
+    return stw;
+}
+
+// 8-connectivity: unions of the runs of closed word c = C[w] (row `row` > 0 of the table) with the runs of the row above
+template <class SM>
+__device__ __forceinline__ void unite_with_row_above(SM &s, int w, int wi, int rw, uint32_t c, int row, int rpr) {
+    const int up = w - rw;
+    const uint32_t u = s.C[up];
+    const uint32_t u_l = (wi > 0) ? (s.C[up - 1] >> 31) : 0u, u_r = (wi + 1 < rw) ? (s.C[up + 1] & 1u) : 0u;
+    const uint32_t c_l = (wi > 0) ? (s.C[w - 1] >> 31) : 0u, c_r = (wi + 1 < rw) ? (s.C[w + 1] & 1u) : 0u;
+    const uint32_t ul = (u << 1) | u_l, ur = (u >> 1) | (u_r << 31);
+    const uint32_t cl = (c << 1) | c_l, cr = (c >> 1) | (c_r << 31);
+    uint32_t needA = c & u & ~(cl & ul);   // pixel above, unless the left neighbour already links to it
+    uint32_t needB = c & ul & ~u & ~cl;    // upper-left only
+    uint32_t needC = c & ur & ~u & ~cr;    // upper-right only
+    const int w0 = w - wi, u0 = up - wi, xb = wi * 32;
+    while (needA) {
+        const int b = __ffs(needA) - 1;
+        needA &= needA - 1;
+        uf_union(s.parent, run_id(s, w0, row, rpr, xb + b), run_id(s, u0, row - 1, rpr, xb + b));
+    }
+    while (needB) {
+        const int b = __ffs(needB) - 1;
+        needB &= needB - 1;
+        uf_union(s.parent, run_id(s, w0, row, rpr, xb + b), run_id(s, u0, row - 1, rpr, xb + b - 1));
+    }
+    while (needC) {
+        const int b = __ffs(needC) - 1;
+        needC &= needC - 1;
+        uf_union(s.parent, run_id(s, w0, row, rpr, xb + b), run_id(s, u0, row - 1, rpr, xb + b + 1));
+    }
+}
+
+template <class SM>
+__device__ __forceinline__ void reset_slot(SM &s, int i) {
+    s.c_key[i] = INT32_MAX; s.c_area[i] = 0; s.c_sx[i] = 0; s.c_sy[i] = 0;
+    s.c_l[i] = INT32_MAX; s.c_t[i] = INT32_MAX; s.c_r[i] = -1; s.c_b[i] = -1;
+}
+
+// length of the run that starts at bit b of closed word c = C[w]
+template <class SM>
+__device__ __forceinline__ int run_length(const SM &s, int w, int wi, int rw, uint32_t c, int b) {
+    const uint32_t inv = ~(c >> b);
+    int len = (inv == 0) ? 32 : (__ffs(inv) - 1);
+    if (b + len >= 32) {  // run continues into the following words
+        len = 32 - b;
+        for (int q = wi + 1; q < rw; ++q) {
+            const uint32_t cn = ~s.C[w - wi + q];
+            if (cn == 0) { len += 32; continue; }
+            len += __ffs(cn) - 1;
+            break;
+        }
+    }
+    return len;
+}
+
+// the run of len pixels from (xs, y) into the statistics of its component's slot
+template <class SM>
+__device__ __forceinline__ void add_run(SM &s, const Geometry &g, int slot, int xs, int y, int len) {
+    atomicMin(&s.c_key[slot], (y >> 1) * g.block_w + (xs >> 1));
+    atomicAdd(&s.c_area[slot], len);
+    atomicAdd(&s.c_sx[slot], len * (2 * xs + len - 1) / 2);
+    atomicAdd(&s.c_sy[slot], len * y);
+    atomicMin(&s.c_l[slot], xs);
+    atomicMax(&s.c_r[slot], xs + len - 1);
+    atomicMin(&s.c_t[slot], y);
+    atomicMax(&s.c_b[slot], y);
+}
+
+// OpenCV label order: rank of slot i among slots 0 .. nslots - 1 by the key of the component's first 2x2 block
+template <class SM>
+__device__ __forceinline__ int slot_rank(const SM &s, int i, int nslots) {
+    const int key = s.c_key[i];
+    int rank = 0;
+    for (int q = 0; q < nslots; ++q) rank += (s.c_key[q] < key);
+    return rank;
+}
+
+// region record of slot i; pixel_variance is K6's
+template <class SM>
+__device__ __forceinline__ cpt_region region_record(const SM &s, int i) {
+    cpt_region r;
+    r.x = s.c_l[i]; r.y = s.c_t[i];
+    r.width = s.c_r[i] - r.x + 1; r.height = s.c_b[i] - r.y + 1;
+    r.area = s.c_area[i]; r.sum_x = s.c_sx[i]; r.sum_y = s.c_sy[i];
+    r.key = s.c_key[i];
+    r.pixel_variance = 0.0;
+    return r;
+}
+
+__device__ __forceinline__ void store_label_run(uint8_t *lab_frame, const Geometry &g, int xs, int y, int len, uint8_t lab) {
+    uint8_t *px = lab_frame + y * g.W + xs;
+    for (int k = 0; k < len; ++k) px[k] = lab;
+}
+
 struct RunCursor {
     uint32_t c, stw;
     int y, wi, base;
 };
 
-// K4 second half + K5 + K6 for the mask in s.M[buf].  Called by all kT threads of the role (kBar: their named barrier).
+// K4 second half + K5 for the mask in s.M[buf]: close, labelling, statistics, label image and region records of output
+// frame o.  Called by all kT threads of the role (kBar: their named barrier).  var_deferred: region_variance_kernel computes
+// the frame's variances (info.reserved[0]).  Returns the number of region records.
 template <class SM, int kT, int kBar>
-__device__ void components_of_frame(const KernelArgs &a, SM &s, const Geometry &g, int ctid, int buf, size_t o,
-                                    const float *fcur, const float *fprev, int cur_fmin, int cur_fmax, int prev_fmin,
-                                    int prev_fmax, bool have_prev, bool defer_variance) {
-    const int W = g.W, lane = ctid & 31, cwarp = ctid >> 5;
+__device__ int components_of_frame(const KernelArgs &a, SM &s, const Geometry &g, int ctid, int buf, size_t o, bool var_deferred) {
+    const int rw = g.row_words;
     constexpr int kIter = (kMaxWords + kT - 1) / kT;  // 3
     RunCursor rc[kIter];
     bool any = false;
     CPT_TICK_START2(ctid == 0);
-    // ---- close: C[y] = M[y-1] | (M[y] & M[y-2]) (C[0] = M[0]); slot tables reset
+    // ---- close; slot tables reset
 #pragma unroll
     for (int it = 0; it < kIter; ++it) {
         int w = ctid + it * kT;
         rc[it].c = 0; rc[it].stw = 0; rc[it].y = 0; rc[it].wi = 0; rc[it].base = 0;
         if (w < g.words) {
             int y = (int)(((uint32_t)w * g.rw_magic) >> 13);
-            uint32_t m0 = s.M[buf][w], c;
-            if (y == 0) c = m0;
-            else {
-                uint32_t m1 = s.M[buf][w - g.row_words];
-                uint32_t m2 = (y >= 2) ? s.M[buf][w - 2 * g.row_words] : 0u;
-                c = m1 | (m0 & m2);
-            }
+            const uint32_t c = closed_word(s.M[buf], w, y, rw);
             s.C[w] = c;
-            rc[it].c = c; rc[it].y = y; rc[it].wi = w - y * g.row_words;
+            rc[it].c = c; rc[it].y = y; rc[it].wi = w - y * rw;
             any |= (c != 0);
         }
     }
     // (a component's slot is initialised by the thread that allocates it; only the overflow sink is reset here)
     if (ctid == 0) {
         s.ncomp = 0;
-        const int i = CPT_MAX_COMPONENTS;
-        s.c_key[i] = INT32_MAX; s.c_area[i] = 0; s.c_sx[i] = 0; s.c_sy[i] = 0;
-        s.c_l[i] = INT32_MAX; s.c_t[i] = INT32_MAX; s.c_r[i] = -1; s.c_b[i] = -1;
+        reset_slot(s, CPT_MAX_COMPONENTS);
     }
-    if (!bar_or(kBar, kT, any)) return;  // no foreground: info.n_components stays 0
+    if (!bar_or(kBar, kT, any)) return 0;  // no foreground: info.n_components stays 0
     CPT_TICK2(ctid == 0, 20);  // close + reset + barrier
 
     // ---- run starts and ids
@@ -167,70 +309,24 @@ __device__ void components_of_frame(const KernelArgs &a, SM &s, const Geometry &
     for (int it = 0; it < kIter; ++it) {
         int w = ctid + it * kT;
         if (w < g.words && rc[it].c != 0) {  // (ST / base of an empty word are never looked up)
-            const int wi = rc[it].wi, y = rc[it].y;
-            uint32_t carry = 0;
-            int base = 0;
-            for (int q = 0; q < wi; ++q) {
-                uint32_t cq = s.C[w - wi + q];
-                base += __popc(cq & ~((cq << 1) | carry));
-                carry = cq >> 31;
-            }
-            uint32_t c = rc[it].c, stw = c & ~((c << 1) | carry);
-            s.ST[w] = stw;
-            s.base[w] = (uint8_t)base;
+            int base;
+            const uint32_t stw = word_run_starts(s, w, rc[it].wi, rc[it].c, base);
             rc[it].stw = stw; rc[it].base = base;
-            uint32_t bitsleft = stw;
-            int n = 0;
-            while (bitsleft) {
-                bitsleft &= bitsleft - 1;
-                int id = y * kRunsPerRow + base + n;
-                s.parent[id] = (uint16_t)id;
-                ++n;
-            }
+            int id = rc[it].y * kRunsPerRow + base;
+            for (uint32_t bitsleft = stw; bitsleft; bitsleft &= bitsleft - 1, ++id) s.parent[id] = (uint16_t)id;
         }
     }
     bar_sync(kBar, kT);
     CPT_TICK2(ctid == 0, 21);  // run starts + barrier
-    // ---- unions with the row above (8-connectivity)
+    // ---- unions with the row above
 #pragma unroll
     for (int it = 0; it < kIter; ++it) {
         int w = ctid + it * kT;
-        const uint32_t c = rc[it].c;
-        const int y = rc[it].y, wi = rc[it].wi;
-        if (w < g.words && y > 0 && c != 0) {
-            const int up = w - g.row_words;
-            uint32_t u = s.C[up];
-            uint32_t u_l = (wi > 0) ? (s.C[up - 1] >> 31) : 0u;
-            uint32_t u_r = (wi + 1 < g.row_words) ? (s.C[up + 1] & 1u) : 0u;
-            uint32_t c_l = (wi > 0) ? (s.C[w - 1] >> 31) : 0u;
-            uint32_t c_r = (wi + 1 < g.row_words) ? (s.C[w + 1] & 1u) : 0u;
-            uint32_t ul = (u << 1) | u_l, ur = (u >> 1) | (u_r << 31);
-            uint32_t cl = (c << 1) | c_l, cr = (c >> 1) | (c_r << 31);
-            uint32_t needA = c & u & ~(cl & ul);   // pixel above, unless the left neighbour already links to it
-            uint32_t needB = c & ul & ~u & ~cl;    // upper-left only
-            uint32_t needC = c & ur & ~u & ~cr;    // upper-right only
-            const int xb = wi * 32;
-            while (needA) {
-                int b = __ffs(needA) - 1;
-                needA &= needA - 1;
-                uf_union(s.parent, run_id(s, g, xb + b, y), run_id(s, g, xb + b, y - 1));
-            }
-            while (needB) {
-                int b = __ffs(needB) - 1;
-                needB &= needB - 1;
-                uf_union(s.parent, run_id(s, g, xb + b, y), run_id(s, g, xb + b - 1, y - 1));
-            }
-            while (needC) {
-                int b = __ffs(needC) - 1;
-                needC &= needC - 1;
-                uf_union(s.parent, run_id(s, g, xb + b, y), run_id(s, g, xb + b + 1, y - 1));
-            }
-        }
+        if (w < g.words && rc[it].y > 0 && rc[it].c != 0) unite_with_row_above(s, w, rc[it].wi, rw, rc[it].c, rc[it].y, kRunsPerRow);
     }
     bar_sync(kBar, kT);
     CPT_TICK2(ctid == 0, 22);  // unions + barrier
-    // ---- roots -> component slots (and the variance sums: in frame_components_kernel they live where the mask and the
-    // run-start bits were, both dead once the unions are done)
+    // ---- roots -> component slots
 #pragma unroll
     for (int it = 0; it < kIter; ++it) {
         uint32_t bitsleft = rc[it].stw;
@@ -240,11 +336,7 @@ __device__ void components_of_frame(const KernelArgs &a, SM &s, const Geometry &
             int id = rc[it].y * kRunsPerRow + rc[it].base + n;
             if (s.parent[id] == id) {
                 int slot = atomicAdd(&s.ncomp, 1);
-                if (slot < CPT_MAX_COMPONENTS) {
-                    s.c_key[slot] = INT32_MAX; s.c_area[slot] = 0; s.c_sx[slot] = 0; s.c_sy[slot] = 0;
-                    s.c_l[slot] = INT32_MAX; s.c_t[slot] = INT32_MAX; s.c_r[slot] = -1; s.c_b[slot] = -1;
-                    s.acc_s[slot] = 0.0; s.acc_s2[slot] = 0.0;
-                }
+                if (slot < CPT_MAX_COMPONENTS) reset_slot(s, slot);
                 s.parent[id] = (uint16_t)(kSlotFlag | (slot < CPT_MAX_COMPONENTS ? slot : CPT_MAX_COMPONENTS));
             }
             ++n;
@@ -310,60 +402,28 @@ __device__ void components_of_frame(const KernelArgs &a, SM &s, const Geometry &
             }
         }
         bar_sync(kBar, kT);
-        for (int slot = ctid; slot < CPT_MAX_COMPONENTS; slot += kT) {
-            s.c_key[slot] = INT32_MAX; s.c_area[slot] = 0; s.c_sx[slot] = 0; s.c_sy[slot] = 0;
-            s.c_l[slot] = INT32_MAX; s.c_t[slot] = INT32_MAX; s.c_r[slot] = -1; s.c_b[slot] = -1;
-            s.acc_s[slot] = 0.0; s.acc_s2[slot] = 0.0;
-        }
+        for (int slot = ctid; slot < CPT_MAX_COMPONENTS; slot += kT) reset_slot(s, slot);
         bar_sync(kBar, kT);
     }
     // ---- per-run statistics into the slot tables
 #pragma unroll
     for (int it = 0; it < kIter; ++it) {
-        int w = ctid + it * kT;
+        const int w = ctid + it * kT;
         uint32_t bitsleft = rc[it].stw;
-        const uint32_t c = rc[it].c;
-        const int y = rc[it].y, wi = rc[it].wi;
-        int n = 0;
+        int id = rc[it].y * kRunsPerRow + rc[it].base;
         while (bitsleft) {
-            int b = __ffs(bitsleft) - 1;
+            const int b = __ffs(bitsleft) - 1;
             bitsleft &= bitsleft - 1;
-            int id = y * kRunsPerRow + rc[it].base + n;
-            ++n;
-            int slot = uf_slot(s.parent, id);
-            s.parent[id] = (uint16_t)(kSlotFlag | slot);
-            int xs = wi * 32 + b;
-            uint32_t inv = ~(c >> b);
-            int len = (inv == 0) ? 32 : (__ffs(inv) - 1);
-            if (b + len >= 32) {  // run continues into the following words
-                len = 32 - b;
-                for (int q = wi + 1; q < g.row_words; ++q) {
-                    uint32_t cn = ~s.C[w - wi + q];
-                    if (cn == 0) { len += 32; continue; }
-                    len += __ffs(cn) - 1;
-                    break;
-                }
-            }
-            atomicMin(&s.c_key[slot], (y >> 1) * g.block_w + (xs >> 1));
-            atomicAdd(&s.c_area[slot], len);
-            atomicAdd(&s.c_sx[slot], len * (2 * xs + len - 1) / 2);
-            atomicAdd(&s.c_sy[slot], len * y);
-            atomicMin(&s.c_l[slot], xs);
-            atomicMax(&s.c_r[slot], xs + len - 1);
-            atomicMin(&s.c_t[slot], y);
-            atomicMax(&s.c_b[slot], y);
+            const int slot = uf_slot(s.parent, id);
+            s.parent[id++] = (uint16_t)(kSlotFlag | slot);
+            add_run(s, g, slot, rc[it].wi * 32 + b, rc[it].y, run_length(s, w, rc[it].wi, rw, rc[it].c, b));
         }
     }
     bar_sync(kBar, kT);
     CPT_TICK2(ctid == 0, 24);  // run statistics + barrier
-    // ---- OpenCV label order: rank by the key of the component's first 2x2 block
     const int nslots = min(ncomp, CPT_MAX_COMPONENTS);
     const int nout = min(nslots, g.max_regions);
-    for (int i = ctid; i < nslots; i += kT) {
-        int key = s.c_key[i], rank = 0;
-        for (int q = 0; q < nslots; ++q) rank += (s.c_key[q] < key);
-        s.c_rank[i] = (uint8_t)rank;
-    }
+    for (int i = ctid; i < nslots; i += kT) s.c_rank[i] = (uint8_t)slot_rank(s, i, nslots);
     bar_sync(kBar, kT);
     CPT_TICK2(ctid == 0, 25);  // rank + barrier
     // ---- label image: the pixel warps already stored zeros for this frame; write the runs
@@ -371,87 +431,34 @@ __device__ void components_of_frame(const KernelArgs &a, SM &s, const Geometry &
         uint8_t *lab_frame = a.labels + o * g.npx;
 #pragma unroll
         for (int it = 0; it < kIter; ++it) {
+            const int w = ctid + it * kT;
             uint32_t bitsleft = rc[it].stw;
-            const int y = rc[it].y, wi = rc[it].wi;
-            int n = 0;
+            int id = rc[it].y * kRunsPerRow + rc[it].base;
             while (bitsleft) {
-                int b = __ffs(bitsleft) - 1;
+                const int b = __ffs(bitsleft) - 1;
                 bitsleft &= bitsleft - 1;
-                int id = y * kRunsPerRow + rc[it].base + n;
-                ++n;
-                int slot = s.parent[id] & 0xff;
-                uint8_t lab = (slot < CPT_MAX_COMPONENTS) ? (uint8_t)(s.c_rank[slot] + 1) : (uint8_t)255;
-                const int w = y * g.row_words + wi;
-                uint32_t inv = ~(rc[it].c >> b);
-                int len = (inv == 0) ? 32 : (__ffs(inv) - 1);
-                if (b + len >= 32) {  // run continues into the following words
-                    len = 32 - b;
-                    for (int q = wi + 1; q < g.row_words; ++q) {
-                        uint32_t cn = ~s.C[w - wi + q];
-                        if (cn == 0) { len += 32; continue; }
-                        len += __ffs(cn) - 1;
-                        break;
-                    }
-                }
-                uint8_t *px = lab_frame + y * W + wi * 32 + b;
-                for (int k = 0; k < len; ++k) px[k] = lab;
+                const int slot = s.parent[id++] & 0xff;
+                const uint8_t lab = (slot < CPT_MAX_COMPONENTS) ? (uint8_t)(s.c_rank[slot] + 1) : (uint8_t)255;
+                store_label_run(lab_frame, g, rc[it].wi * 32 + b, rc[it].y, run_length(s, w, rc[it].wi, rw, rc[it].c, b), lab);
             }
         }
     }
     CPT_TICK2(ctid == 0, 26);  // label writes
-    // ---- delta-frame variance over each component's bounding box (K6)
-    if (have_prev && !defer_variance) {
-        const bool exact = 255ll * max(cur_fmax - cur_fmin, prev_fmax - prev_fmin) < (1ll << 24) &&
-                           max(max(abs(cur_fmax), abs(cur_fmin)), max(abs(prev_fmax), abs(prev_fmin))) < (1 << 24);
-        for (int slot = 0; slot < nslots; ++slot) {
-            if (s.c_rank[slot] >= nout) continue;
-            const int l = s.c_l[slot], tp = s.c_t[slot];
-            const int bw = s.c_r[slot] - l + 1, bh = s.c_b[slot] - tp + 1;
-            if (cwarp >= bh) continue;
-            double s1 = 0.0, s2 = 0.0;
-            for (int yy = tp + cwarp; yy < tp + bh; yy += (kT / 32))
-                for (int xx = l + lane; xx < l + bw; xx += 32) {
-                    int fc = (int)fcur[yy * W + xx], fp = (int)fprev[yy * W + xx];
-                    float d = fabsf(norm255(fc, cur_fmin, cur_fmax, exact) - norm255(fp, prev_fmin, prev_fmax, exact));
-                    s1 += (double)d;
-                    s2 += (double)d * (double)d;
-                }
-            for (int off = 16; off; off >>= 1) {
-                s1 += __shfl_xor_sync(0xffffffffu, s1, off);
-                s2 += __shfl_xor_sync(0xffffffffu, s2, off);
-            }
-            if (lane == 0) {
-                atomicAdd(&s.acc_s[slot], s1);
-                atomicAdd(&s.acc_s2[slot], s2);
-            }
-        }
-    }
-    bar_sync(kBar, kT);
-    CPT_TICK2(ctid == 0, 27);  // variance + barrier
     for (int i = ctid; i < nslots; i += kT) {
         const int rank = s.c_rank[i];
-        if (rank < nout) {
-            cpt_region r;
-            r.x = s.c_l[i]; r.y = s.c_t[i];
-            r.width = s.c_r[i] - r.x + 1; r.height = s.c_b[i] - r.y + 1;
-            r.area = s.c_area[i]; r.sum_x = s.c_sx[i]; r.sum_y = s.c_sy[i];
-            r.key = s.c_key[i];
-            double n = (double)r.width * (double)r.height;
-            double mean = s.acc_s[i] / n;
-            double var = s.acc_s2[i] / n - mean * mean;
-            r.pixel_variance = (have_prev && !defer_variance && var > 0.0) ? var : 0.0;
-            a.regions[o * g.max_regions + rank] = r;
-        }
+        if (rank < nout) a.regions[o * g.max_regions + rank] = region_record(s, i);
     }
     if (ctid == 0) {
         a.info[o].n_components = ncomp;
-        if (have_prev && defer_variance) a.info[o].reserved[0] = 1;  // region_variance_kernel fills pixel_variance
+        if (var_deferred) a.info[o].reserved[0] = 1;  // region_variance_kernel fills pixel_variance
     }
+    return nout;
 }
 
 __device__ void component_warps(const KernelArgs &a, Smem &s, const cpt_clip &clip, int ctid, float *scratch,
                                 const StateHeader *st_hdr, const float *st_F) {
     const Geometry &g = a.g;
+    const int lane = ctid & 31;
     int prev_fmin = 0, prev_fmax = 0;
     bool have_prev = false;
     if (clip.flags & CPT_CLIP_RESUME) {
@@ -469,17 +476,30 @@ __device__ void component_warps(const KernelArgs &a, Smem &s, const cpt_clip &cl
         bar_sync(BAR_FULL + buf, kMThreads + kCThreads);  // mask of frame t is in s.M[buf]
         CPT_TICK(ctid == 0, 11);  // waiting for a mask
         const int cur_fmin = s.msg[buf][0], cur_fmax = s.msg[buf][1];
-        const float *fcur = filtered_ptr(a, clip, scratch, t);
-        const float *fprev = (t == 0) ? st_F : filtered_ptr(a, clip, scratch, t - 1);
+        const size_t o = (size_t)(clip.out_offset + t);
         // frames after the first of a launch have both filtered images in the caller's buffer: their variances
         // are left to region_variance_kernel (a wide second launch) instead of this 7-warp critical path
-        components_of_frame<Smem, kCThreads, BAR_C>(a, s, g, ctid, buf, (size_t)(clip.out_offset + t), fcur, fprev, cur_fmin, cur_fmax, prev_fmin,
-                            prev_fmax, have_prev, a.defer_variance && t > 0);
+        const bool var_later = a.defer_variance && t > 0;
+        const int nout = components_of_frame<Smem, kCThreads, BAR_C>(a, s, g, ctid, buf, o, have_prev && var_later);
+        if (have_prev && !var_later && nout > 0) {
+            // K6 of the other frames: one warp per region record
+            CPT_TICK_START2(ctid == 0);
+            bar_sync(BAR_C, kCThreads);  // the records are stored
+            const float *fcur = filtered_ptr(a, clip, scratch, t);
+            const float *fprev = (t == 0) ? st_F : filtered_ptr(a, clip, scratch, t - 1);
+            const bool exact = norm255_exact(cur_fmin, cur_fmax, prev_fmin, prev_fmax);
+            for (int r = ctid >> 5; r < nout; r += kCWarps) {
+                cpt_region *reg = a.regions + o * g.max_regions + r;
+                region_variance<false>(g, reg->x, reg->y, reg->width, reg->height, fcur, fprev, cur_fmin, cur_fmax, prev_fmin,
+                                       prev_fmax, exact, lane, &reg->pixel_variance);
+            }
+            CPT_TICK2(ctid == 0, 27);  // variance + barrier (0 for the frames left to region_variance_kernel)
+        }
         prev_fmin = cur_fmin;
         prev_fmax = cur_fmax;
         have_prev = true;
-        // all component threads are done with s.M[buf] (and s.C etc.): hand it back zeroed, the pixel warps only
-        // write the bytes of the groups they blurred
+        // all component threads are past the close, the only reader of s.M[buf]: hand it back zeroed, the pixel warps
+        // only write the bytes of the groups they blurred
         for (int i = ctid; i < g.words; i += kCThreads) s.M[buf][i] = 0;
         CPT_TICK(ctid == 0, 12);  // components of the frame
         if (t + 2 < n_here) bar_arrive(BAR_EMPTY + buf, kMThreads + kCThreads);
@@ -1361,32 +1381,27 @@ __device__ __forceinline__ unsigned long long quad_row_bits_bytes(const Geometry
 }
 
 // ---- components of a small mask inside frame_regions_kernel's CTA ---------------------------------------------------------
-// The same algorithm as components_of_frame (close, runs, unions with the row above, statistics, OpenCV label order, label
-// runs, region records), restricted to the rows [r0, r1] the mask stage can have set and sized for the masks real frames
-// have: run ids are (row of the extent) * rpr + index with rpr = min(80, 2048 / rows), at most kLeanSlots components.
+// The passes of components_of_frame (close, runs, unions with the row above, statistics, OpenCV label order, label runs,
+// region records), restricted to the rows [r0, r1] the mask stage can have set and sized for the masks real frames have:
+// the tables are indexed by word of the extent, run ids are (row of the extent) * rpr + index with
+// rpr = min(80, kLeanParents / rows), at most kLeanSlots components.
 // Returns 0 when the frame is done; when it does not fit (a row with more runs, more components) -- found before anything is
 // written to global memory -- the number of threads that are still there (threads 0 .. n - 1; the others got 0 and left):
 // they store the mask for frame_components_kernel, which redoes the frame.  Called by all kFThreads threads.
-__device__ __forceinline__ int lean_run_id(const MaskSmem &s, int lw, int ry, int rpr, int b) {
-    return ry * rpr + (int)s.base[lw] + __popc(s.ST[lw] & (0xffffffffu >> (31 - b))) - 1;
-}
-
 __device__ int components_lean(const KernelArgs &a, MaskSmem &s, const Geometry &g, int tid, size_t o, int r0, int r1, bool have_prev) {
-    const int rw = g.row_words, W = g.W;
+    const int rw = g.row_words;
     const int c0 = r0, c1 = min(r1 + 1, g.H - 1), nrows = c1 - c0 + 1, nw = nrows * rw;
     const int rpr = min(kRunsPerRow, kLeanParents / nrows);
-    // ---- close: C[y] = M[y-1] | (M[y] & M[y-2]) (C[0] = M[0]); rows outside [c0, c1] are empty.  The non-empty words go
-    // on a list (any order): every later pass walks the list, a few dozen words for the masks real frames have.
+    // ---- close; rows outside [c0, c1] are empty.  The non-empty words go on a list (any order): every later pass walks the
+    // list, a few dozen words for the masks real frames have.
     // (s.ncomp, s.overflow and s.nwords were zeroed by the caller before its last barrier)
     const int lane = tid & 31;
     for (int lw0 = 0; lw0 < nw; lw0 += kFThreads) {
         const int lw = lw0 + tid;
         uint32_t c = 0u;
         if (lw < nw) {
-            const int ry = (int)(((uint32_t)lw * g.rw_magic) >> 13), y = c0 + ry, w = lw + c0 * rw;
-            const uint32_t m0 = s.M[0][w];
-            c = m0;
-            if (y > 0) c = s.M[0][w - rw] | (m0 & (y >= 2 ? s.M[0][w - 2 * rw] : 0u));
+            const int ry = (int)(((uint32_t)lw * g.rw_magic) >> 13);
+            c = closed_word(s.M[0], lw + c0 * rw, c0 + ry, rw);
             s.C[lw] = c;
         }
         const uint32_t nz = __ballot_sync(0xffffffffu, c != 0u);
@@ -1407,57 +1422,19 @@ __device__ int components_lean(const KernelArgs &a, MaskSmem &s, const Geometry 
     // ---- run starts and ids
     for (int i = tid; i < nwl; i += nact) {
         const int lw = s.wlist[i];
-        const uint32_t c = s.C[lw];
-        const int ry = (int)(((uint32_t)lw * g.rw_magic) >> 13), wi = lw - ry * rw;
-        uint32_t carry = 0;
-        int base = 0;
-        for (int q = 0; q < wi; ++q) {
-            const uint32_t cq = s.C[lw - wi + q];
-            base += __popc(cq & ~((cq << 1) | carry));
-            carry = cq >> 31;
-        }
-        const uint32_t stw = c & ~((c << 1) | carry);
-        s.ST[lw] = stw;
-        s.base[lw] = (uint8_t)base;
-        const int n = __popc(stw);
+        const int ry = (int)(((uint32_t)lw * g.rw_magic) >> 13);
+        int base;
+        const int n = __popc(word_run_starts(s, lw, lw - ry * rw, s.C[lw], base));
         if (base + n > rpr) { s.overflow = 1; continue; }
         for (int k = 0; k < n; ++k) s.parent[ry * rpr + base + k] = (uint16_t)(ry * rpr + base + k);
     }
     sync_act();
     if (s.overflow) return nact;
-    // ---- unions with the row above (8-connectivity)
+    // ---- unions with the row above
     for (int i = tid; i < nwl; i += nact) {
         const int lw = s.wlist[i];
-        const uint32_t c = s.C[lw];
-        const int ry = (int)(((uint32_t)lw * g.rw_magic) >> 13), wi = lw - ry * rw;
-        if (ry == 0) continue;  // (the row above the extent is empty)
-        const int up = lw - rw;
-        const uint32_t u = s.C[up];
-        const uint32_t u_l = (wi > 0) ? (s.C[up - 1] >> 31) : 0u, u_r = (wi + 1 < rw) ? (s.C[up + 1] & 1u) : 0u;
-        const uint32_t c_l = (wi > 0) ? (s.C[lw - 1] >> 31) : 0u, c_r = (wi + 1 < rw) ? (s.C[lw + 1] & 1u) : 0u;
-        const uint32_t ul = (u << 1) | u_l, ur = (u >> 1) | (u_r << 31);
-        const uint32_t cl = (c << 1) | c_l, cr = (c >> 1) | (c_r << 31);
-        uint32_t needA = c & u & ~(cl & ul);   // pixel above, unless the left neighbour already links to it
-        uint32_t needB = c & ul & ~u & ~cl;    // upper-left only
-        uint32_t needC = c & ur & ~u & ~cr;    // upper-right only
-        while (needA) {
-            const int b = __ffs(needA) - 1;
-            needA &= needA - 1;
-            uf_union(s.parent, lean_run_id(s, lw, ry, rpr, b), lean_run_id(s, up, ry - 1, rpr, b));
-        }
-        while (needB) {
-            const int b = __ffs(needB) - 1;
-            needB &= needB - 1;
-            // (the upper-left pixel of bit 0 is bit 31 of the previous word)
-            const int id_up = b > 0 ? lean_run_id(s, up, ry - 1, rpr, b - 1) : lean_run_id(s, up - 1, ry - 1, rpr, 31);
-            uf_union(s.parent, lean_run_id(s, lw, ry, rpr, b), id_up);
-        }
-        while (needC) {
-            const int b = __ffs(needC) - 1;
-            needC &= needC - 1;
-            const int id_up = b < 31 ? lean_run_id(s, up, ry - 1, rpr, b + 1) : lean_run_id(s, up + 1, ry - 1, rpr, 0);
-            uf_union(s.parent, lean_run_id(s, lw, ry, rpr, b), id_up);
-        }
+        const int ry = (int)(((uint32_t)lw * g.rw_magic) >> 13);
+        if (ry > 0) unite_with_row_above(s, lw, lw - ry * rw, rw, s.C[lw], ry, rpr);  // (the row above the extent is empty)
     }
     sync_act();
     // ---- roots -> component slots
@@ -1469,8 +1446,7 @@ __device__ int components_lean(const KernelArgs &a, MaskSmem &s, const Geometry 
             const int id = id0 + k;
             if (s.parent[id] == id) {
                 const int slot = min(atomicAdd(&s.ncomp, 1), kLeanSlots);
-                s.c_key[slot] = INT32_MAX; s.c_area[slot] = 0; s.c_sx[slot] = 0; s.c_sy[slot] = 0;
-                s.c_l[slot] = INT32_MAX; s.c_t[slot] = INT32_MAX; s.c_r[slot] = -1; s.c_b[slot] = -1;
+                reset_slot(s, slot);
                 s.parent[id] = (uint16_t)(kSlotFlag | slot);
             }
         }
@@ -1482,54 +1458,23 @@ __device__ int components_lean(const KernelArgs &a, MaskSmem &s, const Geometry 
     for (int i = tid; i < nwl; i += nact) {
         const int lw = s.wlist[i];
         const uint32_t c = s.C[lw];
-        const int ry = (int)(((uint32_t)lw * g.rw_magic) >> 13), wi = lw - ry * rw, y = c0 + ry;
+        const int ry = (int)(((uint32_t)lw * g.rw_magic) >> 13), wi = lw - ry * rw;
         uint32_t bitsleft = s.ST[lw];
         int id = ry * rpr + (int)s.base[lw];
         while (bitsleft) {
             const int b = __ffs(bitsleft) - 1;
             bitsleft &= bitsleft - 1;
             const int slot = uf_slot(s.parent, id);
-            s.parent[id] = (uint16_t)(kSlotFlag | slot);
-            ++id;
-            const int xs = wi * 32 + b;
-            const uint32_t inv = ~(c >> b);
-            int len = (inv == 0) ? 32 : (__ffs(inv) - 1);
-            if (b + len >= 32) {  // run continues into the following words
-                len = 32 - b;
-                for (int q = wi + 1; q < rw; ++q) {
-                    const uint32_t cn = ~s.C[lw - wi + q];
-                    if (cn == 0) { len += 32; continue; }
-                    len += __ffs(cn) - 1;
-                    break;
-                }
-            }
-            atomicMin(&s.c_key[slot], (y >> 1) * g.block_w + (xs >> 1));
-            atomicAdd(&s.c_area[slot], len);
-            atomicAdd(&s.c_sx[slot], len * (2 * xs + len - 1) / 2);
-            atomicAdd(&s.c_sy[slot], len * y);
-            atomicMin(&s.c_l[slot], xs);
-            atomicMax(&s.c_r[slot], xs + len - 1);
-            atomicMin(&s.c_t[slot], y);
-            atomicMax(&s.c_b[slot], y);
+            s.parent[id++] = (uint16_t)(kSlotFlag | slot);
+            add_run(s, g, slot, wi * 32 + b, c0 + ry, run_length(s, lw, wi, rw, c, b));
         }
     }
     sync_act();
-    // ---- OpenCV label order: rank by the key of the component's first 2x2 block
     const int nout = min(ncomp, g.max_regions);
     if (tid < ncomp) {
-        const int key = s.c_key[tid];
-        int rank = 0;
-        for (int q = 0; q < ncomp; ++q) rank += (s.c_key[q] < key);
+        const int rank = slot_rank(s, tid, ncomp);
         s.c_rank[tid] = (uint8_t)rank;
-        if (rank < nout) {
-            cpt_region r;
-            r.x = s.c_l[tid]; r.y = s.c_t[tid];
-            r.width = s.c_r[tid] - r.x + 1; r.height = s.c_b[tid] - r.y + 1;
-            r.area = s.c_area[tid]; r.sum_x = s.c_sx[tid]; r.sum_y = s.c_sy[tid];
-            r.key = key;
-            r.pixel_variance = 0.0;  // region_variance_kernel
-            a.regions[o * g.max_regions + rank] = r;
-        }
+        if (rank < nout) a.regions[o * g.max_regions + rank] = region_record(s, tid);
     }
     if (tid == 0) {
         a.info[o].n_components = ncomp;
@@ -1542,27 +1487,14 @@ __device__ int components_lean(const KernelArgs &a, MaskSmem &s, const Geometry 
     for (int i = tid; i < nwl; i += nact) {
         const int lw = s.wlist[i];
         const uint32_t c = s.C[lw];
-        const int ry = (int)(((uint32_t)lw * g.rw_magic) >> 13), wi = lw - ry * rw, y = c0 + ry;
+        const int ry = (int)(((uint32_t)lw * g.rw_magic) >> 13), wi = lw - ry * rw;
         uint32_t bitsleft = s.ST[lw];
         int id = ry * rpr + (int)s.base[lw];
         while (bitsleft) {
             const int b = __ffs(bitsleft) - 1;
             bitsleft &= bitsleft - 1;
-            const uint8_t lab = (uint8_t)(s.c_rank[s.parent[id] & 0xff] + 1);
-            ++id;
-            const uint32_t inv = ~(c >> b);
-            int len = (inv == 0) ? 32 : (__ffs(inv) - 1);
-            if (b + len >= 32) {
-                len = 32 - b;
-                for (int q = wi + 1; q < rw; ++q) {
-                    const uint32_t cn = ~s.C[lw - wi + q];
-                    if (cn == 0) { len += 32; continue; }
-                    len += __ffs(cn) - 1;
-                    break;
-                }
-            }
-            uint8_t *px = lab_frame + y * W + wi * 32 + b;
-            for (int k = 0; k < len; ++k) px[k] = lab;
+            const uint8_t lab = (uint8_t)(s.c_rank[s.parent[id++] & 0xff] + 1);
+            store_label_run(lab_frame, g, wi * 32 + b, c0 + ry, run_length(s, lw, wi, rw, c, b), lab);
         }
     }
     return 0;
@@ -1785,32 +1717,6 @@ __global__ void __launch_bounds__(kFThreads, kFMinBlocks) frame_regions_kernel(c
     if (tid == 0) a.fallback[1 + atomicAdd(a.fallback, 1)] = (int)o;
 }
 
-// K6 for one region record: variance of |norm255(F_t) - norm255(F_t-1)| over the component's bounding box; one warp.
-// (one summation order everywhere it is used, so both launch plans give identical bits)
-__device__ __forceinline__ void region_variance_warp(const Geometry &g, cpt_region *reg, const float *fcur, const float *fprev, int cur_fmin,
-                                                     int cur_fmax, int prev_fmin, int prev_fmax, bool exact, int lane) {
-    const int l = reg->x, tp = reg->y, bw = reg->width, bh = reg->height, npix = bw * bh;
-    if (l < 0 || tp < 0 || bw < 1 || bh < 1 || l + bw > g.W || tp + bh > g.H) return;  // not a record of this launch
-    double s1 = 0.0, s2 = 0.0;
-    const uint32_t rcp = 0xffffffffu / (uint32_t)bw + 1u;  // i / bw == umulhi(i, rcp) for i * bw < 2^32
-    // pixels lane, lane + 32, ... in this order
-    for (int i = lane; i < npix; i += 32) {
-        const int yy = bw == 1 ? i : (int)__umulhi((uint32_t)i, rcp), xx = i - yy * bw, p = (tp + yy) * g.W + l + xx;  // (rcp wraps to 0 for bw == 1)
-        const float fc = __ldg(fcur + p), fp = __ldg(fprev + p);
-        const float d = fabsf(norm255((int)fc, cur_fmin, cur_fmax, exact) - norm255((int)fp, prev_fmin, prev_fmax, exact));
-        s1 += (double)d;
-        s2 += (double)d * (double)d;
-    }
-    for (int off = 16; off; off >>= 1) {
-        s1 += __shfl_xor_sync(0xffffffffu, s1, off);
-        s2 += __shfl_xor_sync(0xffffffffu, s2, off);
-    }
-    if (lane == 0) {
-        const double cnt = (double)npix, mean = s1 / cnt, var = s2 / cnt - mean * mean;
-        reg->pixel_variance = var > 0.0 ? var : 0.0;
-    }
-}
-
 // Split path, third launch: the frames frame_regions_kernel could not finish in place (a.fallback: very busy masks -- more than
 // kLeanSlots components or more runs in a row than its run table holds).  The stored mask -> close -> components, statistics,
 // labels (K4, K5) with the full-size tables; the variances are left to region_variance_kernel.  A small persistent grid
@@ -1825,18 +1731,15 @@ __global__ void __launch_bounds__(kGThreads, 6) frame_components_kernel(const Ke
         const long long o = a.fallback[1 + idx];
         if (o < 0 || o >= total_frames) continue;
         __syncthreads();  // the previous frame is done with the tables
-        const cpt_frame_info *fi = a.info + o;
         const uint32_t *min_ = a.maskbits + (size_t)o * kMaxWords;
         const uint32_t hflags = a.fhdr[o].flags;
         for (int i = tid; i < g.words; i += kGThreads) s.M[0][i] = min_[i];
         __syncthreads();
-        const float *fcur = a.filtered + (size_t)o * g.npx;
         const bool have_prev = !(hflags & kHdrFirst);  // not the first frame of its clip
         // (variances in this kernel were measured slower than the separate wide pass, whose warps hide the cold reads of
-        // the filtered images: components_of_frame's own path +4.1 ms, one warp per region record as a tail here +7.9 ms,
+        // the filtered images: all warps over each box +4.1 ms, one warp per region record as a tail here +7.9 ms,
         // against the 2.4 ms of region_variance_kernel)
-        components_of_frame<CompSmem, kGThreads, 1>(a, s, g, tid, 0, (size_t)o, fcur, fcur, fi->filtered_min, fi->filtered_max, 0, 0,
-                                                     have_prev, true);
+        components_of_frame<CompSmem, kGThreads, 1>(a, s, g, tid, 0, (size_t)o, have_prev);
     }
 }
 
@@ -1860,13 +1763,8 @@ __global__ void __launch_bounds__(kThreads, 1) mask_components_kernel(const Kern
         if (tid < kThreads - kCThreads)
             for (int grp = tid; grp < g.groups; grp += kThreads - kCThreads) blur_group(s, g, grp, 3u, 0, ith);
         __syncthreads();
-        if (tid >= kThreads - kCThreads) {
-            const bool have_prev = marker == 2;
-            const float *fcur = a.filtered + (size_t)o * g.npx;
-            const int fmin = a.info[o].filtered_min, fmax = a.info[o].filtered_max;
-            components_of_frame<Smem, kCThreads, BAR_C>(a, s, g, tid - (kThreads - kCThreads), 0, (size_t)o, fcur, have_prev ? fcur - g.npx : fcur, fmin, fmax,
-                                have_prev ? a.info[o - 1].filtered_min : 0, have_prev ? a.info[o - 1].filtered_max : 0, have_prev, true);
-        }
+        if (tid >= kThreads - kCThreads)
+            components_of_frame<Smem, kCThreads, BAR_C>(a, s, g, tid - (kThreads - kCThreads), 0, (size_t)o, marker == 2);
         __syncthreads();
         if (tid == 0) a.info[o].reserved[1] = 0;
     }
@@ -1885,11 +1783,14 @@ __global__ void __launch_bounds__(kVarThreads, 2048 / kVarThreads > 32 ? 32 : 20
     const int n = min(fi->n_components, g.max_regions);
     const int cur_fmin = fi->filtered_min, cur_fmax = fi->filtered_max;
     const int prev_fmin = fi[-1].filtered_min, prev_fmax = fi[-1].filtered_max;
-    const bool exact = 255ll * max(cur_fmax - cur_fmin, prev_fmax - prev_fmin) < (1ll << 24) &&
-                       max(max(abs(cur_fmax), abs(cur_fmin)), max(abs(prev_fmax), abs(prev_fmin))) < (1 << 24);
+    const bool exact = norm255_exact(cur_fmin, cur_fmax, prev_fmin, prev_fmax);
     const float *fcur = filtered + (size_t)o * g.npx, *fprev = fcur - g.npx;
-    for (int r = 0; r < n; ++r)
-        region_variance_warp(g, regions + (size_t)o * g.max_regions + r, fcur, fprev, cur_fmin, cur_fmax, prev_fmin, prev_fmax, exact, lane);
+    for (int r = 0; r < n; ++r) {
+        cpt_region *reg = regions + (size_t)o * g.max_regions + r;
+        const int l = reg->x, tp = reg->y, bw = reg->width, bh = reg->height;
+        if (l < 0 || tp < 0 || bw < 1 || bh < 1 || l + bw > g.W || tp + bh > g.H) continue;  // not a record of this launch
+        region_variance<true>(g, l, tp, bw, bh, fcur, fprev, cur_fmin, cur_fmax, prev_fmin, prev_fmax, exact, lane, &reg->pixel_variance);
+    }
     if (lane == 0) fi->reserved[0] = 0;
 }
 

@@ -23,17 +23,17 @@ def _clips(ex, designs, repeat=1):
     return ds, np.concatenate([d.frames for d in ds]), clips
 
 
-def _device(ex, frames, clips, single):
+def _device(ex, frames, clips, single, keep_filtered=True):
     import torch
 
     d_frames = torch.from_numpy(frames.view(np.int16)).cuda().view(torch.uint16)
     ex.ctx.force_single_kernel(single)
     try:
-        out = ex.extract_device(d_frames, clips, keep_filtered=True, keep_labels=True, out={})
+        out = ex.extract_device(d_frames, clips, keep_filtered=keep_filtered, keep_labels=True, out={})
         torch.cuda.synchronize()
     finally:
         ex.ctx.force_single_kernel(False)
-    return dict(filtered=out["filtered"].cpu().numpy(), labels=out["labels"].cpu().numpy(),
+    return dict(filtered=out["filtered"].cpu().numpy() if keep_filtered else None, labels=out["labels"].cpu().numpy(),
                 info=ex.info_numpy(out["info"]).copy(), regions=ex.regions_numpy(out["regions"]).copy())
 
 
@@ -77,15 +77,20 @@ def test_lean_designs_with_fewer_region_slots_than_components():
 
 
 def test_both_plans_agree_on_the_designs(extractor):
+    """The split plan against the single kernel with the filtered images kept (which leaves the variances of all frames but
+    the first to region_variance_kernel) and without them (regions only: the single kernel computes every variance)."""
     ds, frames, clips = _clips(extractor, DESIGNS)
-    a, b = (_device(extractor, frames, clips, single) for single in (False, True))
-    assert np.array_equal(a["filtered"], b["filtered"]) and np.array_equal(a["labels"], b["labels"])
-    for f in ("threshold", "n_components", "norm_min", "norm_max", "avg_change"):
-        assert np.array_equal(a["info"][f], b["info"][f]), f
-    for t in range(len(frames)):
-        k = min(int(a["info"]["n_components"][t]), extractor.max_regions)
-        for f in FIELDS + ("pixel_variance",):
-            assert np.array_equal(a["regions"][t, :k][f], b["regions"][t, :k][f]), (t, f)
+    a = _device(extractor, frames, clips, False)
+    for keep_filtered in (True, False):
+        b = _device(extractor, frames, clips, True, keep_filtered=keep_filtered)
+        assert not keep_filtered or np.array_equal(a["filtered"], b["filtered"])
+        assert np.array_equal(a["labels"], b["labels"]), keep_filtered
+        for f in ("threshold", "n_components", "norm_min", "norm_max", "avg_change"):
+            assert np.array_equal(a["info"][f], b["info"][f]), (keep_filtered, f)
+        for t in range(len(frames)):
+            k = min(int(a["info"]["n_components"][t]), extractor.max_regions)
+            for f in FIELDS + ("pixel_variance",):
+                assert np.array_equal(a["regions"][t, :k][f], b["regions"][t, :k][f]), (keep_filtered, t, f)
 
 
 def test_host_staged_chunks_and_a_larger_second_call(extractor):
