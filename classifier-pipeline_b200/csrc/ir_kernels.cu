@@ -107,6 +107,7 @@ int cpt_ir_motion_gray(cpt_ir_motion *m, const uint8_t *h_bgr, int slot_new, uin
     cpt_ctx *c = m->ctx;
     CUDA_TRY(cudaSetDevice(c->device));
     const int n = m->W * m->H;
+    CUDA_TRY(cudaStreamSynchronize(c->stream));  // without h_gray_out the previous frame's copy from h_pin may still run
     memcpy(m->h_pin, h_bgr, 3 * (size_t)n);
     CUDA_TRY(cudaMemcpyAsync(m->d_bgr, m->h_pin, 3 * (size_t)n, cudaMemcpyHostToDevice, c->stream));
     uint8_t *gray = m->d_ring + (size_t)slot_new * n;
@@ -120,13 +121,25 @@ int cpt_ir_motion_gray(cpt_ir_motion *m, const uint8_t *h_bgr, int slot_new, uin
     return CPT_OK;
 }
 
-int cpt_ir_motion_detect(cpt_ir_motion *m, int slot_new, int slot_oldest, int threshold, int erode_k, const uint8_t *h_mask,
-                         int32_t *h_diff_pixels, int32_t *h_mask_pixels) {
+const uint8_t *cpt_ir_motion_ring_slot(cpt_ir_motion *m, int slot) {
+    if (!m) {
+        fail(CPT_ERR_INVALID, "null argument");
+        return nullptr;
+    }
+    if (slot < 0 || slot >= m->ring_frames) {
+        fail(CPT_ERR_INVALID, "ring slot out of range");
+        return nullptr;
+    }
+    return m->d_ring + (size_t)slot * m->W * m->H;
+}
+
+int cpt_ir_motion_detect_ex(cpt_ir_motion *m, int slot_new, int slot_oldest, int threshold, int erode_k, const uint8_t *d_mask,
+                            int32_t *h_diff_pixels, int32_t *h_mask_pixels) {
     if (!m || !h_diff_pixels) return fail(CPT_ERR_INVALID, "null argument");
     if (slot_new < 0 || slot_new >= m->ring_frames || slot_oldest < 0 || slot_oldest >= m->ring_frames)
         return fail(CPT_ERR_INVALID, "ring slot out of range");
     if (erode_k < 1 || erode_k > 64) return fail(CPT_ERR_INVALID, "erosion box must be 1..64 pixels");
-    if (h_mask && !h_mask_pixels) return fail(CPT_ERR_INVALID, "h_mask_pixels is required with h_mask");
+    if (d_mask && !h_mask_pixels) return fail(CPT_ERR_INVALID, "h_mask_pixels is required with a mask");
     cpt_ctx *c = m->ctx;
     CUDA_TRY(cudaSetDevice(c->device));
     const int n = m->W * m->H;
@@ -135,10 +148,8 @@ int cpt_ir_motion_detect(cpt_ir_motion *m, int slot_new, int slot_oldest, int th
     cpt::delta_mask_kernel<<<(n + 255) / 256, 256, 0, st>>>(m->d_ring + (size_t)slot_oldest * n, m->d_ring + (size_t)slot_new * n, n, threshold, m->d_mask);
     cpt::erode_rows_kernel<<<(m->H + 127) / 128, 128, 0, st>>>(m->d_mask, m->W, m->H, erode_k, m->d_rows);
     cpt::erode_cols_kernel<<<(m->W + 127) / 128, 128, 0, st>>>(m->d_rows, m->W, m->H, erode_k, m->d_counts);
-    if (h_mask) {
-        memcpy(m->h_pin, h_mask, n);
-        CUDA_TRY(cudaMemcpyAsync(m->d_in_mask, m->h_pin, n, cudaMemcpyHostToDevice, st));
-        cpt::erode_rows_kernel<<<(m->H + 127) / 128, 128, 0, st>>>(m->d_in_mask, m->W, m->H, erode_k, m->d_rows);
+    if (d_mask) {
+        cpt::erode_rows_kernel<<<(m->H + 127) / 128, 128, 0, st>>>(d_mask, m->W, m->H, erode_k, m->d_rows);
         cpt::erode_cols_kernel<<<(m->W + 127) / 128, 128, 0, st>>>(m->d_rows, m->W, m->H, erode_k, m->d_counts + 1);
     }
     CUDA_TRY(cudaGetLastError());
@@ -146,8 +157,24 @@ int cpt_ir_motion_detect(cpt_ir_motion *m, int slot_new, int slot_oldest, int th
     CUDA_TRY(cudaMemcpyAsync(h_counts, m->d_counts, 2 * sizeof(int), cudaMemcpyDeviceToHost, st));
     CUDA_TRY(cudaStreamSynchronize(st));
     *h_diff_pixels = h_counts[0];
-    if (h_mask_pixels) *h_mask_pixels = h_mask ? h_counts[1] : 0;
+    if (h_mask_pixels) *h_mask_pixels = d_mask ? h_counts[1] : 0;
     return CPT_OK;
+}
+
+int cpt_ir_motion_detect(cpt_ir_motion *m, int slot_new, int slot_oldest, int threshold, int erode_k, const uint8_t *h_mask,
+                         int32_t *h_diff_pixels, int32_t *h_mask_pixels) {
+    if (!m) return fail(CPT_ERR_INVALID, "null argument");
+    if (h_mask && !h_mask_pixels) return fail(CPT_ERR_INVALID, "h_mask_pixels is required with h_mask");
+    if (h_mask) {
+        // the host mask goes through pinned staging into the detector's own device buffer
+        const int n = m->W * m->H;
+        CUDA_TRY(cudaSetDevice(m->ctx->device));
+        CUDA_TRY(cudaStreamSynchronize(m->ctx->stream));  // h_pin may still be the source of an earlier copy
+        memcpy(m->h_pin, h_mask, n);
+        CUDA_TRY(cudaMemcpyAsync(m->d_in_mask, m->h_pin, n, cudaMemcpyHostToDevice, m->ctx->stream));
+    }
+    return cpt_ir_motion_detect_ex(m, slot_new, slot_oldest, threshold, erode_k, h_mask ? m->d_in_mask : nullptr, h_diff_pixels,
+                                   h_mask_pixels);
 }
 
 }  // extern "C"

@@ -73,6 +73,12 @@ class CptMotionResult(ctypes.Structure):
                 ("mean_frames", ctypes.c_int32), ("reserved", ctypes.c_int32)]
 
 
+class CptMog2Params(ctypes.Structure):
+    _fields_ = [("history", ctypes.c_int), ("var_threshold", ctypes.c_double), ("background_ratio", ctypes.c_double),
+                ("var_threshold_gen", ctypes.c_float), ("var_init", ctypes.c_float), ("var_min", ctypes.c_float),
+                ("var_max", ctypes.c_float), ("complexity_reduction", ctypes.c_float), ("detect_shadows", ctypes.c_int)]
+
+
 DETECT_CLOSE, DETECT_OPEN_GRAY, DETECT_DILATE, DETECT_OTSU, DETECT_MASK_ONLY = 1, 2, 4, 8, 16
 MOTION_MEAN, MOTION_MEAN_RESTART, MOTION_BACKGROUND, MOTION_DETECT, MOTION_WARMER_ONLY, MOTION_ONE_DIFF = 1, 2, 4, 8, 16, 32
 
@@ -159,6 +165,13 @@ SYMBOLS = {
     "cpt_ir_motion_close": (None, [_vp]),
     "cpt_ir_motion_gray": (_i, [_vp, _vp, _i, _vp]),
     "cpt_ir_motion_detect": (_i, [_vp, _i, _i, _i, _i, _vp, ctypes.POINTER(ctypes.c_int32), ctypes.POINTER(ctypes.c_int32)]),
+    "cpt_ir_motion_ring_slot": (_vp, [_vp, _i]),
+    "cpt_ir_motion_detect_ex": (_i, [_vp, _i, _i, _i, _i, _vp, ctypes.POINTER(ctypes.c_int32), ctypes.POINTER(ctypes.c_int32)]),
+    "cpt_mog2_open": (_vp, [_vp, _i, _i, ctypes.POINTER(CptMog2Params)]),
+    "cpt_mog2_close": (None, [_vp]),
+    "cpt_mog2_apply": (_i, [_vp, _vp, _i, _i64, _vp, _vp]),
+    "cpt_mog2_background": (_i, [_vp, _vp]),
+    "cpt_mog2_frames": (_i, [_vp]),
     "cpt_cptv_decode": (_i, [_vp, _vp, _vp, _i, _vp, _i, _vp]),
     "cpt_extract_batch_cptv_host": (_i, [_vp, _vp, _u64, _vp, _vp, _vp, _i, _i64, _vp, _vp, _i]),
     "cpt_motion_open": (_vp, [_vp, _i, _i, _i, _i]),
@@ -417,16 +430,33 @@ class IrMotion:
         if not self._h:
             raise NativeError("cpt_ir_motion_open failed: {}".format(ctx.lib.cpt_last_error().decode()))
 
-    def gray(self, bgr, slot):
+    def gray(self, bgr, slot, copy_out=True):
+        """BGR frame -> grey into ring slot ``slot``; returns the grey frame as a host array, or None with copy_out=False
+        (the frame then stays on the device: ``ring_slot(slot)``)."""
         bgr = np.ascontiguousarray(bgr, dtype=np.uint8)
         if bgr.shape != (self.height, self.width, 3):
             raise ValueError("IR frames must be ({}, {}, 3) uint8".format(self.height, self.width))
-        out = np.empty((self.height, self.width), np.uint8)
+        out = np.empty((self.height, self.width), np.uint8) if copy_out else None
         check(self.ctx.lib.cpt_ir_motion_gray(self._h, _ptr(bgr), int(slot), _ptr(out)))
         return out
 
-    def detect(self, slot_new, slot_oldest, threshold, erode_k, mask=None):
+    def ring_slot(self, slot):
+        """Device address of the grey frame in ring slot ``slot`` ([H][W] uint8)."""
+        p = self.ctx.lib.cpt_ir_motion_ring_slot(self._h, int(slot))
+        if not p:
+            raise NativeError("cpt_ir_motion_ring_slot failed: {}".format(self.ctx.lib.cpt_last_error().decode()))
+        return p
+
+    def detect(self, slot_new, slot_oldest, threshold, erode_k, mask=None, d_mask=None):
+        """(eroded difference pixels, eroded mask pixels).  The foreground mask is a host array (``mask``) or device memory
+        (``d_mask``: a uint8 CUDA tensor or a device address, e.g. ``Mog2.apply``'s output); at most one of them."""
         diff, cnt = ctypes.c_int32(), ctypes.c_int32()
+        if d_mask is not None:
+            if mask is not None:
+                raise ValueError("pass mask or d_mask, not both")
+            check(self.ctx.lib.cpt_ir_motion_detect_ex(self._h, int(slot_new), int(slot_oldest), int(threshold), int(erode_k),
+                                                       _dptr(d_mask, self.height * self.width), ctypes.byref(diff), ctypes.byref(cnt)))
+            return diff.value, cnt.value
         if mask is not None:
             mask = np.ascontiguousarray(mask, dtype=np.uint8)
         check(self.ctx.lib.cpt_ir_motion_detect(self._h, int(slot_new), int(slot_oldest), int(threshold), int(erode_k), _ptr(mask),
@@ -436,6 +466,77 @@ class IrMotion:
     def close(self):
         if self._h:
             self.ctx.lib.cpt_ir_motion_close(self._h)
+            self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+def _dptr(t, min_bytes):
+    """Device address of a uint8 CUDA tensor (at least min_bytes, contiguous) or a raw device address (int)."""
+    if isinstance(t, int):
+        return t
+    if not (getattr(t, "is_cuda", False) and str(t.dtype) == "torch.uint8" and t.is_contiguous() and t.numel() >= min_bytes):
+        raise ValueError("expected a contiguous uint8 CUDA tensor of at least {} bytes".format(min_bytes))
+    return t.data_ptr()
+
+
+class Mog2:
+    """OpenCV's BackgroundSubtractorMOG2 (detectShadows=False, one uint8 channel) on the device, bit for bit (cpt_mog2_*).
+    The model's state stays in device memory; frames and masks are uint8 CUDA tensors or device addresses.  Calls launch on
+    the context's stream and return without waiting."""
+
+    def __init__(self, ctx, width, height, history=500, var_threshold=16.0, background_ratio=0.9, var_threshold_gen=9.0,
+                 var_init=15.0, var_min=4.0, var_max=75.0, complexity_reduction=0.05, detect_shadows=False):
+        self.ctx = ctx
+        self.width, self.height = int(width), int(height)
+        self.params = CptMog2Params(int(history), float(var_threshold), float(background_ratio), float(var_threshold_gen), float(var_init),
+                                    float(var_min), float(var_max), float(complexity_reduction), int(bool(detect_shadows)))
+        self._h = ctx.lib.cpt_mog2_open(ctx._h, self.width, self.height, ctypes.byref(self.params))
+        if not self._h:
+            raise NativeError("cpt_mog2_open failed: {}".format(ctx.lib.cpt_last_error().decode()))
+
+    @property
+    def frame_bytes(self):
+        return self.width * self.height
+
+    def apply(self, d_frames, learning_rates, d_masks=None, n_frames=None, frame_stride=None):
+        """apply() for consecutive frames: d_frames [n][H][W] (or [H][W]) uint8 on the device, learning_rates one cv2
+        learningRate per frame (a number applies to all).  Writes n masks (0 / 255) to d_masks when given."""
+        n = n_frames
+        if n is None:
+            if isinstance(d_frames, int):
+                raise ValueError("n_frames is required with a device address")
+            if tuple(d_frames.shape[-2:]) != (self.height, self.width):
+                raise ValueError("MOG2 frames must be [..., {}, {}] uint8".format(self.height, self.width))
+            n = 1 if d_frames.dim() == 2 else int(d_frames.shape[0])
+        stride = self.frame_bytes if frame_stride is None else int(frame_stride)
+        lrs = np.full(n, float(learning_rates), np.float64) if np.isscalar(learning_rates) else np.ascontiguousarray(learning_rates, np.float64)
+        if lrs.shape != (n,):
+            raise ValueError("one learning rate per frame")
+        if n == 0:
+            return
+        fp = _dptr(d_frames, stride * (n - 1) + self.frame_bytes)
+        mp = None if d_masks is None else _dptr(d_masks, n * self.frame_bytes)
+        check(self.ctx.lib.cpt_mog2_apply(self._h, fp, int(n), int(stride), lrs.ctypes.data, mp))
+
+    def background(self, d_out):
+        """getBackgroundImage() into d_out ([H][W] uint8 on the device)."""
+        check(self.ctx.lib.cpt_mog2_background(self._h, _dptr(d_out, self.frame_bytes)))
+
+    @property
+    def frames(self):
+        n = self.ctx.lib.cpt_mog2_frames(self._h)
+        if n < 0:
+            check(n)
+        return n
+
+    def close(self):
+        if getattr(self, "_h", None):
+            self.ctx.lib.cpt_mog2_close(self._h)
             self._h = None
 
     def __del__(self):

@@ -3,15 +3,18 @@
 Per frame the reference converts BGR to grey, updates its background model, and erodes two binary images with a 15x15
 (idle) or 10x10 (recording) box: ``absdiff(oldest grey, grey) > 12`` and the background model's foreground mask.  The grey
 conversion, the difference mask, both erosions and the pixel counts run on the device (csrc/ir_kernels.cu), with the grey
-ring resident in device memory.  The background model itself is OpenCV's MOG2 (``track.cliptracker.CVBackground``): a
-third-party algorithm, not restated here -- it runs on the host through cv2 when cv2 is importable, and any object with
-``update_background(gray, learning_rate=)`` / ``compute_filtered(None)`` / ``background`` can be passed instead.
+ring resident in device memory.  The background model is OpenCV's MOG2: by default ``track.cliptracker.CVBackground``, cv2 on
+the host, which needs the grey frame copied out and the mask copied back every frame.  ``MOG2Background`` (the same model
+bit for bit, csrc/mog2_kernels.cu) on the detector's engine keeps both on the device: the grey frame goes from its ring slot
+into the model and the mask from the model into the erosion, so per frame only the BGR frame goes in and two counts come
+out.  Any other object with ``update_background(gray, learning_rate=)`` / ``compute_filtered(None)`` / ``background`` can be
+passed as well.
 """
 import numpy as np
 
 from .. import engine as _engine
 from .. import native
-from ..track.cliptracker import Background, CVBackground, get_diff_back_filtered
+from ..track.cliptracker import Background, CVBackground, MOG2Background, get_diff_back_filtered
 from .motiondetector import MotionDetector, SlidingWindow
 
 
@@ -74,6 +77,9 @@ class IRMotionDetector(MotionDetector):
         self.processed = 0
         eng = _engine.get_engine(device)
         self._dev = native.IrMotion(eng.ctx, headers.res_x, headers.res_y, max(self.num_preview_frames, 1))
+        self._device_background = isinstance(self._background, MOG2Background) and self._background.ctx is eng.ctx
+        if self._device_background:
+            eng.ctx.use_torch_stream()  # grey ring, model and erosion in one stream order from the first frame on
 
     def disconnected(self):
         self.rgb_window.reset()
@@ -103,15 +109,21 @@ class IRMotionDetector(MotionDetector):
             # the grey ring lives on the device: the host window only tracks which slot is the oldest / the newest
             self.gray_window.add(None)
             slot = self.gray_window.last_index
-            gray = self._dev.gray(frame, slot)
+            gray = self._dev.gray(frame, slot, copy_out=not self._device_background)
             if self.gray_window.oldest_index is None:
                 return False
             learning_rate = 0 if self.movement_detected else -1
-            self._background.update_background(gray, learning_rate=learning_rate)
+            if self._device_background:
+                self._background.update_background_device(self._dev.ring_slot(slot), self._dev.width, self._dev.height, learning_rate)
+            else:
+                self._background.update_background(gray, learning_rate=learning_rate)
             if self.num_frames > MIN_FRAMES:
                 k = self.get_kernel().shape[0]
-                diff_erosion_pixels, erosion_pixels = self._dev.detect(slot, self.gray_window.oldest_index, THRESHOLD, k,
-                                                                       mask=self._background.compute_filtered(None))
+                if self._device_background:
+                    mask = dict(d_mask=self._background.device_mask)
+                else:
+                    mask = dict(mask=self._background.compute_filtered(None))
+                diff_erosion_pixels, erosion_pixels = self._dev.detect(slot, self.gray_window.oldest_index, THRESHOLD, k, **mask)
                 # with the background frozen while motion lasts, a real change of the scene would keep the trigger up
                 # forever: the frame difference bounds it
                 if self.movement_detected:

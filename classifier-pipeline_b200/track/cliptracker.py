@@ -280,6 +280,108 @@ class CVBackground(Background):
         return self._background
 
 
+class MOG2Background(Background):
+    """``CVBackground`` on the device: cv2.createBackgroundSubtractorMOG2(history, var_threshold, detectShadows=False) bit for
+    bit (csrc/mog2_kernels.cu), with the model's state in device memory.  Frames are host uint8 arrays or uint8 CUDA tensors
+    of one geometry (fixed by the first frame).  ``update_backgrounds`` runs a whole clip's frames in one launch."""
+
+    def __init__(self, history=1000, var_threshold=16, device=None):
+        super().__init__()
+        from .. import engine
+
+        self.history, self.var_threshold = int(history), float(var_threshold)
+        self.ctx = engine.get_engine(device).ctx
+        self._model = None
+        self._mask = None       # last foreground mask, [H][W] uint8 on the device
+        self._mask_host = None  # its host copy, made on first request
+
+    def _open(self, height, width):
+        if self._model is None:
+            from ..native import Mog2
+
+            self._model = Mog2(self.ctx, width, height, history=self.history, var_threshold=self.var_threshold)
+        elif (self._model.height, self._model.width) != (height, width):
+            raise ValueError("MOG2Background holds {}x{} frames, got {}x{}".format(self._model.width, self._model.height, width, height))
+        return self._model
+
+    def _to_device(self, frames):
+        import torch
+
+        if isinstance(frames, torch.Tensor):
+            if frames.dtype != torch.uint8 or not frames.is_cuda:
+                raise ValueError("MOG2Background takes uint8 frames (host arrays or CUDA tensors)")
+            return frames.contiguous()
+        frames = np.ascontiguousarray(frames)
+        if frames.dtype != np.uint8:
+            raise ValueError("MOG2Background takes uint8 frames (host arrays or CUDA tensors)")
+        return torch.from_numpy(frames).to("cuda:{}".format(self.ctx.device))
+
+    def update_background_device(self, d_frame, width, height, learning_rate=-1):
+        """One apply() on a [height][width] uint8 frame already in device memory, given by its address (the IR detector's
+        grey ring slot)."""
+        import torch
+
+        model = self._open(height, width)
+        self.ctx.use_torch_stream()
+        self._mask = torch.empty((height, width), dtype=torch.uint8, device="cuda:{}".format(self.ctx.device))
+        self._mask_host = None
+        model.apply(d_frame, [learning_rate], d_masks=self._mask, n_frames=1)
+        self._frames += 1
+
+    def set_background(self, background, frames=1):
+        self.update_background(background, learning_rate=1)
+
+    def update_background(self, thermal, filtered=None, learning_rate=-1):
+        frame = self._to_device(thermal)
+        if frame.dim() != 2:
+            raise ValueError("update_background takes one [H][W] frame")
+        self.update_background_device(frame.data_ptr(), frame.shape[1], frame.shape[0], learning_rate)
+
+    def update_backgrounds(self, frames, learning_rate=-1):
+        """apply() on frames [N][H][W] in one launch; learning_rate is a number or one per frame.  Returns the N masks, as
+        host arrays for host input and as a CUDA tensor for device input."""
+        import torch
+
+        d = self._to_device(frames)
+        if d.dim() != 3:
+            raise ValueError("update_backgrounds takes frames [N][H][W]")
+        n, h, w = d.shape
+        model = self._open(h, w)
+        self.ctx.use_torch_stream()
+        masks = torch.empty((n, h, w), dtype=torch.uint8, device=d.device)
+        lrs = np.full(n, float(learning_rate)) if np.isscalar(learning_rate) else learning_rate
+        model.apply(d, lrs, d_masks=masks)
+        self._frames += n
+        if n:
+            self._mask, self._mask_host = masks[n - 1], None
+        return masks if isinstance(frames, torch.Tensor) else masks.cpu().numpy()
+
+    @property
+    def background(self):
+        """getBackgroundImage() as a host array."""
+        import torch
+
+        if self._model is None:
+            return None
+        self.ctx.use_torch_stream()
+        out = torch.empty((self._model.height, self._model.width), dtype=torch.uint8, device="cuda:{}".format(self.ctx.device))
+        self._model.background(out)
+        return out.cpu().numpy()
+
+    @property
+    def device_mask(self):
+        """The last foreground mask (0 / 255) on the device, without a copy."""
+        return self._mask
+
+    def compute_filtered(self, thermal, threshold=None):
+        """The last foreground mask as a host array (copied once, on first request)."""
+        if self._mask is None:
+            return None
+        if self._mask_host is None:
+            self._mask_host = self._mask.cpu().numpy()
+        return self._mask_host
+
+
 def get_diff_back_filtered(background, frame, back_thresh):
     """|frame - background| with everything below back_thresh zeroed, normalised to 0..255 (cliptracker.py:652-668);
     the normalisation runs on the device (ml_tools.imageprocessing.normalize)."""

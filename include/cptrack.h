@@ -358,21 +358,50 @@ int cpt_motion_step(cpt_motion *m, const uint16_t *h_pix, void *d_background_sta
                     double init_average, cpt_motion_result *h_result);
 
 /* ---- IRMotionDetector (piclassifier/irmotiondetector.py:55-153), streaming, 640x480 BGR frames ----
- * Per frame the reference does cv2.cvtColor(BGR2GRAY), feeds the grey frame to its background model (OpenCV's MOG2: third
- * party, stays on the host), then absdiff(oldest grey, grey) -> threshold 12 -> erode with a k x k box (15 idle / 10 while
- * recording) -> count, and the same erode + count on the background model's foreground mask.  The detector owns a ring of
- * grey frames on the device (SlidingWindow of preview_secs * fps frames).
- *   cpt_ir_motion_gray    h_bgr [H][W][3] -> grey (OpenCV's fixed point: (B*3735 + G*19235 + R*9798 + 2^14) >> 15) into ring
- *                         slot slot_new; h_gray_out (may be NULL) receives it for the host's background model
- *   cpt_ir_motion_detect  *h_diff_pixels = count(erode(|ring[slot_oldest] - ring[slot_new]| > threshold)); with h_mask (the
- *                         background model's foreground mask, [H][W], non-zero = set; may be NULL) *h_mask_pixels =
- *                         count(erode(h_mask)).  Pixels outside the image do not constrain the erosion (cv2's default). */
+ * Per frame the reference does cv2.cvtColor(BGR2GRAY), feeds the grey frame to its background model (OpenCV's MOG2, on the
+ * host through cv2 or on the device through cpt_mog2 below), then absdiff(oldest grey, grey) -> threshold 12 -> erode with a
+ * k x k box (15 idle / 10 while recording) -> count, and the same erode + count on the background model's foreground mask.
+ * The detector owns a ring of grey frames on the device (SlidingWindow of preview_secs * fps frames).
+ *   cpt_ir_motion_gray       h_bgr [H][W][3] -> grey (OpenCV's fixed point: (B*3735 + G*19235 + R*9798 + 2^14) >> 15) into
+ *                            ring slot slot_new; h_gray_out (may be NULL) receives it for a host background model
+ *   cpt_ir_motion_ring_slot  device address of ring slot `slot` ([H][W] uint8), NULL (CPT_ERR_INVALID) out of range
+ *   cpt_ir_motion_detect     *h_diff_pixels = count(erode(|ring[slot_oldest] - ring[slot_new]| > threshold)); with h_mask (the
+ *                            background model's foreground mask, [H][W], non-zero = set; may be NULL) *h_mask_pixels =
+ *                            count(erode(h_mask)).  Pixels outside the image do not constrain the erosion (cv2's default).
+ *   cpt_ir_motion_detect_ex  the same with the mask in device memory (d_mask, e.g. cpt_mog2_apply's output; may be NULL) */
 typedef struct cpt_ir_motion cpt_ir_motion;
 cpt_ir_motion *cpt_ir_motion_open(cpt_ctx *ctx, int width, int height, int ring_frames);
 void cpt_ir_motion_close(cpt_ir_motion *m);
 int cpt_ir_motion_gray(cpt_ir_motion *m, const uint8_t *h_bgr, int slot_new, uint8_t *h_gray_out);
 int cpt_ir_motion_detect(cpt_ir_motion *m, int slot_new, int slot_oldest, int threshold, int erode_k, const uint8_t *h_mask,
                          int32_t *h_diff_pixels, int32_t *h_mask_pixels);
+const uint8_t *cpt_ir_motion_ring_slot(cpt_ir_motion *m, int slot);
+int cpt_ir_motion_detect_ex(cpt_ir_motion *m, int slot_new, int slot_oldest, int threshold, int erode_k, const uint8_t *d_mask,
+                            int32_t *h_diff_pixels, int32_t *h_mask_pixels);
+
+/* ---- OpenCV's BackgroundSubtractorMOG2 (track/cliptracker.py:560-609 CVBackground; the IR detector's background model) ----
+ * cv2.createBackgroundSubtractorMOG2(history, varThreshold, detectShadows=False) on one uint8 channel with five modes, bit for
+ * bit: every foreground mask of apply() and getBackgroundImage().  The model's state (61 bytes per pixel) stays on the
+ * device; one cpt_mog2_apply runs any number of consecutive frames (one launch per 256 frames, a new launch where a frame
+ * re-initialises the model).  Launches go on the ctx stream and do not synchronise. */
+typedef struct cpt_mog2_params {       /* cv2.createBackgroundSubtractorMOG2 defaults in brackets */
+    int history;                       /* [500]; the reference's CVBackground uses 1000 */
+    double var_threshold;              /* Tb [16] */
+    double background_ratio;           /* TB [0.9] */
+    float var_threshold_gen;           /* Tg [9] */
+    float var_init, var_min, var_max;  /* [15, 4, 75] */
+    float complexity_reduction;        /* fCT [0.05f] -- prune = (float)(-lr * (double)fCT) */
+    int detect_shadows;                /* must be 0: the reference creates MOG2 with detectShadows=False */
+} cpt_mog2_params;
+typedef struct cpt_mog2 cpt_mog2;
+cpt_mog2 *cpt_mog2_open(cpt_ctx *ctx, int width, int height, const cpt_mog2_params *p);
+void cpt_mog2_close(cpt_mog2 *m);
+/* n_frames uint8 frames at d_frames (frame_stride bytes apart) -> n_frames masks (0 / 255) at d_masks (may be NULL);
+ * h_learning_rates[n_frames]: cv2's learningRate argument per frame (-1 = automatic, >= 1 re-initialises the model) */
+int cpt_mog2_apply(cpt_mog2 *m, const uint8_t *d_frames, int n_frames, int64_t frame_stride,
+                   const double *h_learning_rates, uint8_t *d_masks);
+int cpt_mog2_background(cpt_mog2 *m, uint8_t *d_out);   /* getBackgroundImage: d_out [H][W] uint8 */
+int cpt_mog2_frames(const cpt_mog2 *m);                 /* nframes as cv2 counts it (frames since the last initialisation) */
 
 /* State access for WeightedBackground.background / .background_weight / .average
  * (motiondetector.py:178-248).  h_background int32 [H][W]; h_weight_count uint16 [(H-2e)][(W-2e)]
