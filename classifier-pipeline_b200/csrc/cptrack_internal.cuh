@@ -123,6 +123,7 @@ struct cpt_ctx {
     cpt::Grow<int32_t, true> pk_h_first[2];  // packed host-staged call: the same, on the host
     cpt::Grow<int32_t> pk_change;  // packed host-staged call: the decoder's change images
     cpt::Grow<int32_t> cptv_scratch;  // cpt_cptv_decode: the decoder's change images
-    cpt::Grow<uint8_t> detect_scratch;  // cpt_detect_objects_ex: images, masks, union-find and component tables
+    cpt::Grow<uint8_t> detect_scratch;  // cpt_detect_objects_ex / _batch: images, masks, union-find and component tables
+    cpt::Grow<int> merge_order;  // cpt_ir_merge_components: list order of every frame of a launch
 };
 

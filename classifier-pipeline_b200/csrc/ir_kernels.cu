@@ -6,6 +6,10 @@
 //   erode_rows_kernel    one thread per image row: a pixel survives the horizontal pass iff its k-wide window (anchor k / 2,
 //                        pixels outside the image count as set) is all set -- run lengths along the row
 //   erode_cols_kernel    one thread per column: the vertical pass on the row result, counting the survivors
+// and the rectangle merging of the IR tracker's detection half for a batch of frames:
+//   ir_merge_kernel      track/irtrackextractor.py merge_components on every frame's stats rows, one warp per frame
+#include <algorithm>
+
 #include "cptrack_internal.cuh"
 
 namespace cpt {
@@ -53,6 +57,149 @@ __global__ void __launch_bounds__(128) erode_cols_kernel(const uint8_t *rows_ok,
     }
     mine = __reduce_add_sync(0xffffffffu, mine);
     if ((threadIdx.x & 31) == 0 && mine) atomicAdd(count, mine);
+}
+
+// merge_components' pair test (track/irtrackextractor.py): rect a = the scanning rectangle, b = the other one.  The squared
+// distance wraps in 32 bits as numpy's int32 arithmetic on the stats rows does.
+__device__ __forceinline__ bool ir_rects_merge(int ax, int ay, int aw, int ah, int bx, int by, int bw, int bh, double max_gap) {
+    bool within = false;
+    if (bw + aw > max(bx + bw, aw + ax) - min(bx, ax)) within = bh + ah > max(by + bh, ay + ah) - min(by, ay);
+    int x1 = 0, x2 = 0, y1 = 0, y2 = 0;
+    if (aw + bw > max(ax + aw, bw + bx) - min(ax, bx)) {
+    } else if (ax < bx) {
+        x1 = ax + aw; x2 = bx;
+    } else {
+        x1 = bx + bw; x2 = ax;
+    }
+    if (ah + bh > max(ay + ah, by + bh) - min(ay, by)) {
+    } else if (ay < by) {
+        y1 = ay + ah; y2 = by;
+    } else {
+        y1 = by + bh; y2 = ay;
+    }
+    const unsigned dx = (unsigned)(x1 - x2), dy = (unsigned)(y1 - y2);
+    const int d2 = (int)(dx * dx + dy * dy);
+    return sqrt((double)d2) < max_gap || within;
+}
+
+// One warp per frame.  stats [frame][max_components + 1][5] with row 0 the background, counts = cv2's label count.  The
+// list lives in the frame's output rows (merged, [max_components][5]) and in order[max_components] (the label of each list
+// position; negative once deleted), so no list length is too long: every step is a warp-wide pass over the list, 32
+// positions at a time.  A deletion only marks the position, which keeps the survivors in the order the Python list keeps
+// them.
+__global__ void __launch_bounds__(128) ir_merge_kernel(const int32_t *stats, const int32_t *counts, int n_frames, int max_components,
+                                                       int min_mass, int min_size, double max_gap, int *order, int32_t *merged,
+                                                       int32_t *merged_counts) {
+    const int f = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
+    if (f >= n_frames) return;  // whole warps
+    const unsigned below = (1u << lane) - 1u;
+    const int n = counts[f];
+    if (n < 1 || n - 1 > max_components) {  // overflowed: the list is truncated, never merge it
+        if (lane == 0) merged_counts[f] = -1;
+        return;
+    }
+    stats += (size_t)f * ((size_t)max_components + 1) * 5;
+    merged += (size_t)f * (size_t)max_components * 5;
+    int *ord = order + (size_t)f * max_components;
+    // filter, in label order
+    int m = 0;
+    for (int b = 0; b < n - 1; b += 32) {
+        const int l = b + lane + 1;
+        bool keep = false;
+        if (l < n) {
+            const int32_t *r = stats + l * 5;
+            keep = r[4] > min_mass || (r[2] > min_size && r[3] > min_size);
+        }
+        const unsigned k = __ballot_sync(0xffffffffu, keep);
+        if (keep) ord[m + __popc(k & below)] = l;
+        m += __popc(k);
+    }
+    __syncwarp();
+    // stable sort by area, descending: the rank counts larger areas and equal areas earlier in the list
+    for (int b = 0; b < m; b += 32) {
+        const int i = b + lane;
+        if (i < m) {
+            const int li = ord[i], ai = stats[li * 5 + 4];
+            int rank = 0;
+            for (int j = 0; j < m; ++j) {
+                const int aj = stats[ord[j] * 5 + 4];
+                rank += aj > ai || (aj == ai && j < i);
+            }
+            merged[rank * 5] = li;
+        }
+    }
+    __syncwarp();
+    for (int p = lane; p < m; p += 32) {
+        const int l = merged[p * 5];
+        ord[p] = l;
+        for (int k = 0; k < 5; ++k) merged[p * 5 + k] = stats[l * 5 + k];
+    }
+    __syncwarp();
+    // the scan: the current rectangle's original against every live original; merges fold in list order
+    int cur = 0;
+    while (cur < m) {
+        const int32_t *rc = stats + ord[cur] * 5;
+        const int rx = rc[0], ry = rc[1], rw = rc[2], rh = rc[3];
+        int mx = merged[cur * 5], my = merged[cur * 5 + 1], mw = merged[cur * 5 + 2], mh = merged[cur * 5 + 3], ma = merged[cur * 5 + 4];
+        bool any = false;
+        for (int b = 0; b < m; b += 32) {
+            const int p = b + lane;
+            const int l = p < m ? ord[p] : 0;
+            int x2 = 0, y2 = 0, w2 = 0, h2 = 0, a2 = 0;
+            bool hit = false;
+            if (l > 0) {
+                const int32_t *r2 = stats + l * 5;
+                x2 = r2[0]; y2 = r2[1]; w2 = r2[2]; h2 = r2[3]; a2 = r2[4];
+                hit = x2 != rx && ir_rects_merge(rx, ry, rw, rh, x2, y2, w2, h2, max_gap);
+            }
+            unsigned hits = __ballot_sync(0xffffffffu, hit);
+            any |= hits != 0;
+            if (hit) ord[p] = -l;
+            while (hits) {
+                const int k = __ffs(hits) - 1;
+                hits &= hits - 1;
+                const int X = __shfl_sync(0xffffffffu, x2, k), Y = __shfl_sync(0xffffffffu, y2, k);
+                const int W2 = __shfl_sync(0xffffffffu, w2, k), H2 = __shfl_sync(0xffffffffu, h2, k), A2 = __shfl_sync(0xffffffffu, a2, k);
+                const int cur_right = mx + mw;
+                mx = min(mx, X);
+                my = min(my, Y);
+                mw = max(cur_right, X + W2) - mx;
+                mh = max(my + mh, Y + H2) - my;  // the bottom edge from the updated y, as the reference writes it
+                ma += A2;
+            }
+        }
+        if (any && lane == 0) {
+            merged[cur * 5] = mx; merged[cur * 5 + 1] = my; merged[cur * 5 + 2] = mw; merged[cur * 5 + 3] = mh; merged[cur * 5 + 4] = ma;
+        }
+        __syncwarp();
+        // a merge restarts the scan at the first live rectangle, otherwise it moves to the next live one
+        const int start = any ? 0 : cur + 1;
+        cur = m;
+        for (int b = start; b < m; b += 32) {
+            const int p = b + lane;
+            const unsigned live = __ballot_sync(0xffffffffu, p < m && ord[p] > 0);
+            if (live) {
+                cur = b + __ffs(live) - 1;
+                break;
+            }
+        }
+    }
+    // compact the live rows in place (a row only moves down, and a chunk is read before it is written)
+    int out = 0;
+    for (int b = 0; b < m; b += 32) {
+        const int p = b + lane;
+        const bool live = p < m && ord[p] > 0;
+        int row[5];
+        if (live)
+            for (int k = 0; k < 5; ++k) row[k] = merged[p * 5 + k];
+        const unsigned lv = __ballot_sync(0xffffffffu, live);
+        __syncwarp();
+        if (live)
+            for (int k = 0; k < 5; ++k) merged[(out + __popc(lv & below)) * 5 + k] = row[k];
+        out += __popc(lv);
+        __syncwarp();
+    }
+    if (lane == 0) merged_counts[f] = out;
 }
 
 }  // namespace cpt
@@ -175,6 +322,27 @@ int cpt_ir_motion_detect(cpt_ir_motion *m, int slot_new, int slot_oldest, int th
     }
     return cpt_ir_motion_detect_ex(m, slot_new, slot_oldest, threshold, erode_k, h_mask ? m->d_in_mask : nullptr, h_diff_pixels,
                                    h_mask_pixels);
+}
+
+int cpt_ir_merge_components(cpt_ctx *c, const int32_t *d_stats, const int32_t *d_counts, int n_frames, int max_components, int min_mass,
+                            int min_size, double max_gap, int32_t *d_merged, int32_t *d_merged_counts) {
+    if (!c || !d_stats || !d_counts || !d_merged || !d_merged_counts) return fail(CPT_ERR_INVALID, "null argument");
+    if (n_frames < 0) return fail(CPT_ERR_INVALID, "n_frames < 0");
+    if (max_components < 1) return fail(CPT_ERR_INVALID, "max_components < 1");
+    if (n_frames == 0) return CPT_OK;
+    CUDA_TRY(cudaSetDevice(c->device));
+    // frames per launch: the list-order scratch stays near 64 MB whatever the call's length
+    const int chunk = (int)std::max<long long>(1, std::min<long long>(n_frames, (16ll << 20) / max_components));
+    CUDA_TRY(c->merge_order.ensure((size_t)chunk * max_components));
+    const size_t rows = (size_t)max_components + 1;
+    for (int f0 = 0; f0 < n_frames; f0 += chunk) {
+        const int nf = std::min(chunk, n_frames - f0);
+        cpt::ir_merge_kernel<<<(nf + 3) / 4, 128, 0, c->stream>>>(d_stats + (size_t)f0 * rows * 5, d_counts + f0, nf, max_components, min_mass,
+                                                                   min_size, max_gap, c->merge_order,
+                                                                   d_merged + (size_t)f0 * max_components * 5, d_merged_counts + f0);
+    }
+    CUDA_TRY(cudaGetLastError());
+    return CPT_OK;
 }
 
 }  // extern "C"

@@ -160,6 +160,8 @@ SYMBOLS = {
     "cpt_detect_objects_u8": (_i, [_vp, _vp, _i, _i, _d, _i, _i, _i, _vp, _vp, _vp, ctypes.POINTER(ctypes.c_int32)]),
     "cpt_detect_objects_ex": (_i, [_vp, _vp, _i, _i, _d, _i, ctypes.c_uint32, _vp, _i, _vp, _vp, _vp, _vp, ctypes.POINTER(ctypes.c_int32),
                                    ctypes.POINTER(_d)]),
+    "cpt_detect_objects_batch": (_i, [_vp, _vp, _i, _i, _i, _d, ctypes.c_uint32, _i, _vp, _vp, _vp, _vp]),
+    "cpt_ir_merge_components": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _d, _vp, _vp]),
     "cpt_nlm_denoise_u8": (_i, [_vp, _vp, _i, _i, _i, _vp]),
     "cpt_ir_motion_open": (_vp, [_vp, _i, _i, _i]),
     "cpt_ir_motion_close": (None, [_vp]),
@@ -212,9 +214,9 @@ def check(rc):
 
 
 def _ptr(t):
-    """Device or host pointer of a torch tensor / numpy array / None."""
-    if t is None:
-        return None
+    """Device or host pointer of a torch tensor / numpy array / address (int) / None."""
+    if t is None or isinstance(t, int):
+        return t
     if isinstance(t, np.ndarray):
         return t.ctypes.data
     return t.data_ptr()
@@ -367,6 +369,20 @@ class Context:
                                              _ptr(d_or_mask), int(max_components), _ptr(d_labels), _ptr(d_stats), _ptr(d_centroids),
                                              _ptr(d_mask_out), ctypes.byref(n), ctypes.byref(thr)))
         return n.value, thr.value
+
+    def detect_objects_batch(self, d_frames, n_frames, width, height, threshold, steps, max_components, d_counts, d_stats, d_centroids=None,
+                             d_labels=None):
+        """detect_objects_ir for n_frames frames [n][H][W] uint8 on the device (CUDA tensors or device addresses): d_counts
+        int32 [n], d_stats int32 [n][max_components + 1][5], d_centroids float64 [n][max_components + 1][2] and d_labels
+        int32 [n][H][W] (both may be None).  Launches on the context's stream without waiting."""
+        check(self.lib.cpt_detect_objects_batch(self._h, _ptr(d_frames), int(n_frames), int(width), int(height), float(threshold), int(steps),
+                                                int(max_components), _ptr(d_counts), _ptr(d_stats), _ptr(d_centroids), _ptr(d_labels)))
+
+    def ir_merge_components(self, d_stats, d_counts, n_frames, max_components, min_mass, min_size, max_gap, d_merged, d_merged_counts):
+        """merge_components for every frame of a detect_objects_batch result: d_merged int32 [n][max_components][5],
+        d_merged_counts int32 [n] (-1: the frame's components overflowed).  Launches without waiting."""
+        check(self.lib.cpt_ir_merge_components(self._h, _ptr(d_stats), _ptr(d_counts), int(n_frames), int(max_components), int(min_mass),
+                                               int(min_size), float(max_gap), _ptr(d_merged), _ptr(d_merged_counts)))
 
     def nlm_denoise_u8(self, d_src, width, height, n_frames, d_dst):
         check(self.lib.cpt_nlm_denoise_u8(self._h, _ptr(d_src), int(width), int(height), int(n_frames), _ptr(d_dst)))

@@ -287,7 +287,8 @@ int cpt_detect_objects_u8(cpt_ctx *ctx, const uint8_t *d_image, int width, int h
  *   detect_objects_both                             imageprocessing.py:202-238  blur, threshold, CPT_DETECT_DILATE, CPT_DETECT_CLOSE,
  *                                                   d_or_mask (the thresholded saliency map, any non-zero = set) OR-ed in
  * CPT_DETECT_MASK_ONLY stops after the binary stages and writes the mask (0 / 255) to d_mask_out.  h_threshold_used (may
- * be NULL) receives the threshold applied (Otsu's when CPT_DETECT_OTSU).  Synchronises the ctx stream. */
+ * be NULL) receives the threshold applied (Otsu's when CPT_DETECT_OTSU).  For an image that is all foreground, the
+ * background row is cv2's [-1, INT_MAX, 0, 0, 0] with a NaN centroid.  Synchronises the ctx stream. */
 #define CPT_DETECT_CLOSE 1u
 #define CPT_DETECT_OPEN_GRAY 2u
 #define CPT_DETECT_DILATE 4u
@@ -296,6 +297,28 @@ int cpt_detect_objects_u8(cpt_ctx *ctx, const uint8_t *d_image, int width, int h
 int cpt_detect_objects_ex(cpt_ctx *ctx, const uint8_t *d_image, int width, int height, double threshold, int blur_ksize,
                           uint32_t steps, const uint8_t *d_or_mask, int max_components, int32_t *d_labels, int32_t *d_stats,
                           double *d_centroids, uint8_t *d_mask_out, int32_t *h_count, double *h_threshold_used);
+
+/* detect_objects_ir (imageprocessing.py:185-199) on n_frames uint8 frames [n_frames][H][W] of one geometry in one call, with
+ * no host synchronisation: steps CPT_DETECT_OPEN_GRAY (or 0) -> threshold -> connectedComponentsWithStats per frame.
+ *   d_counts     [n_frames]: cv2's label count of each frame (background included)
+ *   d_stats      [n_frames][max_components + 1][5], row 0 = background; rows beyond the frame's count are not written
+ *   d_centroids  [n_frames][max_components + 1][2] double, or NULL
+ *   d_labels     [n_frames][H][W] int32, or NULL
+ * A frame with more than max_components components reports its true count and keeps its first max_components rows in
+ * label order (its label image stays complete); the call does not fail.  Other steps return CPT_ERR_UNSUPPORTED.
+ * Launches go on the ctx stream. */
+int cpt_detect_objects_batch(cpt_ctx *ctx, const uint8_t *d_frames, int n_frames, int width, int height, double threshold,
+                             uint32_t steps, int max_components, int32_t *d_counts, int32_t *d_stats, double *d_centroids,
+                             int32_t *d_labels);
+
+/* IRTrackExtractor's rectangle merging (track/irtrackextractor.py:324-389, merge_components) for every frame of a
+ * cpt_detect_objects_batch result (d_stats, d_counts, the same max_components): keep rows with area > min_mass or with
+ * width and height > min_size, sort by area (descending, stable), merge pairs that overlap or lie closer than max_gap.
+ * The caller derives min_mass = int(40 * scale), min_size = int(16 * scale), max_gap = 40 * scale (40, 16, 40 without a
+ * scale).  d_merged [n_frames][max_components][5] (x, y, w, h, area), d_merged_counts [n_frames]: rectangles per frame,
+ * -1 for a frame whose components overflowed max_components.  Launches go on the ctx stream. */
+int cpt_ir_merge_components(cpt_ctx *ctx, const int32_t *d_stats, const int32_t *d_counts, int n_frames, int max_components,
+                            int min_mass, int min_size, double max_gap, int32_t *d_merged, int32_t *d_merged_counts);
 
 /* cv2.fastNlMeansDenoising(uint8, None) (track/cliptracker.py:116-117; h = 3, 7x7 template, 21x21 search), OpenCV's
  * integer algorithm bit for bit, on n_frames images [n_frames][H][W].  The batched extractor runs the same kernel for clips
