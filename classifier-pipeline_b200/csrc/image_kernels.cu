@@ -7,6 +7,7 @@
 #include <cfloat>
 
 #include "cptrack_internal.cuh"
+#include "resize_cv.cuh"
 
 namespace cpt {
 
@@ -56,8 +57,8 @@ __global__ void __launch_bounds__(256) normalize_kernel(const float *in, long lo
 
 // ------------------------------------------------------------------------------------------------
 // cv2.resize of an fp32 image (sw x sh) to (fw x fh), pasted at (ox, oy) into a (dw x dh) image filled with pad.
-// interpolation 1 = INTER_LINEAR (half-pixel centres, fp32 taps, horizontal then vertical, each pair as
-// fma(b - a, w, a) -- the form the x86 OpenCV 4.x build uses), 0 = INTER_NEAREST (floor(dst * src/dst)).
+// interpolation 1 = INTER_LINEAR (the measured cv2 arithmetic of resize_cv.cuh; a same-size resize is a copy, as in cv2:
+// the taps, all of weight 0, would still turn -0.0 into +0.0), 0 = INTER_NEAREST (floor(dst * src/dst)).
 __global__ void __launch_bounds__(256) resize_pad_kernel(const float *src, int sw, int sh, int fw, int fh, int ox, int oy,
                                                          int dw, int dh, float pad, int interpolation, float *dst) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -70,29 +71,14 @@ __global__ void __launch_bounds__(256) resize_pad_kernel(const float *src, int s
             const int sx = min((int)floor((double)dx * (1.0 / ((double)fw / (double)sw))), sw - 1);
             const int sy = min((int)floor((double)dy * (1.0 / ((double)fh / (double)sh))), sh - 1);
             v = __ldg(src + sy * sw + sx);
+        } else if (fw == sw && fh == sh) {
+            v = __ldg(src + dy * sw + dx);
         } else {
-            int x0, x1, y0, y1;
-            float wx, wy;
-            {
-                const double fx = ((double)dx + 0.5) * (1.0 / ((double)fw / (double)sw)) - 0.5;
-                if (sh == 1 && sw > 1) { const float ff = (float)fx, fl = floorf(ff); x0 = (int)fl; wx = __fsub_rn(ff, fl); }
-                else { const double fl = floor(fx); x0 = (int)fl; wx = (float)(fx - fl); }
-                if (x0 < 0) { x0 = 0; wx = 0.f; }
-                if (x0 >= sw - 1) { x0 = sw - 1; wx = 0.f; }
-                x1 = min(x0 + 1, sw - 1);
-            }
-            {
-                const double fy = ((double)dy + 0.5) * (1.0 / ((double)fh / (double)sh)) - 0.5;
-                if (sw == 1 && sh > 1) { const float ff = (float)fy, fl = floorf(ff); y0 = (int)fl; wy = __fsub_rn(ff, fl); }
-                else { const double fl = floor(fy); y0 = (int)fl; wy = (float)(fy - fl); }
-                if (y0 < 0) { y0 = 0; wy = 0.f; }
-                if (y0 >= sh - 1) { y0 = sh - 1; wy = 0.f; }
-                y1 = min(y0 + 1, sh - 1);
-            }
-            const float a = __ldg(src + y0 * sw + x0), b = __ldg(src + y0 * sw + x1);
-            const float c = __ldg(src + y1 * sw + x0), d = __ldg(src + y1 * sw + x1);
-            const float r0 = __fmaf_rn(__fsub_rn(b, a), wx, a), r1 = __fmaf_rn(__fsub_rn(d, c), wx, c);
-            v = __fmaf_rn(__fsub_rn(r1, r0), wy, r0);
+            const bool thin = sw == 1 || sh == 1;
+            const ResizeTaps X = linear_taps(dx, fw, sw, thin, true), Y = linear_taps(dy, fh, sh, thin, !thin);
+            const float r0 = lerp_cv(__ldg(src + Y.i0 * sw + X.i0), __ldg(src + Y.i0 * sw + X.i1), X.w, thin);
+            const float r1 = lerp_cv(__ldg(src + Y.i1 * sw + X.i0), __ldg(src + Y.i1 * sw + X.i1), X.w, thin);
+            v = lerp_cv(r0, r1, Y.w, thin);
         }
     }
     dst[i] = v;

@@ -21,6 +21,7 @@
 
 #include "cptrack_internal.cuh"
 #include "median.cuh"
+#include "resize_cv.cuh"
 
 namespace cpt {
 
@@ -247,36 +248,6 @@ __global__ void track_thermal_limits_stats_kernel(const cpt_sample *regions, con
 }
 
 // ------------------------------------------------------------------------------------------------
-struct ResizeTaps {
-    int i0, i1;
-    float w;
-};
-
-// cv2.resize INTER_LINEAR source taps for destination index d (OpenCV 4.x resizeGeneric, float path):
-// fx = (d + 0.5) * scale - 0.5 in double, sx = floor(fx), weight = float(fx - sx), clamped at both ends.
-// one_d: measured against cv2 4.13 -- a 1-D resize rounds the coordinate to fp32 before taking the fraction.
-__device__ __forceinline__ ResizeTaps linear_taps(int d, int dn, int sn, bool one_d) {
-    const double scale = 1.0 / ((double)dn / (double)sn);
-    const double fx = ((double)d + 0.5) * scale - 0.5;
-    ResizeTaps t;
-    if (one_d) {
-        const float ff = (float)fx;
-        const float fl = floorf(ff);
-        t.i0 = (int)fl;
-        t.w = __fsub_rn(ff, fl);
-    } else {
-        const double fl = floor(fx);
-        t.i0 = (int)fl;
-        t.w = (float)(fx - fl);
-    }
-    if (t.i0 < 0) { t.i0 = 0; t.w = 0.0f; }
-    if (t.i0 >= sn - 1) { t.i0 = sn - 1; t.w = 0.0f; }
-    t.i1 = min(t.i0 + 1, sn - 1);
-    return t;
-}
-
-__device__ __forceinline__ float lerp_cv(float a, float b, float w) { return __fmaf_rn(__fsub_rn(b, a), w, a); }
-
 // normalize(data, min, max, new_max=255) of imageprocessing.py:151-169 on fp32
 __device__ __forceinline__ float normalize255(float v, float mn, float mx) {
     if (mx == mn) return (mx == 0.0f) ? 0.0f : __fdiv_rn(v, mx);
@@ -328,8 +299,10 @@ __global__ void __launch_bounds__(kTileThreads) segment_tiles_kernel(const Segme
         if (r.y <= a.crop_y) oy = min(0, size - fh);
         else if (r.y + sh >= a.crop_y + a.crop_h) oy = max(size - fh, 0);
     }
-    if (tid < fw) tx[tid] = linear_taps(tid, fw, sw, sh == 1 && sw > 1);
-    if (tid >= 64 && tid - 64 < fh) ty[tid - 64] = linear_taps(tid - 64, fh, sh, sw == 1 && sh > 1);
+    // cv2.resize INTER_LINEAR (resize_cv.cuh); a same-size resize is a copy, as cv2 makes it
+    const bool thin = sw == 1 || sh == 1, copy = fw == sw && fh == sh;
+    if (tid < fw) tx[tid] = linear_taps(tid, fw, sw, thin, true);
+    if (tid >= 64 && tid - 64 < fh) ty[tid - 64] = linear_taps(tid - 64, fh, sh, thin, !thin);
 
     // (index arithmetic without divisions: i / sw by a reciprocal multiply, i / size by a shift for the usual power of two)
     const uint32_t sw_rcp = 0xffffffffu / (uint32_t)sw + 1u;  // i / sw == umulhi(i, sw_rcp) for i * sw < 2^32 (wraps to 0 for sw == 1)
@@ -351,12 +324,18 @@ __global__ void __launch_bounds__(kTileThreads) segment_tiles_kernel(const Segme
         const int dx = x - ox, dy = y - oy;
         float t = pad, f = 0.0f;
         if (dx >= 0 && dx < fw && dy >= 0 && dy < fh) {
-            const ResizeTaps X = tx[dx], Y = ty[dy];
-            const uint16_t *r0 = th + Y.i0 * a.W, *r1 = th + Y.i1 * a.W;
-            t = lerp_cv(lerp_cv((float)__ldg(r0 + X.i0), (float)__ldg(r0 + X.i1), X.w),
-                        lerp_cv((float)__ldg(r1 + X.i0), (float)__ldg(r1 + X.i1), X.w), Y.w);
-            const float *g0 = fl + Y.i0 * a.W, *g1 = fl + Y.i1 * a.W;
-            f = lerp_cv(lerp_cv(__ldg(g0 + X.i0), __ldg(g0 + X.i1), X.w), lerp_cv(__ldg(g1 + X.i0), __ldg(g1 + X.i1), X.w), Y.w);
+            if (copy) {
+                t = (float)__ldg(th + dy * a.W + dx);
+                f = __ldg(fl + dy * a.W + dx);
+            } else {
+                const ResizeTaps X = tx[dx], Y = ty[dy];
+                const uint16_t *r0 = th + Y.i0 * a.W, *r1 = th + Y.i1 * a.W;
+                t = lerp_cv(lerp_cv((float)__ldg(r0 + X.i0), (float)__ldg(r0 + X.i1), X.w, thin),
+                            lerp_cv((float)__ldg(r1 + X.i0), (float)__ldg(r1 + X.i1), X.w, thin), Y.w, thin);
+                const float *g0 = fl + Y.i0 * a.W, *g1 = fl + Y.i1 * a.W;
+                f = lerp_cv(lerp_cv(__ldg(g0 + X.i0), __ldg(g0 + X.i1), X.w, thin),
+                            lerp_cv(__ldg(g1 + X.i0), __ldg(g1 + X.i1), X.w, thin), Y.w, thin);
+            }
         }
         t = __fsub_rn(t, r.median);
         if (clip0) t = fmaxf(t, 0.0f);

@@ -20,47 +20,78 @@ INTER_NEAREST = 0
 INTER_LINEAR = 1
 
 
+def linear_taps(dn, sn, thin):
+    """Source taps of cv2.resize INTER_LINEAR along one axis for destination indices 0..dn-1: (i0, i1, w), the
+    fp32 weight w of the second tap, before any edge rule.  Two coordinate rules, measured against cv2 4.13 (x86):
+      * not thin (both source sides > 1, IPP's linear resize): f = (d + 0.5) * (sn / dn) - 0.5 in double, the
+        ratio taken directly (not as 1 / (dn / sn): that misplaces coordinates that land exactly on an integer),
+        product and difference rounded separately; i0 = floor(f), w = fp32(f - i0);
+      * thin (a source side is 1, OpenCV's own resizeGeneric_): f = fp32((d + 0.5) * (1 / (dn / sn)) - 0.5), the
+        coordinate rounded to fp32 before the floor; i0 = floor(f), w = f - i0 in fp32."""
+    d = np.arange(dn, dtype=np.float64) + 0.5
+    if thin:
+        f = (d * (1.0 / (dn / sn)) - 0.5).astype(np.float32)
+        i0 = np.floor(f).astype(np.int64)
+        w = f - i0.astype(np.float32)
+    else:
+        f = d * (sn / dn) - 0.5
+        i0 = np.floor(f).astype(np.int64)
+        w = (f - i0).astype(np.float32)
+    return i0, i0 + 1, w
+
+
+def clamp_taps(i0, i1, w, sn, zero_weight):
+    """The edge rule: taps outside [0, sn-1] are clamped; with zero_weight an index clamped at either end also
+    gets weight 0 (i0 < 0 -> (0, 1, 0); i0 >= sn-1 -> (sn-1, sn-1, 0)), without it the weight is kept."""
+    w = w.copy()
+    if zero_weight:
+        w[(i0 < 0) | (i0 >= sn - 1)] = 0
+        i0 = np.clip(i0, 0, sn - 1)
+        return i0, np.minimum(i0 + 1, sn - 1), w
+    return np.clip(i0, 0, sn - 1), np.clip(i1, 0, sn - 1), w
+
+
 def resize_linear(src, dw, dh):
-    """cv2.resize(float32, (dw, dh), INTER_LINEAR): half-pixel centres, edge clamp, fp32 weights,
-    horizontal pass then vertical pass, each tap pair combined as fma(b - a, w, a)."""
+    """cv2.resize(float32, (dw, dh), INTER_LINEAR), bit for bit with cv2 4.13 on x86 (IPP build).  Half-pixel
+    centres; horizontal pass (fp32 rows) then vertical pass.  Measured with live cv2 (tests/test_resize_cv2.py):
+      * identity (dw, dh) == (sw, sh): a copy;
+      * both source sides > 1 (IPP): taps of linear_taps(thin=False) in both directions, clamped with the weight
+        zeroed at both ends in both directions, each pair as fma(b - a, w, a) (the fp32 difference, then one fused
+        multiply-add).  One side unchanged, integer up- and downscales and exact 2x downscales all take this form:
+        there is no INTER_AREA switch for fp32 here;
+      * a source side of 1, 1x1 included (OpenCV's generic path): taps of linear_taps(thin=True); horizontally the
+        index is clamped with the weight zeroed, vertically only the row index is clamped and the weight is kept;
+        each pair as fl(a * fl(1 - w)) + fl(b * w), two rounded products and a rounded sum, no fused multiply-add.
+        So a 1-row source resized to dh rows gives rows that differ from the source row by ULPs."""
     src = np.asarray(src, np.float32)
     sh, sw = src.shape
     if (dw, dh) == (sw, sh):
         return src.copy()
-
-    def taps(dn, sn, cast_first):
-        scale = 1.0 / (dn / sn)  # OpenCV: inv_scale = dsize/ssize (double); scale = 1/inv_scale
-        f = (np.arange(dn, dtype=np.float64) + 0.5) * scale - 0.5
-        if cast_first:
-            # measured against cv2 4.13: only when the other source dimension is 1 (a 1-D resize) is the
-            # coordinate rounded to fp32 before the fraction is taken
-            f = f.astype(np.float32)
-            i0 = np.floor(f).astype(np.int64)
-            w = f - i0.astype(np.float32)
-        else:
-            i0 = np.floor(f).astype(np.int64)
-            w = (f - i0).astype(np.float32)
-        low = i0 < 0
-        i0[low] = 0
-        w[low] = 0
-        high = i0 >= sn - 1
-        i0[high] = sn - 1
-        w[high] = 0
-        i1 = np.minimum(i0 + 1, sn - 1)
-        return i0, i1, w
-
-    x0, x1, wx = taps(dw, sw, sh == 1 and sw > 1)
-    y0, y1, wy = taps(dh, sh, sw == 1 and sh > 1)
+    thin = sw == 1 or sh == 1
+    x0, x1, wx = clamp_taps(*linear_taps(dw, sw, thin), sw, zero_weight=True)
+    y0, y1, wy = clamp_taps(*linear_taps(dh, sh, thin), sh, zero_weight=not thin)
 
     def lerp(a, b, w):
-        # fma(b - a, w, a): the form the installed cv2 (4.13, x86 AVX2/IPP build) was measured to use -- bit-exact
-        # on 300/300 random aspect-preserving resizes; the fp32 difference first, then one fused multiply-add
-        # (emulated in fp64: the product of two fp32 values is exact there)
-        d = (b - a).astype(np.float64)
-        return (a.astype(np.float64) + d * w.astype(np.float64)).astype(np.float32)
+        if thin:
+            return a * (np.float32(1) - w) + b * w  # (fp32 numpy: each product and the sum rounded)
+        return fma32(b - a, np.broadcast_to(w, a.shape), a)
 
     rows = lerp(src[:, x0], src[:, x1], wx[None, :])  # (sh, dw)
     return lerp(rows[y0], rows[y1], wy[:, None])
+
+
+def fma32(x, y, z):
+    """fp32 fma(x, y, z) with one rounding, elementwise.  The product of two fp32 values is exact in fp64; the fp64
+    sum is turned into its round-to-odd value (TwoSum gives the exact error), whose rounding to fp32 is the correct
+    rounding of the exact x * y + z -- a plain fp64 sum would round twice."""
+    p = np.asarray(x, np.float32).astype(np.float64) * np.asarray(y, np.float32).astype(np.float64)
+    z = np.asarray(z, np.float32).astype(np.float64)
+    s = p + z
+    t = s - p
+    err = (p - (s - t)) + (z - t)
+    even = (s.view(np.int64) & 1) == 0
+    s = np.where((err != 0) & even, np.nextafter(s, np.where(err > 0, np.inf, -np.inf)), s)
+    return s.astype(np.float32)
 
 
 def resize_nearest(src, dw, dh):

@@ -91,12 +91,12 @@ def test_resize_helpers_match_oracle():
         region = Rectangle(x, y, w, h)
         got = ip.resize_and_pad(src, (32, 32), region, crop, keep_edge=True)
         ref = po.resize_and_pad(src, (32, 32), (x, y, w, h), (1, 1, 158, 118), keep_edge=True)
-        np.testing.assert_allclose(got, ref, rtol=1e-6, atol=1e-4)
+        assert np.array_equal(got, ref)
         got = ip.resize_and_pad(src, (32, 32), region, crop, keep_edge=True, pad=0, interpolation=ip.INTER_NEAREST)
         ref = po.resize_and_pad(src, (32, 32), (x, y, w, h), (1, 1, 158, 118), keep_edge=True, pad=0, interpolation=po.INTER_NEAREST)
         assert np.array_equal(got, ref)
         dw, dh = int(rng.integers(1, 40)), int(rng.integers(1, 40))
-        np.testing.assert_allclose(ip.resize_cv(src, (dw, dh)), po.resize_linear(src, dw, dh), rtol=1e-6, atol=1e-4)
+        assert np.array_equal(ip.resize_cv(src, (dw, dh)), po.resize_linear(src, dw, dh))
 
 
 def test_preprocess_frame_single_matches_oracle():
@@ -126,11 +126,11 @@ def test_preprocess_frame_single_matches_oracle():
         out = preprocess_frame(fr, (32, 32), Region(20 + t, 30, 24, 18), None, crop, calculate_filtered=False,
                                filtered_norm_limits=(lo, hi), median=np.median(pix[t]), clip_thermals_at_zero=clip_zero)
         r, c = divmod(i, 5)
-        np.testing.assert_allclose(out.thermal, oracle[r * 32 : (r + 1) * 32, c * 32 : (c + 1) * 32, 0], rtol=1e-6, atol=1e-4)
-        np.testing.assert_allclose(out.filtered, oracle[r * 32 : (r + 1) * 32, c * 32 : (c + 1) * 32, 1], rtol=1e-6, atol=1e-4)
+        assert np.array_equal(out.thermal, oracle[r * 32 : (r + 1) * 32, c * 32 : (c + 1) * 32, 0])
+        assert np.array_equal(out.filtered, oracle[r * 32 : (r + 1) * 32, c * 32 : (c + 1) * 32, 1])
         frames.append(out)
     tiled = preprocess_movement(frames, 5, 32, ["thermal", "filtered"])
-    np.testing.assert_allclose(tiled, oracle, rtol=1e-6, atol=1e-4)
+    assert np.array_equal(tiled, oracle)
 
 
 def test_nlm_denoise_matches_oracle_and_reference_fixture():

@@ -101,7 +101,7 @@ def test_tiling_matches_oracle(dev, fs, sw):
             for regions, segs in tracks:
                 want = po.preprocess_track(thermal, filtered, regions, crop, segs, dim=(fs, fs), frames_per_row=sw, seed=77,
                                            diff_norm=diff_norm)
-                np.testing.assert_allclose(got[at : at + len(segs)], want, rtol=1e-6, atol=1e-4)
+                np.testing.assert_array_equal(got[at : at + len(segs)], want)
                 at += len(segs)
             assert got.shape == bp.output_shape(at) == (at, sw * fs, sw * fs, 2)
             # the flat track: thermal all zero after the median (mx == mn == 0), filtered constant (data / max)
@@ -125,7 +125,7 @@ def test_inc3_at_a_non_default_size(dev):
     at = 0
     for regions, segs in tracks:
         want = po.preprocess_track(thermal, filtered, regions, CROP, segs, dim=(fs, fs), frames_per_row=sw, seed=5, preprocess_fn="inc3")
-        np.testing.assert_allclose(got[at : at + len(segs)], want, rtol=1e-6, atol=1e-4)
+        np.testing.assert_array_equal(got[at : at + len(segs)], want)
         at += len(segs)
     assert at == len(got)
 
@@ -169,8 +169,8 @@ def test_interpreter_square_width_4_frame_size_48_matches_oracle():
         want = po.preprocess_track(thermal, filtered, regions, crop, [s.frame_indices for s in segments], dim=(48, 48), frames_per_row=4,
                                    seed=1234)
         assert got.shape == got_clips_data.shape == (len(segments), 192, 192, 2)
-        np.testing.assert_allclose(got, want, rtol=1e-6, atol=1e-4)
-        np.testing.assert_allclose(got_clips_data, want, rtol=1e-6, atol=1e-4)
+        np.testing.assert_array_equal(got, want)
+        np.testing.assert_array_equal(got_clips_data, want)
         n_checked += len(segments)
     assert n_checked
 
