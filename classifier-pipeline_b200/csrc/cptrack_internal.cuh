@@ -125,5 +125,6 @@ struct cpt_ctx {
     cpt::Grow<int32_t> cptv_scratch;  // cpt_cptv_decode: the decoder's change images
     cpt::Grow<uint8_t> detect_scratch;  // cpt_detect_objects_ex / _batch: images, masks, union-find and component tables
     cpt::Grow<int> merge_order;  // cpt_ir_merge_components: list order of every frame of a launch
+    cpt::Grow<uint8_t> motion_scratch;  // cpt_motion_clips: detector records, steps, mean rows, results, ring copies
 };
 

@@ -8,6 +8,7 @@
 //            (cptvmotiondetector.py:74-120), with the optional second delta ring (one_diff_only False)
 // The frame ring, the sum and the delta ring live in HBM for the life of the detector.
 #include <cstring>
+#include <vector>
 
 #include "background_step.cuh"
 #include "cptrack_internal.cuh"
@@ -56,26 +57,34 @@ __global__ void __launch_bounds__(256) motion_mean_init_kernel(const uint16_t *r
     if (i == 0) *mean_count = n;
 }
 
-__global__ void __launch_bounds__(1024, 1) motion_step_kernel(const MotionArgs a) {
-    __shared__ unsigned long long red_sum[32];
-    __shared__ int red_changed;
-    __shared__ int red_count[32];
-    __shared__ int s_error;
-    const Geometry &g = a.g;
+struct MotionShared {
+    unsigned long long red_sum[32];
+    int red_changed;
+    int red_count[32];
+    int error;
+};
+
+// One process_frame on the device: the three phases of the file comment for one frame.  `cur`, `old` (the ring's
+// oldest frame, read when the running mean is full) and `nonffc` (the oldest non-FFC frame, read with
+// CPT_MOTION_DETECT) may come from the ring or from a staged frame array.  `n` is RunningMean.running_mean_frames
+// before the step; the new count is returned to every thread.  Every thread of the CTA must call; thread 0 writes
+// *result.  Ends with a barrier, so a CTA may run steps back to back.
+__device__ __forceinline__ int motion_phases(const Geometry &g, const uint16_t *cur, const uint16_t *old, const uint16_t *nonffc,
+                                             uint32_t *sum, int n, int mean_frames, double *diff, int diff_slot_new,
+                                             int diff_slot_old, uint8_t *bg_state, const WeightTable &wt, uint32_t flags,
+                                             int delta_thresh, double init_average, MotionShared &sh,
+                                             cpt_motion_result *result) {
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const uint16_t *cur = a.ring + (size_t)a.slot_new * g.npx;
-    if (tid == 0) s_error = 0;
+    if (tid == 0) sh.error = 0;
     __syncthreads();
 
     // ---- phase 1: running mean
-    int n = *a.mean_count;
-    if (a.flags & CPT_MOTION_MEAN) {
-        const bool restart = (a.flags & CPT_MOTION_MEAN_RESTART) || n == 0;
-        const bool full = !restart && n == a.mean_frames;
-        const uint16_t *old = a.ring + (size_t)(a.slot_oldest < 0 ? a.slot_new : a.slot_oldest) * g.npx;
+    if (flags & CPT_MOTION_MEAN) {
+        const bool restart = (flags & CPT_MOTION_MEAN_RESTART) || n == 0;
+        const bool full = !restart && n == mean_frames;
         for (int i = tid; i < g.npx / 2; i += blockDim.x) {
             const uint32_t c2 = reinterpret_cast<const uint32_t *>(cur)[i];
-            uint2 s = reinterpret_cast<uint2 *>(a.sum)[i];
+            uint2 s = reinterpret_cast<uint2 *>(sum)[i];
             if (restart) {
                 s.x = c2 & 0xffffu;
                 s.y = c2 >> 16;
@@ -88,39 +97,37 @@ __global__ void __launch_bounds__(1024, 1) motion_step_kernel(const MotionArgs a
                 s.x += c2 & 0xffffu;
                 s.y += c2 >> 16;
             }
-            reinterpret_cast<uint2 *>(a.sum)[i] = s;
+            reinterpret_cast<uint2 *>(sum)[i] = s;
         }
         n = restart ? 1 : (full ? n : n + 1);
     }
     __syncthreads();
-    if (tid == 0) *a.mean_count = n;
 
     // ---- phase 2: background from the running mean (np.int32(sum / n): truncation == floor division here)
-    if ((a.flags & CPT_MOTION_BACKGROUND) && n > 0) {
-        const uint32_t *S = a.sum;
+    if ((flags & CPT_MOTION_BACKGROUND) && n > 0) {
+        const uint32_t *S = sum;
         const uint32_t un = (uint32_t)n;
-        int *err = &s_error;
-        background_step(g, a.bg_state, [S, un, err](int p) {
+        int *err = &sh.error;
+        background_step(g, bg_state, [S, un, err](int p) {
             const uint32_t v = S[p] / un;
             if (v > 65535u) { *err = 1; return 65535; }
             return (int)v;
-        }, a.wt, red_sum, &red_changed);
+        }, wt, sh.red_sum, &sh.red_changed);
     }
 
     // ---- phase 3: motion count against the oldest non-FFC frame
     int count = 0;
-    const StateHeader *bg_hdr = reinterpret_cast<const StateHeader *>(a.bg_state);
-    const double T = bg_hdr->initialised ? bg_hdr->average : a.init_average;
-    if (a.flags & CPT_MOTION_DETECT) {
-        const uint16_t *old = a.ring + (size_t)a.slot_nonffc * g.npx;
-        const double dt = (double)a.delta_thresh;
-        const bool warmer = a.flags & CPT_MOTION_WARMER_ONLY, one = a.flags & CPT_MOTION_ONE_DIFF;
-        double *dnew = a.diff ? a.diff + (size_t)a.diff_slot_new * g.ncrop : nullptr;
-        const double *dold = (a.diff && a.diff_slot_old >= 0) ? a.diff + (size_t)a.diff_slot_old * g.ncrop : nullptr;
+    const StateHeader *bg_hdr = reinterpret_cast<const StateHeader *>(bg_state);
+    const double T = bg_hdr->initialised ? bg_hdr->average : init_average;
+    if (flags & CPT_MOTION_DETECT) {
+        const double dt = (double)delta_thresh;
+        const bool warmer = flags & CPT_MOTION_WARMER_ONLY, one = flags & CPT_MOTION_ONE_DIFF;
+        double *dnew = diff ? diff + (size_t)diff_slot_new * g.ncrop : nullptr;
+        const double *dold = (diff && diff_slot_old >= 0) ? diff + (size_t)diff_slot_old * g.ncrop : nullptr;
         for (int i = tid; i < g.ncrop; i += blockDim.x) {
             const int y = i / g.crop_w + g.edge, x = i - (y - g.edge) * g.crop_w + g.edge;
             const int p = y * g.W + x;
-            double d = fmax((double)cur[p], T) - fmax((double)old[p], T);
+            double d = fmax((double)cur[p], T) - fmax((double)nonffc[p], T);
             if (!warmer) d = fabs(d);
             if (one) {
                 count += d > dt;
@@ -132,19 +139,88 @@ __global__ void __launch_bounds__(1024, 1) motion_step_kernel(const MotionArgs a
         }
     }
     count = __reduce_add_sync(0xffffffffu, count);
-    if (lane == 0) red_count[warp] = count;
+    if (lane == 0) sh.red_count[warp] = count;
     __syncthreads();
     if (tid == 0) {
         int total = 0;
-        for (int w = 0; w < (int)(blockDim.x >> 5); ++w) total += red_count[w];
+        for (int w = 0; w < (int)(blockDim.x >> 5); ++w) total += sh.red_count[w];
         cpt_motion_result r;
         r.average = T;
         r.diff = total;
-        r.error = s_error;
+        r.error = sh.error;
         r.mean_frames = n;
         r.reserved = 0;
-        *a.result = r;
+        *result = r;
     }
+    __syncthreads();
+    return n;
+}
+
+__global__ void __launch_bounds__(1024, 1) motion_step_kernel(const MotionArgs a) {
+    __shared__ MotionShared sh;
+    const size_t npx = a.g.npx;
+    const uint16_t *cur = a.ring + (size_t)a.slot_new * npx;
+    const uint16_t *old = a.ring + (size_t)(a.slot_oldest < 0 ? a.slot_new : a.slot_oldest) * npx;
+    const uint16_t *nonffc = a.slot_nonffc < 0 ? nullptr : a.ring + (size_t)a.slot_nonffc * npx;
+    const int n = motion_phases(a.g, cur, old, nonffc, a.sum, *a.mean_count, a.mean_frames, a.diff, a.diff_slot_new,
+                                a.diff_slot_old, a.bg_state, a.wt, a.flags, a.delta_thresh, a.init_average, sh, a.result);
+    if (threadIdx.x == 0) *a.mean_count = n;
+}
+
+// Per detector of a cpt_motion_clips launch.
+struct MotionClipArgs {
+    uint16_t *ring;
+    uint32_t *sum;
+    double *diff;
+    int32_t *mean_count;
+    uint8_t *bg_state;
+    WeightTable wt;
+    double init_average;
+    int delta_thresh, mean_frames, first_step, n_steps;
+};
+
+// A frame reference of cpt_motion_clip_step: row r >= 0 of the staged frames, or ring slot -1 - r as it stood before
+// the launch (the ring is refreshed only after this kernel, by motion_ring_gather_kernel).
+__device__ __forceinline__ const uint16_t *motion_frame(const uint16_t *frames, const uint16_t *ring, int npx, int ref) {
+    return ref >= 0 ? frames + (size_t)ref * npx : ring + (size_t)(-1 - ref) * npx;
+}
+
+// cpt_motion_clips: one CTA per detector walks that detector's steps in order, one cpt_motion_result per step.
+__global__ void __launch_bounds__(1024, 1) motion_clips_kernel(const Geometry g, const MotionClipArgs *clips,
+                                                               const cpt_motion_clip_step *steps, const int32_t *mean_rows,
+                                                               const uint16_t *frames, cpt_motion_result *results) {
+    __shared__ MotionShared sh;
+    const MotionClipArgs c = clips[blockIdx.x];
+    int n = *c.mean_count;
+    for (int s = c.first_step; s < c.first_step + c.n_steps; ++s) {
+        const cpt_motion_clip_step st = steps[s];
+        if (st.mean_count > 0) {  // RunningMean(frames, window) (motiondetector.py:161-164) before this step
+            for (int i = threadIdx.x; i < g.npx; i += blockDim.x) {
+                uint32_t v = 0;
+                for (int k = 0; k < st.mean_count; ++k) v += motion_frame(frames, c.ring, g.npx, mean_rows[st.mean_first + k])[i];
+                c.sum[i] = v;
+            }
+            n = st.mean_count;
+            __syncthreads();
+        }
+        n = motion_phases(g, motion_frame(frames, c.ring, g.npx, st.frame), motion_frame(frames, c.ring, g.npx, st.oldest),
+                          (st.flags & CPT_MOTION_DETECT) ? motion_frame(frames, c.ring, g.npx, st.nonffc) : nullptr, c.sum, n, c.mean_frames, c.diff, st.diff_slot_new,
+                          st.diff_slot_old, c.bg_state, c.wt, st.flags, c.delta_thresh, c.init_average, sh, results + s);
+    }
+    if (threadIdx.x == 0) *c.mean_count = n;
+}
+
+struct RingCopy {
+    uint16_t *dst;
+    int64_t row;
+};
+
+// After motion_clips_kernel: each listed ring slot takes the staged frame the per-frame loop would have left there.
+__global__ void __launch_bounds__(256) motion_ring_gather_kernel(const RingCopy *copies, const uint16_t *frames, int npx) {
+    const RingCopy c = copies[blockIdx.x];
+    const uint32_t *src = reinterpret_cast<const uint32_t *>(frames + c.row * npx);
+    uint32_t *dst = reinterpret_cast<uint32_t *>(c.dst);
+    for (int i = threadIdx.x; i < npx / 2; i += blockDim.x) dst[i] = src[i];
 }
 
 }  // namespace cpt
@@ -271,6 +347,85 @@ int cpt_motion_step(cpt_motion *m, const uint16_t *h_pix, void *d_background_sta
     CUDA_TRY(cudaStreamSynchronize(c->stream));
     *h_result = *m->h_result;
     if (h_result->error) return fail(CPT_ERR_INVALID, "running mean left the uint16 range (inconsistent ring / mean window)");
+    return CPT_OK;
+}
+
+int cpt_motion_clips(cpt_ctx *c, const cpt_motion_clip *h_clips, int n, const uint16_t *d_frames, int64_t n_frames,
+                     const cpt_motion_clip_step *h_steps, int n_steps, const int32_t *h_mean_rows, int n_mean_rows,
+                     cpt_motion_result *h_results) {
+    if (!c || n < 0 || n_frames < 0 || n_steps < 0 || n_mean_rows < 0) return fail(CPT_ERR_INVALID, "cpt_motion_clips: bad argument");
+    if ((n && !h_clips) || (n_frames && !d_frames) || (n_steps && (!h_steps || !h_results)) || (n_mean_rows && !h_mean_rows))
+        return fail(CPT_ERR_INVALID, "cpt_motion_clips: null argument");
+    std::vector<cpt::MotionClipArgs> args(n);
+    std::vector<cpt::RingCopy> copies;
+    for (int d = 0; d < n; ++d) {
+        const cpt_motion_clip &k = h_clips[d];
+        const cpt_motion *m = k.m;
+        if (!m || m->ctx != c) return fail(CPT_ERR_INVALID, "cpt_motion_clips: detector %d does not belong to this context", d);
+        if (!k.d_background_state) return fail(CPT_ERR_INVALID, "cpt_motion_clips: detector %d has no background state", d);
+        if (!c->tables[m->weight_slot].d_thr) return fail(CPT_ERR_INVALID, "weight table slot %d is not set", m->weight_slot);
+        for (int e = 0; e < d; ++e)
+            if (h_clips[e].m == m || h_clips[e].d_background_state == k.d_background_state)
+                return fail(CPT_ERR_INVALID, "cpt_motion_clips: detectors %d and %d share a handle or a state record", e, d);
+        if (k.first_step < 0 || k.n_steps < 0 || k.n_steps > n_steps - k.first_step)
+            return fail(CPT_ERR_INVALID, "cpt_motion_clips: detector %d: steps out of range", d);
+        auto ref_ok = [&](int32_t r) { return r >= 0 ? r < n_frames : -1 - (int64_t)r < m->ring_frames; };
+        for (int i = k.first_step; i < k.first_step + k.n_steps; ++i) {
+            const cpt_motion_clip_step &st = h_steps[i];
+            if (!ref_ok(st.frame) || !ref_ok(st.oldest)) return fail(CPT_ERR_INVALID, "step %d: frame reference out of range", i);
+            if (st.flags & CPT_MOTION_DETECT) {
+                if (!ref_ok(st.nonffc)) return fail(CPT_ERR_INVALID, "step %d: oldest non-FFC reference out of range", i);
+                if (!(st.flags & CPT_MOTION_ONE_DIFF)) {
+                    if (!m->d_diff) return fail(CPT_ERR_INVALID, "step %d: the detector was opened without a delta ring", i);
+                    if (st.diff_slot_new < 0 || st.diff_slot_new >= m->diff_frames || st.diff_slot_old >= m->diff_frames)
+                        return fail(CPT_ERR_INVALID, "step %d: delta ring slot out of range", i);
+                }
+            }
+            if (st.mean_count < 0 || st.mean_count > m->mean_frames || st.mean_first < 0 || st.mean_count > n_mean_rows - st.mean_first)
+                return fail(CPT_ERR_INVALID, "step %d: mean rows out of range", i);
+            for (int j = 0; j < st.mean_count; ++j)
+                if (!ref_ok(h_mean_rows[st.mean_first + j])) return fail(CPT_ERR_INVALID, "step %d: mean frame reference out of range", i);
+        }
+        for (int s = 0; k.ring_rows && s < m->ring_frames; ++s) {
+            const int32_t r = k.ring_rows[s];
+            if (r < -1 || r >= n_frames) return fail(CPT_ERR_INVALID, "detector %d: ring row out of range", d);
+            if (r >= 0) copies.push_back({m->d_ring + (size_t)s * c->g.npx, r});
+        }
+        cpt::MotionClipArgs &a = args[d];
+        a.ring = m->d_ring; a.sum = m->d_sum; a.diff = m->d_diff; a.mean_count = m->d_mean_count;
+        a.bg_state = (uint8_t *)k.d_background_state;
+        a.wt = c->tables[m->weight_slot].device();
+        a.init_average = k.init_average;
+        a.delta_thresh = k.delta_thresh; a.mean_frames = m->mean_frames;
+        a.first_step = k.first_step; a.n_steps = k.n_steps;
+    }
+    if (n == 0) return CPT_OK;
+    CUDA_TRY(cudaSetDevice(c->device));
+    // one scratch block: detector records | steps | mean rows | results | ring copies, each 256-byte aligned
+    auto up = [](size_t b) { return (b + 255) & ~(size_t)255; };
+    const size_t o_steps = up(sizeof(cpt::MotionClipArgs) * n), o_mean = o_steps + up(sizeof(cpt_motion_clip_step) * n_steps),
+                 o_res = o_mean + up(sizeof(int32_t) * n_mean_rows), o_copy = o_res + up(sizeof(cpt_motion_result) * n_steps),
+                 total = o_copy + up(sizeof(cpt::RingCopy) * copies.size());
+    CUDA_TRY(c->motion_scratch.ensure(total));
+    uint8_t *base = c->motion_scratch;
+    auto *d_args = reinterpret_cast<cpt::MotionClipArgs *>(base);
+    auto *d_steps = reinterpret_cast<cpt_motion_clip_step *>(base + o_steps);
+    auto *d_mean = reinterpret_cast<int32_t *>(base + o_mean);
+    auto *d_res = reinterpret_cast<cpt_motion_result *>(base + o_res);
+    auto *d_copy = reinterpret_cast<cpt::RingCopy *>(base + o_copy);
+    CUDA_TRY(cudaMemcpyAsync(d_args, args.data(), sizeof(cpt::MotionClipArgs) * n, cudaMemcpyHostToDevice, c->stream));
+    if (n_steps) CUDA_TRY(cudaMemcpyAsync(d_steps, h_steps, sizeof(cpt_motion_clip_step) * n_steps, cudaMemcpyHostToDevice, c->stream));
+    if (n_mean_rows) CUDA_TRY(cudaMemcpyAsync(d_mean, h_mean_rows, sizeof(int32_t) * n_mean_rows, cudaMemcpyHostToDevice, c->stream));
+    if (!copies.empty())
+        CUDA_TRY(cudaMemcpyAsync(d_copy, copies.data(), sizeof(cpt::RingCopy) * copies.size(), cudaMemcpyHostToDevice, c->stream));
+    cpt::motion_clips_kernel<<<n, 1024, 0, c->stream>>>(c->g, d_args, d_steps, d_mean, d_frames, d_res);
+    CUDA_TRY(cudaGetLastError());
+    if (!copies.empty()) {  // stream order: the ring changes only after every step has read it
+        cpt::motion_ring_gather_kernel<<<(unsigned)copies.size(), 256, 0, c->stream>>>(d_copy, d_frames, c->g.npx);
+        CUDA_TRY(cudaGetLastError());
+    }
+    if (n_steps) CUDA_TRY(cudaMemcpyAsync(h_results, d_res, sizeof(cpt_motion_result) * n_steps, cudaMemcpyDeviceToHost, c->stream));
+    CUDA_TRY(cudaStreamSynchronize(c->stream));  // the host vectors above and the scratch block are free again
     return CPT_OK;
 }
 

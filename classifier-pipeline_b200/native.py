@@ -73,6 +73,18 @@ class CptMotionResult(ctypes.Structure):
                 ("mean_frames", ctypes.c_int32), ("reserved", ctypes.c_int32)]
 
 
+class CptMotionClipStep(ctypes.Structure):
+    _fields_ = [("frame", ctypes.c_int32), ("oldest", ctypes.c_int32), ("nonffc", ctypes.c_int32), ("diff_slot_new", ctypes.c_int32),
+                ("diff_slot_old", ctypes.c_int32), ("mean_first", ctypes.c_int32), ("mean_count", ctypes.c_int32),
+                ("flags", ctypes.c_uint32)]
+
+
+class CptMotionClip(ctypes.Structure):
+    _fields_ = [("m", ctypes.c_void_p), ("d_background_state", ctypes.c_void_p), ("ring_rows", ctypes.c_void_p),
+                ("init_average", ctypes.c_double), ("delta_thresh", ctypes.c_int32), ("first_step", ctypes.c_int32),
+                ("n_steps", ctypes.c_int32), ("reserved", ctypes.c_int32)]
+
+
 class CptMog2Params(ctypes.Structure):
     _fields_ = [("history", ctypes.c_int), ("var_threshold", ctypes.c_double), ("background_ratio", ctypes.c_double),
                 ("var_threshold_gen", ctypes.c_float), ("var_init", ctypes.c_float), ("var_min", ctypes.c_float),
@@ -118,6 +130,7 @@ assert TRACK_NORM_DTYPE.itemsize == ctypes.sizeof(CptTrackNorm) == 32
 assert REGION_DTYPE.itemsize == ctypes.sizeof(CptRegion) == 40
 assert INFO_DTYPE.itemsize == ctypes.sizeof(CptFrameInfo) == 64
 assert CLIP_DTYPE.itemsize == ctypes.sizeof(CptClip) == 48
+assert ctypes.sizeof(CptMotionClipStep) == 32 and ctypes.sizeof(CptMotionClip) == 48
 
 # every symbol include/cptrack.h declares: (name, restype, argtypes)
 _vp, _i, _i64, _u64, _d, _f = ctypes.c_void_p, ctypes.c_int, ctypes.c_int64, ctypes.c_uint64, ctypes.c_double, ctypes.c_float
@@ -181,6 +194,7 @@ SYMBOLS = {
     "cpt_motion_store": (_i, [_vp, _vp, _i]),
     "cpt_motion_mean_init": (_i, [_vp, _vp, _i]),
     "cpt_motion_step": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _i, ctypes.c_uint32, _i, _d, ctypes.POINTER(CptMotionResult)]),
+    "cpt_motion_clips": (_i, [_vp, _vp, _i, _vp, _i64, _vp, _i, _vp, _i, _vp]),
     "cpt_state_read": (_i, [_vp, _vp, _i, _vp, _vp, ctypes.POINTER(_d), _vp, ctypes.POINTER(ctypes.c_int32)]),
     "cpt_state_write": (_i, [_vp, _vp, _i, _vp, _vp, _d]),
     "cpt_weight_value": (_d, [_vp, _i, _i]),

@@ -380,6 +380,40 @@ int cpt_motion_step(cpt_motion *m, const uint16_t *h_pix, void *d_background_sta
                     int slot_nonffc, int diff_slot_new, int diff_slot_old, uint32_t flags, int delta_thresh,
                     double init_average, cpt_motion_result *h_result);
 
+/* Whole recordings, many detectors, one launch (cptvmotiondetector.py:135-205, motiondetector.py:160-244 for every frame
+ * of each detector's frame list): the host plans every frame with the same ring bookkeeping as cpt_motion_step's caller,
+ * and one CTA per detector then runs that detector's steps in order.  d_frames is [n_frames][H][W] uint16 in device
+ * memory.  A frame reference r >= 0 is row r of d_frames; r < 0 is slot -1 - r of the detector's ring as it stood before
+ * the call (a detector resumed after streaming).  After the steps, each ring slot with ring_rows[slot] >= 0 takes that
+ * row, so the ring holds what the per-frame calls would have left; the running sum, the delta ring and the background
+ * state record are updated in place as by those calls.  Every detector must belong to ctx and appear once, with its own
+ * state record.  Every index (frame references, delta-ring slots, mean rows, ring_rows, step ranges) is checked before
+ * anything is launched: CPT_ERR_INVALID.  h_results[i] is step i's result as cpt_motion_step returns it; a step whose
+ * running mean left the uint16 range has error = 1 (the call itself returns CPT_OK). */
+typedef struct {
+    int32_t frame;          /* the new frame (SlidingWindow.current after add) */
+    int32_t oldest;         /* SlidingWindow.oldest after the add */
+    int32_t nonffc;         /* SlidingWindow.oldest_nonffc; read with CPT_MOTION_DETECT only */
+    int32_t diff_slot_new;  /* delta ring slots as in cpt_motion_step (CPT_MOTION_DETECT without CPT_MOTION_ONE_DIFF) */
+    int32_t diff_slot_old;
+    int32_t mean_first;     /* mean_count > 0: RunningMean(frames) from h_mean_rows[mean_first .. mean_first + mean_count) */
+    int32_t mean_count;     /*   before this step (at most the detector's mean_frames), as cpt_motion_mean_init */
+    uint32_t flags;         /* CPT_MOTION_* */
+} cpt_motion_clip_step;
+typedef struct {
+    cpt_motion *m;
+    void *d_background_state;  /* the detector's WeightedBackground state record */
+    const int32_t *ring_rows;  /* host [ring_frames]: row of d_frames each ring slot holds afterwards, -1 = unchanged; NULL = none */
+    double init_average;       /* as cpt_motion_step */
+    int32_t delta_thresh;
+    int32_t first_step;        /* this detector's steps: h_steps[first_step .. first_step + n_steps) */
+    int32_t n_steps;
+    int32_t reserved;
+} cpt_motion_clip;
+int cpt_motion_clips(cpt_ctx *ctx, const cpt_motion_clip *h_clips, int n, const uint16_t *d_frames, int64_t n_frames,
+                     const cpt_motion_clip_step *h_steps, int n_steps, const int32_t *h_mean_rows, int n_mean_rows,
+                     cpt_motion_result *h_results);
+
 /* ---- IRMotionDetector (piclassifier/irmotiondetector.py:55-153), streaming, 640x480 BGR frames ----
  * Per frame the reference does cv2.cvtColor(BGR2GRAY), feeds the grey frame to its background model (OpenCV's MOG2, on the
  * host through cv2 or on the device through cpt_mog2 below), then absdiff(oldest grey, grey) -> threshold 12 -> erode with a
