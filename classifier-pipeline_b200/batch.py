@@ -317,13 +317,14 @@ class BatchPreprocessor:
             d_lim_rows = torch.from_numpy(row_map[limit_regions["frame"]]).to(self.device)
             d_smp_rows = torch.from_numpy(row_map[samples["frame"]]).to(self.device)
         # (always resets the rows)
-        ctx.preprocess_limits_ex(d_filtered, d_lim_rows, d_lim, n_lim if self.diff_norm else 0, d_tracks, n_tracks)
+        ctx.preprocess_limits(d_filtered, d_lim, n_lim if self.diff_norm else 0, d_tracks, n_tracks, d_filtered_rows=d_lim_rows)
         if self.thermal_diff_norm:
-            ctx.preprocess_thermal_limits_ex(d_thermal, d_lim_rows, d_lim, n_lim, d_tracks, n_tracks, frame_medians, frame_info)
-        ctx.preprocess_medians_ex(d_thermal, frame_medians, d_smp, n_smp, d_tracks)
+            ctx.preprocess_thermal_limits(d_thermal, d_lim, n_lim, d_tracks, n_tracks, d_filtered_rows=d_lim_rows,
+                                          d_frame_medians=frame_medians, d_frame_info=frame_info)
+        ctx.preprocess_medians(d_thermal, d_smp, n_smp, d_tracks, d_frame_medians=frame_medians)
         fn = int(self.preprocess_fn) | (0 if self.diff_norm else native.PREPROCESS_PER_TILE)
-        ctx.preprocess_segments_ex(d_thermal, d_filtered, d_smp_rows, d_smp, d_tracks, d_seg, n_seg, launched, self.frames_per_row,
-                                   self.frame_size, crop_rectangle, fn, d_out)
+        ctx.preprocess_segments(d_thermal, d_filtered, d_smp, d_tracks, d_seg, n_seg, launched, self.frames_per_row, self.frame_size,
+                                crop_rectangle, fn, d_out, d_filtered_rows=d_smp_rows)
         return dict(segments=d_out, tracks=d_tracks, samples=d_smp)
 
     def run(self, d_thermal, d_filtered, tracks, crop_rectangle, seed=None, out=None, row_map=None, frame_medians=None, frame_info=None):

@@ -321,21 +321,6 @@ int cpt_debug_force_single_kernel(cpt_ctx *c, int enable) {
     return CPT_OK;
 }
 
-int cpt_debug_kernel_times(cpt_ctx *c, int enable, float *h_ms4) {
-    if (!c) return fail(CPT_ERR_INVALID, "null ctx");
-    CUDA_TRY(cudaSetDevice(c->device));
-    float ms5[5];
-    int rc = cpt_debug_kernel_times_ex(c, enable, h_ms4 ? ms5 : nullptr, 5);
-    if (rc) return rc;
-    if (h_ms4) {
-        h_ms4[0] = ms5[0];
-        h_ms4[1] = ms5[1] + ms5[2];
-        h_ms4[2] = ms5[3];
-        h_ms4[3] = ms5[4];
-    }
-    return CPT_OK;
-}
-
 int cpt_debug_kernel_times_ex(cpt_ctx *c, int enable, float *h_ms, int n) {
     if (!c) return fail(CPT_ERR_INVALID, "null ctx");
     if (h_ms && (n < 1 || n > 5)) return fail(CPT_ERR_INVALID, "n must be in [1,5]");

@@ -91,7 +91,7 @@ struct cpt_ctx {
     int num_sms = 0;
     cpt::HostWeightTable tables[4];
     bool force_single = false;  // cpt_debug_force_single_kernel
-    bool time_kernels = false;  // cpt_debug_kernel_times
+    bool time_kernels = false;  // cpt_debug_kernel_times_ex
     bool timed_valid = false;
     cudaEvent_t ev_k[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
     int *work_counter = nullptr;
@@ -123,7 +123,7 @@ struct cpt_ctx {
     cpt::Grow<int32_t, true> pk_h_first[2];  // packed host-staged call: the same, on the host
     cpt::Grow<int32_t> pk_change;  // packed host-staged call: the decoder's change images
     cpt::Grow<int32_t> cptv_scratch;  // cpt_cptv_decode: the decoder's change images
-    cpt::Grow<uint8_t> detect_scratch;  // cpt_detect_objects_ex / _batch: images, masks, union-find and component tables
+    cpt::Grow<uint8_t> detect_scratch;  // cpt_detect_objects / _batch: images, masks, union-find and component tables
     cpt::Grow<int> merge_order;  // cpt_ir_merge_components: list order of every frame of a launch
     cpt::Grow<uint8_t> motion_scratch;  // cpt_motion_clips: detector records, steps, mean rows, results, ring copies
 };

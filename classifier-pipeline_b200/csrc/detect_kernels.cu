@@ -2,8 +2,6 @@
 // and detect_objects_ir for a batch of frames of one geometry (the extraction kernel fuses the same steps for 160x120 clips
 // in shared memory; this is the stand-alone primitive, also the building block for the 640x480 IR frames of SURVEY.md
 // section 8f-4):
-//   blur_threshold_kernel   cv2.GaussianBlur(u8, (5,5), 0): (sum k_i k_j U + 128) >> 8, BORDER_REFLECT_101, then
-//                           cv2.threshold: U > floor(thresh)
 //   close_init_kernel       cv2.morphologyEx(MORPH_CLOSE, <tuple>): the tuple becomes a 2x1 element, i.e.
 //                           C[y] = M[y-1] | (M[y] & M[y-2]), C[0] = C[1] = M[0]; seeds the union-find
 //   merge / flatten         8-connected label equivalence in global memory (union by smaller index, atomicMin); flatten
@@ -63,29 +61,6 @@ __device__ __forceinline__ size_t frame_off(size_t per_frame) { return (size_t)b
 __host__ __device__ __forceinline__ int key_words(int W, int H) { return (((W + 1) >> 1) * ((H + 1) >> 1) + 31) >> 5; }
 
 }  // namespace
-
-__global__ void __launch_bounds__(256) blur_threshold_kernel(const uint8_t *img, int W, int H, int ithresh, int blur, uint8_t *mask) {
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= W * H) return;
-    const int y = i / W, x = i - y * W;
-    int v;
-    if (blur) {
-        const int k[5] = {1, 4, 6, 4, 1};
-        int acc = 0;
-#pragma unroll
-        for (int dy = -2; dy <= 2; ++dy) {
-            const uint8_t *row = img + reflect(y + dy, H) * W;
-            int r = 0;
-#pragma unroll
-            for (int dx = -2; dx <= 2; ++dx) r += k[dx + 2] * (int)__ldg(row + reflect(x + dx, W));
-            acc += k[dy + 2] * r;
-        }
-        v = (acc + 128) >> 8;
-    } else {
-        v = img[i];
-    }
-    mask[i] = v > ithresh ? 1 : 0;
-}
 
 // cv2.GaussianBlur(u8, (k, k), 0) for k in {3, 5, 7, 15}: OpenCV's 8-bit path uses fixed-point taps that sum to 256 and
 // rounds once, (sum_y K_y sum_x K_x U + 2^15) >> 16, BORDER_REFLECT_101 (taps of 15 probed from cv2 4.13: a column of 255
@@ -450,9 +425,9 @@ static int int_threshold(double threshold) {
     return fl >= 255.0 ? 255 : (fl < -1.0 ? -1 : (int)fl);
 }
 
-int cpt_detect_objects_ex(cpt_ctx *c, const uint8_t *d_image, int width, int height, double threshold, int blur_ksize,
-                          uint32_t steps, const uint8_t *d_or_mask, int max_components, int32_t *d_labels, int32_t *d_stats,
-                          double *d_centroids, uint8_t *d_mask_out, int32_t *h_count, double *h_threshold_used) {
+int cpt_detect_objects(cpt_ctx *c, const uint8_t *d_image, int width, int height, double threshold, int blur_ksize,
+                       uint32_t steps, const uint8_t *d_or_mask, int max_components, int32_t *d_labels, int32_t *d_stats,
+                       double *d_centroids, uint8_t *d_mask_out, int32_t *h_count, double *h_threshold_used) {
     const bool mask_only = (steps & CPT_DETECT_MASK_ONLY) != 0;
     if (!c || !d_image || !h_count) return fail(CPT_ERR_INVALID, "null argument");
     if (!mask_only && (!d_labels || !d_stats || !d_centroids)) return fail(CPT_ERR_INVALID, "null output");
@@ -524,13 +499,6 @@ int cpt_detect_objects_ex(cpt_ctx *c, const uint8_t *d_image, int width, int hei
     if (n > max_components) return fail(CPT_ERR_INVALID, "%d components exceed max_components %d", n, max_components);
     *h_count = n + 1;  // cv2 counts the background label
     return CPT_OK;
-}
-
-int cpt_detect_objects_u8(cpt_ctx *c, const uint8_t *d_image, int width, int height, double threshold, int blur_ksize,
-                          int close, int max_components, int32_t *d_labels, int32_t *d_stats, double *d_centroids,
-                          int32_t *h_count) {
-    return cpt_detect_objects_ex(c, d_image, width, height, threshold, blur_ksize, close ? CPT_DETECT_CLOSE : 0u, nullptr, max_components,
-                                 d_labels, d_stats, d_centroids, nullptr, h_count, nullptr);
 }
 
 int cpt_detect_objects_batch(cpt_ctx *c, const uint8_t *d_frames, int n_frames, int width, int height, double threshold, uint32_t steps,

@@ -12,9 +12,9 @@
 //                            image (preprocess_movement / square_clip, preprocess.py:151-202,
 //                            imageprocessing.py:85-104): one CTA per (segment, tile); the crop is read from
 //                            HBM/L2 once, the only large traffic is the coalesced float2 output rows.
-// The *_ex entry points run the same kernels on an extraction's own buffers, where a frame's thermal row (its row of the
-// input) and its filtered row (its row of every per-frame output) differ, and reuse the per-frame statistics the extraction
-// has already computed:
+// The same entry points also run on an extraction's own buffers, where a frame's thermal row (its row of the input) and its
+// filtered row (its row of every per-frame output) differ, and reuse the per-frame statistics the extraction has already
+// computed when the caller passes them:
 //   sample_crop_median_kernel        pass 1 with the frame medians of cpt_frame_medians: only the crop is read
 //   track_thermal_limits_stats_kernel  thermal_diff_norm limits from cpt_frame_info.thermal_min / thermal_max: no frame read
 #include <cfloat>
@@ -380,8 +380,8 @@ using cpt::fail;
 
 extern "C" {
 
-int cpt_preprocess_limits_ex(cpt_ctx *c, const float *d_filtered, const int64_t *d_filtered_rows, const cpt_sample *d_regions,
-                             int n_regions, cpt_track_norm *d_tracks, int n_tracks) {
+int cpt_preprocess_limits(cpt_ctx *c, const float *d_filtered, const int64_t *d_filtered_rows, const cpt_sample *d_regions,
+                          int n_regions, cpt_track_norm *d_tracks, int n_tracks) {
     if (!c || !d_tracks) return fail(CPT_ERR_INVALID, "null argument");
     if (n_regions < 0 || n_tracks < 0) return fail(CPT_ERR_INVALID, "negative count");
     if (n_tracks == 0) return CPT_OK;
@@ -396,14 +396,9 @@ int cpt_preprocess_limits_ex(cpt_ctx *c, const float *d_filtered, const int64_t 
     return CPT_OK;
 }
 
-int cpt_preprocess_limits(cpt_ctx *c, const float *d_filtered, const cpt_sample *d_regions, int n_regions,
-                          cpt_track_norm *d_tracks, int n_tracks) {
-    return cpt_preprocess_limits_ex(c, d_filtered, nullptr, d_regions, n_regions, d_tracks, n_tracks);
-}
-
-int cpt_preprocess_thermal_limits_ex(cpt_ctx *c, const uint16_t *d_thermal, const int64_t *d_filtered_rows, const cpt_sample *d_regions,
-                                     int n_regions, cpt_track_norm *d_tracks, int n_tracks, const float *d_frame_medians,
-                                     const cpt_frame_info *d_frame_info) {
+int cpt_preprocess_thermal_limits(cpt_ctx *c, const uint16_t *d_thermal, const int64_t *d_filtered_rows, const cpt_sample *d_regions,
+                                  int n_regions, cpt_track_norm *d_tracks, int n_tracks, const float *d_frame_medians,
+                                  const cpt_frame_info *d_frame_info) {
     if (!c || !d_tracks) return fail(CPT_ERR_INVALID, "null argument");
     if (n_regions < 0 || n_tracks < 0) return fail(CPT_ERR_INVALID, "negative count");
     if (n_tracks == 0) return CPT_OK;
@@ -424,13 +419,8 @@ int cpt_preprocess_thermal_limits_ex(cpt_ctx *c, const uint16_t *d_thermal, cons
     return CPT_OK;
 }
 
-int cpt_preprocess_thermal_limits(cpt_ctx *c, const uint16_t *d_thermal, const cpt_sample *d_regions, int n_regions,
-                                  cpt_track_norm *d_tracks, int n_tracks) {
-    return cpt_preprocess_thermal_limits_ex(c, d_thermal, nullptr, d_regions, n_regions, d_tracks, n_tracks, nullptr, nullptr);
-}
-
-int cpt_preprocess_medians_ex(cpt_ctx *c, const uint16_t *d_thermal, const float *d_frame_medians, cpt_sample *d_samples, int n_samples,
-                              cpt_track_norm *d_tracks) {
+int cpt_preprocess_medians(cpt_ctx *c, const uint16_t *d_thermal, const float *d_frame_medians, cpt_sample *d_samples, int n_samples,
+                           cpt_track_norm *d_tracks) {
     if (!c) return fail(CPT_ERR_INVALID, "null ctx");
     if (n_samples < 0) return fail(CPT_ERR_INVALID, "negative count");
     if (n_samples == 0) return CPT_OK;
@@ -447,15 +437,10 @@ int cpt_preprocess_medians_ex(cpt_ctx *c, const uint16_t *d_thermal, const float
     return CPT_OK;
 }
 
-int cpt_preprocess_medians(cpt_ctx *c, const uint16_t *d_thermal, cpt_sample *d_samples, int n_samples,
-                           cpt_track_norm *d_tracks) {
-    return cpt_preprocess_medians_ex(c, d_thermal, nullptr, d_samples, n_samples, d_tracks);
-}
-
-int cpt_preprocess_segments_ex(cpt_ctx *c, const uint16_t *d_thermal, const float *d_filtered, const int64_t *d_filtered_rows,
-                               const cpt_sample *d_samples, const cpt_track_norm *d_tracks, const int32_t *d_segment_samples,
-                               int n_segments, int tiles_per_segment, int frames_per_row, int frame_size,
-                               const int32_t *crop_rectangle, int preprocess_fn, float *d_out) {
+int cpt_preprocess_segments(cpt_ctx *c, const uint16_t *d_thermal, const float *d_filtered, const int64_t *d_filtered_rows,
+                            const cpt_sample *d_samples, const cpt_track_norm *d_tracks, const int32_t *d_segment_samples,
+                            int n_segments, int tiles_per_segment, int frames_per_row, int frame_size,
+                            const int32_t *crop_rectangle, int preprocess_fn, float *d_out) {
     if (!c) return fail(CPT_ERR_INVALID, "null ctx");
     if (n_segments < 0) return fail(CPT_ERR_INVALID, "negative count");
     if (n_segments == 0) return CPT_OK;
@@ -479,14 +464,6 @@ int cpt_preprocess_segments_ex(cpt_ctx *c, const uint16_t *d_thermal, const floa
     cpt::segment_tiles_kernel<<<(unsigned)(n_segments * tiles_per_segment), cpt::kTileThreads, smem, c->stream>>>(a);
     CUDA_TRY(cudaGetLastError());
     return CPT_OK;
-}
-
-int cpt_preprocess_segments(cpt_ctx *c, const uint16_t *d_thermal, const float *d_filtered, const cpt_sample *d_samples,
-                            const cpt_track_norm *d_tracks, const int32_t *d_segment_samples, int n_segments,
-                            int tiles_per_segment, int frames_per_row, int frame_size, const int32_t *crop_rectangle,
-                            int preprocess_fn, float *d_out) {
-    return cpt_preprocess_segments_ex(c, d_thermal, d_filtered, nullptr, d_samples, d_tracks, d_segment_samples, n_segments,
-                                      tiles_per_segment, frames_per_row, frame_size, crop_rectangle, preprocess_fn, d_out);
 }
 
 }  // extern "C"

@@ -34,7 +34,7 @@ def _run(image, threshold, blur, steps, or_mask=None, stats_only=False):
     d_labels = torch.empty((H, W), dtype=torch.int32, device=eng.device)
     d_stats = torch.empty((MAX_COMPONENTS + 1, 5), dtype=torch.int32, device=eng.device)
     d_cent = torch.empty((MAX_COMPONENTS + 1, 2), dtype=torch.float64, device=eng.device)
-    n, _ = eng.ctx.detect_objects_ex(d_img, W, H, threshold, blur, steps, MAX_COMPONENTS, d_labels, d_stats, d_cent, d_or_mask=d_or)
+    n, _ = eng.ctx.detect_objects(d_img, W, H, threshold, blur, steps, MAX_COMPONENTS, d_labels, d_stats, d_cent, d_or_mask=d_or)
     return n, d_labels.cpu().numpy(), d_stats[:n].cpu().numpy(), d_cent[:n].cpu().numpy()
 
 
@@ -63,7 +63,7 @@ def _binary_mask(image, threshold, steps):
     eng.ctx.use_torch_stream()
     d_img = torch.from_numpy(np.ascontiguousarray(image)).to(eng.device)
     d_mask = torch.empty((H, W), dtype=torch.uint8, device=eng.device)
-    eng.ctx.detect_objects_ex(d_img, W, H, threshold, 0, steps | native.DETECT_MASK_ONLY, 1, None, None, None, d_mask_out=d_mask)
+    eng.ctx.detect_objects(d_img, W, H, threshold, 0, steps | native.DETECT_MASK_ONLY, 1, None, None, None, d_mask_out=d_mask)
     return d_mask.cpu().numpy()
 
 

@@ -102,26 +102,11 @@ class CptOutputs(ctypes.Structure):
     ]
 
 
-REGION_DTYPE = np.dtype(
-    [("x", "<i4"), ("y", "<i4"), ("width", "<i4"), ("height", "<i4"), ("area", "<i4"), ("sum_x", "<i4"),
-     ("sum_y", "<i4"), ("key", "<i4"), ("pixel_variance", "<f8")]
-)
-INFO_DTYPE = np.dtype(
-    [("background_average", "<f8"), ("threshold", "<f4"), ("norm_min", "<i4"), ("norm_max", "<i4"),
-     ("avg_change", "<i4"), ("filtered_min", "<i4"), ("filtered_max", "<i4"), ("n_components", "<i4"),
-     ("thermal_min", "<i4"), ("thermal_max", "<i4"), ("thermal_sum", "<u4"), ("abs_filtered_sum", "<u4"),
-     ("thermal_median", "<f4"), ("reserved", "<i4", (2,))]
-)
-CLIP_DTYPE = np.dtype(
-    [("frame_offset", "<i8"), ("init_offset", "<i8"), ("out_offset", "<i8"), ("n_frames", "<i4"),
-     ("first_frame", "<i4"), ("ring_frames", "<i4"), ("background_thresh", "<i4"), ("weight_table", "<i4"),
-     ("flags", "<u4")]
-)
-SAMPLE_DTYPE = np.dtype(
-    [("frame", "<i8"), ("x", "<i4"), ("y", "<i4"), ("width", "<i4"), ("height", "<i4"), ("track", "<i4"), ("median", "<f4")]
-)
-TRACK_NORM_DTYPE = np.dtype([("filtered_min", "<f4"), ("filtered_max", "<f4"), ("clip_at_zero", "<i4"), ("has_limits", "<i4"),
-                             ("thermal_min", "<f4"), ("thermal_max", "<f4"), ("has_thermal_limits", "<i4"), ("reserved", "<i4")])
+REGION_DTYPE = np.dtype(CptRegion)
+INFO_DTYPE = np.dtype(CptFrameInfo)
+CLIP_DTYPE = np.dtype(CptClip)
+SAMPLE_DTYPE = np.dtype(CptSample)
+TRACK_NORM_DTYPE = np.dtype(CptTrackNorm)
 PREPROCESS_INC3 = 1       # x / 127.5 - 1
 PREPROCESS_PER_TILE = 2   # HyperParams.diff_norm off: both channels normalised by the tile's own extrema
 CPTV_FRAME_DTYPE = np.dtype([("payload_offset", "<u8"), ("bit_width", "<i4"), ("reserved", "<i4")])
@@ -145,7 +130,6 @@ SYMBOLS = {
     "cpt_set_weight_table": (_i, [_vp, _i, _d, _i]),
     "cpt_build_weight_table": (_i, [_d, _i, _vp, _vp]),
     "cpt_debug_phase_cycles": (_i, [_vp, _vp, _i]),
-    "cpt_debug_kernel_times": (_i, [_vp, _i, _vp]),
     "cpt_debug_kernel_times_ex": (_i, [_vp, _i, _vp, _i]),
     "cpt_debug_force_single_kernel": (_i, [_vp, _i]),
     "cpt_device_alloc": (_i, [_vp, ctypes.POINTER(_vp), _u64]),
@@ -159,20 +143,15 @@ SYMBOLS = {
     "cpt_extract_batch_host": (_i, [_vp, _vp, _vp, _i, _i64, _vp, _vp, _vp, _vp, _i]),
     "cpt_background_process": (_i, [_vp, _vp, _vp, _i, _vp, _i]),
     "cpt_frame_medians": (_i, [_vp, _vp, _i64, _vp]),
-    "cpt_preprocess_limits": (_i, [_vp, _vp, _vp, _i, _vp, _i]),
-    "cpt_preprocess_thermal_limits": (_i, [_vp, _vp, _vp, _i, _vp, _i]),
-    "cpt_preprocess_medians": (_i, [_vp, _vp, _vp, _i, _vp]),
-    "cpt_preprocess_segments": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp, _i, _vp]),
-    "cpt_preprocess_limits_ex": (_i, [_vp, _vp, _vp, _vp, _i, _vp, _i]),
-    "cpt_preprocess_thermal_limits_ex": (_i, [_vp, _vp, _vp, _vp, _i, _vp, _i, _vp, _vp]),
-    "cpt_preprocess_medians_ex": (_i, [_vp, _vp, _vp, _vp, _i, _vp]),
-    "cpt_preprocess_segments_ex": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp, _i, _vp]),
+    "cpt_preprocess_limits": (_i, [_vp, _vp, _vp, _vp, _i, _vp, _i]),
+    "cpt_preprocess_thermal_limits": (_i, [_vp, _vp, _vp, _vp, _i, _vp, _i, _vp, _vp]),
+    "cpt_preprocess_medians": (_i, [_vp, _vp, _vp, _vp, _i, _vp]),
+    "cpt_preprocess_segments": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp, _i, _vp]),
     "cpt_minmax_f32": (_i, [_vp, _vp, _i64, _vp]),
     "cpt_normalize_f32": (_i, [_vp, _vp, _i64, _d, _d, _d, _i, _vp]),
     "cpt_resize_pad_f32": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _f, _i, _vp]),
-    "cpt_detect_objects_u8": (_i, [_vp, _vp, _i, _i, _d, _i, _i, _i, _vp, _vp, _vp, ctypes.POINTER(ctypes.c_int32)]),
-    "cpt_detect_objects_ex": (_i, [_vp, _vp, _i, _i, _d, _i, ctypes.c_uint32, _vp, _i, _vp, _vp, _vp, _vp, ctypes.POINTER(ctypes.c_int32),
-                                   ctypes.POINTER(_d)]),
+    "cpt_detect_objects": (_i, [_vp, _vp, _i, _i, _d, _i, ctypes.c_uint32, _vp, _i, _vp, _vp, _vp, _vp, ctypes.POINTER(ctypes.c_int32),
+                                ctypes.POINTER(_d)]),
     "cpt_detect_objects_batch": (_i, [_vp, _vp, _i, _i, _i, _d, ctypes.c_uint32, _i, _vp, _vp, _vp, _vp]),
     "cpt_ir_merge_components": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _d, _vp, _vp]),
     "cpt_nlm_denoise_u8": (_i, [_vp, _vp, _i, _i, _i, _vp]),
@@ -319,41 +298,26 @@ class Context:
     def frame_medians(self, d_frames, n_frames, d_medians):
         check(self.lib.cpt_frame_medians(self._h, _ptr(d_frames), int(n_frames), _ptr(d_medians)))
 
-    def preprocess_limits(self, d_filtered, d_regions, n_regions, d_tracks, n_tracks):
-        check(self.lib.cpt_preprocess_limits(self._h, _ptr(d_filtered), _ptr(d_regions), int(n_regions), _ptr(d_tracks), int(n_tracks)))
+    # d_filtered_rows: int64 filtered row per entry on an extraction's buffers (None: the entry's frame); d_frame_medians
+    # float32 per thermal row and d_frame_info the extraction's INFO_DTYPE records (None: the frames are read).  Either
+    # choice gives bit-identical results (include/cptrack.h)
+    def preprocess_limits(self, d_filtered, d_regions, n_regions, d_tracks, n_tracks, d_filtered_rows=None):
+        check(self.lib.cpt_preprocess_limits(self._h, _ptr(d_filtered), _ptr(d_filtered_rows), _ptr(d_regions), int(n_regions),
+                                             _ptr(d_tracks), int(n_tracks)))
 
-    def preprocess_thermal_limits(self, d_thermal, d_regions, n_regions, d_tracks, n_tracks):
-        check(self.lib.cpt_preprocess_thermal_limits(self._h, _ptr(d_thermal), _ptr(d_regions), int(n_regions), _ptr(d_tracks), int(n_tracks)))
+    def preprocess_thermal_limits(self, d_thermal, d_regions, n_regions, d_tracks, n_tracks, d_filtered_rows=None, d_frame_medians=None,
+                                  d_frame_info=None):
+        check(self.lib.cpt_preprocess_thermal_limits(self._h, _ptr(d_thermal), _ptr(d_filtered_rows), _ptr(d_regions), int(n_regions),
+                                                     _ptr(d_tracks), int(n_tracks), _ptr(d_frame_medians), _ptr(d_frame_info)))
 
-    def preprocess_medians(self, d_thermal, d_samples, n_samples, d_tracks):
-        check(self.lib.cpt_preprocess_medians(self._h, _ptr(d_thermal), _ptr(d_samples), int(n_samples), _ptr(d_tracks)))
+    def preprocess_medians(self, d_thermal, d_samples, n_samples, d_tracks, d_frame_medians=None):
+        check(self.lib.cpt_preprocess_medians(self._h, _ptr(d_thermal), _ptr(d_frame_medians), _ptr(d_samples), int(n_samples),
+                                              _ptr(d_tracks)))
 
     def preprocess_segments(self, d_thermal, d_filtered, d_samples, d_tracks, d_segment_samples, n_segments, tiles, per_row,
-                            frame_size, crop_rectangle, preprocess_fn, d_out):
+                            frame_size, crop_rectangle, preprocess_fn, d_out, d_filtered_rows=None):
         crop = None if crop_rectangle is None else (ctypes.c_int32 * 4)(*[int(v) for v in crop_rectangle])
         check(self.lib.cpt_preprocess_segments(
-            self._h, _ptr(d_thermal), _ptr(d_filtered), _ptr(d_samples), _ptr(d_tracks), _ptr(d_segment_samples), int(n_segments),
-            int(tiles), int(per_row), int(frame_size), crop, int(preprocess_fn), _ptr(d_out)))
-
-    # the same passes on an extraction's buffers (include/cptrack.h, cpt_preprocess_*_ex): d_filtered_rows int64 per entry
-    # (None: the entry's frame), d_frame_medians float32 per thermal row, d_frame_info the extraction's INFO_DTYPE records
-    def preprocess_limits_ex(self, d_filtered, d_filtered_rows, d_regions, n_regions, d_tracks, n_tracks):
-        check(self.lib.cpt_preprocess_limits_ex(self._h, _ptr(d_filtered), _ptr(d_filtered_rows), _ptr(d_regions), int(n_regions),
-                                                _ptr(d_tracks), int(n_tracks)))
-
-    def preprocess_thermal_limits_ex(self, d_thermal, d_filtered_rows, d_regions, n_regions, d_tracks, n_tracks, d_frame_medians=None,
-                                     d_frame_info=None):
-        check(self.lib.cpt_preprocess_thermal_limits_ex(self._h, _ptr(d_thermal), _ptr(d_filtered_rows), _ptr(d_regions), int(n_regions),
-                                                        _ptr(d_tracks), int(n_tracks), _ptr(d_frame_medians), _ptr(d_frame_info)))
-
-    def preprocess_medians_ex(self, d_thermal, d_frame_medians, d_samples, n_samples, d_tracks):
-        check(self.lib.cpt_preprocess_medians_ex(self._h, _ptr(d_thermal), _ptr(d_frame_medians), _ptr(d_samples), int(n_samples),
-                                                 _ptr(d_tracks)))
-
-    def preprocess_segments_ex(self, d_thermal, d_filtered, d_filtered_rows, d_samples, d_tracks, d_segment_samples, n_segments, tiles,
-                               per_row, frame_size, crop_rectangle, preprocess_fn, d_out):
-        crop = None if crop_rectangle is None else (ctypes.c_int32 * 4)(*[int(v) for v in crop_rectangle])
-        check(self.lib.cpt_preprocess_segments_ex(
             self._h, _ptr(d_thermal), _ptr(d_filtered), _ptr(d_filtered_rows), _ptr(d_samples), _ptr(d_tracks), _ptr(d_segment_samples),
             int(n_segments), int(tiles), int(per_row), int(frame_size), crop, int(preprocess_fn), _ptr(d_out)))
 
@@ -367,21 +331,14 @@ class Context:
         check(self.lib.cpt_resize_pad_f32(self._h, _ptr(d_src), int(sw), int(sh), int(fw), int(fh), int(ox), int(oy), int(dw),
                                           int(dh), float(pad), int(interpolation), _ptr(d_out)))
 
-    def detect_objects_u8(self, d_image, width, height, threshold, blur_ksize, close, max_components, d_labels, d_stats, d_centroids):
-        n = ctypes.c_int32()
-        check(self.lib.cpt_detect_objects_u8(self._h, _ptr(d_image), int(width), int(height), float(threshold), int(blur_ksize),
-                                             int(close), int(max_components), _ptr(d_labels), _ptr(d_stats), _ptr(d_centroids),
-                                             ctypes.byref(n)))
-        return n.value
-
-    def detect_objects_ex(self, d_image, width, height, threshold, blur_ksize, steps, max_components, d_labels, d_stats, d_centroids,
-                          d_or_mask=None, d_mask_out=None):
+    def detect_objects(self, d_image, width, height, threshold, blur_ksize, steps, max_components, d_labels, d_stats, d_centroids,
+                       d_or_mask=None, d_mask_out=None):
         """Returns (n_labels, threshold used)."""
         n = ctypes.c_int32()
         thr = ctypes.c_double()
-        check(self.lib.cpt_detect_objects_ex(self._h, _ptr(d_image), int(width), int(height), float(threshold), int(blur_ksize), int(steps),
-                                             _ptr(d_or_mask), int(max_components), _ptr(d_labels), _ptr(d_stats), _ptr(d_centroids),
-                                             _ptr(d_mask_out), ctypes.byref(n), ctypes.byref(thr)))
+        check(self.lib.cpt_detect_objects(self._h, _ptr(d_image), int(width), int(height), float(threshold), int(blur_ksize), int(steps),
+                                          _ptr(d_or_mask), int(max_components), _ptr(d_labels), _ptr(d_stats), _ptr(d_centroids),
+                                          _ptr(d_mask_out), ctypes.byref(n), ctypes.byref(thr)))
         return n.value, thr.value
 
     def detect_objects_batch(self, d_frames, n_frames, width, height, threshold, steps, max_components, d_counts, d_stats, d_centroids=None,
@@ -397,6 +354,13 @@ class Context:
         d_merged_counts int32 [n] (-1: the frame's components overflowed).  Launches without waiting."""
         check(self.lib.cpt_ir_merge_components(self._h, _ptr(d_stats), _ptr(d_counts), int(n_frames), int(max_components), int(min_mass),
                                                int(min_size), float(max_gap), _ptr(d_merged), _ptr(d_merged_counts)))
+
+    def motion_clips(self, h_clips, n_clips, d_frames, n_frames, h_steps, n_steps, h_mean_rows, n_mean_rows, h_results):
+        """cpt_motion_clips: h_clips CptMotionClip [n_clips] (``Motion.clip_record``), h_steps CptMotionClipStep [n_steps],
+        h_mean_rows int32 [n_mean_rows] and h_results CptMotionResult [n_steps] on the host; d_frames uint16 [n_frames][H][W]
+        on the device."""
+        check(self.lib.cpt_motion_clips(self._h, h_clips, int(n_clips), _ptr(d_frames), int(n_frames), h_steps, int(n_steps),
+                                        _ptr(h_mean_rows), int(n_mean_rows), h_results))
 
     def nlm_denoise_u8(self, d_src, width, height, n_frames, d_dst):
         check(self.lib.cpt_nlm_denoise_u8(self._h, _ptr(d_src), int(width), int(height), int(n_frames), _ptr(d_dst)))
@@ -450,15 +414,39 @@ def pinned_empty(shape, dtype):
 _PINNED_OWNERS = {}
 
 
-class IrMotion:
+class _Handle:
+    """A device object of a Context: ``open(ctx, *args)`` returns its handle (NULL: NativeError), ``close`` frees it once."""
+
+    def __init__(self, ctx, open_fn, close_fn, *args):
+        self.ctx = ctx
+        self._close = close_fn
+        self._h = open_fn(ctx._h, *args)
+        if not self._h:
+            raise NativeError("{} failed: {}".format(open_fn.__name__, ctx.lib.cpt_last_error().decode()))
+
+    @property
+    def address(self):
+        """Address of the native object (None once closed), for inspecting its device buffers."""
+        return self._h
+
+    def close(self):
+        if getattr(self, "_h", None):
+            self._close(self._h)
+            self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+class IrMotion(_Handle):
     """Device half of IRMotionDetector (cpt_ir_motion_*): a ring of grey frames, grey conversion and the eroded-pixel counts."""
 
     def __init__(self, ctx, width, height, ring_frames):
-        self.ctx = ctx
         self.width, self.height, self.ring_frames = width, height, ring_frames
-        self._h = ctx.lib.cpt_ir_motion_open(ctx._h, int(width), int(height), int(ring_frames))
-        if not self._h:
-            raise NativeError("cpt_ir_motion_open failed: {}".format(ctx.lib.cpt_last_error().decode()))
+        super().__init__(ctx, ctx.lib.cpt_ir_motion_open, ctx.lib.cpt_ir_motion_close, int(width), int(height), int(ring_frames))
 
     def gray(self, bgr, slot, copy_out=True):
         """BGR frame -> grey into ring slot ``slot``; returns the grey frame as a host array, or None with copy_out=False
@@ -493,17 +481,6 @@ class IrMotion:
                                                 ctypes.byref(diff), ctypes.byref(cnt)))
         return diff.value, cnt.value
 
-    def close(self):
-        if self._h:
-            self.ctx.lib.cpt_ir_motion_close(self._h)
-            self._h = None
-
-    def __del__(self):
-        try:
-            self.close()
-        except Exception:
-            pass
-
 
 def _dptr(t, min_bytes):
     """Device address of a uint8 CUDA tensor (at least min_bytes, contiguous) or a raw device address (int)."""
@@ -514,20 +491,17 @@ def _dptr(t, min_bytes):
     return t.data_ptr()
 
 
-class Mog2:
+class Mog2(_Handle):
     """OpenCV's BackgroundSubtractorMOG2 (detectShadows=False, one uint8 channel) on the device, bit for bit (cpt_mog2_*).
     The model's state stays in device memory; frames and masks are uint8 CUDA tensors or device addresses.  Calls launch on
     the context's stream and return without waiting."""
 
     def __init__(self, ctx, width, height, history=500, var_threshold=16.0, background_ratio=0.9, var_threshold_gen=9.0,
                  var_init=15.0, var_min=4.0, var_max=75.0, complexity_reduction=0.05, detect_shadows=False):
-        self.ctx = ctx
         self.width, self.height = int(width), int(height)
         self.params = CptMog2Params(int(history), float(var_threshold), float(background_ratio), float(var_threshold_gen), float(var_init),
                                     float(var_min), float(var_max), float(complexity_reduction), int(bool(detect_shadows)))
-        self._h = ctx.lib.cpt_mog2_open(ctx._h, self.width, self.height, ctypes.byref(self.params))
-        if not self._h:
-            raise NativeError("cpt_mog2_open failed: {}".format(ctx.lib.cpt_last_error().decode()))
+        super().__init__(ctx, ctx.lib.cpt_mog2_open, ctx.lib.cpt_mog2_close, self.width, self.height, ctypes.byref(self.params))
 
     @property
     def frame_bytes(self):
@@ -564,13 +538,34 @@ class Mog2:
             check(n)
         return n
 
-    def close(self):
-        if getattr(self, "_h", None):
-            self.ctx.lib.cpt_mog2_close(self._h)
-            self._h = None
 
-    def __del__(self):
-        try:
-            self.close()
-        except Exception:
-            pass
+class Motion(_Handle):
+    """Device half of CPTVMotionDetector (cpt_motion_*): the ring of frames, the running sum and the ring of delta frames.
+    Ring bookkeeping (which slot is newest / oldest / oldest non-FFC) stays with the caller."""
+
+    def __init__(self, ctx, ring_frames, mean_frames, diff_frames, weight_slot):
+        super().__init__(ctx, ctx.lib.cpt_motion_open, ctx.lib.cpt_motion_close, int(ring_frames), int(mean_frames), int(diff_frames),
+                         int(weight_slot))
+
+    def store(self, h_pix, slot):
+        """Host uint16 frame [H][W] into ring slot ``slot`` without processing it."""
+        check(self.ctx.lib.cpt_motion_store(self._h, _ptr(h_pix), int(slot)))
+
+    def mean_init(self, slots):
+        """Start the running sum from the frames in ring slots ``slots``."""
+        arr = (ctypes.c_int32 * len(slots))(*slots)
+        check(self.ctx.lib.cpt_motion_mean_init(self._h, arr, len(slots)))
+
+    def step(self, h_pix, d_background_state, slot_new, slot_oldest, slot_nonffc, diff_slot_new, diff_slot_old, flags, delta_thresh,
+             init_average):
+        """One process_frame (include/cptrack.h, cpt_motion_step); waits for it and returns its CptMotionResult."""
+        result = CptMotionResult()
+        check(self.ctx.lib.cpt_motion_step(self._h, _ptr(h_pix), _ptr(d_background_state), int(slot_new), int(slot_oldest),
+                                           int(slot_nonffc), int(diff_slot_new), int(diff_slot_old), int(flags), int(delta_thresh),
+                                           float(init_average), ctypes.byref(result)))
+        return result
+
+    def clip_record(self, d_background_state, ring_rows, init_average, delta_thresh, first_step, n_steps):
+        """This detector's CptMotionClip of a ``Context.motion_clips`` call (ring_rows: host int32 [ring_frames])."""
+        return CptMotionClip(self._h, _ptr(d_background_state), _ptr(ring_rows), float(init_average), int(delta_thresh), int(first_step),
+                             int(n_steps), 0)

@@ -1,5 +1,4 @@
 """``CPTVMotionDetector`` and ``is_affected_by_ffc`` (piclassifier/cptvmotiondetector.py:14-234)."""
-import ctypes
 from collections import namedtuple
 from datetime import timedelta
 from typing import NamedTuple
@@ -90,23 +89,15 @@ class CPTVMotionDetector(MotionDetector):
         self.ffc_affected = False
         self.detect_after = self.thermal_window.size * 2 if detect_after is None else detect_after
         self._ctx = self._background.ctx
-        lib = self._ctx.lib
-        self._lib = lib
-        self._m = lib.cpt_motion_open(self._ctx._h, self.thermal_window.size, self.MEAN_FRAMES,
-                                      0 if self.config.one_diff_only else self.compare_gap, self._background.weight_slot)
-        if not self._m:
-            raise native.NativeError("cpt_motion_open failed: " + lib.cpt_last_error().decode())
-        self._result = native.CptMotionResult()
+        self._motion = native.Motion(self._ctx, self.thermal_window.size, self.MEAN_FRAMES,
+                                     0 if self.config.one_diff_only else self.compare_gap, self._background.weight_slot)
         self._average = None
         self.last_diff = 0
 
-    def __del__(self):
-        try:
-            if getattr(self, "_m", None):
-                self._lib.cpt_motion_close(self._m)
-                self._m = None
-        except Exception:
-            pass
+    @property
+    def _m(self):
+        """Address of the detector's struct cpt_motion, whose leading members name its device buffers."""
+        return self._motion.address
 
     @property
     def calibrating(self):
@@ -209,19 +200,16 @@ class CPTVMotionDetector(MotionDetector):
     def process_frame(self, cptv_frame, force_process=False):
         pix = self._pix(cptv_frame)
         step = self._plan(cptv_frame, force_process)
-        win = self.thermal_window
+        result = None
         if step is None:
-            native.check(self._lib.cpt_motion_store(self._m, pix.ctypes.data, win.last_index))
+            self._motion.store(pix, self.thermal_window.last_index)
         else:
             if step.mean_slots:
-                native.check(self._lib.cpt_motion_store(self._m, pix.ctypes.data, step.new))
-                arr = (ctypes.c_int32 * len(step.mean_slots))(*step.mean_slots)
-                native.check(self._lib.cpt_motion_mean_init(self._m, arr, len(step.mean_slots)))
-            native.check(self._lib.cpt_motion_step(
-                self._m, pix.ctypes.data, self._background.d_state.data_ptr(), step.new, step.oldest,
-                -1 if step.nonffc is None else step.nonffc, step.diff_new, step.diff_old, step.flags,
-                int(self.config.delta_thresh), self._init_average(), ctypes.byref(self._result)))
-        self._apply(step, self._result)
+                self._motion.store(pix, step.new)
+                self._motion.mean_init(step.mean_slots)
+            result = self._motion.step(pix, self._background.d_state, step.new, step.oldest, -1 if step.nonffc is None else step.nonffc,
+                                       step.diff_new, step.diff_old, step.flags, self.config.delta_thresh, self._init_average())
+        self._apply(step, result)
         return self.movement_detected
 
     def process_frames(self, cptv_frames, force_process=False):
@@ -270,8 +258,8 @@ class ClipSteps:
             self._processed.append(processed)
             self.offsets[i + 1] = self.offsets[i] + len(frames)
             self._ring_rows.append(ring_rows)
-            self._clips[i] = native.CptMotionClip(det._m, det._background.d_state.data_ptr(), ring_rows.ctypes.data,
-                                                  det._init_average(), int(det.config.delta_thresh), first, len(steps) - first, 0)
+            self._clips[i] = det._motion.clip_record(det._background.d_state, ring_rows, det._init_average(), det.config.delta_thresh,
+                                                     first, len(steps) - first)
         self.n_steps = len(steps)
         self._steps = (native.CptMotionClipStep * max(1, len(steps)))(*[native.CptMotionClipStep(*s) for s in steps])
         self._mean_rows = np.array(mean_rows, dtype=np.int32)
@@ -285,9 +273,8 @@ class ClipSteps:
         """One ``cpt_motion_clips`` launch over ``d_frames`` (device uint16 [n_frames][H][W], any tensor or address)."""
         ctx = self.detectors[0]._ctx
         ctx.use_torch_stream()
-        native.check(ctx.lib.cpt_motion_clips(ctx._h, self._clips, len(self.detectors), native._ptr(d_frames), self.n_frames,
-                                              self._steps, self.n_steps, self._mean_rows.ctypes.data, len(self._mean_rows),
-                                              self.results))
+        ctx.motion_clips(self._clips, len(self.detectors), d_frames, self.n_frames, self._steps, self.n_steps, self._mean_rows,
+                         len(self._mean_rows), self.results)
         return self.results
 
     def apply(self):

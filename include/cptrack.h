@@ -141,12 +141,8 @@ int cpt_copy_to_host(cpt_ctx *ctx, void *h_dst, const void *d_src, uint64_t byte
 int cpt_debug_phase_cycles(cpt_ctx *ctx, long long *h_out32, int reset);
 
 /* Diagnostics: with enable != 0, every following cpt_extract_batch call brackets its launches with CUDA events on the
- * ctx stream.  h_ms4 (may be NULL) receives the durations of the last timed call in milliseconds after synchronising:
- * [0] the recurrence kernel (strip_sweep_kernel, or extract_clips_kernel on the single-kernel path), [1]
- * frame_scalars_kernel + the per-frame mask / component launches (0 on the single-kernel path), [2] the denoise passes,
- * [3] region_variance_kernel. */
-int cpt_debug_kernel_times(cpt_ctx *ctx, int enable, float *h_ms4);
-/* Same, finer: h_ms[0..n-1], n <= 5: [0] strip_sweep_kernel (the recurrence; extract_clips_kernel on the single-kernel path),
+ * ctx stream.  h_ms (may be NULL) receives the durations of the last timed call in milliseconds after synchronising,
+ * h_ms[0..n-1], n <= 5: [0] strip_sweep_kernel (the recurrence; extract_clips_kernel on the single-kernel path),
  * [1] frame_scalars_kernel, [2] the per-frame mask / component launches, [3] the denoise passes, [4] region_variance_kernel. */
 int cpt_debug_kernel_times_ex(cpt_ctx *ctx, int enable, float *h_ms, int n);
 
@@ -206,54 +202,46 @@ typedef struct {
     int32_t reserved;
 } cpt_track_norm;
 
+/* On an extraction's own buffers (ClipTrackExtractor.parse_clips(keep_on_device=True)) a tracked frame lives at two rows:
+ * its thermal row (sample.frame: the row of d_frames it was read from, also its row of cpt_frame_medians) and its filtered
+ * row (out_offset + n: its row of d_filtered and of every other per-frame output).  d_filtered_rows holds one int64 filtered
+ * row per entry of d_regions / d_samples, d_frame_medians and d_frame_info the extraction's per-frame statistics.  Each
+ * may be NULL, as each entry point below says, and every choice gives bit-identical results on the same frames. */
+
 /* get_limits: resets all n_tracks rows (min unset, max 0, clip_at_zero 1), then folds the min / max of
- * region.subimage(frame.filtered) of every entry of d_regions (all non-blank regions of each track). */
-int cpt_preprocess_limits(cpt_ctx *ctx, const float *d_filtered, const cpt_sample *d_regions, int n_regions,
-                          cpt_track_norm *d_tracks, int n_tracks);
+ * region.subimage(frame.filtered) of every entry of d_regions (all non-blank regions of each track), read at the entry's
+ * filtered row (d_filtered_rows, or NULL: sample.frame). */
+int cpt_preprocess_limits(cpt_ctx *ctx, const float *d_filtered, const int64_t *d_filtered_rows, const cpt_sample *d_regions,
+                          int n_regions, cpt_track_norm *d_tracks, int n_tracks);
 /* get_limits with HyperParams.thermal_diff_norm (interpreter.py:338-345,358-359): after cpt_preprocess_limits, folds the
  * min / max of frame.thermal - np.median(frame.thermal) over the WHOLE frame of every entry of d_regions into the
- * track rows (one full-frame median per entry). */
-int cpt_preprocess_thermal_limits(cpt_ctx *ctx, const uint16_t *d_thermal, const cpt_sample *d_regions, int n_regions,
-                                  cpt_track_norm *d_tracks, int n_tracks);
+ * track rows.  With d_frame_medians (float32 per thermal row, as cpt_frame_medians writes them) and d_frame_info (the
+ * extraction's cpt_frame_info per filtered row, computed with CPT_CLIP_FRAME_STATS; d_filtered_rows, or NULL: sample.frame)
+ * both given, the limits are (thermal_min - median, thermal_max - median) and no frame is read; with either NULL each
+ * entry's thermal frame is read and its full-frame median computed (d_filtered_rows is then unused). */
+int cpt_preprocess_thermal_limits(cpt_ctx *ctx, const uint16_t *d_thermal, const int64_t *d_filtered_rows, const cpt_sample *d_regions,
+                                  int n_regions, cpt_track_norm *d_tracks, int n_tracks, const float *d_frame_medians,
+                                  const cpt_frame_info *d_frame_info);
 /* Pass 1 of preprocess_segments over the unique track-frames: fills sample.median and clears the track's
- * clip_at_zero when np.median(region.subimage(thermal) - median) <= 0. */
-int cpt_preprocess_medians(cpt_ctx *ctx, const uint16_t *d_thermal, cpt_sample *d_samples, int n_samples,
+ * clip_at_zero when np.median(region.subimage(thermal) - median) <= 0.  d_frame_medians (float32 per thermal row, as
+ * cpt_frame_medians writes them): sample.median is looked up and only the crop is read; NULL: each sample's thermal frame
+ * is read and its median computed. */
+int cpt_preprocess_medians(cpt_ctx *ctx, const uint16_t *d_thermal, const float *d_frame_medians, cpt_sample *d_samples, int n_samples,
                            cpt_track_norm *d_tracks);
 /* Pass 2 + preprocess_movement (ml_tools/preprocess.py:56-113,151-202; imageprocessing.py:11-104): every
  * segment is tiles_per_segment sample indices (d_segment_samples [n_segments][tiles_per_segment], already padded
  * and sorted as preprocess_movement does); tile i lands in row i / frames_per_row, column i % frames_per_row of
- * d_out [n_segments][rows*frame_size][frames_per_row*frame_size][2] float32 (channels thermal, filtered).
+ * d_out [n_segments][rows*frame_size][frames_per_row*frame_size][2] float32 (channels thermal, filtered).  The thermal
+ * crop is read at sample.frame, the filtered crop at the sample's filtered row (d_filtered_rows, or NULL: sample.frame).
  * crop_rectangle = {x, y, width, height} of Clip.crop_rectangle (keep_edge anchoring) or NULL;
  * preprocess_fn: CPT_PREPROCESS_INC3 = x / 127.5 - 1 (interpreter.py:563-566); CPT_PREPROCESS_PER_TILE = HyperParams.diff_norm
  * off: no track-wide limits, both channels are normalised by the tile's own extrema (Frame.normalize, preprocess.py:111). */
 #define CPT_PREPROCESS_INC3 1
 #define CPT_PREPROCESS_PER_TILE 2
-int cpt_preprocess_segments(cpt_ctx *ctx, const uint16_t *d_thermal, const float *d_filtered, const cpt_sample *d_samples,
-                            const cpt_track_norm *d_tracks, const int32_t *d_segment_samples, int n_segments,
-                            int tiles_per_segment, int frames_per_row, int frame_size, const int32_t *crop_rectangle,
-                            int preprocess_fn, float *d_out);
-
-/* The same passes on an extraction's own buffers (ClipTrackExtractor.parse_clips(keep_on_device=True)).  There a tracked frame
- * lives at different rows: its thermal row (sample.frame; the row of d_frames it was read from, also its row of
- * cpt_frame_medians) and its filtered row (out_offset + n, its row of d_filtered and of every other per-frame output).
- *   d_filtered_rows    one int64 per entry of d_regions / d_samples: the entry's filtered row (NULL: the same as sample.frame)
- *   d_frame_medians    float32 per thermal row as cpt_frame_medians writes them (NULL: recompute them from the frames).  Given,
- *                      the medians pass looks sample.median up and reads only the crop for the clip_thermals_at_zero test
- *   d_frame_info       the extraction's cpt_frame_info per filtered row, computed with CPT_CLIP_FRAME_STATS.  With
- *                      d_frame_medians as well, the thermal_diff_norm limits are (thermal_min - median, thermal_max - median)
- *                      folded per track without reading a frame; otherwise the frames are read as cpt_preprocess_thermal_limits does
- * Results are bit-identical to the entry points above on the same frames. */
-int cpt_preprocess_limits_ex(cpt_ctx *ctx, const float *d_filtered, const int64_t *d_filtered_rows, const cpt_sample *d_regions,
-                             int n_regions, cpt_track_norm *d_tracks, int n_tracks);
-int cpt_preprocess_thermal_limits_ex(cpt_ctx *ctx, const uint16_t *d_thermal, const int64_t *d_filtered_rows, const cpt_sample *d_regions,
-                                     int n_regions, cpt_track_norm *d_tracks, int n_tracks, const float *d_frame_medians,
-                                     const cpt_frame_info *d_frame_info);
-int cpt_preprocess_medians_ex(cpt_ctx *ctx, const uint16_t *d_thermal, const float *d_frame_medians, cpt_sample *d_samples, int n_samples,
-                              cpt_track_norm *d_tracks);
-int cpt_preprocess_segments_ex(cpt_ctx *ctx, const uint16_t *d_thermal, const float *d_filtered, const int64_t *d_filtered_rows,
-                               const cpt_sample *d_samples, const cpt_track_norm *d_tracks, const int32_t *d_segment_samples,
-                               int n_segments, int tiles_per_segment, int frames_per_row, int frame_size,
-                               const int32_t *crop_rectangle, int preprocess_fn, float *d_out);
+int cpt_preprocess_segments(cpt_ctx *ctx, const uint16_t *d_thermal, const float *d_filtered, const int64_t *d_filtered_rows,
+                            const cpt_sample *d_samples, const cpt_track_norm *d_tracks, const int32_t *d_segment_samples,
+                            int n_segments, int tiles_per_segment, int frames_per_row, int frame_size,
+                            const int32_t *crop_rectangle, int preprocess_fn, float *d_out);
 
 /* ---- ml_tools/imageprocessing.py helpers on single images (device buffers) ----
  * normalize() (imageprocessing.py:151-169): cpt_minmax_f32 writes {min, max} of d_in to d_out2; cpt_normalize_f32
@@ -269,23 +257,19 @@ int cpt_normalize_f32(cpt_ctx *ctx, const float *d_in, int64_t n, double min, do
 int cpt_resize_pad_f32(cpt_ctx *ctx, const float *d_src, int src_w, int src_h, int resized_w, int resized_h, int offset_x,
                        int offset_y, int out_w, int out_h, float pad, int interpolation, float *d_out);
 
-/* detect_objects() (imageprocessing.py:240-248) on one uint8 image of any size: GaussianBlur (blur_ksize 5, or 0
- * for none) -> threshold (src > floor(threshold)) -> morphologyEx CLOSE with a tuple kernel (close != 0; OpenCV turns
- * the tuple into a 2x1 element) -> connectedComponentsWithStats (8-connectivity, OpenCV label numbering).
- * d_labels int32 [H][W]; d_stats int32 [max_components + 1][5] = left, top, width, height, area; d_centroids double
- * [max_components + 1][2]; row 0 is the background.  *h_count = number of labels including the background.
- * Synchronises the ctx stream. */
-int cpt_detect_objects_u8(cpt_ctx *ctx, const uint8_t *d_image, int width, int height, double threshold, int blur_ksize,
-                          int close, int max_components, int32_t *d_labels, int32_t *d_stats, double *d_centroids,
-                          int32_t *h_count);
-
-/* The same pipeline with every stage the imageprocessing.py variants use, on one uint8 image of any size:
+/* detect_objects() (imageprocessing.py:240-248) and its variants on one uint8 image of any size: the grey stages, a
+ * threshold (src > floor(threshold)), the binary stages, then connectedComponentsWithStats (8-connectivity, OpenCV label
+ * numbering).  steps selects the stages each variant uses:
  *   detect_objects(kernel=(15,15) default, otsus)   imageprocessing.py:240-248  blur_ksize 3 / 5 / 7 / 15 (cv2.GaussianBlur 8-bit
- *                                                   fixed-point taps), CPT_DETECT_OTSU (cv2.threshold THRESH_OTSU), CPT_DETECT_CLOSE
+ *                                                   fixed-point taps, 0 for none), CPT_DETECT_OTSU (cv2.threshold THRESH_OTSU),
+ *                                                   CPT_DETECT_CLOSE (morphologyEx CLOSE with a tuple kernel: OpenCV turns the
+ *                                                   tuple into a 2x1 element)
  *   detect_objects_ir (IR 640x480 frames)           imageprocessing.py:185-199  CPT_DETECT_OPEN_GRAY (cv2.morphologyEx MORPH_OPEN
  *                                                   with a tuple kernel = 2x1 element, on the grey image), threshold, components
  *   detect_objects_both                             imageprocessing.py:202-238  blur, threshold, CPT_DETECT_DILATE, CPT_DETECT_CLOSE,
  *                                                   d_or_mask (the thresholded saliency map, any non-zero = set) OR-ed in
+ * d_labels int32 [H][W]; d_stats int32 [max_components + 1][5] = left, top, width, height, area; d_centroids double
+ * [max_components + 1][2]; row 0 is the background.  *h_count = number of labels including the background.
  * CPT_DETECT_MASK_ONLY stops after the binary stages and writes the mask (0 / 255) to d_mask_out.  h_threshold_used (may
  * be NULL) receives the threshold applied (Otsu's when CPT_DETECT_OTSU).  For an image that is all foreground, the
  * background row is cv2's [-1, INT_MAX, 0, 0, 0] with a NaN centroid.  Synchronises the ctx stream. */
@@ -294,9 +278,9 @@ int cpt_detect_objects_u8(cpt_ctx *ctx, const uint8_t *d_image, int width, int h
 #define CPT_DETECT_DILATE 4u
 #define CPT_DETECT_OTSU 8u
 #define CPT_DETECT_MASK_ONLY 16u
-int cpt_detect_objects_ex(cpt_ctx *ctx, const uint8_t *d_image, int width, int height, double threshold, int blur_ksize,
-                          uint32_t steps, const uint8_t *d_or_mask, int max_components, int32_t *d_labels, int32_t *d_stats,
-                          double *d_centroids, uint8_t *d_mask_out, int32_t *h_count, double *h_threshold_used);
+int cpt_detect_objects(cpt_ctx *ctx, const uint8_t *d_image, int width, int height, double threshold, int blur_ksize,
+                       uint32_t steps, const uint8_t *d_or_mask, int max_components, int32_t *d_labels, int32_t *d_stats,
+                       double *d_centroids, uint8_t *d_mask_out, int32_t *h_count, double *h_threshold_used);
 
 /* detect_objects_ir (imageprocessing.py:185-199) on n_frames uint8 frames [n_frames][H][W] of one geometry in one call, with
  * no host synchronisation: steps CPT_DETECT_OPEN_GRAY (or 0) -> threshold -> connectedComponentsWithStats per frame.

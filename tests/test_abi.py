@@ -69,13 +69,28 @@ def test_product_never_imports_oracle():
                 assert "oracle" not in src.replace("no oracle", ""), os.path.join(dirpath, f)
 
 
+def test_no_product_module_calls_the_library_directly():
+    """native.py is the only caller of libcptrack.so: every other product module goes through its wrappers."""
+    pkg = os.path.join(ROOT, "classifier-pipeline_b200")
+    for dirpath, _, files in os.walk(pkg):
+        for f in files:
+            path = os.path.join(dirpath, f)
+            if f.endswith(".py") and path != os.path.join(pkg, "native.py"):
+                src = open(path).read()
+                assert "lib.cpt_" not in src and not re.search(r"\._h\b", src), path
+
+
 def test_clip_flags_match_header():
-    """The Python constants of the clip flags are the header's #defines."""
+    """The Python constants of the clip, detect, motion and preprocessing flags are the header's #defines."""
     from classifier_pipeline_b200 import native
 
     text = open(os.path.join(ROOT, "include", "cptrack.h")).read()
-    flags = {m.group(1): int(m.group(2)) for m in re.finditer(r"#define\s+CPT_CLIP_([A-Z_]+)\s+(\d+)u", text)}
-    assert set(flags) >= {"UPDATE_BACKGROUND", "RESUME", "DENOISE", "FRAME_STATS", "SKIP_FIRST_UPDATE", "PREV_IN_OUTPUT"}
-    for name, value in flags.items():
-        assert getattr(native, "CLIP_" + name) == value, name
-    assert len(set(flags.values())) == len(flags) and all(v & (v - 1) == 0 for v in flags.values())
+    for group, expected in (("CLIP", {"UPDATE_BACKGROUND", "RESUME", "DENOISE", "FRAME_STATS", "SKIP_FIRST_UPDATE", "PREV_IN_OUTPUT"}),
+                            ("DETECT", {"CLOSE", "OPEN_GRAY", "DILATE", "OTSU", "MASK_ONLY"}),
+                            ("MOTION", {"MEAN", "MEAN_RESTART", "BACKGROUND", "DETECT", "WARMER_ONLY", "ONE_DIFF"}),
+                            ("PREPROCESS", {"INC3", "PER_TILE"})):
+        flags = {m.group(1): int(m.group(2)) for m in re.finditer(r"#define\s+CPT_%s_([A-Z0-9_]+)\s+(\d+)u?\b" % group, text)}
+        assert set(flags) >= expected, group
+        for name, value in flags.items():
+            assert getattr(native, group + "_" + name) == value, group + "_" + name
+        assert len(set(flags.values())) == len(flags) and all(v & (v - 1) == 0 for v in flags.values()), group

@@ -1,6 +1,7 @@
-"""Classifier inputs straight from an extraction's device buffers: the cpt_preprocess_*_ex entry points against the
-existing ones on repacked frames, and ClipTrackExtractor.parse_clips(keep_on_device=True) + Interpreter.preprocess_clips
-against parse_clips + per-clip Interpreter.preprocess."""
+"""Classifier inputs straight from an extraction's device buffers: the cpt_preprocess_* entry points given the extraction's
+filtered rows, frame medians and frame records against the same entry points on repacked frames, and
+ClipTrackExtractor.parse_clips(keep_on_device=True) + Interpreter.preprocess_clips against parse_clips + per-clip
+Interpreter.preprocess."""
 import json
 import os
 

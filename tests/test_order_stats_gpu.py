@@ -162,7 +162,7 @@ def test_crop_medians_and_clip_decision_equal_numpy(kernel):
     else:
         d_med = torch.empty(len(frames), dtype=torch.float32, device="cuda")
         eng.ctx.frame_medians(d_thermal, len(frames), d_med)
-        eng.ctx.preprocess_medians_ex(d_thermal, d_med, d_smp, len(smp), d_tracks)
+        eng.ctx.preprocess_medians(d_thermal, d_smp, len(smp), d_tracks, d_frame_medians=d_med)
     got = d_smp.cpu().numpy().view(native.SAMPLE_DTYPE)
     tracks = BatchPreprocessor.tracks_numpy(d_tracks)
     assert np.array_equal(got["median"].astype(np.float64), want_median)
@@ -208,7 +208,8 @@ def test_thermal_limits_on_wide_range_frames_equal_oracle(kernel):
         info = np.zeros(n_frames, native.INFO_DTYPE)
         info["thermal_min"] = frames.reshape(n_frames, -1).min(1)
         info["thermal_max"] = frames.reshape(n_frames, -1).max(1)
-        eng.ctx.preprocess_thermal_limits_ex(d_thermal, None, d_lim, len(lim), d_tracks, len(tracks), d_med, _dev_bytes(torch, info))
+        eng.ctx.preprocess_thermal_limits(d_thermal, d_lim, len(lim), d_tracks, len(tracks), d_frame_medians=d_med,
+                                          d_frame_info=_dev_bytes(torch, info))
     got = BatchPreprocessor.tracks_numpy(d_tracks)
     assert (got["has_thermal_limits"] == 1).all()
     for ti, regs in enumerate(tracks):
