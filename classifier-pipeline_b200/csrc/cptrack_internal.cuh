@@ -126,5 +126,6 @@ struct cpt_ctx {
     cpt::Grow<uint8_t> detect_scratch;  // cpt_detect_objects / _batch: images, masks, union-find and component tables
     cpt::Grow<int> merge_order;  // cpt_ir_merge_components: list order of every frame of a launch
     cpt::Grow<uint8_t> motion_scratch;  // cpt_motion_clips: detector records, steps, mean rows, results, ring copies
+    cpt::Grow<uint8_t> ir_clips_scratch;  // cpt_ir_motion_clips: clip records, flags, steps, results, staged host frames
 };
 

@@ -4,119 +4,18 @@
 //   mog2_apply_kernel        apply() for T consecutive frames of one model: one thread per pixel, the pixel's modes in
 //                            registers for all T frames, the state read once at the start and written once at the end
 //   mog2_background_kernel   getBackgroundImage()
-// Every product, sum and quotient is a separately rounded intrinsic: cv2 evaluates a*b+c as two rounded operations, and a
-// fused multiply-add gives different background pixels.  The library is built with one set of nvcc flags, so the
-// rounding is pinned here rather than with -fmad=false.
-#include <algorithm>
-#include <cfloat>
-
-#include "cptrack_internal.cuh"
+// The per-pixel update, the state layout and the learning-rate rule are in mog2.cuh, shared with the IR motion detector's
+// kernel of whole clips (ir_kernels.cu).
+#include "mog2.cuh"
 
 namespace cpt {
 
-constexpr int kMog2Modes = 5;
 constexpr int kMog2MaxT = 256;  // frames per launch: the per-frame rates travel as kernel parameters (2 KB)
 
-struct Mog2Consts {
-    float Tb, TB, Tg, var_init, var_min, var_max;
-};
 struct Mog2Rates {
     float alpha[kMog2MaxT];  // alphaT = (float)learning rate
     float prune[kMog2MaxT];  // (float)(-learning rate * (double)complexity_reduction)
 };
-
-// State in HBM, structure of arrays over the npx pixels: float weight[5][npx], var[5][npx], mean[5][npx], then
-// uint8 used[npx] (the mode count).
-__host__ __device__ inline size_t mog2_state_bytes(int64_t npx) { return (size_t)npx * (3 * kMog2Modes * sizeof(float) + 1); }
-
-template <int N>
-__device__ __forceinline__ void swap_mode(float (&w)[N], float (&v)[N], float (&m)[N], int i) {
-    float t = w[i]; w[i] = w[i - 1]; w[i - 1] = t;
-    t = v[i]; v[i] = v[i - 1]; v[i - 1] = t;
-    t = m[i]; m[i] = m[i - 1]; m[i - 1] = t;
-}
-
-// One apply() of one pixel.  Indices into w / v / m are compile-time constants after unrolling (a runtime index would put
-// the arrays in local memory): the loops of the scalar algorithm become predicated chains with the same break conditions.
-// Returns 1 when the pixel is background.
-__device__ __forceinline__ int mog2_pixel(float (&w)[kMog2Modes], float (&v)[kMog2Modes], float (&m)[kMog2Modes], int &nmodes,
-                                          float data, float alphaT, float prune, const Mog2Consts &c) {
-    const float alpha1 = __fsub_rn(1.f, alphaT);
-    int background = 0, fits = 0;
-    float totalWeight = 0.f;
-#pragma unroll
-    for (int mode = 0; mode < kMog2Modes; ++mode) {
-        if (mode >= nmodes) break;  // nmodes shrinks inside the loop (a pruned mode stays in place with weight 0)
-        float weight = __fadd_rn(__fmul_rn(alpha1, w[mode]), prune);
-        int swap_count = 0;
-        if (!fits) {
-            const float var = v[mode];
-            const float d = __fsub_rn(m[mode], data);
-            const float dist2 = __fmul_rn(d, d);
-            if (totalWeight < c.TB && dist2 < __fmul_rn(c.Tb, var)) background = 1;
-            if (dist2 < __fmul_rn(c.Tg, var)) {
-                fits = 1;
-                weight = __fadd_rn(weight, alphaT);
-                const float k = __fdiv_rn(alphaT, weight);
-                m[mode] = __fsub_rn(m[mode], __fmul_rn(k, d));
-                float varnew = __fadd_rn(var, __fmul_rn(k, __fsub_rn(dist2, var)));
-                varnew = varnew > c.var_min ? varnew : c.var_min;
-                varnew = varnew < c.var_max ? varnew : c.var_max;
-                v[mode] = varnew;
-                // bubble the mode up while its new weight is >= the one above (equal weights swap)
-                bool moving = true;
-#pragma unroll
-                for (int i = mode; i > 0; --i) {
-                    moving = moving && !(weight < w[i - 1]);
-                    if (moving) {
-                        swap_mode(w, v, m, i);
-                        ++swap_count;
-                    }
-                }
-            }
-        }
-        if (weight < -prune) {
-            weight = 0.f;
-            --nmodes;
-        }
-#pragma unroll
-        for (int j = 0; j <= mode; ++j)
-            if (j == mode - swap_count) w[j] = weight;
-        totalWeight = __fadd_rn(totalWeight, weight);
-    }
-    // cv2 4.x renormalises with 0 when every mode it visited was pruned (a learning rate near 1 prunes all modes before the
-    // fitting one); 1 / totalWeight would turn the remaining weights into NaN
-    const float invWeight = fabsf(totalWeight) > FLT_EPSILON ? __fdiv_rn(1.f, totalWeight) : 0.f;
-#pragma unroll
-    for (int j = 0; j < kMog2Modes; ++j)
-        if (j < nmodes) w[j] = __fmul_rn(w[j], invWeight);
-    if (!fits && alphaT > 0.f) {
-        const int mode = nmodes == kMog2Modes ? kMog2Modes - 1 : nmodes++;
-#pragma unroll
-        for (int j = 0; j < kMog2Modes; ++j) {
-            if (nmodes == 1) {
-                if (j == mode) w[j] = 1.f;
-            } else if (j == mode) {
-                w[j] = alphaT;
-            } else if (j < nmodes - 1) {
-                w[j] = __fmul_rn(w[j], alpha1);
-            }
-            if (j == mode) {
-                m[j] = data;
-                v[j] = c.var_init;
-            }
-        }
-        bool moving = true;
-#pragma unroll
-        for (int i = kMog2Modes - 1; i > 0; --i) {
-            if (i < nmodes) {
-                moving = moving && !(alphaT < w[i - 1]);
-                if (moving) swap_mode(w, v, m, i);
-            }
-        }
-    }
-    return background;
-}
 
 // fresh != 0: the model starts empty (cv2's initialisation: zero modes) and the state is not read.  masks may be null.
 __global__ void __launch_bounds__(256) mog2_apply_kernel(float *__restrict__ state, int64_t npx, const uint8_t *__restrict__ frames,
@@ -124,22 +23,9 @@ __global__ void __launch_bounds__(256) mog2_apply_kernel(float *__restrict__ sta
                                                           uint8_t *__restrict__ masks) {
     const int64_t x = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (x >= npx) return;
-    float *sw = state, *sv = state + kMog2Modes * npx, *sm = state + 2 * kMog2Modes * npx;
-    uint8_t *used = reinterpret_cast<uint8_t *>(state + 3 * kMog2Modes * npx);
     float w[kMog2Modes], v[kMog2Modes], m[kMog2Modes];
-    int nmodes = 0;
-    if (fresh) {
-#pragma unroll
-        for (int j = 0; j < kMog2Modes; ++j) w[j] = v[j] = m[j] = 0.f;
-    } else {
-#pragma unroll
-        for (int j = 0; j < kMog2Modes; ++j) {
-            w[j] = sw[j * npx + x];
-            v[j] = sv[j * npx + x];
-            m[j] = sm[j * npx + x];
-        }
-        nmodes = used[x];
-    }
+    int nmodes;
+    mog2_load(state, npx, x, fresh, w, v, m, nmodes);
     const uint8_t *f = frames + x;
     uint8_t next = __ldg(f);
     for (int t = 0; t < T; ++t) {
@@ -148,13 +34,7 @@ __global__ void __launch_bounds__(256) mog2_apply_kernel(float *__restrict__ sta
         const int bg = mog2_pixel(w, v, m, nmodes, data, r.alpha[t], r.prune[t], c);
         if (masks) masks[(int64_t)t * npx + x] = bg ? 0 : 255;
     }
-#pragma unroll
-    for (int j = 0; j < kMog2Modes; ++j) {
-        sw[j * npx + x] = w[j];
-        sv[j * npx + x] = v[j];
-        sm[j * npx + x] = m[j];
-    }
-    used[x] = (uint8_t)nmodes;
+    mog2_store(state, npx, x, w, v, m, nmodes);
 }
 
 __global__ void __launch_bounds__(256) mog2_background_kernel(const float *__restrict__ state, int64_t npx, float TB,
@@ -180,17 +60,6 @@ __global__ void __launch_bounds__(256) mog2_background_kernel(const float *__res
 }  // namespace cpt
 
 using cpt::fail;
-
-struct cpt_mog2 {
-    cpt_ctx *ctx;
-    int W, H;
-    int64_t npx;
-    int history;
-    float complexity_reduction;
-    cpt::Mog2Consts c;
-    int nframes;     // cv2's nframes: frames since the last initialisation
-    float *d_state;  // mog2_state_bytes(npx)
-};
 
 extern "C" {
 
@@ -263,15 +132,11 @@ int cpt_mog2_apply(cpt_mog2 *m, const uint8_t *d_frames, int n_frames, int64_t f
         int fresh = 0, t = 0;
         while (i < n_frames && t < cpt::kMog2MaxT) {
             const double lr_arg = h_learning_rates[i];
-            if (m->nframes == 0 || lr_arg >= 1) {
+            if (cpt::mog2_reinitialises(m->nframes, lr_arg)) {
                 if (t > 0) break;
                 fresh = 1;
-                m->nframes = 0;
             }
-            ++m->nframes;
-            const double lr = (lr_arg >= 0 && m->nframes > 1) ? lr_arg : 1.0 / (double)std::min(2 * m->nframes, m->history);
-            r.alpha[t] = (float)lr;
-            r.prune[t] = (float)(-lr * (double)m->complexity_reduction);
+            cpt::mog2_next_rate(*m, m->nframes, lr_arg, r.alpha[t], r.prune[t]);
             ++t;
             ++i;
         }

@@ -85,6 +85,26 @@ class CptMotionClip(ctypes.Structure):
                 ("n_steps", ctypes.c_int32), ("reserved", ctypes.c_int32)]
 
 
+class CptIrMotionClipStep(ctypes.Structure):
+    _fields_ = [("row", ctypes.c_int64), ("slot_new", ctypes.c_int32), ("slot_oldest", ctypes.c_int32), ("detect", ctypes.c_int32),
+                ("reserved", ctypes.c_int32)]
+
+
+class CptIrMotionClip(ctypes.Structure):
+    _fields_ = [("m", ctypes.c_void_p), ("mog2", ctypes.c_void_p), ("d_mask", ctypes.c_void_p), ("first_step", ctypes.c_int32),
+                ("n_steps", ctypes.c_int32), ("movement", ctypes.c_int32), ("triggered", ctypes.c_int32)]
+
+
+class CptIrMotionClipParams(ctypes.Structure):
+    _fields_ = [("threshold", ctypes.c_int32), ("trigger_frames", ctypes.c_int32), ("max_triggered", ctypes.c_int32),
+                ("erode_idle", ctypes.c_int32), ("erode_recording", ctypes.c_int32), ("host_frames", ctypes.c_int32)]
+
+
+class CptIrMotionClipResult(ctypes.Structure):
+    _fields_ = [("movement", ctypes.c_int32), ("triggered", ctypes.c_int32), ("diff_pixels", ctypes.c_int32),
+                ("mask_pixels", ctypes.c_int32)]
+
+
 class CptMog2Params(ctypes.Structure):
     _fields_ = [("history", ctypes.c_int), ("var_threshold", ctypes.c_double), ("background_ratio", ctypes.c_double),
                 ("var_threshold_gen", ctypes.c_float), ("var_init", ctypes.c_float), ("var_min", ctypes.c_float),
@@ -116,6 +136,8 @@ assert REGION_DTYPE.itemsize == ctypes.sizeof(CptRegion) == 40
 assert INFO_DTYPE.itemsize == ctypes.sizeof(CptFrameInfo) == 64
 assert CLIP_DTYPE.itemsize == ctypes.sizeof(CptClip) == 48
 assert ctypes.sizeof(CptMotionClipStep) == 32 and ctypes.sizeof(CptMotionClip) == 48
+assert ctypes.sizeof(CptIrMotionClipStep) == 24 and ctypes.sizeof(CptIrMotionClip) == 40
+assert ctypes.sizeof(CptIrMotionClipParams) == 24 and ctypes.sizeof(CptIrMotionClipResult) == 16
 
 # every symbol include/cptrack.h declares: (name, restype, argtypes)
 _vp, _i, _i64, _u64, _d, _f = ctypes.c_void_p, ctypes.c_int, ctypes.c_int64, ctypes.c_uint64, ctypes.c_double, ctypes.c_float
@@ -161,6 +183,7 @@ SYMBOLS = {
     "cpt_ir_motion_detect": (_i, [_vp, _i, _i, _i, _i, _vp, ctypes.POINTER(ctypes.c_int32), ctypes.POINTER(ctypes.c_int32)]),
     "cpt_ir_motion_ring_slot": (_vp, [_vp, _i]),
     "cpt_ir_motion_detect_ex": (_i, [_vp, _i, _i, _i, _i, _vp, ctypes.POINTER(ctypes.c_int32), ctypes.POINTER(ctypes.c_int32)]),
+    "cpt_ir_motion_clips": (_i, [_vp, _vp, _i, _vp, _i64, _vp, _i, ctypes.POINTER(CptIrMotionClipParams), _vp]),
     "cpt_mog2_open": (_vp, [_vp, _i, _i, ctypes.POINTER(CptMog2Params)]),
     "cpt_mog2_close": (None, [_vp]),
     "cpt_mog2_apply": (_i, [_vp, _vp, _i, _i64, _vp, _vp]),
@@ -362,6 +385,14 @@ class Context:
         check(self.lib.cpt_motion_clips(self._h, h_clips, int(n_clips), _ptr(d_frames), int(n_frames), h_steps, int(n_steps),
                                         _ptr(h_mean_rows), int(n_mean_rows), h_results))
 
+    def ir_motion_clips(self, h_clips, n_clips, h_frames, n_frames, h_steps, n_steps, params, h_results):
+        """cpt_ir_motion_clips: h_clips CptIrMotionClip [n_clips] (``IrMotion.clip_record``; movement / triggered are updated),
+        h_frames uint64 [n_frames] frame addresses (host or device as ``params.host_frames`` says), h_steps
+        CptIrMotionClipStep [n_steps], params CptIrMotionClipParams and h_results CptIrMotionClipResult [n_steps], all on the
+        host.  Waits for the steps to finish."""
+        check(self.lib.cpt_ir_motion_clips(self._h, h_clips, int(n_clips), _ptr(h_frames), int(n_frames), h_steps, int(n_steps),
+                                           ctypes.byref(params), h_results))
+
     def nlm_denoise_u8(self, d_src, width, height, n_frames, d_dst):
         check(self.lib.cpt_nlm_denoise_u8(self._h, _ptr(d_src), int(width), int(height), int(n_frames), _ptr(d_dst)))
 
@@ -480,6 +511,12 @@ class IrMotion(_Handle):
         check(self.ctx.lib.cpt_ir_motion_detect(self._h, int(slot_new), int(slot_oldest), int(threshold), int(erode_k), _ptr(mask),
                                                 ctypes.byref(diff), ctypes.byref(cnt)))
         return diff.value, cnt.value
+
+    def clip_record(self, mog2, d_mask, first_step, n_steps, movement, triggered):
+        """This detector's CptIrMotionClip of a ``Context.ir_motion_clips`` call: ``mog2`` its ``Mog2`` model, ``d_mask`` the
+        [H][W] uint8 CUDA tensor that receives the foreground masks."""
+        return CptIrMotionClip(self._h, mog2.address, _dptr(d_mask, self.height * self.width), int(first_step), int(n_steps),
+                               int(bool(movement)), int(triggered))
 
 
 def _dptr(t, min_bytes):

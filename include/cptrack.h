@@ -420,6 +420,54 @@ const uint8_t *cpt_ir_motion_ring_slot(cpt_ir_motion *m, int slot);
 int cpt_ir_motion_detect_ex(cpt_ir_motion *m, int slot_new, int slot_oldest, int threshold, int erode_k, const uint8_t *d_mask,
                             int32_t *h_diff_pixels, int32_t *h_mask_pixels);
 
+/* Whole IR recordings, many detectors, with each frame's trigger decided on the device (irmotiondetector.py:103-153 for
+ * every frame of each detector's frame list, with the device MOG2 of cpt_mog2 as background model).  The host plans the
+ * ring cursors and which frames detect; the device runs, for every step: grey into ring slot slot_new, the MOG2 update of
+ * the clip's model with learning rate 0 while the clip's movement flag is set and cv2's automatic rate otherwise, the
+ * foreground mask into the clip's d_mask, and with detect the two eroded counts (box erode_recording while recording,
+ * erode_idle otherwise) and the trigger rule: the mask count is min(diff, mask) while recording, triggered moves by one
+ * within [0, max_triggered], movement starts at triggered >= trigger_frames and ends at triggered <= 0.  Steps of one clip
+ * run in order; the movement flag each step reads is the one the clip's previous step left, with no host round trip.
+ * h_frames holds n_frames addresses of [H][W][3] uint8 BGR frames: device memory, or host memory with host_frames = 1
+ * (copied with cudaMemcpyAsync, in chunks of about 256 MB of the context's scratch).  Each clip's model advances its frame
+ * count as cpt_mog2_apply with learning rates -1 / 0 would.  Every handle (on ctx, one geometry, each ir / MOG2 handle and
+ * mask once), frame row, ring slot, step range and erosion size is checked before anything is launched or changed:
+ * CPT_ERR_INVALID.  The call synchronises once, at the end; movement / triggered of each clip record then hold the
+ * clip's state after its last step. */
+typedef struct {
+    int64_t row;          /* the step's BGR frame: h_frames[row] */
+    int32_t slot_new;     /* ring slot the grey frame goes to (SlidingWindow.last_index after add) */
+    int32_t slot_oldest;  /* the ring slot it is compared with (SlidingWindow.oldest_index; == slot_new in a ring of one) */
+    int32_t detect;       /* 1: erode, count and decide (num_frames > MIN_FRAMES); 0: grey and MOG2 only */
+    int32_t reserved;
+} cpt_ir_motion_clip_step;
+typedef struct {
+    cpt_ir_motion *m;     /* the detector's grey ring */
+    struct cpt_mog2 *mog2; /* its background model (cpt_mog2 below), of the same geometry */
+    uint8_t *d_mask;      /* [H][W]: each step's foreground mask (0 / 255); the last one stays */
+    int32_t first_step;   /* this clip's steps: h_steps[first_step .. first_step + n_steps) */
+    int32_t n_steps;
+    int32_t movement;     /* movement_detected on entry; on return, after the last step */
+    int32_t triggered;    /* triggered on entry; on return, after the last step */
+} cpt_ir_motion_clip;
+typedef struct {
+    int32_t threshold;        /* |oldest grey - grey| > threshold is a changed pixel (THRESHOLD) */
+    int32_t trigger_frames;   /* TRIGGER_FRAMES */
+    int32_t max_triggered;    /* the cap of triggered */
+    int32_t erode_idle;       /* erosion box while not recording, 1..64 */
+    int32_t erode_recording;  /* erosion box while recording, 1..64 */
+    int32_t host_frames;      /* 1: h_frames are host addresses */
+} cpt_ir_motion_clip_params;
+typedef struct {
+    int32_t movement;     /* movement_detected after the step */
+    int32_t triggered;    /* triggered after the step */
+    int32_t diff_pixels;  /* eroded counts before the min rule; -1 for a step without detect */
+    int32_t mask_pixels;
+} cpt_ir_motion_clip_result;
+int cpt_ir_motion_clips(cpt_ctx *ctx, cpt_ir_motion_clip *h_clips, int n, const uint8_t *const *h_frames, int64_t n_frames,
+                        const cpt_ir_motion_clip_step *h_steps, int n_steps, const cpt_ir_motion_clip_params *params,
+                        cpt_ir_motion_clip_result *h_results);
+
 /* ---- OpenCV's BackgroundSubtractorMOG2 (track/cliptracker.py:560-609 CVBackground; the IR detector's background model) ----
  * cv2.createBackgroundSubtractorMOG2(history, varThreshold, detectShadows=False) on one uint8 channel with five modes, bit for
  * bit: every foreground mask of apply() and getBackgroundImage().  The model's state (61 bytes per pixel) stays on the
