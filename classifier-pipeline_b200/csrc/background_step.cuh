@@ -1,5 +1,5 @@
 // background_step.cuh -- WeightedBackground.process_frame (piclassifier/motiondetector.py:197-244) on one state
-// record by one CTA; shared by background_step_kernel (aux_kernels.cu) and motion_step_kernel (motion_kernels.cu).
+// record by one CTA; shared by background_step_kernel (aux_kernels.cu) and motion_phases (motion_kernels.cu).
 #pragma once
 #include "cptrack_kernels.cuh"
 

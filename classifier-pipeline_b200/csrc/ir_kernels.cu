@@ -45,7 +45,7 @@ struct IrStep {
 };
 struct IrRule {
     int threshold, trigger_frames, max_triggered, erode_idle, erode_recording;
-    int decide;  // 0: counts only (cpt_ir_motion_detect_ex)
+    int decide;  // 0: counts only (cpt_ir_motion_detect)
 };
 
 __device__ __forceinline__ uint8_t bgr_to_gray(const uint8_t *p) {
@@ -363,18 +363,70 @@ __global__ void __launch_bounds__(128) ir_merge_kernel(const int32_t *stats, con
 
 using cpt::fail;
 
+// The leading members (ctx, W, H, ring_frames, d_ring) are read through the handle's address (native.py, _IrMotionHead);
+// keep their order.
 struct cpt_ir_motion {
     cpt_ctx *ctx;
     int W, H, ring_frames;
-    uint8_t *d_bgr, *d_ring, *d_in_mask;
+    uint8_t *d_ring;   // [ring_frames][H][W] grey
+    uint8_t *d_bgr;    // [H][W][3] BGR, then at ir_records_offset cpt_ir_motion_step's IrStepRecords and cpt_ir_motion_detect's
+    uint8_t *d_in_mask;
     uint32_t *d_bits;  // [2][H][words per row]: bit planes of the difference and of the foreground mask
-    // cpt_ir_motion_detect_ex's one-clip, one-step launch of ir_erode_kernel: its records, set once at open
-    cpt::IrClipArgs *d_args;
-    cpt::IrStep *d_step;
-    cpt::IrClipFlag *d_flag;
-    cpt_ir_motion_clip_result *d_result;
-    uint8_t *h_pin;  // pinned staging: bgr in, grey / counts out
+    struct IrStepRecords *d_detect;  // the one-clip, one-step records of cpt_ir_motion_detect's ir_erode_kernel, set at open
+    uint8_t *h_pin;  // pinned staging laid out as d_bgr: BGR and records in; grey, counts and records out
 };
+
+// A one-clip, one-step launch's records (cpt_ir_motion_step's go up with the frame; flag and result come back together).
+struct IrStepRecords {
+    cpt::IrClipArgs args;
+    cpt::IrStep step;
+    cpt::IrClipFlag flag;
+    cpt_ir_motion_clip_result result;
+};
+static_assert(offsetof(IrStepRecords, result) == offsetof(IrStepRecords, flag) + sizeof(cpt::IrClipFlag), "flag, then result");
+static size_t ir_records_offset(size_t npx) { return (3 * npx + 255) & ~(size_t)255; }
+
+static int ir_check_params(const cpt_ir_motion_clip_params *p) {
+    if (p->erode_idle < 1 || p->erode_idle > cpt::kErodeMaxK || p->erode_recording < 1 || p->erode_recording > cpt::kErodeMaxK)
+        return fail(CPT_ERR_INVALID, "erosion boxes must be 1..64 pixels");
+    return CPT_OK;
+}
+
+// Clip d: both handles on ctx c, of the call's W x H geometry (W == 0: clip d sets it), and a mask buffer.
+static int ir_check_clip(cpt_ctx *c, const cpt_ir_motion_clip &k, int d, int &W, int &H) {
+    const cpt_ir_motion *m = k.m;
+    const cpt_mog2 *g = k.mog2;
+    if (!m || !g || m->ctx != c || g->ctx != c) return fail(CPT_ERR_INVALID, "clip %d: a handle is missing or belongs to another context", d);
+    if (W == 0) { W = m->W; H = m->H; }
+    if (m->W != W || m->H != H || g->W != W || g->H != H)
+        return fail(CPT_ERR_INVALID, "clip %d: the handles do not share one %d x %d geometry", d, W, H);
+    if (!k.d_mask) return fail(CPT_ERR_INVALID, "clip %d has no mask buffer", d);
+    return CPT_OK;
+}
+
+static int ir_check_slots(const cpt_ir_motion *m, const cpt_ir_motion_clip_step &st, int i) {
+    if (st.slot_new < 0 || st.slot_new >= m->ring_frames || st.slot_oldest < 0 || st.slot_oldest >= m->ring_frames)
+        return fail(CPT_ERR_INVALID, "step %d: ring slot out of range", i);
+    return CPT_OK;
+}
+
+// The device records of clip k and of its steps h_steps[k.first_step .. + k.n_steps), all but each step's frame address:
+// each step's rate pair of both learning rates it may take, from cv2's rule (mog2.cuh), with the model's frame count
+// advanced once per step.
+static void ir_clip_records(const cpt_ir_motion_clip &k, const cpt_ir_motion_clip_step *h_steps, cpt::IrClipArgs &args,
+                            cpt::IrClipFlag &flag, cpt::IrStep *steps) {
+    args = cpt::IrClipArgs{k.m->d_ring, k.mog2->d_state, k.d_mask, k.m->d_bits, k.mog2->c, k.first_step, k.n_steps};
+    flag = cpt::IrClipFlag{k.movement != 0, k.triggered, 0, 0, 0u, {0, 0, 0}};
+    for (int i = k.first_step; i < k.first_step + k.n_steps; ++i) {
+        const cpt_ir_motion_clip_step &st = h_steps[i];
+        cpt::IrStep &s = steps[i];
+        s.slot_new = st.slot_new; s.slot_oldest = st.slot_oldest; s.detect = st.detect != 0;
+        s.fresh = cpt::mog2_reinitialises(k.mog2->nframes, -1.0);
+        int frozen = k.mog2->nframes;
+        cpt::mog2_next_rate(*k.mog2, frozen, 0.0, s.alpha[1], s.prune[1]);
+        cpt::mog2_next_rate(*k.mog2, k.mog2->nframes, -1.0, s.alpha[0], s.prune[0]);
+    }
+}
 
 extern "C" {
 
@@ -390,24 +442,21 @@ cpt_ir_motion *cpt_ir_motion_open(cpt_ctx *c, int width, int height, int ring_fr
     cpt_ir_motion *m = new cpt_ir_motion();
     m->ctx = c; m->W = width; m->H = height; m->ring_frames = ring_frames;
     const size_t n = (size_t)width * height, wpr = (width + 31) / 32;
-    if (cudaMalloc(&m->d_bgr, 3 * n) != cudaSuccess || cudaMalloc(&m->d_ring, n * ring_frames) != cudaSuccess ||
+    const size_t stage = ir_records_offset(n) + sizeof(IrStepRecords);
+    if (cudaMalloc(&m->d_bgr, stage + sizeof(IrStepRecords)) != cudaSuccess || cudaMalloc(&m->d_ring, n * ring_frames) != cudaSuccess ||
         cudaMalloc(&m->d_in_mask, n) != cudaSuccess || cudaMalloc(&m->d_bits, 2 * height * wpr * sizeof(uint32_t)) != cudaSuccess ||
-        cudaMalloc(&m->d_args, sizeof(cpt::IrClipArgs)) != cudaSuccess || cudaMalloc(&m->d_step, sizeof(cpt::IrStep)) != cudaSuccess ||
-        cudaMalloc(&m->d_flag, sizeof(cpt::IrClipFlag)) != cudaSuccess ||
-        cudaMalloc(&m->d_result, sizeof(cpt_ir_motion_clip_result)) != cudaSuccess ||
-        cudaHostAlloc((void **)&m->h_pin, 3 * n + 64, cudaHostAllocDefault) != cudaSuccess) {
+        cudaHostAlloc((void **)&m->h_pin, stage, cudaHostAllocDefault) != cudaSuccess) {
         fail(CPT_ERR_NOMEM, "IR motion detector allocation failed");
         cpt_ir_motion_close(m);
         return nullptr;
     }
-    cpt::IrClipArgs args{};
-    args.bits = m->d_bits;
-    args.first_step = 0; args.n_steps = 1;
-    cpt::IrStep step{};
-    step.detect = 1;
-    if (cudaMemset(m->d_ring, 0, n * ring_frames) != cudaSuccess || cudaMemset(m->d_flag, 0, sizeof(cpt::IrClipFlag)) != cudaSuccess ||
-        cudaMemcpy(m->d_args, &args, sizeof(args), cudaMemcpyHostToDevice) != cudaSuccess ||
-        cudaMemcpy(m->d_step, &step, sizeof(step), cudaMemcpyHostToDevice) != cudaSuccess) {
+    m->d_detect = reinterpret_cast<IrStepRecords *>(m->d_bgr + stage);
+    IrStepRecords detect{};
+    detect.args.bits = m->d_bits;
+    detect.args.n_steps = 1;
+    detect.step.detect = 1;
+    if (cudaMemset(m->d_ring, 0, n * ring_frames) != cudaSuccess ||
+        cudaMemcpy(m->d_detect, &detect, sizeof(detect), cudaMemcpyHostToDevice) != cudaSuccess) {
         fail(CPT_ERR_CUDA, "IR motion detector initialisation failed");
         cpt_ir_motion_close(m);
         return nullptr;
@@ -420,7 +469,6 @@ void cpt_ir_motion_close(cpt_ir_motion *m) {
     cudaSetDevice(m->ctx->device);
     cudaStreamSynchronize(m->ctx->stream);
     cudaFree(m->d_bgr); cudaFree(m->d_ring); cudaFree(m->d_in_mask); cudaFree(m->d_bits);
-    cudaFree(m->d_args); cudaFree(m->d_step); cudaFree(m->d_flag); cudaFree(m->d_result);
     cudaFreeHost(m->h_pin);
     delete m;
 }
@@ -445,58 +493,74 @@ int cpt_ir_motion_gray(cpt_ir_motion *m, const uint8_t *h_bgr, int slot_new, uin
     return CPT_OK;
 }
 
-const uint8_t *cpt_ir_motion_ring_slot(cpt_ir_motion *m, int slot) {
-    if (!m) {
-        fail(CPT_ERR_INVALID, "null argument");
-        return nullptr;
-    }
-    if (slot < 0 || slot >= m->ring_frames) {
-        fail(CPT_ERR_INVALID, "ring slot out of range");
-        return nullptr;
-    }
-    return m->d_ring + (size_t)slot * m->W * m->H;
-}
-
-int cpt_ir_motion_detect_ex(cpt_ir_motion *m, int slot_new, int slot_oldest, int threshold, int erode_k, const uint8_t *d_mask,
-                            int32_t *h_diff_pixels, int32_t *h_mask_pixels) {
+int cpt_ir_motion_detect(cpt_ir_motion *m, int slot_new, int slot_oldest, int threshold, int erode_k, const uint8_t *h_mask,
+                         int32_t *h_diff_pixels, int32_t *h_mask_pixels) {
     if (!m || !h_diff_pixels) return fail(CPT_ERR_INVALID, "null argument");
     if (slot_new < 0 || slot_new >= m->ring_frames || slot_oldest < 0 || slot_oldest >= m->ring_frames)
         return fail(CPT_ERR_INVALID, "ring slot out of range");
     if (erode_k < 1 || erode_k > cpt::kErodeMaxK) return fail(CPT_ERR_INVALID, "erosion box must be 1..64 pixels");
-    if (d_mask && !h_mask_pixels) return fail(CPT_ERR_INVALID, "h_mask_pixels is required with a mask");
+    if (h_mask && !h_mask_pixels) return fail(CPT_ERR_INVALID, "h_mask_pixels is required with h_mask");
     cpt_ctx *c = m->ctx;
     CUDA_TRY(cudaSetDevice(c->device));
     const int W = m->W, H = m->H, wpr = (W + 31) / 32;
     const size_t n = (size_t)W * H;
     cudaStream_t st = c->stream;
+    if (h_mask) {
+        // the host mask goes through pinned staging into the detector's own device buffer
+        CUDA_TRY(cudaStreamSynchronize(st));  // h_pin may still be the source of an earlier copy
+        memcpy(m->h_pin, h_mask, n);
+        CUDA_TRY(cudaMemcpyAsync(m->d_in_mask, m->h_pin, n, cudaMemcpyHostToDevice, st));
+    }
+    const uint8_t *d_mask = h_mask ? m->d_in_mask : nullptr;
     cpt::ir_pack_kernel<<<(H * wpr + 7) / 8, 256, 0, st>>>(m->d_ring + slot_oldest * n, m->d_ring + slot_new * n, d_mask, W, H, wpr,
                                                            threshold, m->d_bits);
     const cpt::IrRule rule{threshold, 0, 0, erode_k, erode_k, 0};
-    cpt::ir_erode_kernel<<<dim3(cpt::erode_ctas(H, wpr), 1), 256, 0, st>>>(m->d_args, m->d_flag, m->d_step, 0, 0, W, H, wpr,
-                                                                          d_mask ? 2 : 1, rule, m->d_result);
+    IrStepRecords *d = m->d_detect;
+    cpt::ir_erode_kernel<<<dim3(cpt::erode_ctas(H, wpr), 1), 256, 0, st>>>(&d->args, &d->flag, &d->step, 0, 0, W, H, wpr,
+                                                                          d_mask ? 2 : 1, rule, &d->result);
     CUDA_TRY(cudaGetLastError());
     auto *h_result = reinterpret_cast<cpt_ir_motion_clip_result *>(m->h_pin + 3 * n);
-    CUDA_TRY(cudaMemcpyAsync(h_result, m->d_result, sizeof(*h_result), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaMemcpyAsync(h_result, &d->result, sizeof(*h_result), cudaMemcpyDeviceToHost, st));
     CUDA_TRY(cudaStreamSynchronize(st));
     *h_diff_pixels = h_result->diff_pixels;
     if (h_mask_pixels) *h_mask_pixels = d_mask ? h_result->mask_pixels : 0;
     return CPT_OK;
 }
 
-int cpt_ir_motion_detect(cpt_ir_motion *m, int slot_new, int slot_oldest, int threshold, int erode_k, const uint8_t *h_mask,
-                         int32_t *h_diff_pixels, int32_t *h_mask_pixels) {
-    if (!m) return fail(CPT_ERR_INVALID, "null argument");
-    if (h_mask && !h_mask_pixels) return fail(CPT_ERR_INVALID, "h_mask_pixels is required with h_mask");
-    if (h_mask) {
-        // the host mask goes through pinned staging into the detector's own device buffer
-        const int n = m->W * m->H;
-        CUDA_TRY(cudaSetDevice(m->ctx->device));
-        CUDA_TRY(cudaStreamSynchronize(m->ctx->stream));  // h_pin may still be the source of an earlier copy
-        memcpy(m->h_pin, h_mask, n);
-        CUDA_TRY(cudaMemcpyAsync(m->d_in_mask, m->h_pin, n, cudaMemcpyHostToDevice, m->ctx->stream));
+int cpt_ir_motion_step(cpt_ir_motion_clip *h_clip, const uint8_t *h_bgr, const cpt_ir_motion_clip_step *h_step,
+                       const cpt_ir_motion_clip_params *p, cpt_ir_motion_clip_result *h_result) {
+    if (!h_clip || !h_bgr || !h_step || !p || !h_result) return fail(CPT_ERR_INVALID, "null argument");
+    cpt_ir_motion_clip k = *h_clip;
+    k.first_step = 0; k.n_steps = 1;
+    int W = 0, H = 0, rc = ir_check_params(p);
+    if (!rc) rc = ir_check_clip(k.m ? k.m->ctx : nullptr, k, 0, W, H);
+    if (!rc) rc = ir_check_slots(k.m, *h_step, 0);
+    if (rc) return rc;
+    cpt_ir_motion *m = k.m;
+    CUDA_TRY(cudaSetDevice(m->ctx->device));
+    cudaStream_t st = m->ctx->stream;
+    CUDA_TRY(cudaStreamSynchronize(st));  // h_pin may still be the source of an earlier copy
+    const size_t n = (size_t)W * H, off = ir_records_offset(n);
+    auto *h = reinterpret_cast<IrStepRecords *>(m->h_pin + off), *d = reinterpret_cast<IrStepRecords *>(m->d_bgr + off);
+    ir_clip_records(k, h_step, h->args, h->flag, &h->step);
+    h->step.bgr = m->d_bgr;
+    // frame and records go up in four slices, each copy overlapping the memcpy of the next slice into the pinned buffer
+    const size_t total = off + sizeof(IrStepRecords), slice = (total + 3) / 4;
+    for (size_t o = 0; o < total; o += slice) {
+        if (o < 3 * n) memcpy(m->h_pin + o, h_bgr + o, std::min(slice, 3 * n - o));
+        CUDA_TRY(cudaMemcpyAsync(m->d_bgr + o, m->h_pin + o, std::min(slice, total - o), cudaMemcpyHostToDevice, st));
     }
-    return cpt_ir_motion_detect_ex(m, slot_new, slot_oldest, threshold, erode_k, h_mask ? m->d_in_mask : nullptr, h_diff_pixels,
-                                   h_mask_pixels);
+    const int wpr = (W + 31) / 32;
+    const cpt::IrRule rule{p->threshold, p->trigger_frames, p->max_triggered, p->erode_idle, p->erode_recording, 1};
+    cpt::ir_frame_kernel<<<dim3((H * wpr + 7) / 8, 1), 256, 0, st>>>(&d->args, &d->flag, &d->step, 0, 0, W, H, wpr, p->threshold);
+    cpt::ir_erode_kernel<<<dim3(cpt::erode_ctas(H, wpr), 1), 256, 0, st>>>(&d->args, &d->flag, &d->step, 0, 0, W, H, wpr, 2, rule, &d->result);
+    CUDA_TRY(cudaGetLastError());
+    CUDA_TRY(cudaMemcpyAsync(&h->flag, &d->flag, sizeof(h->flag) + sizeof(h->result), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    h_clip->movement = h->flag.movement;
+    h_clip->triggered = h->flag.triggered;
+    *h_result = h->result;
+    return CPT_OK;
 }
 
 int cpt_ir_motion_clips(cpt_ctx *c, cpt_ir_motion_clip *h_clips, int n, const uint8_t *const *h_frames, int64_t n_frames,
@@ -505,23 +569,16 @@ int cpt_ir_motion_clips(cpt_ctx *c, cpt_ir_motion_clip *h_clips, int n, const ui
     if (!c || !p || n < 0 || n_frames < 0 || n_steps < 0) return fail(CPT_ERR_INVALID, "cpt_ir_motion_clips: bad argument");
     if ((n && !h_clips) || (n_frames && !h_frames) || (n_steps && (!h_steps || !h_results)))
         return fail(CPT_ERR_INVALID, "cpt_ir_motion_clips: null argument");
-    if (p->erode_idle < 1 || p->erode_idle > cpt::kErodeMaxK || p->erode_recording < 1 || p->erode_recording > cpt::kErodeMaxK)
-        return fail(CPT_ERR_INVALID, "cpt_ir_motion_clips: erosion boxes must be 1..64 pixels");
+    int rc = ir_check_params(p);
+    if (rc) return rc;
     // everything is checked before any model's frame count or any device buffer changes
     std::vector<int> owner(n_steps, -1);
     int W = 0, H = 0, max_steps = 0;
     for (int d = 0; d < n; ++d) {
         const cpt_ir_motion_clip &k = h_clips[d];
-        const cpt_ir_motion *m = k.m;
-        const cpt_mog2 *g = k.mog2;
-        if (!m || !g || m->ctx != c || g->ctx != c)
-            return fail(CPT_ERR_INVALID, "cpt_ir_motion_clips: clip %d: a handle is missing or belongs to another context", d);
-        if (d == 0) { W = m->W; H = m->H; }
-        if (m->W != W || m->H != H || g->W != W || g->H != H)
-            return fail(CPT_ERR_INVALID, "cpt_ir_motion_clips: clip %d: the handles do not share one %d x %d geometry", d, W, H);
-        if (!k.d_mask) return fail(CPT_ERR_INVALID, "cpt_ir_motion_clips: clip %d has no mask buffer", d);
+        if ((rc = ir_check_clip(c, k, d, W, H))) return rc;
         for (int e = 0; e < d; ++e)
-            if (h_clips[e].m == m || h_clips[e].mog2 == g || h_clips[e].d_mask == k.d_mask)
+            if (h_clips[e].m == k.m || h_clips[e].mog2 == k.mog2 || h_clips[e].d_mask == k.d_mask)
                 return fail(CPT_ERR_INVALID, "cpt_ir_motion_clips: clips %d and %d share a handle or a mask buffer", e, d);
         if (k.first_step < 0 || k.n_steps < 0 || k.n_steps > n_steps - k.first_step)
             return fail(CPT_ERR_INVALID, "cpt_ir_motion_clips: clip %d: steps out of range", d);
@@ -531,8 +588,7 @@ int cpt_ir_motion_clips(cpt_ctx *c, cpt_ir_motion_clip *h_clips, int n, const ui
             const cpt_ir_motion_clip_step &st = h_steps[i];
             if (st.row < 0 || st.row >= n_frames || !h_frames[st.row])
                 return fail(CPT_ERR_INVALID, "cpt_ir_motion_clips: step %d: frame row out of range", i);
-            if (st.slot_new < 0 || st.slot_new >= m->ring_frames || st.slot_oldest < 0 || st.slot_oldest >= m->ring_frames)
-                return fail(CPT_ERR_INVALID, "cpt_ir_motion_clips: step %d: ring slot out of range", i);
+            if ((rc = ir_check_slots(k.m, st, i))) return rc;
         }
         max_steps = std::max(max_steps, k.n_steps);
     }
@@ -583,25 +639,13 @@ int cpt_ir_motion_clips(cpt_ctx *c, cpt_ir_motion_clip *h_clips, int n, const ui
     auto *d_steps = reinterpret_cast<cpt::IrStep *>(base + o_step);
     auto *d_res = reinterpret_cast<cpt_ir_motion_clip_result *>(base + o_res);
     uint8_t *d_stage = base + o_stage;
-    // the records, and each model's learning rates: the rate pair of both learning rates the step may take, from cv2's
-    // rule (mog2.cuh), with the model's frame count advanced once per step
     std::vector<cpt::IrClipArgs> args(n);
     std::vector<cpt::IrClipFlag> flags(n);
     std::vector<cpt::IrStep> steps(n_steps);
     for (int d = 0; d < n; ++d) {
         const cpt_ir_motion_clip &k = h_clips[d];
-        args[d] = cpt::IrClipArgs{k.m->d_ring, k.mog2->d_state, k.d_mask, k.m->d_bits, k.mog2->c, k.first_step, k.n_steps};
-        flags[d] = cpt::IrClipFlag{k.movement != 0, k.triggered, 0, 0, 0u, {0, 0, 0}};
-        for (int i = k.first_step; i < k.first_step + k.n_steps; ++i) {
-            const cpt_ir_motion_clip_step &st = h_steps[i];
-            cpt::IrStep &s = steps[i];
-            s.bgr = h_frames[st.row];
-            s.slot_new = st.slot_new; s.slot_oldest = st.slot_oldest; s.detect = st.detect != 0;
-            s.fresh = cpt::mog2_reinitialises(k.mog2->nframes, -1.0);
-            int frozen = k.mog2->nframes;
-            cpt::mog2_next_rate(*k.mog2, frozen, 0.0, s.alpha[1], s.prune[1]);
-            cpt::mog2_next_rate(*k.mog2, k.mog2->nframes, -1.0, s.alpha[0], s.prune[0]);
-        }
+        ir_clip_records(k, h_steps, args[d], flags[d], steps.data());
+        for (int i = k.first_step; i < k.first_step + k.n_steps; ++i) steps[i].bgr = h_frames[h_steps[i].row];
     }
     struct Copy { int64_t row; size_t offset; };
     std::vector<Copy> copies;  // host frames: the staging offset of each step's frame within its chunk

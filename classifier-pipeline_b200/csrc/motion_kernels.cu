@@ -1,12 +1,13 @@
 // motion_kernels.cu -- CPTVMotionDetector.process_frame (piclassifier/cptvmotiondetector.py:74-205) as ONE launch
 // per frame (M1 of SURVEY.md section 8a): batch-1 latency is the metric, so the running mean, the weighted
 // background update and the motion count are fused into a single 1024-thread CTA and the host reads back one
-// 32-byte result record.
+// 32-byte result record.  motion_step_kernel (per frame) and motion_clips_kernel (recordings) both run motion_step:
 //   phase 1  RunningMean.add (motiondetector.py:160-175): uint32 sum += new - oldest-in-ring (modular, as numpy)
 //   phase 2  WeightedBackground.process_frame(sum / n) (motiondetector.py:197-244) unless FFC affected
 //   phase 3  detect(): count(clip(cur, T) - clip(oldest_nonffc, T) > delta_thresh), T = background average
 //            (cptvmotiondetector.py:74-120), with the optional second delta ring (one_diff_only False)
 // The frame ring, the sum and the delta ring live in HBM for the life of the detector.
+#include <algorithm>
 #include <cstring>
 #include <vector>
 
@@ -23,39 +24,9 @@ struct cpt_motion {
     cpt_motion_result *d_result = nullptr;
     cpt_motion_result *h_result = nullptr;  // pinned
     uint16_t *h_stage = nullptr;            // pinned frame
-    bool mean_started = false;
 };
 
 namespace cpt {
-
-struct MotionArgs {
-    Geometry g;
-    uint16_t *ring;
-    uint32_t *sum;
-    double *diff;
-    int32_t *mean_count;
-    uint8_t *bg_state;
-    WeightTable wt;
-    cpt_motion_result *result;
-    int slot_new, slot_oldest, slot_nonffc;
-    int diff_slot_new, diff_slot_old;
-    int mean_frames;
-    uint32_t flags;
-    int delta_thresh;
-    double init_average;  // WeightedBackground(init_average=...) until the background has seen a frame
-};
-
-// RunningMean(frames, window) constructor (motiondetector.py:161-164): sum of the listed ring slots
-__global__ void __launch_bounds__(256) motion_mean_init_kernel(const uint16_t *ring, int npx, const int *slots, int n,
-                                                               uint32_t *sum, int32_t *mean_count) {
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < npx) {
-        uint32_t s = 0;
-        for (int k = 0; k < n; ++k) s += ring[(size_t)slots[k] * npx + i];
-        sum[i] = s;
-    }
-    if (i == 0) *mean_count = n;
-}
 
 struct MotionShared {
     unsigned long long red_sum[32];
@@ -156,18 +127,7 @@ __device__ __forceinline__ int motion_phases(const Geometry &g, const uint16_t *
     return n;
 }
 
-__global__ void __launch_bounds__(1024, 1) motion_step_kernel(const MotionArgs a) {
-    __shared__ MotionShared sh;
-    const size_t npx = a.g.npx;
-    const uint16_t *cur = a.ring + (size_t)a.slot_new * npx;
-    const uint16_t *old = a.ring + (size_t)(a.slot_oldest < 0 ? a.slot_new : a.slot_oldest) * npx;
-    const uint16_t *nonffc = a.slot_nonffc < 0 ? nullptr : a.ring + (size_t)a.slot_nonffc * npx;
-    const int n = motion_phases(a.g, cur, old, nonffc, a.sum, *a.mean_count, a.mean_frames, a.diff, a.diff_slot_new,
-                                a.diff_slot_old, a.bg_state, a.wt, a.flags, a.delta_thresh, a.init_average, sh, a.result);
-    if (threadIdx.x == 0) *a.mean_count = n;
-}
-
-// Per detector of a cpt_motion_clips launch.
+// Per detector of a cpt_motion_clips launch, and the detector of a cpt_motion_step launch.
 struct MotionClipArgs {
     uint16_t *ring;
     uint32_t *sum;
@@ -185,6 +145,26 @@ __device__ __forceinline__ const uint16_t *motion_frame(const uint16_t *frames, 
     return ref >= 0 ? frames + (size_t)ref * npx : ring + (size_t)(-1 - ref) * npx;
 }
 
+// One step of a detector, the one copy for both entry points: the RunningMean(frames, window) start from the step's mean
+// rows (motiondetector.py:161-164) when it has any, then motion_phases.  `n` is the mean count before the step; returns
+// the count after it.  Every thread of the CTA must call.
+__device__ __forceinline__ int motion_step(const Geometry &g, const MotionClipArgs &c, const cpt_motion_clip_step &st,
+                                           const int32_t *mean_rows, const uint16_t *frames, int n, MotionShared &sh,
+                                           cpt_motion_result *result) {
+    if (st.mean_count > 0) {
+        for (int i = threadIdx.x; i < g.npx; i += blockDim.x) {
+            uint32_t v = 0;
+            for (int k = 0; k < st.mean_count; ++k) v += motion_frame(frames, c.ring, g.npx, mean_rows[st.mean_first + k])[i];
+            c.sum[i] = v;
+        }
+        n = st.mean_count;
+        __syncthreads();
+    }
+    return motion_phases(g, motion_frame(frames, c.ring, g.npx, st.frame), motion_frame(frames, c.ring, g.npx, st.oldest),
+                         (st.flags & CPT_MOTION_DETECT) ? motion_frame(frames, c.ring, g.npx, st.nonffc) : nullptr, c.sum, n, c.mean_frames, c.diff, st.diff_slot_new,
+                         st.diff_slot_old, c.bg_state, c.wt, st.flags, c.delta_thresh, c.init_average, sh, result);
+}
+
 // cpt_motion_clips: one CTA per detector walks that detector's steps in order, one cpt_motion_result per step.
 __global__ void __launch_bounds__(1024, 1) motion_clips_kernel(const Geometry g, const MotionClipArgs *clips,
                                                                const cpt_motion_clip_step *steps, const int32_t *mean_rows,
@@ -192,21 +172,19 @@ __global__ void __launch_bounds__(1024, 1) motion_clips_kernel(const Geometry g,
     __shared__ MotionShared sh;
     const MotionClipArgs c = clips[blockIdx.x];
     int n = *c.mean_count;
-    for (int s = c.first_step; s < c.first_step + c.n_steps; ++s) {
-        const cpt_motion_clip_step st = steps[s];
-        if (st.mean_count > 0) {  // RunningMean(frames, window) (motiondetector.py:161-164) before this step
-            for (int i = threadIdx.x; i < g.npx; i += blockDim.x) {
-                uint32_t v = 0;
-                for (int k = 0; k < st.mean_count; ++k) v += motion_frame(frames, c.ring, g.npx, mean_rows[st.mean_first + k])[i];
-                c.sum[i] = v;
-            }
-            n = st.mean_count;
-            __syncthreads();
-        }
-        n = motion_phases(g, motion_frame(frames, c.ring, g.npx, st.frame), motion_frame(frames, c.ring, g.npx, st.oldest),
-                          (st.flags & CPT_MOTION_DETECT) ? motion_frame(frames, c.ring, g.npx, st.nonffc) : nullptr, c.sum, n, c.mean_frames, c.diff, st.diff_slot_new,
-                          st.diff_slot_old, c.bg_state, c.wt, st.flags, c.delta_thresh, c.init_average, sh, results + s);
-    }
+    for (int s = c.first_step; s < c.first_step + c.n_steps; ++s)  // each step record read once, into registers
+        n = motion_step(g, c, cpt_motion_clip_step(steps[s]), mean_rows, frames, n, sh, results + s);
+    if (threadIdx.x == 0) *c.mean_count = n;
+}
+
+// cpt_motion_step's records, passed by value: no upload besides the frame.  Every frame reference is a ring slot.
+constexpr int kMotionStepMeanRows = 64;
+struct MotionMeanRows { int32_t row[kMotionStepMeanRows]; };
+
+__global__ void __launch_bounds__(1024, 1) motion_step_kernel(const Geometry g, const MotionClipArgs c, const cpt_motion_clip_step st,
+                                                              const __grid_constant__ MotionMeanRows mean, cpt_motion_result *result) {
+    __shared__ MotionShared sh;
+    const int n = motion_step(g, c, st, mean.row, nullptr, *c.mean_count, sh, result);
     if (threadIdx.x == 0) *c.mean_count = n;
 }
 
@@ -226,6 +204,38 @@ __global__ void __launch_bounds__(256) motion_ring_gather_kernel(const RingCopy 
 }  // namespace cpt
 
 using cpt::fail;
+
+// The detector record of a step of either entry point: its handle on ctx c, its state record and its weight table.
+static int motion_clip_args(cpt_ctx *c, const cpt_motion_clip &k, int d, cpt::MotionClipArgs &a) {
+    const cpt_motion *m = k.m;
+    if (!m || m->ctx != c) return fail(CPT_ERR_INVALID, "detector %d does not belong to this context", d);
+    if (!k.d_background_state) return fail(CPT_ERR_INVALID, "detector %d has no background state", d);
+    if (!c->tables[m->weight_slot].d_thr) return fail(CPT_ERR_INVALID, "weight table slot %d is not set", m->weight_slot);
+    a = cpt::MotionClipArgs{m->d_ring, m->d_sum, m->d_diff, m->d_mean_count, (uint8_t *)k.d_background_state, c->tables[m->weight_slot].device(),
+                            k.init_average, k.delta_thresh, m->mean_frames, k.first_step, k.n_steps};
+    return CPT_OK;
+}
+
+// Step i of detector m, checked before anything runs: its frame references (r >= 0 a row of the call's n_frames frames,
+// r < 0 ring slot -1 - r), delta-ring slots and the delta ring itself, and its mean rows in h_mean_rows[0 .. n_mean_rows).
+static int motion_check_step(const cpt_motion *m, const cpt_motion_clip_step &st, int64_t n_frames, const int32_t *h_mean_rows,
+                             int n_mean_rows, int i) {
+    auto ref_ok = [&](int32_t r) { return r >= 0 ? r < n_frames : -1 - (int64_t)r < m->ring_frames; };
+    if (!ref_ok(st.frame) || !ref_ok(st.oldest)) return fail(CPT_ERR_INVALID, "step %d: frame reference out of range", i);
+    if (st.flags & CPT_MOTION_DETECT) {
+        if (!ref_ok(st.nonffc)) return fail(CPT_ERR_INVALID, "step %d: oldest non-FFC reference out of range", i);
+        if (!(st.flags & CPT_MOTION_ONE_DIFF)) {
+            if (!m->d_diff) return fail(CPT_ERR_INVALID, "step %d: the detector was opened without a delta ring", i);
+            if (st.diff_slot_new < 0 || st.diff_slot_new >= m->diff_frames || st.diff_slot_old >= m->diff_frames)
+                return fail(CPT_ERR_INVALID, "step %d: delta ring slot out of range", i);
+        }
+    }
+    if (st.mean_count < 0 || st.mean_count > m->mean_frames || st.mean_first < 0 || st.mean_count > n_mean_rows - st.mean_first)
+        return fail(CPT_ERR_INVALID, "step %d: mean rows out of range", i);
+    for (int j = 0; j < st.mean_count; ++j)
+        if (!ref_ok(h_mean_rows[st.mean_first + j])) return fail(CPT_ERR_INVALID, "step %d: mean frame reference out of range", i);
+    return CPT_OK;
+}
 
 extern "C" {
 
@@ -293,55 +303,21 @@ int cpt_motion_store(cpt_motion *m, const uint16_t *h_pix, int slot) {
     return CPT_OK;
 }
 
-int cpt_motion_mean_init(cpt_motion *m, const int32_t *h_slots, int n) {
-    if (!m || !h_slots) return fail(CPT_ERR_INVALID, "null argument");
-    if (n < 1 || n > m->mean_frames || n > 64) return fail(CPT_ERR_INVALID, "bad frame count %d", n);
-    for (int k = 0; k < n; ++k)
-        if (h_slots[k] < 0 || h_slots[k] >= m->ring_frames) return fail(CPT_ERR_INVALID, "ring slot out of range");
+int cpt_motion_step(const cpt_motion_clip *h_clip, const uint16_t *h_pix, const cpt_motion_clip_step *h_step, const int32_t *h_mean_rows,
+                    int n_mean_rows, cpt_motion_result *h_result) {
+    if (!h_clip || !h_clip->m || !h_pix || !h_step || !h_result || (n_mean_rows > 0 && !h_mean_rows))
+        return fail(CPT_ERR_INVALID, "null argument");
+    if (n_mean_rows < 0 || n_mean_rows > cpt::kMotionStepMeanRows) return fail(CPT_ERR_INVALID, "bad mean row count %d", n_mean_rows);
+    cpt_motion *m = h_clip->m;
     cpt_ctx *c = m->ctx;
-    CUDA_TRY(cudaSetDevice(c->device));
-    int *d_slots = nullptr;
-    CUDA_TRY(cudaMalloc(&d_slots, sizeof(int) * n));
-    cudaError_t e = cudaMemcpyAsync(d_slots, h_slots, sizeof(int) * n, cudaMemcpyHostToDevice, c->stream);
-    if (e == cudaSuccess) {
-        cpt::motion_mean_init_kernel<<<(c->g.npx + 255) / 256, 256, 0, c->stream>>>(m->d_ring, c->g.npx, d_slots, n, m->d_sum, m->d_mean_count);
-        e = cudaGetLastError();
-    }
-    if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
-    cudaFree(d_slots);
-    if (e != cudaSuccess) return fail(CPT_ERR_CUDA, "cpt_motion_mean_init: %s", cudaGetErrorString(e));
-    return CPT_OK;
-}
-
-int cpt_motion_step(cpt_motion *m, const uint16_t *h_pix, void *d_background_state, int slot_new, int slot_oldest,
-                    int slot_nonffc, int diff_slot_new, int diff_slot_old, uint32_t flags, int delta_thresh,
-                    double init_average, cpt_motion_result *h_result) {
-    if (!m || !h_pix || !d_background_state || !h_result) return fail(CPT_ERR_INVALID, "null argument");
-    if (slot_new < 0 || slot_new >= m->ring_frames || slot_oldest >= m->ring_frames) return fail(CPT_ERR_INVALID, "ring slot out of range");
-    if (flags & CPT_MOTION_DETECT) {
-        if (slot_nonffc < 0 || slot_nonffc >= m->ring_frames) return fail(CPT_ERR_INVALID, "oldest non-FFC slot out of range");
-        if (!(flags & CPT_MOTION_ONE_DIFF)) {
-            if (!m->d_diff) return fail(CPT_ERR_INVALID, "the detector was opened without a delta ring (one_diff_only)");
-            if (diff_slot_new < 0 || diff_slot_new >= m->diff_frames || diff_slot_old >= m->diff_frames)
-                return fail(CPT_ERR_INVALID, "delta ring slot out of range");
-        }
-    }
-    int rc = cpt_motion_store(m, h_pix, slot_new);
+    cpt::MotionClipArgs a;
+    int rc = motion_clip_args(c, *h_clip, 0, a);
+    if (!rc) rc = motion_check_step(m, *h_step, 0, h_mean_rows, n_mean_rows, 0);
+    if (!rc) rc = cpt_motion_store(m, h_pix, -1 - h_step->frame);
     if (rc) return rc;
-    cpt_ctx *c = m->ctx;
-    cpt::MotionArgs a{};
-    a.g = c->g;
-    a.ring = m->d_ring; a.sum = m->d_sum; a.diff = m->d_diff; a.mean_count = m->d_mean_count;
-    a.bg_state = (uint8_t *)d_background_state;
-    a.wt = c->tables[m->weight_slot].device();
-    a.result = m->d_result;
-    a.slot_new = slot_new; a.slot_oldest = slot_oldest; a.slot_nonffc = slot_nonffc;
-    a.diff_slot_new = diff_slot_new; a.diff_slot_old = diff_slot_old;
-    a.mean_frames = m->mean_frames;
-    a.flags = flags;
-    a.delta_thresh = delta_thresh;
-    a.init_average = init_average;
-    cpt::motion_step_kernel<<<1, 1024, 0, c->stream>>>(a);
+    cpt::MotionMeanRows mean{};
+    std::copy(h_mean_rows, h_mean_rows + n_mean_rows, mean.row);
+    cpt::motion_step_kernel<<<1, 1024, 0, c->stream>>>(c->g, a, *h_step, mean, m->d_result);
     CUDA_TRY(cudaGetLastError());
     CUDA_TRY(cudaMemcpyAsync(m->h_result, m->d_result, sizeof(cpt_motion_result), cudaMemcpyDeviceToHost, c->stream));
     CUDA_TRY(cudaStreamSynchronize(c->stream));
@@ -360,44 +336,21 @@ int cpt_motion_clips(cpt_ctx *c, const cpt_motion_clip *h_clips, int n, const ui
     std::vector<cpt::RingCopy> copies;
     for (int d = 0; d < n; ++d) {
         const cpt_motion_clip &k = h_clips[d];
+        int rc = motion_clip_args(c, k, d, args[d]);
+        if (rc) return rc;
         const cpt_motion *m = k.m;
-        if (!m || m->ctx != c) return fail(CPT_ERR_INVALID, "cpt_motion_clips: detector %d does not belong to this context", d);
-        if (!k.d_background_state) return fail(CPT_ERR_INVALID, "cpt_motion_clips: detector %d has no background state", d);
-        if (!c->tables[m->weight_slot].d_thr) return fail(CPT_ERR_INVALID, "weight table slot %d is not set", m->weight_slot);
         for (int e = 0; e < d; ++e)
             if (h_clips[e].m == m || h_clips[e].d_background_state == k.d_background_state)
                 return fail(CPT_ERR_INVALID, "cpt_motion_clips: detectors %d and %d share a handle or a state record", e, d);
         if (k.first_step < 0 || k.n_steps < 0 || k.n_steps > n_steps - k.first_step)
             return fail(CPT_ERR_INVALID, "cpt_motion_clips: detector %d: steps out of range", d);
-        auto ref_ok = [&](int32_t r) { return r >= 0 ? r < n_frames : -1 - (int64_t)r < m->ring_frames; };
-        for (int i = k.first_step; i < k.first_step + k.n_steps; ++i) {
-            const cpt_motion_clip_step &st = h_steps[i];
-            if (!ref_ok(st.frame) || !ref_ok(st.oldest)) return fail(CPT_ERR_INVALID, "step %d: frame reference out of range", i);
-            if (st.flags & CPT_MOTION_DETECT) {
-                if (!ref_ok(st.nonffc)) return fail(CPT_ERR_INVALID, "step %d: oldest non-FFC reference out of range", i);
-                if (!(st.flags & CPT_MOTION_ONE_DIFF)) {
-                    if (!m->d_diff) return fail(CPT_ERR_INVALID, "step %d: the detector was opened without a delta ring", i);
-                    if (st.diff_slot_new < 0 || st.diff_slot_new >= m->diff_frames || st.diff_slot_old >= m->diff_frames)
-                        return fail(CPT_ERR_INVALID, "step %d: delta ring slot out of range", i);
-                }
-            }
-            if (st.mean_count < 0 || st.mean_count > m->mean_frames || st.mean_first < 0 || st.mean_count > n_mean_rows - st.mean_first)
-                return fail(CPT_ERR_INVALID, "step %d: mean rows out of range", i);
-            for (int j = 0; j < st.mean_count; ++j)
-                if (!ref_ok(h_mean_rows[st.mean_first + j])) return fail(CPT_ERR_INVALID, "step %d: mean frame reference out of range", i);
-        }
+        for (int i = k.first_step; i < k.first_step + k.n_steps; ++i)
+            if ((rc = motion_check_step(m, h_steps[i], n_frames, h_mean_rows, n_mean_rows, i))) return rc;
         for (int s = 0; k.ring_rows && s < m->ring_frames; ++s) {
             const int32_t r = k.ring_rows[s];
             if (r < -1 || r >= n_frames) return fail(CPT_ERR_INVALID, "detector %d: ring row out of range", d);
             if (r >= 0) copies.push_back({m->d_ring + (size_t)s * c->g.npx, r});
         }
-        cpt::MotionClipArgs &a = args[d];
-        a.ring = m->d_ring; a.sum = m->d_sum; a.diff = m->d_diff; a.mean_count = m->d_mean_count;
-        a.bg_state = (uint8_t *)k.d_background_state;
-        a.wt = c->tables[m->weight_slot].device();
-        a.init_average = k.init_average;
-        a.delta_thresh = k.delta_thresh; a.mean_frames = m->mean_frames;
-        a.first_step = k.first_step; a.n_steps = k.n_steps;
     }
     if (n == 0) return CPT_OK;
     CUDA_TRY(cudaSetDevice(c->device));

@@ -181,9 +181,9 @@ SYMBOLS = {
     "cpt_ir_motion_close": (None, [_vp]),
     "cpt_ir_motion_gray": (_i, [_vp, _vp, _i, _vp]),
     "cpt_ir_motion_detect": (_i, [_vp, _i, _i, _i, _i, _vp, ctypes.POINTER(ctypes.c_int32), ctypes.POINTER(ctypes.c_int32)]),
-    "cpt_ir_motion_ring_slot": (_vp, [_vp, _i]),
-    "cpt_ir_motion_detect_ex": (_i, [_vp, _i, _i, _i, _i, _vp, ctypes.POINTER(ctypes.c_int32), ctypes.POINTER(ctypes.c_int32)]),
     "cpt_ir_motion_clips": (_i, [_vp, _vp, _i, _vp, _i64, _vp, _i, ctypes.POINTER(CptIrMotionClipParams), _vp]),
+    "cpt_ir_motion_step": (_i, [ctypes.POINTER(CptIrMotionClip), _vp, ctypes.POINTER(CptIrMotionClipStep), ctypes.POINTER(CptIrMotionClipParams),
+                                ctypes.POINTER(CptIrMotionClipResult)]),
     "cpt_mog2_open": (_vp, [_vp, _i, _i, ctypes.POINTER(CptMog2Params)]),
     "cpt_mog2_close": (None, [_vp]),
     "cpt_mog2_apply": (_i, [_vp, _vp, _i, _i64, _vp, _vp]),
@@ -194,8 +194,7 @@ SYMBOLS = {
     "cpt_motion_open": (_vp, [_vp, _i, _i, _i, _i]),
     "cpt_motion_close": (None, [_vp]),
     "cpt_motion_store": (_i, [_vp, _vp, _i]),
-    "cpt_motion_mean_init": (_i, [_vp, _vp, _i]),
-    "cpt_motion_step": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _i, ctypes.c_uint32, _i, _d, ctypes.POINTER(CptMotionResult)]),
+    "cpt_motion_step": (_i, [ctypes.POINTER(CptMotionClip), _vp, ctypes.POINTER(CptMotionClipStep), _vp, _i, ctypes.POINTER(CptMotionResult)]),
     "cpt_motion_clips": (_i, [_vp, _vp, _i, _vp, _i64, _vp, _i, _vp, _i, _vp]),
     "cpt_state_read": (_i, [_vp, _vp, _i, _vp, _vp, ctypes.POINTER(_d), _vp, ctypes.POINTER(ctypes.c_int32)]),
     "cpt_state_write": (_i, [_vp, _vp, _i, _vp, _vp, _d]),
@@ -472,6 +471,10 @@ class _Handle:
             pass
 
 
+class _IrMotionHead(ctypes.Structure):  # the leading members of struct cpt_ir_motion (csrc/ir_kernels.cu)
+    _fields_ = [("ctx", _vp), ("W", _i), ("H", _i), ("ring_frames", _i), ("d_ring", _vp)]
+
+
 class IrMotion(_Handle):
     """Device half of IRMotionDetector (cpt_ir_motion_*): a ring of grey frames, grey conversion and the eroded-pixel counts."""
 
@@ -480,8 +483,7 @@ class IrMotion(_Handle):
         super().__init__(ctx, ctx.lib.cpt_ir_motion_open, ctx.lib.cpt_ir_motion_close, int(width), int(height), int(ring_frames))
 
     def gray(self, bgr, slot, copy_out=True):
-        """BGR frame -> grey into ring slot ``slot``; returns the grey frame as a host array, or None with copy_out=False
-        (the frame then stays on the device: ``ring_slot(slot)``)."""
+        """BGR frame -> grey into ring slot ``slot``; returns the grey frame as a host array, or None with copy_out=False."""
         bgr = np.ascontiguousarray(bgr, dtype=np.uint8)
         if bgr.shape != (self.height, self.width, 3):
             raise ValueError("IR frames must be ({}, {}, 3) uint8".format(self.height, self.width))
@@ -490,30 +492,30 @@ class IrMotion(_Handle):
         return out
 
     def ring_slot(self, slot):
-        """Device address of the grey frame in ring slot ``slot`` ([H][W] uint8)."""
-        p = self.ctx.lib.cpt_ir_motion_ring_slot(self._h, int(slot))
-        if not p:
-            raise NativeError("cpt_ir_motion_ring_slot failed: {}".format(self.ctx.lib.cpt_last_error().decode()))
-        return p
+        """Device address of the grey frame in ring slot ``slot`` ([H][W] uint8), for inspecting the ring."""
+        if not 0 <= slot < self.ring_frames:
+            raise NativeError("ring slot {} out of range".format(slot))
+        return _IrMotionHead.from_address(self._h).d_ring + slot * self.width * self.height
 
-    def detect(self, slot_new, slot_oldest, threshold, erode_k, mask=None, d_mask=None):
-        """(eroded difference pixels, eroded mask pixels).  The foreground mask is a host array (``mask``) or device memory
-        (``d_mask``: a uint8 CUDA tensor or a device address, e.g. ``Mog2.apply``'s output); at most one of them."""
+    def detect(self, slot_new, slot_oldest, threshold, erode_k, mask=None):
+        """(eroded difference pixels, eroded mask pixels) with the host foreground mask ``mask`` (or None)."""
         diff, cnt = ctypes.c_int32(), ctypes.c_int32()
-        if d_mask is not None:
-            if mask is not None:
-                raise ValueError("pass mask or d_mask, not both")
-            check(self.ctx.lib.cpt_ir_motion_detect_ex(self._h, int(slot_new), int(slot_oldest), int(threshold), int(erode_k),
-                                                       _dptr(d_mask, self.height * self.width), ctypes.byref(diff), ctypes.byref(cnt)))
-            return diff.value, cnt.value
         if mask is not None:
             mask = np.ascontiguousarray(mask, dtype=np.uint8)
         check(self.ctx.lib.cpt_ir_motion_detect(self._h, int(slot_new), int(slot_oldest), int(threshold), int(erode_k), _ptr(mask),
                                                 ctypes.byref(diff), ctypes.byref(cnt)))
         return diff.value, cnt.value
 
+    def step(self, clip, bgr, step, params):
+        """One step of ``Context.ir_motion_clips`` for this detector alone (cpt_ir_motion_step): ``clip`` its CptIrMotionClip
+        (``clip_record``; movement / triggered are updated), bgr a host [H][W][3] uint8 frame, ``step`` its CptIrMotionClipStep
+        and ``params`` the CptIrMotionClipParams.  Waits and returns the CptIrMotionClipResult."""
+        result, bgr = CptIrMotionClipResult(), np.ascontiguousarray(bgr)  # bgr: a contiguous copy lives until the call returns
+        check(self.ctx.lib.cpt_ir_motion_step(ctypes.byref(clip), _ptr(bgr), ctypes.byref(step), ctypes.byref(params), ctypes.byref(result)))
+        return result
+
     def clip_record(self, mog2, d_mask, first_step, n_steps, movement, triggered):
-        """This detector's CptIrMotionClip of a ``Context.ir_motion_clips`` call: ``mog2`` its ``Mog2`` model, ``d_mask`` the
+        """This detector's CptIrMotionClip of a ``Context.ir_motion_clips`` call or of ``step``: ``mog2`` its ``Mog2`` model, ``d_mask`` the
         [H][W] uint8 CUDA tensor that receives the foreground masks."""
         return CptIrMotionClip(self._h, mog2.address, _dptr(d_mask, self.height * self.width), int(first_step), int(n_steps),
                                int(bool(movement)), int(triggered))
@@ -588,21 +590,17 @@ class Motion(_Handle):
         """Host uint16 frame [H][W] into ring slot ``slot`` without processing it."""
         check(self.ctx.lib.cpt_motion_store(self._h, _ptr(h_pix), int(slot)))
 
-    def mean_init(self, slots):
-        """Start the running sum from the frames in ring slots ``slots``."""
-        arr = (ctypes.c_int32 * len(slots))(*slots)
-        check(self.ctx.lib.cpt_motion_mean_init(self._h, arr, len(slots)))
-
-    def step(self, h_pix, d_background_state, slot_new, slot_oldest, slot_nonffc, diff_slot_new, diff_slot_old, flags, delta_thresh,
-             init_average):
-        """One process_frame (include/cptrack.h, cpt_motion_step); waits for it and returns its CptMotionResult."""
+    def step(self, clip, h_pix, step, mean_rows=()):
+        """One process_frame (cpt_motion_step) of the detector record ``clip`` (``clip_record``): h_pix (host uint16 [H][W])
+        into ring slot -1 - step[0], then the step with the cpt_motion_clip_step fields ``step`` (every frame reference a ring
+        slot; the RunningMean start reads ``mean_rows``).  Waits for it and returns its CptMotionResult."""
         result = CptMotionResult()
-        check(self.ctx.lib.cpt_motion_step(self._h, _ptr(h_pix), _ptr(d_background_state), int(slot_new), int(slot_oldest),
-                                           int(slot_nonffc), int(diff_slot_new), int(diff_slot_old), int(flags), int(delta_thresh),
-                                           float(init_average), ctypes.byref(result)))
+        rows = (ctypes.c_int32 * len(mean_rows))(*mean_rows) if len(mean_rows) else None
+        check(self.ctx.lib.cpt_motion_step(ctypes.byref(clip), _ptr(h_pix), ctypes.byref(CptMotionClipStep(*step)), rows, len(mean_rows),
+                                           ctypes.byref(result)))
         return result
 
     def clip_record(self, d_background_state, ring_rows, init_average, delta_thresh, first_step, n_steps):
-        """This detector's CptMotionClip of a ``Context.motion_clips`` call (ring_rows: host int32 [ring_frames])."""
+        """This detector's CptMotionClip of a ``Context.motion_clips`` call (ring_rows: host int32 [ring_frames]) or of ``step``."""
         return CptMotionClip(self._h, _ptr(d_background_state), _ptr(ring_rows), float(init_average), int(delta_thresh), int(first_step),
                              int(n_steps), 0)

@@ -91,6 +91,8 @@ class CPTVMotionDetector(MotionDetector):
         self._ctx = self._background.ctx
         self._motion = native.Motion(self._ctx, self.thermal_window.size, self.MEAN_FRAMES,
                                      0 if self.config.one_diff_only else self.compare_gap, self._background.weight_slot)
+        self._ring_refs = [-1 - s for s in range(self.thermal_window.size)]  # each ring slot as a frame reference
+        self._clip = self._motion.clip_record(self._background.d_state, None, 0.0, 0, 0, 1)  # process_frame's detector record
         self._average = None
         self.last_diff = 0
 
@@ -204,11 +206,10 @@ class CPTVMotionDetector(MotionDetector):
         if step is None:
             self._motion.store(pix, self.thermal_window.last_index)
         else:
-            if step.mean_slots:
-                self._motion.store(pix, step.new)
-                self._motion.mean_init(step.mean_slots)
-            result = self._motion.step(pix, self._background.d_state, step.new, step.oldest, -1 if step.nonffc is None else step.nonffc,
-                                       step.diff_new, step.diff_old, step.flags, self.config.delta_thresh, self._init_average())
+            mean_rows = []
+            record = _step_record(step, self._ring_refs, mean_rows)
+            self._clip.init_average, self._clip.delta_thresh = self._init_average(), self.config.delta_thresh
+            result = self._motion.step(self._clip, pix, record, mean_rows)
         self._apply(step, result)
         return self.movement_detected
 
@@ -219,6 +220,14 @@ class CPTVMotionDetector(MotionDetector):
 
     def skip_frame(self):
         return
+
+
+def _step_record(step, ref, mean_rows):
+    """The cpt_motion_clip_step of a planned step; ``ref[slot]`` is ring slot ``slot``'s frame reference (a row, or -1 - slot)."""
+    mean_first, mean_slots = len(mean_rows), step.mean_slots or ()
+    mean_rows += [ref[s] for s in mean_slots]  # the RunningMean start's frame references
+    return (ref[step.new], ref[step.oldest], _NO_FRAME if step.nonffc is None else ref[step.nonffc], step.diff_new, step.diff_old,
+            mean_first, len(mean_slots), step.flags)
 
 
 class ClipSteps:
@@ -237,7 +246,7 @@ class ClipSteps:
         self._clips = (native.CptMotionClip * len(detectors))()
         for i, (det, frames) in enumerate(zip(detectors, frame_lists)):
             win = det.thermal_window
-            ref = [-1 - s for s in range(win.size)]  # what each ring slot holds: a row of this call, or itself
+            ref = list(det._ring_refs)  # what each ring slot holds: a row of this call, or itself
             ring_rows = np.full(win.size, -1, dtype=np.int32)
             first, plan, processed = len(steps), [], []
             for t, frame in enumerate(frames):
@@ -246,14 +255,8 @@ class ClipSteps:
                 ref[win.last_index] = ring_rows[win.last_index] = row
                 plan.append(step)
                 processed.append(det.processed)
-                if step is None:
-                    continue
-                mean_first, mean_count = len(mean_rows), 0
-                if step.mean_slots:
-                    mean_rows += [ref[s] for s in step.mean_slots]
-                    mean_count = len(step.mean_slots)
-                steps.append((row, ref[step.oldest], _NO_FRAME if step.nonffc is None else ref[step.nonffc], step.diff_new,
-                              step.diff_old, mean_first, mean_count, step.flags))
+                if step is not None:
+                    steps.append(_step_record(step, ref, mean_rows))
             self.plans.append(plan)
             self._processed.append(processed)
             self.offsets[i + 1] = self.offsets[i] + len(frames)

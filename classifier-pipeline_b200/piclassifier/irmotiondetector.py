@@ -5,10 +5,10 @@ Per frame the reference converts BGR to grey, updates its background model, and 
 conversion, the difference mask, both erosions and the pixel counts run on the device (csrc/ir_kernels.cu), with the grey
 ring resident in device memory.  The background model is OpenCV's MOG2: by default ``track.cliptracker.CVBackground``, cv2 on
 the host, which needs the grey frame copied out and the mask copied back every frame.  ``MOG2Background`` (the same model
-bit for bit, csrc/mog2_kernels.cu) on the detector's engine keeps both on the device: the grey frame goes from its ring slot
-into the model and the mask from the model into the erosion, so per frame only the BGR frame goes in and two counts come
-out.  Any other object with ``update_background(gray, learning_rate=)`` / ``compute_filtered(None)`` / ``background`` can be
-passed as well.
+bit for bit, csrc/mog2.cuh) on the detector's engine keeps both on the device: ``process_frame`` is then one step of the
+whole-recording call below (cpt_ir_motion_step), so per frame only the BGR frame goes in and the counts and the trigger
+decision come out.  Any other object with ``update_background(gray, learning_rate=)`` / ``compute_filtered(None)`` /
+``background`` can be passed as well.
 
 With ``MOG2Background``, ``IRMotionDetector.process_frames`` and ``process_clips`` run whole recordings of many detectors
 in one native call (cpt_ir_motion_clips): every frame's grey conversion, model update, erosion and trigger decision stay on
@@ -70,6 +70,7 @@ TRIGGER_FRAMES = 2
 MAX_TRIGGERED = 30
 ERODE_IDLE = 15       # erosion box when not recording
 ERODE_RECORDING = 10  # erosion box when recording
+_PARAMS = native.CptIrMotionClipParams(THRESHOLD, TRIGGER_FRAMES, MAX_TRIGGERED, ERODE_IDLE, ERODE_RECORDING, 0)
 
 # One planned device step: the ring slot the grey frame goes to, the oldest slot it is compared with, and whether the
 # erosion and the trigger rule run (num_frames > MIN_FRAMES).
@@ -164,26 +165,37 @@ class IRMotionDetector(MotionDetector):
         elif self.movement_detected and self.triggered <= 0:
             self.movement_detected = False
 
+    def _apply_device(self, step, r, where=""):
+        """``_apply`` on a device step's CptIrMotionClipResult ``r``; the device's trigger decision must agree."""
+        diff, mask = (int(r.diff_pixels), int(r.mask_pixels)) if step.detect else (-1, -1)
+        self._apply(step, diff, mask)
+        if (self.movement_detected, self.triggered) != (bool(r.movement), int(r.triggered)):
+            raise native.NativeError("{}the device's trigger decision differs from the host's".format(where))
+        return diff, mask
+
+    def _clip_record(self, first, n):
+        """This detector's CptIrMotionClip of n device steps from step ``first``, on its MOG2Background's model and a new mask."""
+        model, mask = self._background._steps(self._dev.height, self._dev.width, n)
+        return self._dev.clip_record(model, mask, first, n, self.movement_detected, self.triggered)
+
     def process_frame(self, frame, force_process=False):
         """Returns True if there is motion (irmotiondetector.py:103-153)."""
         self._check_frame(frame)
         step = self._plan(frame, force_process)
-        counts = (None, None)
-        if step is not None:
-            gray = self._dev.gray(frame, step.slot, copy_out=not self._device_background)
-            learning_rate = 0 if self.movement_detected else -1
-            if self._device_background:
-                self._background.update_background_device(self._dev.ring_slot(step.slot), self._dev.width, self._dev.height, learning_rate)
-            else:
-                self._background.update_background(gray, learning_rate=learning_rate)
+        if step is None:
+            self._apply(None, None, None)
+        elif self._device_background:
+            self._dev.ctx.use_torch_stream()
+            r = self._dev.step(self._clip_record(0, 1), frame, native.CptIrMotionClipStep(0, step.slot, step.oldest, int(step.detect), 0),
+                               _PARAMS)
+            self._apply_device(step, r)
+        else:
+            gray = self._dev.gray(frame, step.slot)
+            self._background.update_background(gray, learning_rate=0 if self.movement_detected else -1)
+            counts = (None, None)
             if step.detect:
-                k = self.get_kernel().shape[0]
-                if self._device_background:
-                    mask = dict(d_mask=self._background.device_mask)
-                else:
-                    mask = dict(mask=self._background.compute_filtered(None))
-                counts = self._dev.detect(step.slot, step.oldest, THRESHOLD, k, **mask)
-        self._apply(step, *counts)
+                counts = self._dev.detect(step.slot, step.oldest, THRESHOLD, self.get_kernel().shape[0], mask=self._background.compute_filtered(None))
+            self._apply(step, *counts)
         return self.movement_detected
 
     def process_frames(self, frames, force_process=False):
@@ -270,23 +282,15 @@ def process_clips(detectors, frame_lists, force_process=False):
                 addresses.append(address)
         plans.append(plan)
         if len(steps) > first:
-            bg = det._background
-            model = bg._open(det._dev.height, det._dev.width)
-            mask = torch.empty((det._dev.height, det._dev.width), dtype=torch.uint8, device="cuda:{}".format(det._dev.ctx.device))
-            clips.append((det, mask, det._dev.clip_record(model, mask, first, len(steps) - first, det.movement_detected, det.triggered)))
+            clips.append(det._clip_record(first, len(steps) - first))
     results = (native.CptIrMotionClipResult * max(1, len(steps)))()
     if clips:
         ctx = detectors[0]._dev.ctx
         ctx.use_torch_stream()
-        records = (native.CptIrMotionClip * len(clips))(*[c[2] for c in clips])
         params = native.CptIrMotionClipParams(THRESHOLD, TRIGGER_FRAMES, MAX_TRIGGERED, ERODE_IDLE, ERODE_RECORDING, int(host))
         table = np.array(addresses, dtype=np.uint64)
-        ctx.ir_motion_clips(records, len(clips), table, len(table), (native.CptIrMotionClipStep * len(steps))(*steps), len(steps), params,
-                            results)
-        for (det, mask, record), rec in zip(clips, records):
-            bg = det._background
-            bg._frames += rec.n_steps
-            bg._mask, bg._mask_host = mask, None
+        ctx.ir_motion_clips((native.CptIrMotionClip * len(clips))(*clips), len(clips), table, len(table),
+                            (native.CptIrMotionClipStep * len(steps))(*steps), len(steps), params, results)
     # the host half, frame by frame; the trigger rule runs again on the device's counts and must agree with its decisions
     traces, k = [], 0
     for i, (det, plan) in enumerate(zip(detectors, plans)):
@@ -294,13 +298,8 @@ def process_clips(detectors, frame_lists, force_process=False):
         for t, step in enumerate(plan):
             diff = mask = -1
             if step is not None:
-                r = results[k]
+                diff, mask = det._apply_device(step, results[k], "detector {} frame {}: ".format(i, t))
                 k += 1
-                if step.detect:
-                    diff, mask = int(r.diff_pixels), int(r.mask_pixels)
-                det._apply(step, diff, mask)
-                if (det.movement_detected, det.triggered) != (bool(r.movement), int(r.triggered)):
-                    raise native.NativeError("detector {} frame {}: the device's trigger decision differs from the host's".format(i, t))
             rows.append((det.movement_detected, det.triggered, diff, mask))
         cols = list(zip(*rows)) if rows else [()] * 4
         traces.append(IrMotionTrace(np.array(cols[0], dtype=bool), np.array(cols[1], dtype=np.int64), np.array(cols[2], dtype=np.int64),

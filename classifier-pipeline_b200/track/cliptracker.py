@@ -316,18 +316,6 @@ class MOG2Background(Background):
             raise ValueError("MOG2Background takes uint8 frames (host arrays or CUDA tensors)")
         return torch.from_numpy(frames).to("cuda:{}".format(self.ctx.device))
 
-    def update_background_device(self, d_frame, width, height, learning_rate=-1):
-        """One apply() on a [height][width] uint8 frame already in device memory, given by its address (the IR detector's
-        grey ring slot)."""
-        import torch
-
-        model = self._open(height, width)
-        self.ctx.use_torch_stream()
-        self._mask = torch.empty((height, width), dtype=torch.uint8, device="cuda:{}".format(self.ctx.device))
-        self._mask_host = None
-        model.apply(d_frame, [learning_rate], d_masks=self._mask, n_frames=1)
-        self._frames += 1
-
     def set_background(self, background, frames=1):
         self.update_background(background, learning_rate=1)
 
@@ -335,7 +323,20 @@ class MOG2Background(Background):
         frame = self._to_device(thermal)
         if frame.dim() != 2:
             raise ValueError("update_background takes one [H][W] frame")
-        self.update_background_device(frame.data_ptr(), frame.shape[1], frame.shape[0], learning_rate)
+        model, mask = self._steps(frame.shape[0], frame.shape[1], 1)
+        self.ctx.use_torch_stream()
+        model.apply(frame, [learning_rate], d_masks=mask)
+
+    def _steps(self, height, width, n):
+        """The model and a new [height][width] mask tensor for n apply() steps about to run on the device, here or in the IR
+        motion detector's native calls; the steps are counted and the tensor becomes the last mask."""
+        import torch
+
+        model = self._open(height, width)
+        self._mask = torch.empty((height, width), dtype=torch.uint8, device="cuda:{}".format(self.ctx.device))
+        self._mask_host = None
+        self._frames += n
+        return model, self._mask
 
     def update_backgrounds(self, frames, learning_rate=-1):
         """apply() on frames [N][H][W] in one launch; learning_rate is a number or one per frame.  Returns the N masks, as

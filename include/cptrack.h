@@ -332,10 +332,12 @@ int cpt_extract_batch_cptv_host(cpt_ctx *ctx, const uint8_t *h_stream, uint64_t 
                                 const int64_t *h_clip_first, const cpt_clip *h_clips, int n_clips, int64_t total_frames,
                                 cpt_region *h_regions, cpt_frame_info *h_info, int chunk_clips);
 
-/* ---- CPTVMotionDetector (piclassifier/cptvmotiondetector.py:14-205), streaming, one launch per frame ----
+/* ---- CPTVMotionDetector (piclassifier/cptvmotiondetector.py:14-205) on the device ----
  * The detector owns a ring of the last ring_frames frames (SlidingWindow of preview_secs * fps + 1 frames), the
  * uint32 running sum (RunningMean over mean_frames = 45) and, for one_diff_only == False, a ring of diff_frames
- * clamped delta frames.  Ring bookkeeping (which slot is newest / oldest / oldest non-FFC) stays on the host. */
+ * clamped delta frames.  Ring bookkeeping (which slot is newest / oldest / oldest non-FFC) stays on the host, which
+ * plans every frame as one cpt_motion_clip_step; cpt_motion_step runs one step and cpt_motion_clips many, with the same
+ * device code and the same checks. */
 typedef struct cpt_motion cpt_motion;
 #define CPT_MOTION_MEAN 1u          /* RunningMean.add(new, oldest) (motiondetector.py:166-172) */
 #define CPT_MOTION_MEAN_RESTART 2u  /* start the running sum from this frame alone */
@@ -350,50 +352,50 @@ typedef struct {
     int32_t mean_frames; /* RunningMean.running_mean_frames */
     int32_t reserved;
 } cpt_motion_result;
-cpt_motion *cpt_motion_open(cpt_ctx *ctx, int ring_frames, int mean_frames, int diff_frames, int weight_slot);
-void cpt_motion_close(cpt_motion *m);
-/* SlidingWindow.update_current_frame / add without processing: host frame -> ring slot. */
-int cpt_motion_store(cpt_motion *m, const uint16_t *h_pix, int slot);
-/* RunningMean(frames, window) from the listed ring slots (first processed frame after frames were only stored). */
-int cpt_motion_mean_init(cpt_motion *m, const int32_t *h_slots, int n);
-/* One process_frame: copies h_pix into ring slot slot_new, runs the fused step on the ctx stream, waits and
- * returns the result.  d_background_state is the WeightedBackground state record (cpt_state_bytes) the detector
- * shares with the streaming extractor; slot_oldest = SlidingWindow.oldest (-1: none); slot_nonffc / diff_slot_old =
- * the oldest non-FFC entries of the two rings (diff_slot_old -1: fewer than 3 frames processed). */
-int cpt_motion_step(cpt_motion *m, const uint16_t *h_pix, void *d_background_state, int slot_new, int slot_oldest,
-                    int slot_nonffc, int diff_slot_new, int diff_slot_old, uint32_t flags, int delta_thresh,
-                    double init_average, cpt_motion_result *h_result);
-
-/* Whole recordings, many detectors, one launch (cptvmotiondetector.py:135-205, motiondetector.py:160-244 for every frame
- * of each detector's frame list): the host plans every frame with the same ring bookkeeping as cpt_motion_step's caller,
- * and one CTA per detector then runs that detector's steps in order.  d_frames is [n_frames][H][W] uint16 in device
- * memory.  A frame reference r >= 0 is row r of d_frames; r < 0 is slot -1 - r of the detector's ring as it stood before
- * the call (a detector resumed after streaming).  After the steps, each ring slot with ring_rows[slot] >= 0 takes that
- * row, so the ring holds what the per-frame calls would have left; the running sum, the delta ring and the background
- * state record are updated in place as by those calls.  Every detector must belong to ctx and appear once, with its own
- * state record.  Every index (frame references, delta-ring slots, mean rows, ring_rows, step ranges) is checked before
- * anything is launched: CPT_ERR_INVALID.  h_results[i] is step i's result as cpt_motion_step returns it; a step whose
- * running mean left the uint16 range has error = 1 (the call itself returns CPT_OK). */
+/* One planned frame (cptvmotiondetector.py:135-205).  A frame reference r >= 0 is row r of cpt_motion_clips' d_frames;
+ * r < 0 is slot -1 - r of the detector's ring as it stood before the call. */
 typedef struct {
     int32_t frame;          /* the new frame (SlidingWindow.current after add) */
     int32_t oldest;         /* SlidingWindow.oldest after the add */
     int32_t nonffc;         /* SlidingWindow.oldest_nonffc; read with CPT_MOTION_DETECT only */
-    int32_t diff_slot_new;  /* delta ring slots as in cpt_motion_step (CPT_MOTION_DETECT without CPT_MOTION_ONE_DIFF) */
-    int32_t diff_slot_old;
+    int32_t diff_slot_new;  /* delta ring slots (CPT_MOTION_DETECT without CPT_MOTION_ONE_DIFF): the new delta frame and the */
+    int32_t diff_slot_old;  /*   oldest non-FFC one (-1: fewer than 3 frames processed) */
     int32_t mean_first;     /* mean_count > 0: RunningMean(frames) from h_mean_rows[mean_first .. mean_first + mean_count) */
-    int32_t mean_count;     /*   before this step (at most the detector's mean_frames), as cpt_motion_mean_init */
+    int32_t mean_count;     /*   before this step (at most the detector's mean_frames): the first processed frame after frames
+                               were only stored */
     uint32_t flags;         /* CPT_MOTION_* */
 } cpt_motion_clip_step;
 typedef struct {
     cpt_motion *m;
-    void *d_background_state;  /* the detector's WeightedBackground state record */
-    const int32_t *ring_rows;  /* host [ring_frames]: row of d_frames each ring slot holds afterwards, -1 = unchanged; NULL = none */
-    double init_average;       /* as cpt_motion_step */
+    void *d_background_state;  /* the WeightedBackground state record (cpt_state_bytes) the detector shares with the
+                                  streaming extractor */
+    const int32_t *ring_rows;  /* cpt_motion_clips: host [ring_frames], row of d_frames each ring slot holds afterwards,
+                                  -1 = unchanged; NULL = none */
+    double init_average;       /* WeightedBackground(init_average=...) until the background has seen a frame */
     int32_t delta_thresh;
-    int32_t first_step;        /* this detector's steps: h_steps[first_step .. first_step + n_steps) */
+    int32_t first_step;        /* cpt_motion_clips: this detector's steps are h_steps[first_step .. first_step + n_steps) */
     int32_t n_steps;
     int32_t reserved;
 } cpt_motion_clip;
+cpt_motion *cpt_motion_open(cpt_ctx *ctx, int ring_frames, int mean_frames, int diff_frames, int weight_slot);
+void cpt_motion_close(cpt_motion *m);
+/* SlidingWindow.update_current_frame / add without processing: host frame -> ring slot. */
+int cpt_motion_store(cpt_motion *m, const uint16_t *h_pix, int slot);
+/* One process_frame of detector h_clip->m (ring_rows, first_step and n_steps are not read): h_pix is stored in ring slot
+ * -1 - h_step->frame, then the step runs on the ctx stream with every frame reference a ring slot and its mean rows in
+ * h_mean_rows[0 .. n_mean_rows), n_mean_rows <= 64.  Waits and returns the result; CPT_ERR_INVALID for a reference, slot or
+ * row out of range (checked before anything changes) and for a step whose running mean left the uint16 range. */
+int cpt_motion_step(const cpt_motion_clip *h_clip, const uint16_t *h_pix, const cpt_motion_clip_step *h_step,
+                    const int32_t *h_mean_rows, int n_mean_rows, cpt_motion_result *h_result);
+
+/* Whole recordings, many detectors, one launch (cptvmotiondetector.py:135-205, motiondetector.py:160-244 for every frame
+ * of each detector's frame list): one CTA per detector runs that detector's steps in order.  d_frames is
+ * [n_frames][H][W] uint16 in device memory.  After the steps, each ring slot with ring_rows[slot] >= 0 takes that row, so
+ * the ring holds what the per-frame calls would have left; the running sum, the delta ring and the background state
+ * record are updated in place as by those calls.  Every detector must belong to ctx and appear once, with its own state
+ * record.  Every index (frame references, delta-ring slots, mean rows, ring_rows, step ranges) is checked before anything
+ * is launched: CPT_ERR_INVALID.  h_results[i] is step i's result as cpt_motion_step returns it; a step whose running mean
+ * left the uint16 range has error = 1 (the call itself returns CPT_OK). */
 int cpt_motion_clips(cpt_ctx *ctx, const cpt_motion_clip *h_clips, int n, const uint16_t *d_frames, int64_t n_frames,
                      const cpt_motion_clip_step *h_steps, int n_steps, const int32_t *h_mean_rows, int n_mean_rows,
                      cpt_motion_result *h_results);
@@ -402,23 +404,20 @@ int cpt_motion_clips(cpt_ctx *ctx, const cpt_motion_clip *h_clips, int n, const 
  * Per frame the reference does cv2.cvtColor(BGR2GRAY), feeds the grey frame to its background model (OpenCV's MOG2, on the
  * host through cv2 or on the device through cpt_mog2 below), then absdiff(oldest grey, grey) -> threshold 12 -> erode with a
  * k x k box (15 idle / 10 while recording) -> count, and the same erode + count on the background model's foreground mask.
- * The detector owns a ring of grey frames on the device (SlidingWindow of preview_secs * fps frames).
+ * The detector owns a ring of grey frames on the device (SlidingWindow of preview_secs * fps frames).  With a host
+ * background model each frame is cpt_ir_motion_gray, the model, then cpt_ir_motion_detect; with the device MOG2 it is one
+ * cpt_ir_motion_step (below).
  *   cpt_ir_motion_gray       h_bgr [H][W][3] -> grey (OpenCV's fixed point: (B*3735 + G*19235 + R*9798 + 2^14) >> 15) into
  *                            ring slot slot_new; h_gray_out (may be NULL) receives it for a host background model
- *   cpt_ir_motion_ring_slot  device address of ring slot `slot` ([H][W] uint8), NULL (CPT_ERR_INVALID) out of range
  *   cpt_ir_motion_detect     *h_diff_pixels = count(erode(|ring[slot_oldest] - ring[slot_new]| > threshold)); with h_mask (the
  *                            background model's foreground mask, [H][W], non-zero = set; may be NULL) *h_mask_pixels =
- *                            count(erode(h_mask)).  Pixels outside the image do not constrain the erosion (cv2's default).
- *   cpt_ir_motion_detect_ex  the same with the mask in device memory (d_mask, e.g. cpt_mog2_apply's output; may be NULL) */
+ *                            count(erode(h_mask)).  Pixels outside the image do not constrain the erosion (cv2's default). */
 typedef struct cpt_ir_motion cpt_ir_motion;
 cpt_ir_motion *cpt_ir_motion_open(cpt_ctx *ctx, int width, int height, int ring_frames);
 void cpt_ir_motion_close(cpt_ir_motion *m);
 int cpt_ir_motion_gray(cpt_ir_motion *m, const uint8_t *h_bgr, int slot_new, uint8_t *h_gray_out);
 int cpt_ir_motion_detect(cpt_ir_motion *m, int slot_new, int slot_oldest, int threshold, int erode_k, const uint8_t *h_mask,
                          int32_t *h_diff_pixels, int32_t *h_mask_pixels);
-const uint8_t *cpt_ir_motion_ring_slot(cpt_ir_motion *m, int slot);
-int cpt_ir_motion_detect_ex(cpt_ir_motion *m, int slot_new, int slot_oldest, int threshold, int erode_k, const uint8_t *d_mask,
-                            int32_t *h_diff_pixels, int32_t *h_mask_pixels);
 
 /* Whole IR recordings, many detectors, with each frame's trigger decided on the device (irmotiondetector.py:103-153 for
  * every frame of each detector's frame list, with the device MOG2 of cpt_mog2 as background model).  The host plans the
@@ -467,6 +466,12 @@ typedef struct {
 int cpt_ir_motion_clips(cpt_ctx *ctx, cpt_ir_motion_clip *h_clips, int n, const uint8_t *const *h_frames, int64_t n_frames,
                         const cpt_ir_motion_clip_step *h_steps, int n_steps, const cpt_ir_motion_clip_params *params,
                         cpt_ir_motion_clip_result *h_results);
+/* One step of cpt_ir_motion_clips for the one clip h_clip (first_step and n_steps are not read, nor h_step->row or
+ * params->host_frames): the host BGR frame h_bgr [H][W][3] goes through the detector's pinned staging with the step's
+ * records in one copy; grey, MOG2 update, mask, erosion and trigger rule run as in cpt_ir_motion_clips, with the same
+ * checks.  Waits; *h_result is the step's result and h_clip->movement / triggered hold the state after it. */
+int cpt_ir_motion_step(cpt_ir_motion_clip *h_clip, const uint8_t *h_bgr, const cpt_ir_motion_clip_step *h_step,
+                       const cpt_ir_motion_clip_params *params, cpt_ir_motion_clip_result *h_result);
 
 /* ---- OpenCV's BackgroundSubtractorMOG2 (track/cliptracker.py:560-609 CVBackground; the IR detector's background model) ----
  * cv2.createBackgroundSubtractorMOG2(history, varThreshold, detectShadows=False) on one uint8 channel with five modes, bit for

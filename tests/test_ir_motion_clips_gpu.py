@@ -383,7 +383,7 @@ def test_no_per_frame_round_trips(monkeypatch):
         calls.append(1)
         return clips(self, *a)
 
-    for name in ("gray", "detect"):
+    for name in ("gray", "detect", "step"):
         monkeypatch.setattr(native.IrMotion, name, fail)
     monkeypatch.setattr(native.Mog2, "apply", fail)
     monkeypatch.setattr(native.Context, "ir_motion_clips", counted)

@@ -144,31 +144,26 @@ def test_mog2_background_surface_equals_cv_background():
 
 def test_ir_motion_detector_with_device_mog2(monkeypatch):
     """IRMotionDetector(background=MOG2Background()) reproduces the motion flags and trigger counts of the cv2 trace in
-    tests/golden/ir.npz, with neither the grey frame nor the mask crossing to the host."""
+    tests/golden/ir.npz, with neither the grey frame nor the mask crossing to the host: one device step per frame."""
     from classifier_pipeline_b200 import native
     from classifier_pipeline_b200.piclassifier.irmotiondetector import IRMotionDetector
     from classifier_pipeline_b200.track.cliptracker import MOG2Background
 
     gold = np.load(os.path.join(helpers.GOLDEN, "ir.npz"))
-    gray, detect = native.IrMotion.gray, native.IrMotion.detect
-    calls = {"gray": 0, "detect": 0}
+    step = native.IrMotion.step
+    calls = {"step": 0}
 
-    def gray_no_copy(self, bgr, slot, copy_out=True):
-        assert not copy_out, "the grey frame was copied to the host"
-        calls["gray"] += 1
-        return gray(self, bgr, slot, copy_out)
+    def counted_step(self, *a):
+        calls["step"] += 1
+        return step(self, *a)
 
-    def detect_device_mask(self, *a, mask=None, d_mask=None):
-        assert mask is None and d_mask is not None, "the mask did not come from the device"
-        calls["detect"] += 1
-        return detect(self, *a, mask=mask, d_mask=d_mask)
+    def no_host_copy(self, *a, **k):
+        raise AssertionError("the grey frame or the foreground mask was copied to the host")
 
-    def no_host_mask(self, *a, **k):
-        raise AssertionError("the foreground mask was copied to the host")
-
-    monkeypatch.setattr(native.IrMotion, "gray", gray_no_copy)
-    monkeypatch.setattr(native.IrMotion, "detect", detect_device_mask)
-    monkeypatch.setattr(MOG2Background, "compute_filtered", no_host_mask)
+    monkeypatch.setattr(native.IrMotion, "step", counted_step)
+    monkeypatch.setattr(native.IrMotion, "gray", no_host_copy)
+    monkeypatch.setattr(native.IrMotion, "detect", no_host_copy)
+    monkeypatch.setattr(MOG2Background, "compute_filtered", no_host_copy)
     cfg, headers = ir_helpers.ir_config()
     det = IRMotionDetector(cfg, headers, background=MOG2Background())
     flags, trig = [], []
@@ -177,7 +172,7 @@ def test_ir_motion_detector_with_device_mog2(monkeypatch):
         trig.append(det.triggered)
     assert np.array_equal(np.array(flags), gold["motion_flags"])
     assert np.array_equal(np.array(trig), gold["motion_triggered"])
-    assert calls["gray"] == len(flags) and calls["detect"] > 0
+    assert calls["step"] == len(flags)
 
 
 def test_invalid_arguments_leave_the_context_usable(ctx):
@@ -206,12 +201,23 @@ def test_invalid_arguments_leave_the_context_usable(ctx):
     with pytest.raises(ValueError):
         m.apply(torch.zeros((61, 96), dtype=torch.uint8, device="cuda"), -1)
     ir = native.IrMotion(ctx, 97, 61, 3)
-    assert not lib.cpt_ir_motion_ring_slot(ir._h, 3) and not lib.cpt_ir_motion_ring_slot(ir._h, -1)
+    model = native.Mog2(ctx, 97, 61)
+    d_mask = torch.empty((61, 97), dtype=torch.uint8, device="cuda")
+    bgr = np.zeros((61, 97, 3), np.uint8)
+    params = native.CptIrMotionClipParams(12, 2, 30, 15, 10, 0)
+    res = native.CptIrMotionClipResult()
+
+    def step(slot_new, slot_oldest, clip=None, result=res):
+        clip = clip or ir.clip_record(model, d_mask, 0, 1, False, 0)
+        st = native.CptIrMotionClipStep(0, slot_new, slot_oldest, 1, 0)
+        return lib.cpt_ir_motion_step(ctypes.byref(clip), bgr.ctypes.data, ctypes.byref(st), ctypes.byref(params), result)
+
     with pytest.raises(native.NativeError):
         ir.ring_slot(3)
-    d, c = ctypes.c_int32(), ctypes.c_int32()
-    assert lib.cpt_ir_motion_detect_ex(ir._h, 3, 0, 12, 15, None, ctypes.byref(d), ctypes.byref(c)) == -1
-    assert lib.cpt_ir_motion_detect_ex(ir._h, 1, 0, 12, 15, frames.data_ptr(), ctypes.byref(d), None) == -1
+    assert step(3, 0) == -1 and step(-1, 0) == -1 and step(0, 3) == -1  # ring slots
+    assert step(1, 0, result=None) == -1                                 # no result record
+    assert step(1, 0, clip=ir.clip_record(model, 0, 0, 1, False, 0)) == -1  # no mask buffer
+    assert model.frames == 0
     # everything still works afterwards, on the same context
     assert m.frames == 0
     compare(ctx, mh.scene("walk", (61, 97), 12, seed=17), [-1.0] * 12, 1000)
@@ -219,6 +225,12 @@ def test_invalid_arguments_leave_the_context_usable(ctx):
     a, b = (rng.integers(0, 256, (61, 97, 3), dtype=np.uint8) for _ in range(2))
     ir.gray(a, 0, copy_out=False)
     gb = ir.gray(b, 1)
-    mask = torch.from_numpy((rng.random((61, 97)) > 0.1).astype(np.uint8) * 255).cuda()
-    assert ir.detect(1, 0, 12, 3, d_mask=mask) == ir.detect(1, 0, 12, 3, mask=mask.cpu().numpy())
     assert np.array_equal(gb, cv2.cvtColor(b, cv2.COLOR_BGR2GRAY))
+    # the per-frame MOG2 step's counts equal cpt_ir_motion_detect's on the same mask: a fresh model takes b as its background,
+    # and its next frame a gives the mask
+    params = native.CptIrMotionClipParams(12, 2, 30, 3, 3, 0)
+    for bgr_t, slot in ((b, 1), (a, 0)):
+        r = ir.step(ir.clip_record(model, d_mask, 0, 1, False, 0), bgr_t, native.CptIrMotionClipStep(0, slot, 1 - slot, 1, 0), params)
+    mask = d_mask.cpu().numpy()
+    assert mask.any() and not mask.all() and r.mask_pixels > 0
+    assert (r.diff_pixels, r.mask_pixels) == ir.detect(0, 1, 12, 3, mask=mask)
